@@ -2,7 +2,7 @@
 """Benchmark of the GeneralGNN hot path (BASELINE.json metric: train graphs/sec and
 GCN-layer edges/sec at 1/2/4/8 B200; SpMM HBM GB/s vs peak).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 One "step" = one full training step on one disjoint batch of 1024 synthetic E. coli-shaped
 graphs per GPU (~500 nodes, stored degree ~12, 32-d features; default GeneralGNN: hidden 256,
@@ -20,6 +20,10 @@ graph across ranks (weak scaling: 1024 graphs per GPU per step).
 `cpu_baseline` / `--impl reference`: the CPU restatement of the reference's op sequence
            (oracle O2, PyTorch-CPU fp32; kind "port" — TensorFlow/Spektral cannot be installed
            here) on the host cores, bounded sample.
+`--dump-outputs DIR`: after the timed steps, rank 0 writes what the last timed step of the `value` arm
+           returned to its caller - {loss, accuracy}, the class probabilities - and the model's gradients,
+           parameters and BatchNorm state after it, as DIR/<name>.npy (float32).  The inputs depend on the
+           arguments only, so two builds run with the same arguments can be compared array by array.
 """
 from __future__ import annotations
 
@@ -68,6 +72,22 @@ def _ncu_traffic():
         return float(d["dram_bytes_read"]) + float(d["dram_bytes_write"])
     except Exception:
         return None
+
+
+DUMP_ARRAY_BYTES = 8 << 20      # per array: the five arrays of --dump-outputs stay well inside 64 MB
+
+
+def dump_outputs(out_dir, arrays):
+    """Write every tensor of ``arrays`` as out_dir/<name>.npy in float32.  An array larger than DUMP_ARRAY_BYTES
+    (the parameters at hidden >= 512) is replaced by a fixed, seeded sample of its flat elements in index order:
+    the same positions in every run, so that two builds still compare element for element."""
+    os.makedirs(out_dir, exist_ok=True)
+    for name, t in arrays.items():
+        a = t.detach().float().cpu().numpy()
+        keep = DUMP_ARRAY_BYTES // a.itemsize
+        if a.size > keep:
+            a = a.ravel()[np.sort(np.random.default_rng(0).choice(a.size, keep, replace=False))]
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 class ClockSampler:
@@ -449,7 +469,7 @@ def run_b200(args):
     def step():
         (x, a, i), y = next(loader)
         stats["n"], stats["nnz"] = a.n_rows, a.nnz
-        trainer.train_step((x, a, i), y)
+        stats["out"] = trainer.train_step((x, a, i), y)
 
     sampler = ClockSampler(local)
     if rank == 0:
@@ -465,6 +485,10 @@ def run_b200(args):
     per_step["device_allocs_in_timed_region"] = torch.cuda.memory_stats().get("num_device_alloc", 0) - segs0
     launches = lib.gcs_debug_launch_count() - launches0
     clocks = sampler.stop() if rank == 0 else None
+    if args.dump_outputs and rank == 0:
+        loss_acc, probs = stats["out"]
+        dump_outputs(args.dump_outputs, {"loss_acc": loss_acc, "probs": probs, "grads": model.grads,
+                                         "params": model.params, "bn_state": model.state})
     ms_step = ms_total / K
     value = world * B * K / (ms_total / 1e3)
 
@@ -650,7 +674,13 @@ def main():
                     "gathered out of pinned host memory by a device kernel (gcs_gather_graphs) instead of sliced copies")
     ap.add_argument("--sync-bn", action="store_true", help="all-reduce the BatchNorm statistics too (a G-GPU step then "
                     "equals one step on the union batch); off by default: the gradient all-reduce is the only collective")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the outputs of the last timed train step as "
+                    "DIR/<name>.npy (default benchmark only)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and (args.impl == "reference" or args.check or args.epoch):
+        ap.error("--dump-outputs applies to the default benchmark only")
     args.warmup = max(args.warmup, 3) if args.impl == "b200" else args.warmup
     if args.impl == "reference":
         return run_reference(args)
