@@ -12,7 +12,7 @@ raises if ``libgcnstring_b200.so`` is missing — there is no CPU fallback.
 from .params import GNNConfig, block_specs, init_params, n_state, n_trainable, named_slices  # noqa: F401
 
 from .data import Dataset, DisjointLoader, Graph, SparseAdjacency  # noqa: F401,E402
-from .layers import GeneralConv, GlobalSumPool, MLP  # noqa: F401,E402
+from .layers import GeneralConv, GlobalAttnSumPool, GlobalAvgPool, GlobalSumPool, MLP  # noqa: F401,E402
 from .losses import CategoricalCrossentropy, categorical_accuracy  # noqa: F401,E402
 from .models import GeneralGNN, GradientTape  # noqa: F401,E402
 from . import optimizers  # noqa: F401,E402

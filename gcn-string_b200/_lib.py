@@ -75,6 +75,11 @@ PROTOTYPES = {
     "gcs_spmm_aggregate": (c_int32, [P, P, P, P, P, I64, P, I64, P, P, P, P, I64, P, I64, I32, I32, P]),
     "gcs_segment_sum_fwd": (c_int32, [P, I64, P, I32, I32, P, I64, P]),
     "gcs_segment_sum_bwd": (c_int32, [P, I64, P, I32, I32, P, I64, P]),
+    "gcs_segment_mean_fwd": (c_int32, [P, I64, P, I32, I32, P, I64, P]),
+    "gcs_segment_mean_bwd": (c_int32, [P, I64, P, I32, I32, P, I64, P]),
+    "gcs_attn_pool_workspace_bytes": (c_int64, [I64, I32, I32]),
+    "gcs_attn_sum_pool_fwd": (c_int32, [P, I64, I64, P, P, I32, I32, P, I64, P, P, P, I64, P]),
+    "gcs_attn_sum_pool_bwd": (c_int32, [P, I64, P, I64, I64, P, P, I32, I32, P, I64, P, P, P, I64, P, P, I64, P]),
     "gcs_softmax_xent": (c_int32, [P, P, I32, I32, P, P, P, F32, P]),
     "gcs_sgd_step": (c_int32, [P, P, I64, F32, F32, P]),
     "gcs_adam_step": (c_int32, [P, P, P, P, I64, F64, F64, F64, F64, I64, F32, P]),

@@ -4,7 +4,9 @@
 //
 //   out = pre(x)                                   MLP: [Dense -> BN -> PReLU] x P
 //   for k in 1..L:  z = A . prelu(bn(out.W_k + b_k));  out = concat([z, out])
-//   out = segment_sum(out, i);  out = post(out)    MLP, last layer Dense -> BN -> softmax
+//   out = pool(out, i);  out = post(out)          MLP, last layer Dense -> BN -> softmax
+//   pool: segment_sum ('sum'), segment_mean ('avg'), attention-weighted sum ('attn_sum', one extra trainable vector
+//   pool.attn_kernel [Wc] after the last post block), or none (node-level output)
 //
 // HBM layout.  The 'cat' skip connection is materialised ONCE: a single [N, H*(L+1)] buffer
 // `cat`; Keras concatenates [z, out] (new block first), so pre() writes the LAST H columns
@@ -41,6 +43,9 @@ int linear_fwd_fused(const float* A, int64_t lda, const float* W, const float* b
 int bn_stats_from_partials(const float* part, int64_t M, int C, float* mean, float* var, void* workspace,
                            int64_t workspace_bytes, gcs_stream stream);
 namespace tc { int amax_merge(float* cell, const float* other, cudaStream_t st); }
+int segment_rows_div_count(float* D, int64_t ld, const int32_t* graph_ptr, int n_graphs, int W, gcs_stream stream);   // pool.cu
+
+enum { kPoolNone = 0, kPoolSum = 1, kPoolAvg = 2, kPoolAttnSum = 3 };
 
 struct BlockDesc {
   int k_in, m_out;
@@ -85,7 +90,8 @@ static int check_config(const gcs_model_config* c) {
     return fail(GCS_ERR_UNSUPPORTED, "model config: pre_process, message_passing, post_process must be >= 1");
   if (c->connectivity < 0 || c->connectivity > 2)
     return fail(GCS_ERR_INVALID_ARGUMENT, "model config: connectivity must be 0 (None), 1 ('cat') or 2 ('sum')");
-  if (c->pool != 0 && c->pool != 1) return fail(GCS_ERR_UNSUPPORTED, "model config: pool must be 'sum' or None");
+  if (c->pool < kPoolNone || c->pool > kPoolAttnSum)
+    return fail(GCS_ERR_UNSUPPORTED, "model config: pool must be 0 (None), 1 ('sum'), 2 ('avg') or 3 ('attn_sum')");
   if (c->final_activation != 0 && c->final_activation != 1)
     return fail(GCS_ERR_UNSUPPORTED, "model config: final activation must be linear or softmax");
   if (c->aggregate < 0 || c->aggregate > 2)
@@ -129,6 +135,12 @@ struct Plan {
   std::vector<float*> act;      // materialised activations of pre blocks 0..P-2
   std::vector<float*> stat;     // per block: mean | var | scale | shift  (4 * m_out)
   float* pooled = nullptr;      // [B, Wc] (unused when pool == 0)
+  int64_t attn_off = 0;         // 'attn_sum': offset of pool.attn_kernel [Wc] in the trainable buffer (after the blocks)
+  int64_t n_params = 0;         // floats in the trainable buffer
+  float* scores = nullptr;      // 'attn_sum', training: [N] attention scores s_n
+  float* gstats = nullptr;      // 'attn_sum', training: [B][2] {max_g, softmax denominator}
+  void* attn_ws = nullptr;      // 'attn_sum': partials of the split graphs
+  int64_t attn_ws_bytes = 0;
   std::vector<float*> post_h;   // [rows_post, m_out]
   std::vector<float*> post_a;   // [rows_post, H], post blocks 0..Q-2
   float* logits = nullptr;      // [rows_post, C]
@@ -137,7 +149,7 @@ struct Plan {
   void* lin_ws = nullptr;       // split weights of the tensor-core GEMM in flight
   int64_t lin_ws_bytes = 0;
   // backward
-  float* gcat = nullptr;        // [N, Wc]  only without pooling (node-level output)
+  float* gcat = nullptr;        // [N, Wc]  without pooling (node-level output) and for 'attn_sum': dLoss/d(emb(L)) in full
   float* dhcat = nullptr;       // [N, H*L] dh of the conv blocks, block k at columns [kH, (k+1)H)
   float* tmp_a = nullptr;       // [N, H]
   float* tmp_b = nullptr;       // [N, H]
@@ -248,6 +260,8 @@ static void make_plan(const gcs_model_config& c, int64_t N, int B, bool training
   p.H = c.hidden; p.Wc = c.connectivity == 1 ? c.hidden * (c.message_passing + 1) : c.hidden; p.C = c.output;
   p.N = N; p.B = B;
   p.rows_post = c.pool ? B : N;
+  p.attn_off = p.blocks.back().off + p.blocks.back().count();
+  p.n_params = p.attn_off + (c.pool == kPoolAttnSum ? p.Wc : 0);
   Arena a(ws);
   p.amax = a.take<float>(64);
   const int64_t NH = N * p.H;
@@ -270,6 +284,14 @@ static void make_plan(const gcs_model_config& c, int64_t N, int B, bool training
   p.stat.clear();
   for (const auto& b : p.blocks) p.stat.push_back(a.take<float>(4LL * b.m_out));
   if (c.pool) p.pooled = a.take<float>(static_cast<int64_t>(B) * p.Wc);
+  if (c.pool == kPoolAttnSum) {
+    if (training) {
+      p.scores = a.take<float>(N);
+      p.gstats = a.take<float>(2LL * B);
+    }
+    p.attn_ws_bytes = gcs_attn_pool_workspace_bytes(N, B, p.Wc);
+    p.attn_ws = a.take<char>(p.attn_ws_bytes);
+  }
   p.post_h.clear(); p.post_a.clear();
   for (int j = 0; j < p.Q; ++j) {
     const auto& b = p.blocks[p.P + p.L + j];
@@ -292,7 +314,7 @@ static void make_plan(const gcs_model_config& c, int64_t N, int B, bool training
   p.lin_ws_bytes = lin_bytes;
   p.lin_ws = a.take<char>(lin_bytes);
   if (training) {
-    if (!c.pool) p.gcat = a.take<float>(N * p.Wc);
+    if (!c.pool || c.pool == kPoolAttnSum) p.gcat = a.take<float>(N * p.Wc);
     p.dhcat = a.take<float>(c.connectivity == 1 ? NH * p.L : NH);
     p.tmp_a = a.take<float>(NH);
     p.tmp_b = a.take<float>(NH);
@@ -464,14 +486,18 @@ static int run_forward(const gcs_model_config& c, const Plan& p, const float* pa
     GCS_TIMED("spmm_fwd", aggregate(bt, false, p.h[bi], H, scale, scale + H, params + b.alpha(),
                                     c.connectivity == 2 ? emb(k) : nullptr, H, emb(k + 1), ld_emb, H, st, c.aggregate));
   }
-  // global sum pool
+  // global pool
   amax_sink() = AmaxSink();                                 // pooled rows and the post-MLP: tf32 kernels / CUDA cores
   const float* pin = emb(L);
   int64_t ld_pin = Wc;
-  if (c.pool) {
+  if (c.pool == kPoolSum)
     GCS_TIMED("pool_fwd", gcs_segment_sum_fwd(emb(L), Wc, bt.graph_ptr, bt.n_graphs, Wc, p.pooled, Wc, st));
-    pin = p.pooled;
-  }
+  else if (c.pool == kPoolAvg)
+    GCS_TIMED("pool_fwd", gcs_segment_mean_fwd(emb(L), Wc, bt.graph_ptr, bt.n_graphs, Wc, p.pooled, Wc, st));
+  else if (c.pool == kPoolAttnSum)
+    GCS_TIMED("pool_fwd", gcs_attn_sum_pool_fwd(emb(L), Wc, N, params + p.attn_off, bt.graph_ptr, bt.n_graphs, Wc, p.pooled, Wc,
+                                                p.scores, p.gstats, p.attn_ws, p.attn_ws_bytes, st));
+  if (c.pool) pin = p.pooled;
   // post-processing MLP
   const int64_t R = p.rows_post;
   for (int j = 0; j < p.Q; ++j) {
@@ -556,7 +582,16 @@ static int run_backward(const gcs_model_config& c, const Plan& p, const float* p
     da = din;
     ldda = lddin;
   }
-  int64_t grads_final_from = p.blocks.back().off + p.blocks.back().count();   // everything from here on is final
+  // From here on the node-level code sees either a pooled gradient dpooled [B, Wc] that every node of graph g receives
+  // ('sum'; 'avg' after dividing row g by n_g) or, for 'attn_sum' and without pooling, dLoss/d(emb(L)) in full in gcat.
+  const bool pooled_grad = c.pool == kPoolSum || c.pool == kPoolAvg;
+  if (c.pool == kPoolAvg)
+    GCS_TIMED("pool_bwd", segment_rows_div_count(p.dpooled, Wc, bt.graph_ptr, bt.n_graphs, Wc, st));
+  else if (c.pool == kPoolAttnSum)
+    GCS_TIMED("pool_bwd", gcs_attn_sum_pool_bwd(p.dpooled, Wc, emb(L), Wc, N, params + p.attn_off, bt.graph_ptr, bt.n_graphs, Wc,
+                                                p.pooled, Wc, p.scores, p.gstats, p.gcat, Wc, grads + p.attn_off, p.attn_ws,
+                                                p.attn_ws_bytes, st));
+  int64_t grads_final_from = p.n_params;                    // everything from here on is final
   auto notify = [&](int first_block) -> int {                // blocks first_block .. have all been differentiated
     const int64_t begin = p.blocks[first_block].off;
     if (ready && begin < grads_final_from) GCS_TRY(ready->fn(ready->user, begin, grads_final_from));
@@ -580,7 +615,7 @@ static int run_backward(const gcs_model_config& c, const Plan& p, const float* p
     }
     const float* dz;
     int64_t lddz;
-    if (c.pool) {
+    if (pooled_grad) {
       const float* rb = p.dpooled + static_cast<int64_t>(L - 1 - k) * H;
       if (nb == 0) {
         GCS_TIMED("pool_bwd", gcs_segment_sum_bwd(rb, Wc, bt.graph_ptr, bt.n_graphs, H, p.tmp_c, H, st));
@@ -616,7 +651,7 @@ static int run_backward(const gcs_model_config& c, const Plan& p, const float* p
   if (!cat) {
     // one running gradient g = dLoss/d(out_k): through z_k into the conv block, and - for 'sum' - straight on to out_{k-1}
     float* g = p.gcat;
-    if (c.pool) {
+    if (pooled_grad) {
       GCS_TIMED("pool_bwd", gcs_segment_sum_bwd(p.dpooled, Wc, bt.graph_ptr, bt.n_graphs, H, p.tmp_c, H, st));
       g = p.tmp_c;
     }
@@ -628,7 +663,7 @@ static int run_backward(const gcs_model_config& c, const Plan& p, const float* p
     }
     da_pre = g;
     ldda_pre = H;
-  } else if (c.pool) {
+  } else if (pooled_grad) {
     GCS_TIMED("linear_bwd_input", dense_dx_concat(p.dhcat, ldd, Wp.data(), roff.data(), L, H, H, p.dpooled + static_cast<int64_t>(L) * H, Wc,
                                                   bt.seg_ids, bt.graph_ptr, bt.n_graphs, p.tmp_c, H, N, 0, p.lin_ws,
                                                   p.lin_ws_bytes, cst));
@@ -664,7 +699,8 @@ extern "C" int64_t gcs_model_num_params(const gcs_model_config* cfg) {
   if (check_config(cfg) != GCS_OK) return -1;
   std::vector<BlockDesc> blocks;
   build_blocks(*cfg, blocks);
-  return blocks.back().off + blocks.back().count();
+  const int64_t wc = cfg->connectivity == 1 ? static_cast<int64_t>(cfg->hidden) * (cfg->message_passing + 1) : cfg->hidden;
+  return blocks.back().off + blocks.back().count() + (cfg->pool == kPoolAttnSum ? wc : 0);
 }
 
 extern "C" int64_t gcs_model_num_state(const gcs_model_config* cfg) {

@@ -1,8 +1,9 @@
-"""Layer-level call surface: ``GeneralConv``, ``GlobalSumPool``, ``MLP``.
+"""Layer-level call surface: ``GeneralConv``, ``GlobalSumPool``, ``GlobalAvgPool``, ``GlobalAttnSumPool``, ``MLP``.
 
 Signatures follow Spektral (SURVEY.md §8b): ``GeneralConv(channels=256, batch_norm=True,
 dropout=0.0, aggregate='sum', activation='prelu', use_bias=True)([x, a]) -> [N, channels]``,
-``GlobalSumPool()([x, i]) -> [B, W]``, ``MLP(output, hidden=256, layers=2, batch_norm=True,
+``GlobalSumPool()([x, i]) -> [B, W]`` (likewise ``GlobalAvgPool()`` and
+``GlobalAttnSumPool()``; ``[x]`` alone pools over all nodes, keepdims), ``MLP(output, hidden=256, layers=2, batch_norm=True,
 dropout=0.0, activation='prelu', final_activation=None)(x)``.  They are inference/forward
 building blocks over the same kernels GeneralGNN uses (the reference only ever reaches them
 through GeneralGNN, src/scripts/gcn.py:320); training goes through the model entry points.
@@ -88,20 +89,49 @@ class GeneralConv:
         return ops.spmm_aggregate(a.rowptr, a.colidx, h, scale, shift, alpha, aggregate=self.aggregate)
 
 
+def _pool_inputs(inputs):
+    """[x, i] -> (x, graph_ptr of the sorted batch index i); [x] or x -> (x, one graph of all nodes: single mode)."""
+    torch = _lib.require_cuda()
+    if isinstance(inputs, (list, tuple)) and len(inputs) == 2:
+        x, i = inputs
+        i = _lib.as_tensor(i)
+        if i.dim() == 2:
+            i = i[:, 0]
+        i = i.to(device="cuda", dtype=torch.int64).contiguous()
+        n_graphs = int(i[-1].item()) + 1 if i.numel() else 0
+        return _lib.as_tensor(x), ops.segment_ptr(i, n_graphs)
+    x = _lib.as_tensor(inputs[0] if isinstance(inputs, (list, tuple)) else inputs)
+    return x, torch.tensor([0, x.shape[0]], dtype=torch.int32, device="cuda")
+
+
 class GlobalSumPool:
     def __call__(self, inputs):
-        torch = _lib.require_cuda()
-        if isinstance(inputs, (list, tuple)) and len(inputs) == 2:
-            x, i = inputs
-            i = _lib.as_tensor(i)
-            if i.dim() == 2:
-                i = i[:, 0]
-            i = i.to(device="cuda", dtype=torch.int64).contiguous()
-            n_graphs = int(i[-1].item()) + 1 if i.numel() else 0
-            return ops.segment_sum_fwd(x, ops.segment_ptr(i, n_graphs))
-        x = inputs[0] if isinstance(inputs, (list, tuple)) else inputs
-        gp = torch.tensor([0, x.shape[0]], dtype=torch.int32, device="cuda")
-        return ops.segment_sum_fwd(x, gp)          # single mode: sum over nodes, keepdims
+        return ops.segment_sum_fwd(*_pool_inputs(inputs))
+
+
+class GlobalAvgPool:
+    """tf.math.segment_mean over the graphs (0 for an empty graph)."""
+
+    def __call__(self, inputs):
+        return ops.segment_mean_fwd(*_pool_inputs(inputs))
+
+
+class GlobalAttnSumPool:
+    """Attention-weighted sum: ``softmax_g(x . attn_kernel)`` per graph weights the rows of x.  ``attn_kernel`` [W, 1]
+    is created on the first call, glorot-uniform from ``seed``."""
+
+    def __init__(self, seed=0):
+        self.seed = seed
+        self.attn_kernel = None
+
+    def __call__(self, inputs):
+        x, gp = _pool_inputs(inputs)
+        if self.attn_kernel is None:
+            w = x.shape[1]
+            lim = np.sqrt(6.0 / (w + 1))
+            self.attn_kernel = _param(np.random.default_rng(self.seed).uniform(-lim, lim, size=(w, 1)))
+        out, _, _ = ops.attn_sum_pool_fwd(x, self.attn_kernel, gp)
+        return out
 
 
 class MLP:

@@ -395,7 +395,7 @@ def spmm_aggregate(rowptr, colidx, x, scale=None, shift=None, alpha=None, values
 
 
 # ------------------------------------------------------------------ pooling (K4/K6)
-def segment_sum_fwd(x, graph_ptr, out=None):
+def _segment_fwd(fn, x, graph_ptr, out):
     torch = _t()
     lib = _lib.load()
     x, ldx = _mat(x, "x")
@@ -404,12 +404,11 @@ def segment_sum_fwd(x, graph_ptr, out=None):
     if out is None:
         out = torch.empty(b, w, dtype=torch.float32, device="cuda")
     out, ldo = _mat(out, "out")
-    check(lib.gcs_segment_sum_fwd(ptr(x), ldx, ptr(graph_ptr), b, w, ptr(out), ldo, stream_ptr()),
-          "gcs_segment_sum_fwd")
+    check(getattr(lib, fn)(ptr(x), ldx, ptr(graph_ptr), b, w, ptr(out), ldo, stream_ptr()), fn)
     return out
 
 
-def segment_sum_bwd(dout, graph_ptr, n_nodes: int, out=None):
+def _segment_bwd(fn, dout, graph_ptr, n_nodes, out):
     torch = _t()
     lib = _lib.load()
     dout, ldo = _mat(dout, "dout")
@@ -417,9 +416,70 @@ def segment_sum_bwd(dout, graph_ptr, n_nodes: int, out=None):
     if out is None:
         out = torch.empty(n_nodes, w, dtype=torch.float32, device="cuda")
     out, ldx = _mat(out, "dx")
-    check(lib.gcs_segment_sum_bwd(ptr(dout), ldo, ptr(graph_ptr), b, w, ptr(out), ldx, stream_ptr()),
-          "gcs_segment_sum_bwd")
+    check(getattr(lib, fn)(ptr(dout), ldo, ptr(graph_ptr), b, w, ptr(out), ldx, stream_ptr()), fn)
     return out
+
+
+def segment_sum_fwd(x, graph_ptr, out=None):
+    return _segment_fwd("gcs_segment_sum_fwd", x, graph_ptr, out)
+
+
+def segment_sum_bwd(dout, graph_ptr, n_nodes: int, out=None):
+    return _segment_bwd("gcs_segment_sum_bwd", dout, graph_ptr, n_nodes, out)
+
+
+def segment_mean_fwd(x, graph_ptr, out=None):
+    """tf.math.segment_mean over the graphs of graph_ptr (0 for an empty graph)."""
+    return _segment_fwd("gcs_segment_mean_fwd", x, graph_ptr, out)
+
+
+def segment_mean_bwd(dout, graph_ptr, n_nodes: int, out=None):
+    return _segment_bwd("gcs_segment_mean_bwd", dout, graph_ptr, n_nodes, out)
+
+
+def attn_sum_pool_fwd(x, kernel, graph_ptr, out=None):
+    """GlobalAttnSumPool: out[g] = sum_{n in g} softmax_g(x . kernel)_n x_n.  ``kernel``: [W] or [W, 1].
+    Returns (out [B, W], scores [N], gstats [B, 2] = {max_g, softmax denominator}); the last two feed the backward."""
+    torch = _t()
+    lib = _lib.load()
+    x, ldx = _mat(x, "x")
+    n, w = x.shape
+    kernel = _vec(as_tensor(kernel).reshape(-1), "kernel", n=w)
+    b = graph_ptr.shape[0] - 1
+    if out is None:
+        out = torch.empty(b, w, dtype=torch.float32, device="cuda")
+    out, ldo = _mat(out, "out")
+    scores = torch.empty(n, dtype=torch.float32, device="cuda")
+    gstats = torch.empty(b, 2, dtype=torch.float32, device="cuda")
+    ws = _ws(lib.gcs_attn_pool_workspace_bytes(n, b, w))
+    check(lib.gcs_attn_sum_pool_fwd(ptr(x), ldx, n, ptr(kernel), ptr(graph_ptr), b, w, ptr(out), ldo, ptr(scores),
+                                    ptr(gstats), ptr(ws), ws.numel(), stream_ptr()), "gcs_attn_sum_pool_fwd")
+    return out, scores, gstats
+
+
+def attn_sum_pool_bwd(dout, x, kernel, graph_ptr, out, scores, gstats, dx=None):
+    """Gradient of ``attn_sum_pool_fwd`` given dout [B, W] and what the forward returned -> (dx [N, W], dkernel [W])."""
+    torch = _t()
+    lib = _lib.load()
+    dout, lddo = _mat(dout, "dout")
+    x, ldx = _mat(x, "x")
+    out, ldo = _mat(out, "out")
+    n, w = x.shape
+    b = graph_ptr.shape[0] - 1
+    kernel = _vec(as_tensor(kernel).reshape(-1), "kernel", n=w)
+    scores = _vec(scores, "scores", n=n)
+    gstats = _vec(as_tensor(gstats).reshape(-1), "gstats", n=2 * b)
+    if tuple(dout.shape) != (b, w) or tuple(out.shape) != (b, w):
+        raise ValueError(f"dout and out must be [{b}, {w}]")
+    if dx is None:
+        dx = torch.empty(n, w, dtype=torch.float32, device="cuda")
+    dx, lddx = _mat(dx, "dx")
+    dkernel = torch.empty(w, dtype=torch.float32, device="cuda")
+    ws = _ws(lib.gcs_attn_pool_workspace_bytes(n, b, w))
+    check(lib.gcs_attn_sum_pool_bwd(ptr(dout), lddo, ptr(x), ldx, n, ptr(kernel), ptr(graph_ptr), b, w, ptr(out), ldo,
+                                    ptr(scores), ptr(gstats), ptr(dx), lddx, ptr(dkernel), ptr(ws), ws.numel(),
+                                    stream_ptr()), "gcs_attn_sum_pool_bwd")
+    return dx, dkernel
 
 
 # ------------------------------------------------------------------ loss (K5) / optimizers (K10)

@@ -10,7 +10,8 @@ A "dense block" is the unit every stage is made of (SURVEY.md §8 a3/a4):
 Blocks, in order: ``pre.0 .. pre.{P-1}``, ``gnn.0 .. gnn.{L-1}``, ``post.0 .. post.{Q-1}``.
 Per block the trainable tensors are laid out ``kernel[K,M], bias[M], gamma[M], beta[M],
 alpha[M]`` (no ``alpha`` on the last post block: its activation is the model's final
-activation, not PReLU) in ONE flat fp32 buffer; the gradient buffer has the same layout
+activation, not PReLU) in ONE flat fp32 buffer; with ``pool='attn_sum'`` the pool's
+``attn_kernel [Wc, 1]`` follows the last block (every block offset stays as for 'sum'); the gradient buffer has the same layout
 (it is the NCCL all-reduce bucket), and the non-trainable BatchNorm statistics
 ``moving_mean[M], moving_variance[M]`` per block live in a second flat buffer.
 """
@@ -20,7 +21,7 @@ from dataclasses import dataclass, field
 from typing import List, Optional, Tuple
 
 CONNECTIVITY = {None: 0, "cat": 1, "sum": 2}
-POOL = {None: 0, "sum": 1}
+POOL = {None: 0, "sum": 1, "avg": 2, "attn_sum": 3}   # spektral GlobalSumPool / GlobalAvgPool / GlobalAttnSumPool
 FINAL_ACT = {None: 0, "linear": 0, "softmax": 1}
 AGGREGATE = {"sum": 0, "mean": 1, "max": 2}          # spektral scatter_sum / scatter_mean / scatter_max
 
@@ -51,7 +52,7 @@ class GNNConfig:
         if self.aggregate == "max" and self.connectivity == "sum":
             raise NotImplementedError("aggregate='max' with connectivity='sum' is not built")
         if self.pool not in POOL:
-            raise NotImplementedError("native path implements pool in {'sum', None}")
+            raise NotImplementedError("native path implements pool in {'sum', 'avg', 'attn_sum', None}")
         if self.connectivity not in CONNECTIVITY:
             raise ValueError("connectivity must be 'cat', 'sum' or None")
         if self.dropout != 0.0:
@@ -142,8 +143,17 @@ def block_specs(cfg: GNNConfig) -> List[BlockSpec]:
     return out
 
 
+def pool_kernel_slice(cfg: GNNConfig) -> Optional[Tuple[int, int]]:
+    """(offset, Wc) of ``pool.attn_kernel`` in the trainable buffer for ``pool='attn_sum'``, else None."""
+    if cfg.pool != "attn_sum":
+        return None
+    last = block_specs(cfg)[-1]
+    return (last.offset + last.n_trainable, cfg.cat_width)
+
+
 def n_trainable(cfg: GNNConfig) -> int:
-    return sum(b.n_trainable for b in block_specs(cfg))
+    pk = pool_kernel_slice(cfg)
+    return sum(b.n_trainable for b in block_specs(cfg)) + (pk[1] if pk else 0)
 
 
 def n_state(cfg: GNNConfig) -> int:
@@ -163,13 +173,17 @@ def named_slices(cfg: GNNConfig):
             out.append((f"{b.name}.prelu.alpha", (b.m_out,), b.alpha[0], "trainable"))
         out.append((f"{b.name}.bn.moving_mean", (b.m_out,), b.moving_mean[0], "state"))
         out.append((f"{b.name}.bn.moving_variance", (b.m_out,), b.moving_variance[0], "state"))
+    pk = pool_kernel_slice(cfg)
+    if pk:
+        out.append(("pool.attn_kernel", (pk[1], 1), pk[0], "trainable"))
     return out
 
 
 def init_params(cfg: GNNConfig, seed: int = 0, perturb: bool = False):
     """Keras-default initialisation as flat fp32 numpy buffers (trainable, state):
     glorot-uniform kernels, zero bias, gamma=1, beta=0, alpha=0, moving_mean=0,
-    moving_variance=1 (SURVEY.md §8 a3/a6/a7).  ``perturb=True`` moves gamma, beta,
+    moving_variance=1 (SURVEY.md §8 a3/a6/a7); ``pool.attn_kernel`` glorot-uniform [Wc, 1], drawn after every
+    block so that the blocks get the same values as with any other pool.  ``perturb=True`` moves gamma, beta,
     alpha, bias and the moving statistics off their defaults so every gradient path is
     exercised in parity tests (SURVEY.md §8d)."""
     import numpy as np
@@ -197,4 +211,9 @@ def init_params(cfg: GNNConfig, seed: int = 0, perturb: bool = False):
             s[o:o + n] = rng.normal(0, 0.3, n)
             o, n = b.moving_variance
             s[o:o + n] = rng.uniform(0.5, 2.0, n)
+    pk = pool_kernel_slice(cfg)
+    if pk:
+        o, n = pk
+        lim = np.sqrt(6.0 / (n + 1))
+        w[o:o + n] = rng.uniform(-lim, lim, size=n).astype(np.float32)
     return w, s

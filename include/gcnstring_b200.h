@@ -247,6 +247,34 @@ int gcs_segment_sum_fwd(const float* X, int64_t ldx, const int32_t* graph_ptr, i
                         int32_t W, float* out, int64_t ldo, gcs_stream stream);
 int gcs_segment_sum_bwd(const float* dout, int64_t ldo, const int32_t* graph_ptr, int32_t n_graphs,
                         int32_t W, float* dX, int64_t ldx, gcs_stream stream);
+/* GlobalAvgPool = tf.math.segment_mean(X, i): the segment sum divided by the graph's row count, 0 for an empty graph;
+ * gradient dX[n] = dOut[i[n]] / n_{i[n]}.  Same parameters as gcs_segment_sum_*. */
+int gcs_segment_mean_fwd(const float* X, int64_t ldx, const int32_t* graph_ptr, int32_t n_graphs,
+                         int32_t W, float* out, int64_t ldo, gcs_stream stream);
+int gcs_segment_mean_bwd(const float* dout, int64_t ldo, const int32_t* graph_ptr, int32_t n_graphs,
+                         int32_t W, float* dX, int64_t ldx, gcs_stream stream);
+
+/* ---------------------------------------------------------------------------------
+ * K4b/K6b  GlobalAttnSumPool (spektral.layers.pooling.GlobalAttnSumPool) over sorted graph ids.
+ *   s_n = X_n . kernel,  p = unsorted_segment_softmax(s, i) = exp(s - max_g) / (sum_g exp(s - max_g) + 1e-9),
+ *   out[g] = sum_{n in g} p_n X_n  (0 for an empty graph).  kernel [W] is Spektral's attn_kernel [W, 1].
+ * fwd: scores [n_rows] (the s_n) and gstats [2 * n_graphs] ({max_g, sum_g exp(s - max_g)}) are NULL-able; the
+ *      backward needs both, together with `out`.
+ * bwd: with u_g = out_g . dOut_g:  ds_n = p_n (X_n . dOut_g - u_g),  dX_n = p_n dOut_g + ds_n kernel (written in full),
+ *      dkernel = sum_n ds_n X_n (overwritten).
+ * One pass over X each; long graphs are split over several thread blocks (fixed by n_rows and n_graphs) whose partials
+ * are combined in a fixed order - bit-identical run to run.  W <= 8192 (W <= 2048 when W, a leading dimension or a
+ * pointer is not a multiple of 4 floats).  workspace: gcs_attn_pool_workspace_bytes(n_rows, n_graphs, W), 16-byte
+ * aligned, for either direction.
+ * --------------------------------------------------------------------------------- */
+int64_t gcs_attn_pool_workspace_bytes(int64_t n_rows, int32_t n_graphs, int32_t W);
+int gcs_attn_sum_pool_fwd(const float* X, int64_t ldx, int64_t n_rows, const float* kernel, const int32_t* graph_ptr,
+                          int32_t n_graphs, int32_t W, float* out, int64_t ldo, float* scores, float* gstats,
+                          void* workspace, int64_t workspace_bytes, gcs_stream stream);
+int gcs_attn_sum_pool_bwd(const float* dout, int64_t lddo, const float* X, int64_t ldx, int64_t n_rows,
+                          const float* kernel, const int32_t* graph_ptr, int32_t n_graphs, int32_t W,
+                          const float* out, int64_t ldo, const float* scores, const float* gstats, float* dX,
+                          int64_t lddx, float* dkernel, void* workspace, int64_t workspace_bytes, gcs_stream stream);
 
 /* ---------------------------------------------------------------------------------
  * K5  softmax + CategoricalCrossentropy (mean over the batch) + categorical_accuracy
@@ -331,7 +359,8 @@ typedef struct gcs_model_config {
   int32_t pre_process;      /* default 2 */
   int32_t post_process;     /* default 2 */
   int32_t connectivity;     /* 0 = None (out = z), 1 = 'cat' (out = concat[z, out]), 2 = 'sum' (out = z + out) */
-  int32_t pool;             /* 1 = 'sum', 0 = None (node-level output) */
+  int32_t pool;             /* 0 = None (node-level output), 1 = 'sum', 2 = 'avg', 3 = 'attn_sum' (adds the trainable
+                               attn_kernel [H*(L+1) or H] after the last post block) */
   int32_t final_activation; /* 0 = linear, 1 = softmax */
   float bn_momentum;        /* 0.99 */
   float bn_epsilon;         /* 1e-3 */
