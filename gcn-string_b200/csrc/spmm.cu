@@ -184,7 +184,9 @@ __global__ void __launch_bounds__(256, 4) spmm_rb4_kernel(
 }
 
 // Row-parallel CSR kernel.  VEC = 4: H % 4 == 0 and 16 B-aligned rows, lanes = H/4 threads per
-// row.  VEC = 1: any H, lanes = H threads per row.  A CTA walks a CONTIGUOUS chunk of rows:
+// row.  VEC = 1: any H, lanes = H threads per row.  Rows wider than 256 lanes are split over
+// gridDim.y into slices of 256 lanes (256 * VEC columns, a multiple of 4: float4 alignment holds);
+// up to that width gridDim.y = 1.  A CTA walks a CONTIGUOUS chunk of rows:
 // consecutive rows of a banded matrix share most of their neighbours, which then hit in L1.
 // kGeneral adds what GeneralConv itself never asks for (SURVEY.md §8 f3): per-entry weights `values` (CSR order),
 // aggregate = mean / max (scatter_mean = unsorted_segment_mean: sum / entry count, 0 for an empty row; scatter_max =
@@ -199,7 +201,7 @@ __global__ void __launch_bounds__(256) spmm_rows_kernel(
     const float* __restrict__ R, int64_t ldr, int agg, float* __restrict__ amax) {
   const int lane = threadIdx.x % lanes;
   const int slot = threadIdx.x / lanes;
-  const int c = lane * VEC;
+  const int c = (static_cast<int>(blockIdx.y) * lanes + lane) * VEC;
   if (slot >= rows_per_block || c >= H) return;
   float sc[VEC], sh[VEC], al[VEC];
 #pragma unroll
@@ -285,7 +287,8 @@ __global__ void __launch_bounds__(256) spmm_rows_kernel(
 //   max : dA[j, c] = sum_i [w_ij * a[j, c] == Z[i, c]] * w_ij * dZ[i, c] / ties[i, c]
 //         (tf.math.unsorted_segment_max's gradient: the maxima of a segment share its gradient equally; ties[i, c] is
 //         the number of neighbours of i that attain the maximum, counted by spmm_max_ties_kernel)
-// One owner thread per output element, entries in ascending column order: deterministic.
+// One owner thread per output element, entries in ascending column order: deterministic.  Lanes own VEC adjacent
+// columns; rows wider than 256 lanes are split over gridDim.y as in spmm_rows_kernel.
 template <int VEC>
 __global__ void __launch_bounds__(256) spmm_agg_bwd_kernel(
     const int32_t* __restrict__ rowptr_t, const int32_t* __restrict__ colidx_t, const float* __restrict__ values_t,
@@ -294,7 +297,7 @@ __global__ void __launch_bounds__(256) spmm_agg_bwd_kernel(
     int64_t ldh, const float* __restrict__ scale, const float* __restrict__ shift, const float* __restrict__ alpha,
     float* __restrict__ dA, int64_t ldda, int H, int lanes, int rows_per_block) {
   const int lane = threadIdx.x % lanes, slot = threadIdx.x / lanes;
-  const int c = lane * VEC;
+  const int c = (static_cast<int>(blockIdx.y) * lanes + lane) * VEC;
   const int64_t j = static_cast<int64_t>(blockIdx.x) * rows_per_block + slot;
   if (slot >= rows_per_block || j >= n_rows || c >= H) return;
   float own[VEC], acc[VEC];
@@ -373,13 +376,21 @@ struct SpmmArgs {
 int g_rows_iters = 16;   // tuning knob (gcs_debug_set_param 1)
 int g_rb4_iters = 2;     // row blocks per slot per CTA (gcs_debug_set_param 2); sweep on 8-row blocks 1/2/3/4: 372/356/358/367 us fwd, 283/277/287/297 us bwd; on 4-row blocks 2/4/8: 338/334/349, 262/264/293
 
+// Lanes per row and column slices (gridDim.y) of the row kernels for H columns, VEC columns per lane.
+struct RowSplit { int lanes; unsigned slices; };
+template <int VEC>
+RowSplit row_split(int H) {
+  const int64_t need = (static_cast<int64_t>(H) + VEC - 1) / VEC;
+  return {static_cast<int>(need < 256 ? need : 256), static_cast<unsigned>(ceil_div(need, static_cast<int64_t>(256)))};
+}
+
 template <int VEC>
 int launch_rows(const SpmmArgs& a) {
-  const int lanes = (a.H + VEC - 1) / VEC;
-  if (lanes > 256) return fail(GCS_ERR_UNSUPPORTED, "gcs_spmm_sum: H=%d too wide for the row kernel", a.H);
+  const RowSplit s = row_split<VEC>(a.H);
+  const int lanes = s.lanes;
   const int rows_per_block = 256 / lanes;
   const int iters = g_rows_iters;                   // rows_per_block * iters contiguous rows per CTA
-  dim3 grid(static_cast<unsigned>(ceil_div(a.n_rows, static_cast<int64_t>(rows_per_block) * iters)));
+  dim3 grid(static_cast<unsigned>(ceil_div(a.n_rows, static_cast<int64_t>(rows_per_block) * iters)), s.slices);
 #define GCS_ROWS_LAUNCH(T, G)                                                                                          \
   spmm_rows_kernel<VEC, T, G><<<grid, 256, 0, a.st>>>(a.rowptr, a.colidx, a.n_rows, a.X, a.ldx, a.scale, a.shift,      \
                                                       a.alpha, a.Y, a.ldy, a.H, lanes, rows_per_block, iters, a.values, \
@@ -538,11 +549,10 @@ extern "C" int gcs_spmm_aggregate_bwd(const int32_t* rowptr_t, const int32_t* co
     spmm_agg_bwd_kernel<1><<<static_cast<unsigned>(ceil_div(n_rows, rpb)), 256, 0, st>>>(
         rowptr_t, colidx_t, values_t, n_rows, dZ, lddz, aggregate, rowptr, Z, ldz, ties, ldt, X, ldx, scale, shift, alpha, dA, ldda, H, H, rpb);
   } else {
-    const int lanes = (H + 3) / 4;
-    GCS_CHECK_ARG(lanes <= 256, "gcs_spmm_aggregate_bwd: H too wide");
-    const int rpb = 256 / lanes;
-    spmm_agg_bwd_kernel<4><<<static_cast<unsigned>(ceil_div(n_rows, rpb)), 256, 0, st>>>(
-        rowptr_t, colidx_t, values_t, n_rows, dZ, lddz, aggregate, rowptr, Z, ldz, ties, ldt, X, ldx, scale, shift, alpha, dA, ldda, H, lanes, rpb);
+    const RowSplit s = row_split<4>(H);
+    const int rpb = 256 / s.lanes;
+    spmm_agg_bwd_kernel<4><<<dim3(static_cast<unsigned>(ceil_div(n_rows, rpb)), s.slices), 256, 0, st>>>(
+        rowptr_t, colidx_t, values_t, n_rows, dZ, lddz, aggregate, rowptr, Z, ldz, ties, ldt, X, ldx, scale, shift, alpha, dA, ldda, H, s.lanes, rpb);
   }
   GCS_CHECK_LAUNCH("spmm_agg_bwd_kernel");
   return GCS_OK;

@@ -203,16 +203,18 @@ class SparseAdjacency:
         return 4
 
     def edge_weight_t(self):
-        """The edge weights in the entry order of the transposed pattern (columns ascending, then rows)."""
+        """The edge weights in the entry order of the transposed pattern (columns ascending, then rows).  Cached per
+        tensor and per in-place version of it: ``a.edge_weight.copy_(w)`` between two steps is seen by the backward."""
         if self.edge_weight is None:
             return None
-        if self._edge_weight_t is None or self._edge_weight_t[0] is not self.edge_weight:
+        w = self.edge_weight
+        if self._edge_weight_t is None or self._edge_weight_t[0] is not w or self._edge_weight_t[1] != w._version:
             torch = _lib.require_cuda()
             counts = (self.rowptr[1:] - self.rowptr[:-1]).to(torch.int64)
             rows = torch.repeat_interleave(torch.arange(self.n_rows, device="cuda"), counts)
             key = self.colidx.to(torch.int64) * self.n_rows + rows
-            self._edge_weight_t = (self.edge_weight, self.edge_weight[torch.argsort(key)].contiguous())
-        return self._edge_weight_t[1]
+            self._edge_weight_t = (w, w._version, w[torch.argsort(key)].contiguous())
+        return self._edge_weight_t[2]
 
     def transposed(self):
         """(rowptr_t, colidx_t) of pattern(A)^T; the same arrays when symmetric."""

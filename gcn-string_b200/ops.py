@@ -394,6 +394,62 @@ def spmm_aggregate(rowptr, colidx, x, scale=None, shift=None, alpha=None, values
     return out
 
 
+def spmm_aggregate_bwd(rowptr_t, colidx_t, rowptr, colidx, dz, aggregate="sum", values_t=None, values=None, x=None,
+                       scale=None, shift=None, alpha=None, z=None, out=None, ties=None):
+    """Gradient of ``spmm_aggregate`` with respect to f(x) (gcs_spmm_aggregate_bwd) -> dA [n, H].
+    ``(rowptr_t, colidx_t)``: the transposed pattern, ``values_t`` the weights in its entry order (with ``values``, the
+    same weights in CSR order); ``dz``: dLoss/dY.  max also takes the forward's ``x`` with its prologue
+    (``scale`` / ``shift`` / ``alpha``) and its output ``z``, and counts the entries that attain each maximum into
+    ``ties`` [n, H] (allocated when not given)."""
+    torch = _t()
+    lib = _lib.load()
+    if aggregate not in AGGREGATE:
+        raise ValueError(f"aggregate must be one of {sorted(AGGREGATE)}")
+    dz, lddz = _mat(dz, "dz")
+    n, hdim = dz.shape
+    if rowptr.shape[0] != n + 1 or rowptr_t.shape[0] != n + 1:
+        raise ValueError(f"A and A^T must have {n} rows, like dz")
+    if colidx_t.shape[0] != colidx.shape[0]:
+        raise ValueError("A and A^T must have the same number of entries")
+    if (values is None) != (values_t is None):
+        raise ValueError("values and values_t go together (the same weights in CSR and transposed order)")
+    if values is not None:
+        if values.shape[0] != colidx.shape[0] or values_t.shape[0] != colidx.shape[0]:
+            raise ValueError("values and values_t must hold one weight per stored entry")
+        values = values.to(device="cuda", dtype=torch.float32).contiguous()
+        values_t = values_t.to(device="cuda", dtype=torch.float32).contiguous()
+    if (scale is None) != (shift is None) or (scale is None) != (alpha is None):
+        raise ValueError("scale, shift and alpha must be all None or all set")
+    if scale is not None:
+        scale, shift, alpha = _vec(scale, "scale", n=hdim), _vec(shift, "shift", n=hdim), _vec(alpha, "alpha", n=hdim)
+    ldx = ldz = ldt = 0
+    if aggregate == "max":
+        if x is None or z is None:
+            raise ValueError("aggregate='max' needs the forward input x and output z")
+        x, ldx = _mat(x, "x")
+        z, ldz = _mat(z, "z")
+        if tuple(x.shape) != (n, hdim) or tuple(z.shape) != (n, hdim):
+            raise ValueError(f"x and z must be [{n}, {hdim}] like dz")
+        if ties is None:
+            ties = torch.empty(n, hdim, dtype=torch.float32, device="cuda")
+    else:
+        x = z = None                                      # read by max only
+    if ties is not None:
+        ties, ldt = _mat(ties, "ties")
+        if tuple(ties.shape) != (n, hdim):
+            raise ValueError(f"ties must be [{n}, {hdim}]")
+    if out is None:
+        out = torch.empty(n, hdim, dtype=torch.float32, device="cuda")
+    out, ldda = _mat(out, "dA")
+    if tuple(out.shape) != (n, hdim):
+        raise ValueError(f"dA must be [{n}, {hdim}]")
+    check(lib.gcs_spmm_aggregate_bwd(ptr(rowptr_t), ptr(colidx_t), ptr(values_t), ptr(rowptr), ptr(colidx), ptr(values), n,
+                                     ptr(dz), lddz, AGGREGATE[aggregate], ptr(x), ldx, ptr(scale), ptr(shift), ptr(alpha),
+                                     ptr(z), ldz, ptr(ties), ldt, ptr(out), ldda, hdim, stream_ptr()),
+          "gcs_spmm_aggregate_bwd")
+    return out
+
+
 # ------------------------------------------------------------------ pooling (K4/K6)
 def _segment_fwd(fn, x, graph_ptr, out):
     torch = _t()

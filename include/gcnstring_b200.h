@@ -221,6 +221,7 @@ int gcs_spmm_sum_graphs(const int32_t* graph_ptr, int32_t n_graphs, int32_t max_
  * residual : optional [n_rows, H] operand added after the aggregation - Keras Add()([z, out]) of
  *            connectivity='sum' - NULL otherwise.
  * The RB4 kernel serves aggregate = 0 without weights (with or without residual); everything else runs row by row.
+ * Any H > 0 (as in gcs_spmm_aggregate_bwd): rows wider than one thread block are split into column slices.
  * gcs_spmm_sum(...) == gcs_spmm_aggregate(..., values = NULL, residual = NULL, aggregate = 0). */
 int gcs_spmm_aggregate(const int32_t* rowptr, const int32_t* colidx, const float* values,
                        const int32_t* rb4_blk_ptr, const uint32_t* rb4_ent, int64_t n_rows, const float* X,

@@ -518,7 +518,7 @@ def test_spmm_graphs_falls_back_without_slab():
         lib.gcs_debug_set_param(11, 0)
 
 
-@pytest.mark.parametrize("H", [64, 6])
+@pytest.mark.parametrize("H", [64, 6, 257, 260, 512, 1028])     # above 256 lanes per row: column slices over gridDim.y
 @pytest.mark.parametrize("aggregate", ["sum", "mean", "max"])
 @pytest.mark.parametrize("weighted", [False, True])
 def test_spmm_aggregate_weights_mean_max_residual(H, aggregate, weighted):
@@ -594,6 +594,30 @@ def test_spmm_is_deterministic_and_handles_empty_rows():
     assert torch.equal(y1, y2) and float(y1[7].abs().max()) == 0.0
     with pytest.raises(ValueError):
         ops.spmm_sum(rp, ci, x, scale=torch.ones(64, device="cuda"))      # partial prologue
+
+
+def test_spmm_sum_and_sum_graphs_at_an_odd_width_above_256():
+    """H = 258: no 16-byte vectors, so both entry points run the scalar row kernel, one lane per column over two column
+    slices; against float64, deterministic, empty rows 0."""
+    rng = np.random.default_rng(258)
+    H = 258
+    a, gp = _block_diag_batch(rng, [60, 1, 130, 17], 0.06)
+    n = a.shape[0]
+    x = rng.standard_normal((n, H)).astype(np.float32)
+    sc, sh, al = (rng.uniform(0.5, 1.5, H).astype(np.float32), rng.normal(0, 0.5, H).astype(np.float32),
+                  rng.uniform(-0.3, 1.4, H).astype(np.float32))
+    rp, ci = dev(a.indptr.astype(np.int32)), dev(a.indices.astype(np.int32))
+    empty = np.diff(a.indptr) == 0
+    assert empty.any()
+    z = x.astype(np.float64) * sc + sh
+    ref = _spmm_ref(a, np.where(z > 0, z, al * z))
+    y1 = ops.spmm_sum(rp, ci, dev(x), dev(sc), dev(sh), dev(al))
+    assert rel_err(host(y1), ref) < TOL and float(y1[dev(empty)].abs().max()) == 0.0
+    assert torch.equal(y1, ops.spmm_sum(rp, ci, dev(x), dev(sc), dev(sh), dev(al)))
+    assert rel_err(host(ops.spmm_sum(rp, ci, dev(x))), _spmm_ref(a, x)) < TOL
+    rb = ops.build_rb(rp, ci, 4)
+    y2 = ops.spmm_sum_graphs(dev(gp), 130, rp, ci, dev(x), dev(sc), dev(sh), dev(al), rb=rb, rb_height=4)
+    assert torch.equal(y2, y1)
 
 
 # ---------------------------------------------------------------- K4/K6 pooling
