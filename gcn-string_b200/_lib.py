@@ -44,6 +44,7 @@ PROTOTYPES = {
     "gcs_set_allreduce_hook": (c_int32, [P, P, I32]),
     "gcs_batch_disjoint": (c_int32, [P, P, P, P, P, I32, I32, P, I32, I64, I64, P, P, P, P, P, P, P, P, P, P]),
     "gcs_gather_graphs": (c_int32, [P, I32, P, P, P, P, P, I32, I32, P, P, P, P, P, P, P]),
+    "gcs_gather_node_rows": (c_int32, [P, I32, P, P, I32, P, P, P]),
     "gcs_coo_to_csr": (c_int32, [P, I64, I64, P, P, P, P]),
     "gcs_segment_ptr": (c_int32, [P, I64, I32, P, P, P]),
     "gcs_csr_is_symmetric": (c_int32, [P, P, I64, P, P]),
@@ -81,6 +82,8 @@ PROTOTYPES = {
     "gcs_attn_sum_pool_fwd": (c_int32, [P, I64, I64, P, P, I32, I32, P, I64, P, P, P, I64, P]),
     "gcs_attn_sum_pool_bwd": (c_int32, [P, I64, P, I64, I64, P, P, I32, I32, P, I64, P, P, P, I64, P, P, I64, P]),
     "gcs_softmax_xent": (c_int32, [P, P, I32, I32, P, P, P, F32, P]),
+    "gcs_softmax_xent_workspace_bytes": (c_int64, [I64, I32]),
+    "gcs_softmax_xent_ws": (c_int32, [P, P, I32, I32, P, P, P, F32, P, I64, P]),
     "gcs_sgd_step": (c_int32, [P, P, I64, F32, F32, P]),
     "gcs_adam_step": (c_int32, [P, P, P, P, I64, F64, F64, F64, F64, I64, F32, P]),
     "gcs_comm_unique_id": (c_int32, [P]),

@@ -337,6 +337,28 @@ __global__ void __launch_bounds__(256) gather_graphs_kernel(
     for (int c = threadIdx.x; c < n_classes; c += blockDim.x) dst_y[static_cast<int64_t>(j) * n_classes + c] = src_y[g * n_classes + c];
 }
 
+// Node-level labels (np.vstack of the graphs' [n_g, width] label blocks): CTA row j copies the contiguous row block of
+// graph ids[j] to batch row graph_ptr[j].  Every access is a coalesced run - 128-bit when width and both addresses allow
+// - so the source may sit in pinned host memory as well as in HBM.  Pure copies: deterministic.
+__global__ void __launch_bounds__(256) gather_node_rows_kernel(
+    const int64_t* __restrict__ ids, const int64_t* __restrict__ src_node_off, const float* __restrict__ src, int width,
+    const int32_t* __restrict__ dst_graph_ptr, float* __restrict__ dst) {
+  const int j = blockIdx.x;
+  const int64_t g = ids[j];
+  const int64_t n0 = src_node_off[g];
+  const int64_t cnt = (src_node_off[g + 1] - n0) * width;
+  const float* s = src + n0 * width;
+  float* d = dst + static_cast<int64_t>(dst_graph_ptr[j]) * width;
+  const int64_t tid = static_cast<int64_t>(blockIdx.y) * blockDim.x + threadIdx.x, nth = static_cast<int64_t>(gridDim.y) * blockDim.x;
+  if ((width & 3) == 0 && ((reinterpret_cast<uintptr_t>(s) | reinterpret_cast<uintptr_t>(d)) & 15u) == 0) {
+    const float4* s4 = reinterpret_cast<const float4*>(s);
+    float4* d4 = reinterpret_cast<float4*>(d);
+    for (int64_t i = tid; i < cnt / 4; i += nth) d4[i] = s4[i];
+  } else {
+    for (int64_t i = tid; i < cnt; i += nth) d[i] = s[i];
+  }
+}
+
 // out[0..n] = exclusive prefix sums of cnt[0..n) (out[n] = total); shared with spmm.cu.
 int exclusive_scan_i64(const int32_t* cnt, int64_t n, int64_t* out, cudaStream_t st) {
   exclusive_scan_kernel<int64_t><<<1, 1024, 0, st>>>(cnt, n, out);
@@ -401,6 +423,20 @@ extern "C" int gcs_gather_graphs(const int64_t* graph_ids, int32_t n_graphs, con
                                                            src_y, n_feat, n_classes, dst_node_off, dst_edge_off, dst_rowptr,
                                                            dst_col, dst_x, dst_y);
   GCS_CHECK_LAUNCH("gather_graphs_kernel");
+  return GCS_OK;
+}
+
+extern "C" int gcs_gather_node_rows(const int64_t* graph_ids, int32_t n_graphs, const int64_t* src_node_off,
+                                    const float* src, int32_t width, const int32_t* dst_graph_ptr, float* dst,
+                                    gcs_stream stream) {
+  GCS_CHECK_ARG(n_graphs >= 0 && width > 0, "gcs_gather_node_rows: bad size");
+  if (n_graphs == 0) return GCS_OK;
+  GCS_CHECK_ARG(graph_ids && src_node_off && src && dst_graph_ptr && dst, "gcs_gather_node_rows: null pointer");
+  int chunks = static_cast<int>(ceil_div(8LL * sm_count(), n_graphs));      // as gcs_gather_graphs: host-link reads in flight
+  chunks = chunks < 1 ? 1 : (chunks > 32 ? 32 : chunks);
+  dim3 grid(n_graphs, chunks);
+  gather_node_rows_kernel<<<grid, 256, 0, as_stream(stream)>>>(graph_ids, src_node_off, src, width, dst_graph_ptr, dst);
+  GCS_CHECK_LAUNCH("gather_node_rows_kernel");
   return GCS_OK;
 }
 

@@ -148,6 +148,8 @@ struct Plan {
   int64_t bn_ws_bytes = 0;
   void* lin_ws = nullptr;       // split weights of the tensor-core GEMM in flight
   int64_t lin_ws_bytes = 0;
+  void* xent_ws = nullptr;      // loss partials of gcs_softmax_xent_ws (0 bytes up to its row threshold)
+  int64_t xent_ws_bytes = 0;
   // backward
   float* gcat = nullptr;        // [N, Wc]  without pooling (node-level output) and for 'attn_sum': dLoss/d(emb(L)) in full
   float* dhcat = nullptr;       // [N, H*L] dh of the conv blocks, block k at columns [kH, (k+1)H)
@@ -334,6 +336,8 @@ static void make_plan(const gcs_model_config& c, int64_t N, int B, bool training
     p.prep_ws_bytes = list_step_weights(c, p, nullptr, nullptr, nullptr, nullptr);
     p.prep_ws = a.take<char>(p.prep_ws_bytes);
   }
+  p.xent_ws_bytes = gcs_softmax_xent_workspace_bytes(p.rows_post, p.C);   // last: graph-level plans keep their layout
+  p.xent_ws = a.take<char>(p.xent_ws_bytes);
   *total = a.used;
 }
 
@@ -735,7 +739,8 @@ extern "C" int gcs_model_forward(const gcs_model_config* cfg, const float* param
   GCS_TRY(run_forward(*cfg, p, params, state, *batch, training != 0, stream));
   if (cfg->final_activation == 1) {
     GCS_CHECK_ARG(p.rows_post < INT32_MAX, "gcs_model_forward: too many output rows");
-    GCS_TRY(gcs_softmax_xent(p.logits, nullptr, static_cast<int32_t>(p.rows_post), p.C, out, nullptr, nullptr, 0.f, stream));
+    GCS_TRY(gcs_softmax_xent_ws(p.logits, nullptr, static_cast<int32_t>(p.rows_post), p.C, out, nullptr, nullptr, 0.f,
+                                p.xent_ws, p.xent_ws_bytes, stream));
   } else {
     GCS_CUDA(cudaMemcpyAsync(out, p.logits, sizeof(float) * p.rows_post * p.C, cudaMemcpyDeviceToDevice, as_stream(stream)));
   }
@@ -763,8 +768,8 @@ extern "C" int gcs_model_train_step(const gcs_model_config* cfg, const float* pa
   GCS_TRY(prepare_step_weights(c, p, params, &prepared, stream));
   PreparedScope prepared_scope(&prepared);
   GCS_TRY(run_forward(c, p, params, state, bt, true, stream));
-  GCS_TRY(gcs_softmax_xent(p.logits, bt.y, static_cast<int32_t>(p.rows_post), p.C, probs, loss_acc, p.dlogits,
-                           grad_scale, stream));
+  GCS_TRY(gcs_softmax_xent_ws(p.logits, bt.y, static_cast<int32_t>(p.rows_post), p.C, probs, loss_acc, p.dlogits,
+                              grad_scale, p.xent_ws, p.xent_ws_bytes, stream));
 
   return run_backward(c, p, params, grads, bt, p.dlogits, stream);
 }
@@ -833,7 +838,8 @@ extern "C" int gcs_model_train_step_dp(const gcs_model_config* cfg, const float*
   GCS_TRY(prepare_step_weights(c, p, params, &prepared, stream));
   PreparedScope prepared_scope(&prepared);
   GCS_TRY(run_forward(c, p, params, state, bt, true, stream));
-  GCS_TRY(gcs_softmax_xent(p.logits, bt.y, static_cast<int32_t>(p.rows_post), p.C, probs, loss_acc, p.dlogits, grad_scale, stream));
+  GCS_TRY(gcs_softmax_xent_ws(p.logits, bt.y, static_cast<int32_t>(p.rows_post), p.C, probs, loss_acc, p.dlogits, grad_scale,
+                              p.xent_ws, p.xent_ws_bytes, stream));
   cudaEvent_t* ev = dp_events();
   DpSync sync{comm, grads, as_stream(stream), as_stream(comm_stream), {}, 0};
   for (int i = 0; i < 8; ++i) sync.ev[i] = ev[i];

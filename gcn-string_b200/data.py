@@ -285,10 +285,12 @@ class DeviceGraphStore:
         self.col = torch.from_numpy(packed.col).cuda()
         self.x = torch.from_numpy(np.ascontiguousarray(packed.x, dtype=np.float32)).cuda()
         self.y = torch.from_numpy(np.ascontiguousarray(packed.y, dtype=np.float32)).cuda() if self.n_classes else None
+        self.node_level = bool(packed.node_level)
         self.symmetric = symmetric
 
     def batch(self, graph_ids_dev, graph_ids_host, want_coo=False, want_labels=True):
-        """Run K0 for the graphs ``graph_ids`` (device int64 tensor + the same ids on host)."""
+        """Run K0 for the graphs ``graph_ids`` (device int64 tensor + the same ids on host); node labels are then
+        gathered by gcs_gather_node_rows at the graph offsets K0 wrote."""
         torch = _lib.require_cuda()
         lib = _lib.load()
         b = int(graph_ids_host.shape[0])
@@ -302,13 +304,21 @@ class DeviceGraphStore:
         colidx = ops.empty_bucketed(nnz, dtype=torch.int32)
         x = ops.empty_bucketed(n, self.n_feat, dtype=torch.float32)
         seg = ops.empty_bucketed(n, dtype=torch.int64)
-        y = torch.empty(b, self.n_classes, dtype=torch.float32, device="cuda") if (want_labels and self.y is not None) else None
+        y = None
+        if want_labels and self.y is not None:
+            y = (ops.empty_bucketed(n, self.n_classes, dtype=torch.float32) if self.node_level
+                 else torch.empty(b, self.n_classes, dtype=torch.float32, device="cuda"))
         coo = ops.empty_bucketed(nnz, 2, dtype=torch.int64) if want_coo else None
         flag = torch.zeros(1, **i32)
-        check(lib.gcs_batch_disjoint(ptr(self.node_off), ptr(self.rowptr), ptr(self.col), ptr(self.x), ptr(self.y),
+        graph_y = None if self.node_level else self.y
+        check(lib.gcs_batch_disjoint(ptr(self.node_off), ptr(self.rowptr), ptr(self.col), ptr(self.x), ptr(graph_y),
                                      self.n_feat, max(self.n_classes, 1), ptr(graph_ids_dev), b, n, nnz,
                                      ptr(graph_ptr), ptr(edge_ptr), ptr(rowptr), ptr(colidx), ptr(x), ptr(seg),
-                                     ptr(y), ptr(coo), ptr(flag), stream_ptr()), "gcs_batch_disjoint")
+                                     None if self.node_level else ptr(y), ptr(coo), ptr(flag), stream_ptr()),
+              "gcs_batch_disjoint")
+        if self.node_level and y is not None:
+            check(lib.gcs_gather_node_rows(ptr(graph_ids_dev), b, ptr(self.node_off), ptr(self.y), self.n_classes,
+                                           ptr(graph_ptr), ptr(y), stream_ptr()), "gcs_gather_node_rows")
         a = SparseAdjacency(rowptr, colidx, n, graph_ptr=graph_ptr, max_graph_nodes=max_nodes, indices=coo,
                             symmetric=self.symmetric)
         a.edge_ptr = edge_ptr
@@ -346,6 +356,7 @@ class HostGraphStore:
         self.node_off, self.rowptr, self.col = pin(packed.node_off), pin(packed.rowptr), pin(packed.col)
         self.x = pin(packed.x.astype(np.float32, copy=False))
         self.y = pin(packed.y.astype(np.float32, copy=False)) if self.n_classes else None
+        self.node_level = bool(packed.node_level)
         self.symmetric = symmetric
         self.h2d_bytes_last = 0
         self._ring = _PinnedRing(depth=6)
@@ -353,7 +364,7 @@ class HostGraphStore:
     def _gather(self, ids):
         """Pack the graphs ``ids`` (any order) into a fresh pinned mini-dataset."""
         torch = _lib.require_cuda()
-        sub = PackedGraphs(*_take_graphs(self, ids))
+        sub = PackedGraphs(*_take_graphs(self, ids), node_level=self.node_level)
         pin = lambda a: torch.from_numpy(np.ascontiguousarray(a)).pin_memory()   # noqa: E731
         return pin(sub.node_off), pin(sub.rowptr), pin(sub.col), pin(sub.x), (pin(sub.y) if self.n_classes else None)
 
@@ -371,8 +382,9 @@ class HostGraphStore:
             g0, g1 = int(ids[0]), int(ids[0]) + b
             n0, n1 = int(self.h_node_off[g0]), int(self.h_node_off[g1])
             e0, e1 = int(self.h_rowptr[n0]), int(self.h_rowptr[n1])
+            y_rows = (n0, n1) if self.node_level else (g0, g1)        # node labels: one contiguous node range
             parts = (self.node_off[g0:g1 + 1], self.rowptr[n0:n1 + 1], self.col[e0:e1], self.x[n0:n1],
-                     self.y[g0:g1] if self.y is not None else None)
+                     self.y[y_rows[0]:y_rows[1]] if self.y is not None else None)
             ids_local = torch.arange(g0, g1, dtype=torch.int64)
         elif self.device_gather:
             parts = None
@@ -390,7 +402,8 @@ class HostGraphStore:
             # loader's asynchronous upload of the epoch order (graph_ids_dev)
             ids_dev = self._ring.upload(ids_local.numpy())
             # bytes the kernel pulls over the host link: per graph its node offsets, row pointers, columns, features, label
-            self.h2d_bytes_last = 16 * b + 8 * (n + b) + 4 * nnz + 4 * self.n_feat * n + 4 * self.n_classes * b + 8 * b
+            self.h2d_bytes_last = (16 * b + 8 * (n + b) + 4 * nnz + 4 * self.n_feat * n
+                                   + 4 * self.n_classes * (n if self.node_level else b) + 8 * b)
         elif parts is None:
             # the selected graphs' offsets in the mini-dataset (host knows the sizes), then one gather kernel
             off = np.zeros((3, b + 1), dtype=np.int64)
@@ -402,13 +415,16 @@ class HostGraphStore:
             d_rowptr = ops.empty_bucketed(n + 1, dtype=torch.int64)
             d_col = ops.empty_bucketed(max(nnz, 1), dtype=torch.int32)
             d_x = ops.empty_bucketed(max(n, 1), self.n_feat, dtype=torch.float32)
-            d_y = torch.empty(b, self.n_classes, dtype=torch.float32, device="cuda") if self.y is not None else None
+            # node labels are gathered straight into the batch after K0 (gcs_gather_node_rows), not into the mini-dataset
+            graph_y = None if self.node_level else self.y
+            d_y = torch.empty(b, self.n_classes, dtype=torch.float32, device="cuda") if graph_y is not None else None
             check(lib.gcs_gather_graphs(ptr(off_dev[2]), b, ptr(self.node_off), ptr(self.rowptr), ptr(self.col), ptr(self.x),
-                                        ptr(self.y), self.n_feat, self.n_classes, ptr(off_dev[0]), ptr(off_dev[1]),
+                                        ptr(graph_y), self.n_feat, self.n_classes, ptr(off_dev[0]), ptr(off_dev[1]),
                                         ptr(d_rowptr), ptr(d_col), ptr(d_x), ptr(d_y), stream_ptr()), "gcs_gather_graphs")
             dev = [d_node_off, d_rowptr, d_col, d_x, d_y]
             ids_dev = self._ring.upload(ids_local.numpy())
-            self.h2d_bytes_last = 16 * b + 8 * (n + b) + 4 * nnz + 4 * self.n_feat * n + 4 * self.n_classes * b + 24 * (b + 1)
+            self.h2d_bytes_last = (16 * b + 8 * (n + b) + 4 * nnz + 4 * self.n_feat * n
+                                   + 4 * self.n_classes * (n if self.node_level else b) + 24 * (b + 1))
         else:
             dev = []
             for t in parts:                              # pinned slices -> bucketed device buffers
@@ -427,17 +443,31 @@ class HostGraphStore:
         rowptr, colidx = ops.empty_bucketed(n + 1, dtype=torch.int32), ops.empty_bucketed(nnz, dtype=torch.int32)
         x = ops.empty_bucketed(n, self.n_feat, dtype=torch.float32)
         seg = ops.empty_bucketed(n, dtype=torch.int64)
-        y = torch.empty(b, self.n_classes, dtype=torch.float32, device="cuda") if (want_labels and d_y is not None) else None
         coo = ops.empty_bucketed(nnz, 2, dtype=torch.int64) if want_coo else None
         flag = torch.zeros(1, **i32)
+        if self.node_level:
+            y, graph_y = None, None
+            if want_labels and self.y is not None:
+                if parts is not None and not self.zero_copy:
+                    y = d_y                      # the copied slice / staged rows are already the batch's rows, in order
+                else:
+                    y = ops.empty_bucketed(n, self.n_classes, dtype=torch.float32)
+        else:
+            y = torch.empty(b, self.n_classes, dtype=torch.float32, device="cuda") if (want_labels and d_y is not None) else None
+            graph_y = (ptr(d_y) - 4 * self.n_classes * g0) if d_y is not None else None
         # the uploaded slices are addressed with DATASET-global ids: rebase the pointers instead
         # of the index arrays (the kernel only touches [g0, g1], [n0, n1], [e0, e1))
         check(lib.gcs_batch_disjoint(ptr(d_node_off) - 8 * g0, ptr(d_rowptr) - 8 * n0, ptr(d_col) - 4 * e0,
-                                     ptr(d_x) - 4 * self.n_feat * n0,
-                                     (ptr(d_y) - 4 * self.n_classes * g0) if d_y is not None else None,
+                                     ptr(d_x) - 4 * self.n_feat * n0, graph_y,
                                      self.n_feat, max(self.n_classes, 1), ptr(ids_dev), b, n, nnz, ptr(graph_ptr),
-                                     ptr(edge_ptr), ptr(rowptr), ptr(colidx), ptr(x), ptr(seg), ptr(y), ptr(coo),
-                                     ptr(flag), stream_ptr()), "gcs_batch_disjoint")
+                                     ptr(edge_ptr), ptr(rowptr), ptr(colidx), ptr(x), ptr(seg),
+                                     None if self.node_level else ptr(y), ptr(coo), ptr(flag), stream_ptr()),
+              "gcs_batch_disjoint")
+        if self.node_level and y is not None and y is not d_y:
+            # zero_copy: the batch's graph ids index the pinned dataset; device_gather: the same ids (off_dev[2])
+            gids = ids_dev if self.zero_copy else off_dev[2]
+            check(lib.gcs_gather_node_rows(ptr(gids), b, ptr(self.node_off), ptr(self.y), self.n_classes, ptr(graph_ptr),
+                                           ptr(y), stream_ptr()), "gcs_gather_node_rows")
         a = SparseAdjacency(rowptr, colidx, n, graph_ptr=graph_ptr, max_graph_nodes=max_nodes, indices=coo,
                             symmetric=self.symmetric)
         a.edge_ptr, a.status = edge_ptr, flag
@@ -452,17 +482,23 @@ def _take_graphs(store, ids):
     hn, hr = store.h_node_off, store.h_rowptr
     col_np, x_np = store.col.numpy(), store.x.numpy()
     rp_np = store.rowptr.numpy()
-    rps, cols, xs = [], [], []
+    rps, cols, xs, ys = [], [], [], []
     e_off = 0
+    y_np = store.y.numpy() if store.y is not None else None
     for g in ids:
         n0, n1 = int(hn[g]), int(hn[g + 1])
         e0, e1 = int(hr[n0]), int(hr[n1])
         rps.append(rp_np[n0:n1] - e0 + e_off)
         cols.append(col_np[e0:e1])
         xs.append(x_np[n0:n1])
+        if store.node_level and y_np is not None:
+            ys.append(y_np[n0:n1])
         e_off += e1 - e0
     rowptr = np.concatenate(rps + [np.array([e_off], dtype=np.int64)])
-    y = store.y.numpy()[ids] if store.y is not None else np.zeros((len(ids), 0), np.float32)
+    if y_np is None:
+        y = np.zeros((len(ids), 0), np.float32)
+    else:
+        y = np.concatenate(ys) if store.node_level else y_np[ids]
     return node_off, rowptr, np.concatenate(cols), np.concatenate(xs), y
 
 
@@ -478,7 +514,8 @@ class _Spec:
 
 class DisjointLoader:
     """``spektral.data.DisjointLoader(dataset, node_level=False, batch_size=1, epochs=None,
-    shuffle=True)``.  Iterating yields ``((x, a, i), y)`` with everything on the device.
+    shuffle=True)``.  Iterating yields ``((x, a, i), y)`` with everything on the device: y [B, C] graph labels, or
+    with ``node_level=True`` y [N, C], the graphs' node labels stacked in batch order (Spektral's np.vstack).
 
     Batch order follows upstream's ``batch_generator``: per epoch an in-place
     ``np.random.shuffle`` (cumulative across epochs, global NumPy RNG), then consecutive
@@ -486,17 +523,21 @@ class DisjointLoader:
     ceil(len / batch_size)``.  With ``device_resident=False`` the dataset stays in pinned host
     memory and each step uploads its own graphs.  ``dataset`` may be a ``Dataset``, a list of ``Graph`` or an
     already packed ``PackedGraphs``.  ``rank`` / ``world_size`` shard every global batch by
-    graph across data-parallel ranks (rank r takes the r-th contiguous part of the slice).
+    graph across data-parallel ranks (rank r takes the r-th contiguous part of the slice); the adjacency carries the
+    global slice's graph and node counts (``a.global_batch_graphs`` / ``a.global_batch_nodes``), the denominators of
+    the graph- and node-level mean loss.
     """
 
     def __init__(self, dataset, node_level=False, batch_size=1, epochs=None, shuffle=True, rank=0, world_size=1,
                  want_coo=False, symmetric=None, device_resident=True, prefetch=None, balance=None, zero_copy=False,
                  device_gather=False):
-        if node_level:
-            raise NotImplementedError("node_level=True labels are not built (reference uses graph labels)")
-        packed = dataset if isinstance(dataset, PackedGraphs) else pack_graphs(list(dataset))
+        node_level = bool(node_level)
+        packed = dataset if isinstance(dataset, PackedGraphs) else pack_graphs(list(dataset), node_level=node_level)
         if packed.n_graphs == 0:
             raise ValueError("Datasets cannot be empty")
+        if bool(packed.node_level) != node_level:
+            raise ValueError(f"DisjointLoader(node_level={node_level}) got a dataset with "
+                             f"{'node' if packed.node_level else 'graph'} labels")
         if symmetric is None:
             symmetric = getattr(packed, "symmetric", None)      # recorded by the shard writer (shards.py)
         self.dataset = dataset
@@ -560,7 +601,7 @@ class DisjointLoader:
         return lo, lo + base + (1 if self.rank < rem else 0)
 
     def _slices(self):
-        """(epoch, lo, hi, host ids, global batch size) of every step, epoch after epoch.  Nothing is uploaded here:
+        """(epoch, lo, hi, host ids, (global batch graphs, global batch nodes)) of every step, epoch after epoch.  Nothing is uploaded here:
         the device copies of the ids are made by _launch on the stream the batching kernels run on."""
         epochs = np.inf if self.epochs is None or self.epochs == -1 else self.epochs
         epoch = 0
@@ -575,21 +616,22 @@ class DisjointLoader:
                 if stop - start < self.world_size:
                     continue                       # a tail shorter than the number of ranks: dropped by every rank alike
                 lo, hi = self._slices_of_rank(start, stop)
+                nodes = int(self.store.h_n_nodes[order_host[start:stop]].sum())
                 if self.balance == "nnz" and self.world_size > 1:
                     from .distributed import balanced_shard
                     ids = order_host[start:stop]
                     cost = self.store.h_n_edges[ids] + 4 * self.store.h_n_nodes[ids]
                     mine = np.ascontiguousarray(balanced_shard(ids, cost, self.rank, self.world_size))
-                    yield epoch, None, None, mine, stop - start, order_host
+                    yield epoch, None, None, mine, (stop - start, nodes), order_host
                 else:
-                    yield epoch, lo, hi, order_host[lo:hi], stop - start, order_host
+                    yield epoch, lo, hi, order_host[lo:hi], (stop - start, nodes), order_host
 
     def _launch(self, item, stream):
         """Enqueue upload + batching kernels for one step on `stream`.  The graph ids go to the device on the SAME
         stream (pinned staging, asynchronous copy): the batching kernels that read them are ordered behind the copy by
         the stream itself, whichever stream the training step runs on."""
         torch = _lib.require_cuda()
-        epoch, lo, hi, ids_host, global_count, order_host = item
+        epoch, lo, hi, ids_host, (global_count, global_nodes), order_host = item
         with torch.cuda.stream(stream):
             # persistent pinned staging (see _PinnedRing: no pinned allocation inside the loop)
             if lo is None:                                     # work-balanced shard: its own id list
@@ -602,6 +644,7 @@ class DisjointLoader:
             staged = None
             x, a, i, y = self.store.batch(ids_dev, ids_host, want_coo=self.want_coo)
             a.global_batch_graphs = global_count
+            a.global_batch_nodes = global_nodes
             a._ids_keepalive = (ids_dev, staged)
             event = torch.cuda.Event()
             event.record(stream)

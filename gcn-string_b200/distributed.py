@@ -8,8 +8,8 @@ collective is one ``all_reduce(SUM)`` over the flat fp32 gradient buffer (4.26 M
 256) through torch.distributed (NCCL over NVLink; gloo on CPU in the tests).
 
 Scaling of the mean loss: every rank back-propagates with grad_scale = 1 / global_batch
-(graphs over ALL ranks), so the summed gradient is the gradient of the mean loss over the
-global batch, also when shards are unequal (short last batch).
+(graphs over ALL ranks; nodes over all ranks for a node-level model, pool=None), so the summed gradient is the
+gradient of the mean loss over the global batch, also when shards are unequal (short last batch).
 
 BatchNorm statistics stay replica-local (the all-reduce is the only collective): a G-GPU
 step equals G reference steps on the shards with count-weighted gradient averaging, not one
@@ -178,7 +178,9 @@ class DataParallelTrainer:
             self._synced = True
         a = inputs[1]
         if global_batch is None:
-            global_batch = getattr(a, "global_batch_graphs", None) or target.shape[0] * ws
+            # the mean loss is over graphs, or over nodes when the model has no pool (node-level output)
+            key = "global_batch_nodes" if self.model.config["pool"] is None else "global_batch_graphs"
+            global_batch = getattr(a, key, None) or target.shape[0] * ws
         if self.comm is not None:                 # the library's own communicator: collectives (and synchronised BatchNorm) per call
             loss_acc, probs = self.model.train_step_grads(inputs, target, grad_scale=1.0 / float(global_batch), comm=self.comm,
                                                           sync_bn=self.sync_bn)

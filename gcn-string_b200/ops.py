@@ -540,7 +540,8 @@ def attn_sum_pool_bwd(dout, x, kernel, graph_ptr, out, scores, gstats, dx=None):
 
 # ------------------------------------------------------------------ loss (K5) / optimizers (K10)
 def softmax_xent(logits, y=None, grad_scale: Optional[float] = None, want_grad=False):
-    """Returns (probs, loss_acc[2] or None, dlogits or None)."""
+    """Returns (probs, loss_acc[2] or None, dlogits or None).  gcs_softmax_xent_ws: one thread block up to 65 536 rows,
+    a grid above - the same rule as the model's fused train step, so both give the same bits."""
     torch = _t()
     lib = _lib.load()
     logits, _ = _mat(logits, "logits")
@@ -553,8 +554,10 @@ def softmax_xent(logits, y=None, grad_scale: Optional[float] = None, want_grad=F
         y, _ = _mat(y, "y")
         y = y.contiguous()
     gs = (1.0 / b if b else 0.0) if grad_scale is None else grad_scale
-    check(lib.gcs_softmax_xent(ptr(logits), ptr(y), b, c, ptr(probs), ptr(loss_acc), ptr(dlogits), gs, stream_ptr()),
-          "gcs_softmax_xent")
+    nbytes = int(lib.gcs_softmax_xent_workspace_bytes(b, c))
+    ws = torch.empty(nbytes, dtype=torch.uint8, device="cuda") if nbytes > 0 else None
+    check(lib.gcs_softmax_xent_ws(ptr(logits), ptr(y), b, c, ptr(probs), ptr(loss_acc), ptr(dlogits), gs, ptr(ws), nbytes,
+                                  stream_ptr()), "gcs_softmax_xent_ws")
     return probs, loss_acc, dlogits
 
 

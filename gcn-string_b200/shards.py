@@ -12,17 +12,22 @@ memory or straight to HBM.
 File layout (little endian, every section 64-byte aligned):
 
     0    8  magic  b"GCSSHRD1"
-    8    4  uint32 version (1)
+    8    4  uint32 version (1: graph labels; 2: node labels)
     12   4  uint32 n_feat
     16   4  uint32 n_classes
     20   4  uint32 flags           bit 0: every graph's pattern is symmetric
+                                   bit 1: node labels (set exactly when version is 2)
     24   8  uint64 n_graphs
     32   8  uint64 n_nodes
     40   8  uint64 nnz
     48   8  uint64 payload checksum (sum of the payload's uint32 words mod 2^64)
     56   8  reserved (0)
     64      node_off int64 [n_graphs+1] | rowptr int64 [n_nodes+1] | col int32 [nnz]
-            | x float32 [n_nodes, n_feat] | y float32 [n_graphs, n_classes]
+            | x float32 [n_nodes, n_feat] | y float32 [n_graphs, n_classes]  (version 1)
+                                           | y float32 [n_nodes, n_classes]   (version 2, node labels)
+
+A node-labelled shard carries version 2 so that a reader that knows only version 1 refuses it instead of misreading
+its y section.  Graph-labelled shards are written as version 1, byte for byte as before.
 """
 from __future__ import annotations
 
@@ -36,21 +41,23 @@ import numpy as np
 from .synthetic import PackedGraphs, pack_graphs
 
 MAGIC = b"GCSSHRD1"
-VERSION = 1
+VERSION = 1                  # graph labels
+VERSION_NODE_LEVEL = 2       # node labels
 _HEADER = struct.Struct("<8sIIIIQQQQQ")          # 64 bytes
 _ALIGN = 64
 FLAG_SYMMETRIC = 1
+FLAG_NODE_LEVEL = 2
 
 
 def _pad(n: int) -> int:
     return (-n) % _ALIGN
 
 
-def _sections(n_graphs: int, n_nodes: int, nnz: int, n_feat: int, n_classes: int):
+def _sections(n_graphs: int, n_nodes: int, nnz: int, n_feat: int, n_classes: int, node_level: bool = False):
     """[(name, dtype, shape, offset)] of the payload, offsets from the start of the file."""
     spec = [("node_off", np.dtype("<i8"), (n_graphs + 1,)), ("rowptr", np.dtype("<i8"), (n_nodes + 1,)),
             ("col", np.dtype("<i4"), (nnz,)), ("x", np.dtype("<f4"), (n_nodes, n_feat)),
-            ("y", np.dtype("<f4"), (n_graphs, n_classes))]
+            ("y", np.dtype("<f4"), (n_nodes if node_level else n_graphs, n_classes))]
     out, off = [], _HEADER.size
     for name, dt, shape in spec:
         nbytes = int(np.prod(shape, dtype=np.int64)) * dt.itemsize
@@ -89,15 +96,17 @@ def write_shard(path: str, packed: PackedGraphs, symmetric: Optional[bool] = Non
     if packed.rowptr.shape[0] != n + 1 or int(packed.rowptr[-1]) != nnz:
         raise ValueError("inconsistent PackedGraphs: rowptr does not match node_off / col")
     x = np.ascontiguousarray(packed.x, dtype="<f4").reshape(n, -1) if n else np.zeros((0, packed.x.shape[-1]), "<f4")
-    y = np.ascontiguousarray(packed.y, dtype="<f4").reshape(g, -1)
+    node_level = bool(getattr(packed, "node_level", False))
+    y = np.ascontiguousarray(packed.y, dtype="<f4").reshape(n if node_level else g, -1)
     if nnz and (packed.col.min() < 0 or (packed.col >= np.repeat(packed.n_nodes, packed.n_edges)).any()):
         raise ValueError("column index outside its graph")
     arrays = [np.ascontiguousarray(packed.node_off, dtype="<i8"), np.ascontiguousarray(packed.rowptr, dtype="<i8"),
               np.ascontiguousarray(packed.col, dtype="<i4"), x, y]
     if symmetric is None:
         symmetric = pattern_is_symmetric(packed)
-    flags = FLAG_SYMMETRIC if symmetric else 0
-    header = _HEADER.pack(MAGIC, VERSION, x.shape[1], y.shape[1], flags, g, n, nnz, _checksum(arrays), 0)
+    flags = (FLAG_SYMMETRIC if symmetric else 0) | (FLAG_NODE_LEVEL if node_level else 0)
+    version = VERSION_NODE_LEVEL if node_level else VERSION
+    header = _HEADER.pack(MAGIC, version, x.shape[1], y.shape[1], flags, g, n, nnz, _checksum(arrays), 0)
     tmp = path + ".tmp"
     with open(tmp, "wb") as f:
         f.write(header)
@@ -117,12 +126,19 @@ class ShardHeader:
             _HEADER.unpack(raw[:_HEADER.size])
         if magic != MAGIC:
             raise ValueError(f"{path}: not a gcn_string_b200 shard (bad magic {magic!r})")
-        if ver != VERSION:
-            raise ValueError(f"{path}: shard version {ver}, this reader understands {VERSION}")
+        if ver not in (VERSION, VERSION_NODE_LEVEL):
+            raise ValueError(f"{path}: shard version {ver}, this reader understands {VERSION} and {VERSION_NODE_LEVEL}")
+        if bool(self.flags & FLAG_NODE_LEVEL) != (ver == VERSION_NODE_LEVEL):
+            raise ValueError(f"{path}: shard version {ver} disagrees with its node-label flag (flags {self.flags:#x})")
+        self.version = ver
 
     @property
     def symmetric(self) -> bool:
         return bool(self.flags & FLAG_SYMMETRIC)
+
+    @property
+    def node_level(self) -> bool:
+        return bool(self.flags & FLAG_NODE_LEVEL)
 
 
 def read_header(path: str) -> ShardHeader:
@@ -134,7 +150,7 @@ def read_shard(path: str, mmap: bool = True, verify: bool = False) -> PackedGrap
     """Open a shard as ``PackedGraphs``.  With ``mmap`` the arrays are read-only views of the file
     (nothing is parsed or copied until the loader uploads it); ``verify`` recomputes the checksum."""
     h = read_header(path)
-    secs, end = _sections(h.n_graphs, h.n_nodes, h.nnz, h.n_feat, h.n_classes)
+    secs, end = _sections(h.n_graphs, h.n_nodes, h.nnz, h.n_feat, h.n_classes, h.node_level)
     size = os.path.getsize(path)
     if size < end:
         raise ValueError(f"{path}: truncated shard ({size} bytes, header implies {end})")
@@ -148,7 +164,7 @@ def read_shard(path: str, mmap: bool = True, verify: bool = False) -> PackedGrap
         arrs[name] = buf[off:off + nbytes].view(dt).reshape(shape)
     if verify and _checksum([arrs[k] for k in ("node_off", "rowptr", "col", "x", "y")]) != h.checksum:
         raise ValueError(f"{path}: payload checksum mismatch")
-    p = PackedGraphs(arrs["node_off"], arrs["rowptr"], arrs["col"], arrs["x"], arrs["y"])
+    p = PackedGraphs(arrs["node_off"], arrs["rowptr"], arrs["col"], arrs["x"], arrs["y"], h.node_level)
     if h.n_graphs and (int(p.node_off[-1]) != h.n_nodes or int(p.rowptr[-1]) != h.nnz or int(p.node_off[0]) != 0):
         raise ValueError(f"{path}: offsets disagree with the header")
     p.symmetric = h.symmetric
@@ -156,7 +172,10 @@ def read_shard(path: str, mmap: bool = True, verify: bool = False) -> PackedGrap
 
 
 def concat_packed(parts: Sequence[PackedGraphs]) -> PackedGraphs:
-    """Concatenate packed datasets (graph order preserved, offsets rebased)."""
+    """Concatenate packed datasets (graph order preserved, offsets rebased).  Graph- and node-labelled parts do not
+    mix."""
+    if len({bool(getattr(p, "node_level", False)) for p in parts}) > 1:
+        raise ValueError("cannot concatenate graph-labelled and node-labelled shards")
     parts = [p for p in parts if p.n_graphs]
     if not parts:
         raise ValueError("nothing to concatenate")
@@ -170,21 +189,23 @@ def concat_packed(parts: Sequence[PackedGraphs]) -> PackedGraphs:
         n0 += int(p.node_off[-1])
         e0 += int(p.rowptr[-1])
     out = PackedGraphs(np.concatenate(node_off), np.concatenate(rowptr), np.concatenate([p.col for p in parts]),
-                       np.concatenate([p.x for p in parts]), np.concatenate([p.y for p in parts]))
+                       np.concatenate([p.x for p in parts]), np.concatenate([p.y for p in parts]), parts[0].node_level)
     out.symmetric = all(getattr(p, "symmetric", False) for p in parts)
     return out
 
 
-def write_dataset(graphs: Iterable, out_dir: str, graphs_per_shard: int = 4096, prefix: str = "shard") -> List[str]:
+def write_dataset(graphs: Iterable, out_dir: str, graphs_per_shard: int = 4096, prefix: str = "shard",
+                  node_level: bool = False) -> List[str]:
     """Convert a dataset (anything iterable over objects with ``.x``, ``.a``, ``.y`` - what
-    ``MyDataset.read`` returns, gcn.py:84-102) into shard files + an ``index.json``; returns the paths."""
+    ``MyDataset.read`` returns, gcn.py:84-102) into shard files + an ``index.json``; returns the paths.
+    ``node_level=True``: every ``.y`` is [n_nodes, C] (version-2 shards; ``index.json`` says ``"labels": "node"``)."""
     os.makedirs(out_dir, exist_ok=True)
     paths, chunk, counts = [], [], []
 
     def flush():
         if chunk:
             path = os.path.join(out_dir, f"{prefix}-{len(paths):05d}.gcss")
-            write_shard(path, pack_graphs(chunk))
+            write_shard(path, pack_graphs(chunk, node_level=node_level))
             paths.append(path)
             counts.append(len(chunk))
             chunk.clear()
@@ -197,7 +218,8 @@ def write_dataset(graphs: Iterable, out_dir: str, graphs_per_shard: int = 4096, 
     if not paths:
         raise ValueError("Datasets cannot be empty")
     with open(os.path.join(out_dir, "index.json"), "w") as f:
-        json.dump({"format": MAGIC.decode(), "version": VERSION,
+        json.dump({"format": MAGIC.decode(), "version": VERSION_NODE_LEVEL if node_level else VERSION,
+                   "labels": "node" if node_level else "graph",
                    "shards": [{"file": os.path.basename(p), "n_graphs": c} for p, c in zip(paths, counts)]}, f, indent=1)
     return paths
 

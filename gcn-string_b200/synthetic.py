@@ -12,7 +12,9 @@ What the reference's offline generator emits per protein pair, restated as a sam
   * adjacency values are all 1 (src/scripts/gcn.py:187-197 pops ``weight``);
   * node features: 16 NetSurfP columns in the real data (gcn_utills.py:293-311),
     mostly probabilities -> U[0,1); width F is a parameter (BASELINE.json uses 32);
-  * labels one-hot [0,1] positive / [1,0] negative, balanced (src/scripts/gcn.py:259,262).
+  * labels one-hot [0,1] positive / [1,0] negative, balanced (src/scripts/gcn.py:259,262);
+    ``node_level=True`` instead labels every residue (a per-residue task such as interface residues): one-hot of the
+    argmax of a fixed random projection of the summed neighbour features, which a GeneralGNN can learn.
 
 Everything is NumPy with ``default_rng(seed + graph_id)`` so any graph can be
 regenerated alone.  The output is the packed layout the device batching kernel consumes
@@ -34,13 +36,14 @@ class PackedGraphs:
     rowptr[sumN+1] int64  start of each node's neighbour list in ``col`` (dataset-global)
     col[sumNNZ]    int32  neighbour index LOCAL to the graph, ascending within a row
     x[sumN, F]     float32
-    y[G, C]        float32 one-hot
+    y[G, C]        float32 one-hot graph labels, or y[sumN, C] node labels (rows in node order) when node_level
     """
     node_off: np.ndarray
     rowptr: np.ndarray
     col: np.ndarray
     x: np.ndarray
     y: np.ndarray
+    node_level: bool = False
 
     @property
     def n_graphs(self) -> int:
@@ -63,7 +66,7 @@ class PackedGraphs:
         n = n1 - n0
         a = sp.csr_matrix((np.ones(e1 - e0, dtype=np.int64), self.col[e0:e1].astype(np.int32),
                            (self.rowptr[n0:n1 + 1] - e0).astype(np.int32)), shape=(n, n))
-        return self.x[n0:n1], a, self.y[g]
+        return self.x[n0:n1], a, (self.y[n0:n1] if self.node_level else self.y[g])
 
 
 def _protein_pairs(rng, n, deg):
@@ -116,9 +119,30 @@ def make_graph(seed: int, graph_id: int, n_mean: int = 500, deg: int = 12, n_fea
     return rowptr, c, x
 
 
+def node_labels(packed: PackedGraphs, n_classes: int, seed: int) -> np.ndarray:
+    """One-hot [sum N, C] node labels of a packed dataset: row n is one-hot at argmax_c of
+    (sum over the stored neighbours j of n of (x_j - 1/2)) . V[:, c], with V [F, C] standard normal from
+    ``default_rng(seed)`` - a function of the graph that one aggregation step can express."""
+    import scipy.sparse as sp
+    n = int(packed.node_off[-1])
+    rows = np.repeat(np.arange(n, dtype=np.int64), np.diff(packed.rowptr))
+    cols = packed.col.astype(np.int64) + np.repeat(packed.node_off[:-1], packed.n_nodes)[rows]
+    a = sp.csr_matrix((np.ones(rows.shape[0]), (rows, cols)), shape=(n, n))
+    v = np.random.default_rng(seed).standard_normal((packed.x.shape[1], n_classes))
+    score = (a @ (np.asarray(packed.x, dtype=np.float64) - 0.5)) @ v
+    y = np.zeros((n, n_classes), dtype=np.float32)
+    y[np.arange(n), np.argmax(score, axis=1)] = 1.0
+    return y
+
+
+def _with_node_labels(p: PackedGraphs, n_classes: int, seed: int) -> PackedGraphs:
+    return PackedGraphs(p.node_off, p.rowptr, p.col, p.x, node_labels(p, n_classes, seed + 0x5EED), node_level=True)
+
+
 def make_dataset(n_graphs: int, seed: int = 0, n_mean: int = 500, deg: int = 12,
-                 n_feat: int = 32, n_classes: int = 2) -> PackedGraphs:
-    """G(seed, n_mean, deg, F) of SURVEY.md §8d, packed."""
+                 n_feat: int = 32, n_classes: int = 2, node_level: bool = False) -> PackedGraphs:
+    """G(seed, n_mean, deg, F) of SURVEY.md §8d, packed.  ``node_level=True``: per-node labels (``node_labels``, one
+    projection for the whole dataset) instead of the balanced graph labels; the graphs themselves are the same."""
     rps: List[np.ndarray] = []
     cols: List[np.ndarray] = []
     xs: List[np.ndarray] = []
@@ -134,6 +158,9 @@ def make_dataset(n_graphs: int, seed: int = 0, n_mean: int = 500, deg: int = 12,
     rowptr = np.concatenate(rps + [np.array([e_off], dtype=np.int64)]) if n_graphs else np.zeros(1, np.int64)
     col = np.concatenate(cols) if n_graphs else np.zeros(0, np.int32)
     x = np.concatenate(xs) if n_graphs else np.zeros((0, n_feat), np.float32)
+    if node_level:
+        return _with_node_labels(PackedGraphs(node_off, rowptr, col, x, np.zeros((0, n_classes), np.float32)), n_classes,
+                                 seed)
     y = np.zeros((n_graphs, n_classes), dtype=np.float32)
     lab = np.arange(n_graphs) % n_classes          # balanced (gcn.py:265-266)
     y[np.arange(n_graphs), lab] = 1.0
@@ -141,7 +168,10 @@ def make_dataset(n_graphs: int, seed: int = 0, n_mean: int = 500, deg: int = 12,
 
 
 def concat_packed(parts: List[PackedGraphs]) -> PackedGraphs:
-    """Concatenate packed datasets (graph order = order of the parts)."""
+    """Concatenate packed datasets (graph order = order of the parts).  Graph- and node-labelled parts do not mix."""
+    kinds = {bool(p.node_level) for p in parts}
+    if len(kinds) > 1:
+        raise ValueError("cannot concatenate graph-labelled and node-labelled datasets")
     if len(parts) == 1:
         return parts[0]
     node_off = [np.zeros(1, dtype=np.int64)]
@@ -154,7 +184,7 @@ def concat_packed(parts: List[PackedGraphs]) -> PackedGraphs:
         e0 += int(p.rowptr[-1])
     rowptr.append(np.array([e0], dtype=np.int64))
     return PackedGraphs(np.concatenate(node_off), np.concatenate(rowptr), np.concatenate([p.col for p in parts]),
-                        np.concatenate([p.x for p in parts]), np.concatenate([p.y for p in parts]))
+                        np.concatenate([p.x for p in parts]), np.concatenate([p.y for p in parts]), kinds.pop())
 
 
 def _make_range(args):
@@ -176,19 +206,20 @@ def _make_range(args):
 
 
 def make_dataset_parallel(n_graphs: int, seed: int = 0, n_mean: int = 500, deg: int = 12, n_feat: int = 32,
-                          n_classes: int = 2, workers: int = 0) -> PackedGraphs:
+                          n_classes: int = 2, workers: int = 0, node_level: bool = False) -> PackedGraphs:
     """make_dataset over a process pool (the same graphs: every graph is seeded by its id).  workers = 0: the cores this
     process may run on."""
     import multiprocessing as mp
     import os
     workers = workers or len(os.sched_getaffinity(0))
     if workers <= 1 or n_graphs < 4 * workers:
-        return make_dataset(n_graphs, seed, n_mean, deg, n_feat, n_classes)
+        return make_dataset(n_graphs, seed, n_mean, deg, n_feat, n_classes, node_level=node_level)
     chunk = -(-n_graphs // (4 * workers))
     jobs = [(seed, g0, min(g0 + chunk, n_graphs), n_mean, deg, n_feat, n_classes) for g0 in range(0, n_graphs, chunk)]
     with mp.get_context("fork").Pool(workers) as pool:
         parts = pool.map(_make_range, jobs)
-    return concat_packed(parts)
+    out = concat_packed(parts)
+    return _with_node_labels(out, n_classes, seed) if node_level else out
 
 
 def tile_dataset(packed: PackedGraphs, n_graphs: int) -> PackedGraphs:
@@ -201,15 +232,17 @@ def tile_dataset(packed: PackedGraphs, n_graphs: int) -> PackedGraphs:
         return out
     n1 = int(out.node_off[n_graphs])
     e1 = int(out.rowptr[n1])
-    return PackedGraphs(out.node_off[:n_graphs + 1], out.rowptr[:n1 + 1], out.col[:e1], out.x[:n1], out.y[:n_graphs])
+    return PackedGraphs(out.node_off[:n_graphs + 1], out.rowptr[:n1 + 1], out.col[:e1], out.x[:n1],
+                        out.y[:n1] if out.node_level else out.y[:n_graphs], out.node_level)
 
 
-def pack_graphs(graphs) -> PackedGraphs:
+def pack_graphs(graphs, node_level: bool = False) -> PackedGraphs:
     """Pack a list of per-graph objects exposing ``.x [n,F]``, ``.a`` (scipy sparse / dense
     [n,n]) and ``.y`` — what the reference's MyDataset.read returns (gcn.py:84-102) — into
     the device-ready layout.  Explicit zeros are dropped and duplicates merged, exactly as
     ``sp.find`` does in Spektral's collate (SURVEY.md §8 a1); values are otherwise ignored
-    (a5: GeneralConv never reads them)."""
+    (a5: GeneralConv never reads them).  ``node_level=True``: every ``.y`` is [n_nodes, C] (one label row per node,
+    all with the same C) and the rows are stacked in node order."""
     import scipy.sparse as sp
     node_off = np.zeros(len(graphs) + 1, dtype=np.int64)
     rps, cols, xs, ys = [], [], [], []
@@ -228,9 +261,19 @@ def pack_graphs(graphs) -> PackedGraphs:
         e_off += int(a.indptr[-1])
         cols.append(a.indices.astype(np.int32))
         xs.append(x.astype(np.float32))
-        ys.append(np.asarray(gr.y, dtype=np.float32).reshape(-1))
+        if node_level:
+            yg = np.asarray(gr.y, dtype=np.float32) if gr.y is not None else None
+            if yg is None or yg.ndim != 2 or yg.shape[0] != n or (ys and yg.shape[1] != ys[0].shape[1]):
+                want = f"[{n}, {ys[0].shape[1]}]" if ys else f"[{n}, C]"
+                raise ValueError(f"graph {g}: node-level labels must be {want}, got "
+                                 f"{None if yg is None else tuple(yg.shape)}")
+            ys.append(yg)
+        else:
+            ys.append(np.asarray(gr.y, dtype=np.float32).reshape(-1))
     rowptr = np.concatenate(rps + [np.array([e_off], dtype=np.int64)]) if graphs else np.zeros(1, np.int64)
     col = np.concatenate(cols) if graphs else np.zeros(0, np.int32)
     x = np.concatenate(xs) if graphs else np.zeros((0, 0), np.float32)
+    if node_level:
+        return PackedGraphs(node_off, rowptr, col, x, np.concatenate(ys) if graphs else np.zeros((0, 0), np.float32), True)
     y = np.stack(ys) if graphs else np.zeros((0, 0), np.float32)
     return PackedGraphs(node_off, rowptr, col, x, y)

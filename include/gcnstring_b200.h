@@ -87,6 +87,15 @@ int gcs_gather_graphs(const int64_t* graph_ids, int32_t n_graphs, const int64_t*
                       int32_t n_feat, int32_t n_classes, const int64_t* dst_node_off, const int64_t* dst_edge_off,
                       int64_t* dst_rowptr, int32_t* dst_col, float* dst_x, float* dst_y, gcs_stream stream);
 
+/* Node-level labels of a disjoint batch.  Replaces Spektral's collate_labels_disjoint(y_list, node_level=True) =
+ * np.vstack(y_list): copies the [n_g, width] row block of every graph graph_ids[0..n_graphs) out of a packed node-row
+ * array src [sum n, width] (row offsets src_node_off [G + 1], as ds_node_off) to batch rows
+ * [dst_graph_ptr[j], dst_graph_ptr[j + 1]) of dst [N, width] - the graph_ptr gcs_batch_disjoint just wrote (which is
+ * then called with ds_y = y = NULL).  src / src_node_off may be in HBM or in pinned host memory (read over the host
+ * link in coalesced runs, 128-bit when width and alignment allow).  One launch; graphs of 0 rows copy nothing. */
+int gcs_gather_node_rows(const int64_t* graph_ids, int32_t n_graphs, const int64_t* src_node_off, const float* src,
+                         int32_t width, const int32_t* dst_graph_ptr, float* dst, gcs_stream stream);
+
 /* Row-major-sorted COO (what tf.sparse.reorder returns; Spektral's
  * sp_matrix_to_sp_tensor) -> int32 CSR.  *status_dev != 0 if unsorted/out of range. */
 int gcs_coo_to_csr(const int64_t* coo_indices, int64_t nnz, int64_t n_rows, int32_t* rowptr,
@@ -285,6 +294,14 @@ int gcs_attn_sum_pool_bwd(const float* dout, int64_t lddo, const float* X, int64
  * --------------------------------------------------------------------------------- */
 int gcs_softmax_xent(const float* logits, const float* y, int32_t B, int32_t C, float* probs,
                      float* loss_acc, float* dlogits, float grad_scale, gcs_stream stream);
+/* The same for any number of rows.  Up to 65 536 rows (B <= 65536) it IS gcs_softmax_xent (one thread block) and
+ * needs no workspace; above, a grid-wide kernel runs the same per-row expressions - probs and dlogits are bit-identical
+ * to gcs_softmax_xent's - and leaves per-block fp64 loss sums and integer hit counts in the workspace, which a second
+ * launch adds in a fixed order (bit-identical run to run).  The choice depends on B alone.  workspace:
+ * gcs_softmax_xent_workspace_bytes(B, C) bytes, 8-byte aligned (only read when loss_acc != NULL). */
+int64_t gcs_softmax_xent_workspace_bytes(int64_t B, int32_t C);
+int gcs_softmax_xent_ws(const float* logits, const float* y, int32_t B, int32_t C, float* probs, float* loss_acc,
+                        float* dlogits, float grad_scale, void* workspace, int64_t workspace_bytes, gcs_stream stream);
 
 /* ---------------------------------------------------------------------------------
  * K11  Residue contact maps of a batch of chains (SURVEY.md 8 f4).  Replaces
@@ -380,7 +397,7 @@ typedef struct gcs_batch {
   const int32_t* graph_ptr; /* [B+1] */
   const float* x;           /* [N, F] */
   int64_t ldx;
-  const float* y;           /* [B, C] one-hot; NULL for inference */
+  const float* y;           /* [B, C] one-hot ([N, C] node labels when pool == 0); NULL for inference */
   const int64_t* seg_ids;       /* [N] graph id of every node (Spektral's i); needed by the pooled backward */
   const int32_t* rb4_blk_ptr;   /* row-block form of pattern(A) (gcs_spmm_build_rb, height rb_height), or NULL */
   const uint32_t* rb4_ent;
@@ -404,9 +421,10 @@ int gcs_model_forward(const gcs_model_config* cfg, const float* params, float* s
                       const gcs_batch* batch, int32_t training, float* out, void* workspace,
                       int64_t workspace_bytes, gcs_stream stream);
 /* Training-mode forward + backward.  grads: flat, same layout as params (overwritten).
- * loss_acc[2] = {mean categorical cross-entropy over this batch, accuracy}; probs [B,C].
- * grad_scale multiplies dLoss (1/B reproduces the reference; use 1/global_B when the
- * gradients are then summed across data-parallel ranks). */
+ * loss_acc[2] = {mean categorical cross-entropy over this batch, accuracy}; probs [B,C] ([N,C] when pool == 0: the
+ * loss is then the mean over nodes).  grad_scale multiplies dLoss (1/B - 1/N node-level - reproduces the reference; use
+ * 1/global_B or 1/global_N when the gradients are then summed across data-parallel ranks).  The loss runs through
+ * gcs_softmax_xent_ws; gcs_model_workspace_bytes includes its workspace. */
 int gcs_model_train_step(const gcs_model_config* cfg, const float* params, float* state,
                          const gcs_batch* batch, float grad_scale, float* grads, float* probs,
                          float* loss_acc, void* workspace, int64_t workspace_bytes,
