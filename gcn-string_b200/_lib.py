@@ -84,6 +84,8 @@ PROTOTYPES = {
     "gcs_softmax_xent": (c_int32, [P, P, I32, I32, P, P, P, F32, P]),
     "gcs_softmax_xent_workspace_bytes": (c_int64, [I64, I32]),
     "gcs_softmax_xent_ws": (c_int32, [P, P, I32, I32, P, P, P, F32, P, I64, P]),
+    "gcs_sigmoid_bce_workspace_bytes": (c_int64, [I64, I32]),
+    "gcs_sigmoid_bce": (c_int32, [P, P, I64, I32, P, P, P, F32, P, I64, P]),
     "gcs_sgd_step": (c_int32, [P, P, I64, F32, F32, P]),
     "gcs_adam_step": (c_int32, [P, P, P, P, I64, F64, F64, F64, F64, I64, F32, P]),
     "gcs_comm_unique_id": (c_int32, [P]),

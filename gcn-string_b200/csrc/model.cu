@@ -4,7 +4,7 @@
 //
 //   out = pre(x)                                   MLP: [Dense -> BN -> PReLU] x P
 //   for k in 1..L:  z = A . prelu(bn(out.W_k + b_k));  out = concat([z, out])
-//   out = pool(out, i);  out = post(out)          MLP, last layer Dense -> BN -> softmax
+//   out = pool(out, i);  out = post(out)          MLP, last layer Dense -> BN -> softmax | sigmoid | linear
 //   pool: segment_sum ('sum'), segment_mean ('avg'), attention-weighted sum ('attn_sum', one extra trainable vector
 //   pool.attn_kernel [Wc] after the last post block), or none (node-level output)
 //
@@ -92,8 +92,8 @@ static int check_config(const gcs_model_config* c) {
     return fail(GCS_ERR_INVALID_ARGUMENT, "model config: connectivity must be 0 (None), 1 ('cat') or 2 ('sum')");
   if (c->pool < kPoolNone || c->pool > kPoolAttnSum)
     return fail(GCS_ERR_UNSUPPORTED, "model config: pool must be 0 (None), 1 ('sum'), 2 ('avg') or 3 ('attn_sum')");
-  if (c->final_activation != 0 && c->final_activation != 1)
-    return fail(GCS_ERR_UNSUPPORTED, "model config: final activation must be linear or softmax");
+  if (c->final_activation < 0 || c->final_activation > 2)
+    return fail(GCS_ERR_UNSUPPORTED, "model config: final activation must be 0 (linear), 1 (softmax) or 2 (sigmoid)");
   if (c->aggregate < 0 || c->aggregate > 2)
     return fail(GCS_ERR_INVALID_ARGUMENT, "model config: aggregate must be 0 ('sum'), 1 ('mean') or 2 ('max')");
   if (c->aggregate == 2 && c->connectivity == 2)
@@ -148,7 +148,8 @@ struct Plan {
   int64_t bn_ws_bytes = 0;
   void* lin_ws = nullptr;       // split weights of the tensor-core GEMM in flight
   int64_t lin_ws_bytes = 0;
-  void* xent_ws = nullptr;      // loss partials of gcs_softmax_xent_ws (0 bytes up to its row threshold)
+  void* xent_ws = nullptr;      // loss partials of gcs_softmax_xent_ws (0 bytes up to its row threshold), or of
+                                // gcs_sigmoid_bce with final_activation = 2
   int64_t xent_ws_bytes = 0;
   // backward
   float* gcat = nullptr;        // [N, Wc]  without pooling (node-level output) and for 'attn_sum': dLoss/d(emb(L)) in full
@@ -336,7 +337,9 @@ static void make_plan(const gcs_model_config& c, int64_t N, int B, bool training
     p.prep_ws_bytes = list_step_weights(c, p, nullptr, nullptr, nullptr, nullptr);
     p.prep_ws = a.take<char>(p.prep_ws_bytes);
   }
-  p.xent_ws_bytes = gcs_softmax_xent_workspace_bytes(p.rows_post, p.C);   // last: graph-level plans keep their layout
+  // last: graph-level softmax plans keep their layout
+  p.xent_ws_bytes = c.final_activation == 2 ? gcs_sigmoid_bce_workspace_bytes(p.rows_post, p.C)
+                                            : gcs_softmax_xent_workspace_bytes(p.rows_post, p.C);
   p.xent_ws = a.take<char>(p.xent_ws_bytes);
   *total = a.used;
 }
@@ -557,6 +560,17 @@ struct GradReady {
   void* user;
 };
 
+// The loss of the fused train step on p.logits: categorical cross-entropy on a softmax head, binary cross-entropy on a
+// sigmoid head; leaves dLoss/dlogits (scaled by grad_scale) in p.dlogits.
+static int run_loss(const gcs_model_config& c, const Plan& p, const float* y, float* probs, float* loss_acc,
+                    float grad_scale, gcs_stream st) {
+  if (c.final_activation == 2)
+    return gcs_sigmoid_bce(p.logits, y, p.rows_post, p.C, probs, loss_acc, p.dlogits, grad_scale, p.xent_ws,
+                           p.xent_ws_bytes, st);
+  return gcs_softmax_xent_ws(p.logits, y, static_cast<int32_t>(p.rows_post), p.C, probs, loss_acc, p.dlogits, grad_scale,
+                             p.xent_ws, p.xent_ws_bytes, st);
+}
+
 // Reverse pass given dlogits = dLoss/d(logits) [rows_post, C]; needs the activations a
 // training-mode run_forward left in the workspace.
 static int run_backward(const gcs_model_config& c, const Plan& p, const float* params, float* grads,
@@ -737,7 +751,10 @@ extern "C" int gcs_model_forward(const gcs_model_config* cfg, const float* param
   if (workspace_bytes < total)
     return fail(GCS_ERR_WORKSPACE, "gcs_model_forward: workspace %lld < %lld bytes", (long long)workspace_bytes, (long long)total);
   GCS_TRY(run_forward(*cfg, p, params, state, *batch, training != 0, stream));
-  if (cfg->final_activation == 1) {
+  if (cfg->final_activation == 2) {
+    GCS_TRY(gcs_sigmoid_bce(p.logits, nullptr, p.rows_post, p.C, out, nullptr, nullptr, 0.f, p.xent_ws, p.xent_ws_bytes,
+                            stream));
+  } else if (cfg->final_activation == 1) {
     GCS_CHECK_ARG(p.rows_post < INT32_MAX, "gcs_model_forward: too many output rows");
     GCS_TRY(gcs_softmax_xent_ws(p.logits, nullptr, static_cast<int32_t>(p.rows_post), p.C, out, nullptr, nullptr, 0.f,
                                 p.xent_ws, p.xent_ws_bytes, stream));
@@ -753,7 +770,9 @@ extern "C" int gcs_model_train_step(const gcs_model_config* cfg, const float* pa
                                     gcs_stream stream) {
   GCS_TRY(check_config(cfg));
   GCS_TRY(check_batch(*cfg, batch, true, true));
-  GCS_CHECK_ARG(cfg->final_activation == 1, "gcs_model_train_step: the loss is categorical cross-entropy on a softmax output");
+  GCS_CHECK_ARG(cfg->final_activation == 1 || cfg->final_activation == 2,
+                "gcs_model_train_step: the loss is categorical cross-entropy on a softmax output or binary cross-entropy "
+                "on a sigmoid output");
   GCS_CHECK_ARG(params && state && grads && loss_acc && workspace, "gcs_model_train_step: null pointer");
   GCS_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 255u) == 0, "gcs_model_train_step: workspace must be 256-byte aligned");
   const gcs_model_config& c = *cfg;
@@ -768,8 +787,7 @@ extern "C" int gcs_model_train_step(const gcs_model_config* cfg, const float* pa
   GCS_TRY(prepare_step_weights(c, p, params, &prepared, stream));
   PreparedScope prepared_scope(&prepared);
   GCS_TRY(run_forward(c, p, params, state, bt, true, stream));
-  GCS_TRY(gcs_softmax_xent_ws(p.logits, bt.y, static_cast<int32_t>(p.rows_post), p.C, probs, loss_acc, p.dlogits,
-                              grad_scale, p.xent_ws, p.xent_ws_bytes, stream));
+  GCS_TRY(run_loss(c, p, bt.y, probs, loss_acc, grad_scale, stream));
 
   return run_backward(c, p, params, grads, bt, p.dlogits, stream);
 }
@@ -821,7 +839,9 @@ extern "C" int gcs_model_train_step_dp(const gcs_model_config* cfg, const float*
                                        gcs_comm* comm, gcs_stream comm_stream, int32_t sync_batchnorm) {
   GCS_TRY(check_config(cfg));
   GCS_TRY(check_batch(*cfg, batch, true, true));
-  GCS_CHECK_ARG(cfg->final_activation == 1, "gcs_model_train_step_dp: the loss is categorical cross-entropy on a softmax output");
+  GCS_CHECK_ARG(cfg->final_activation == 1 || cfg->final_activation == 2,
+                "gcs_model_train_step_dp: the loss is categorical cross-entropy on a softmax output or binary "
+                "cross-entropy on a sigmoid output");
   GCS_CHECK_ARG(params && state && grads && loss_acc && workspace && comm, "gcs_model_train_step_dp: null pointer");
   GCS_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 255u) == 0, "gcs_model_train_step_dp: workspace must be 256-byte aligned");
   GCS_CHECK_ARG(comm_stream != stream, "gcs_model_train_step_dp: the collective needs its own stream");
@@ -838,8 +858,7 @@ extern "C" int gcs_model_train_step_dp(const gcs_model_config* cfg, const float*
   GCS_TRY(prepare_step_weights(c, p, params, &prepared, stream));
   PreparedScope prepared_scope(&prepared);
   GCS_TRY(run_forward(c, p, params, state, bt, true, stream));
-  GCS_TRY(gcs_softmax_xent_ws(p.logits, bt.y, static_cast<int32_t>(p.rows_post), p.C, probs, loss_acc, p.dlogits, grad_scale,
-                              p.xent_ws, p.xent_ws_bytes, stream));
+  GCS_TRY(run_loss(c, p, bt.y, probs, loss_acc, grad_scale, stream));
   cudaEvent_t* ev = dp_events();
   DpSync sync{comm, grads, as_stream(stream), as_stream(comm_stream), {}, 0};
   for (int i = 0; i < 8; ++i) sync.ev[i] = ev[i];

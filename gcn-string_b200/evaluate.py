@@ -4,7 +4,8 @@ final curve kept on the device.
 
 ``evaluate`` runs ``model(inputs, training=False)`` (BatchNorm on moving statistics, folded into
 scale/shift; gcs_model_forward) over one pass of the loader, evaluates loss and accuracy with the
-fused softmax/cross-entropy kernel (gcs_softmax_xent) and returns the batch-size-weighted averages
+fused softmax/cross-entropy kernel (gcs_softmax_xent; sigmoid/binary cross-entropy, gcs_sigmoid_bce, for a model
+built with activation='sigmoid') and returns the batch-size-weighted averages
 plus the per-batch predictions, like the reference.  ``roc_curve`` / ``auc`` follow scikit-learn's
 definitions (the reference calls ``sklearn.metrics.roc_curve(labels, probas)`` and ``auc``); they
 are sort + prefix sums and run on whatever device the scores live on.
@@ -14,14 +15,18 @@ from __future__ import annotations
 import numpy as np
 
 from . import _lib
-from .losses import CategoricalCrossentropy, categorical_accuracy
+from .losses import BinaryCrossentropy, CategoricalCrossentropy, binary_accuracy, categorical_accuracy
 
 
 def evaluate(model, loader, loss_fn=None):
     """One pass over ``loader`` -> (np.array([loss, acc]) weighted by batch size, [pred per batch]).
-    Mirrors gcn.py:342-362; the only host transfers are the two scalars per batch."""
+    Mirrors gcn.py:342-362; the only host transfers are the two scalars per batch.  The loss and accuracy default to
+    BinaryCrossentropy / binary_accuracy for a model built with activation='sigmoid', to CategoricalCrossentropy /
+    categorical_accuracy otherwise."""
     torch = _lib.require_cuda()
-    loss_fn = loss_fn or CategoricalCrossentropy()
+    sigmoid = getattr(model, "config", {}).get("activation") == "sigmoid"
+    loss_fn = loss_fn or (BinaryCrossentropy() if sigmoid else CategoricalCrossentropy())
+    metric = binary_accuracy if sigmoid else categorical_accuracy
     stats, preds = [], []
     step = 0
     while step < loader.steps_per_epoch:
@@ -29,14 +34,15 @@ def evaluate(model, loader, loss_fn=None):
         inputs, target = next(loader)
         pred = model(inputs, training=False)
         preds.append(pred)
-        stats.append(torch.stack([loss_fn(target, pred).reshape(()), categorical_accuracy(target, pred).mean().reshape(()),
+        stats.append(torch.stack([loss_fn(target, pred).reshape(()), metric(target, pred).mean().reshape(()),
                                   torch.tensor(float(target.shape[0]), device=pred.device)]))
     out = torch.stack(stats).cpu().numpy().astype(np.float64)
     return np.average(out[:, :-1], 0, weights=out[:, -1]), preds
 
 
 def positive_scores(preds, column: int = 1):
-    """gcn.py:390-391: stack the per-batch softmax outputs and keep the positive-class column."""
+    """gcn.py:390-391: stack the per-batch softmax outputs and keep the positive-class column (``column=0`` for the
+    one-column output of a sigmoid head)."""
     torch = _lib.require_cuda()
     return torch.cat([p[:, column] for p in preds])
 

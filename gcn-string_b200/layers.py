@@ -141,8 +141,8 @@ class MLP:
             raise NotImplementedError("native path implements dropout=0.0 only")
         if activation != "prelu":
             raise NotImplementedError("native path implements activation='prelu' only")
-        if final_activation not in (None, "linear", "softmax", "prelu"):
-            raise NotImplementedError("final_activation must be None, 'prelu' or 'softmax'")
+        if final_activation not in (None, "linear", "softmax", "sigmoid", "prelu"):
+            raise NotImplementedError("final_activation must be None, 'prelu', 'softmax' or 'sigmoid'")
         self.output, self.hidden, self.layers, self.batch_norm = output, hidden, layers, batch_norm
         self.final_activation = final_activation
         self.seed = seed
@@ -167,4 +167,6 @@ class MLP:
             out = ops.bn_prelu_fwd(h, scale, shift, blk.alpha)
         if self.final_activation == "softmax":
             out, _, _ = ops.softmax_xent(out)
+        elif self.final_activation == "sigmoid":
+            out, _, _ = ops.sigmoid_bce(out)
         return out

@@ -3,7 +3,11 @@
 calls, :339,:355 accuracy).  Keras evaluates the loss on the LOGITS of a softmax output
 (it recovers them from the activation); the model attaches them to its output the same way
 (``_gcs_logits``), and the native kernel computes loss, accuracy and dLoss/dlogits in one
-launch (csrc/loss.cu).  Reduction is the Keras default: mean over the batch."""
+launch (csrc/loss.cu).  Reduction is the Keras default: mean over the batch.
+
+``BinaryCrossentropy`` and ``binary_accuracy`` are the Keras pair for a sigmoid head (binary and multi-label targets):
+on the logits of a ``GeneralGNN(activation='sigmoid')`` output, or with ``from_logits=True``, they run the fused kernel
+of csrc/loss_bce.cu."""
 from __future__ import annotations
 
 from . import _lib, ops
@@ -38,3 +42,47 @@ def categorical_accuracy(y_true, y_pred):
     torch = _lib.require_cuda()
     y = _lib.as_tensor(y_true).to(device="cuda")
     return (y.argmax(dim=-1) == y_pred.argmax(dim=-1)).to(torch.float32)
+
+
+class BinaryCrossentropy:
+    """tf.keras.losses.BinaryCrossentropy: per element ``max(z, 0) - z*y + log1p(exp(-|z|))`` on the logits z, the mean
+    over the last axis, then over the rows.  Labels may be multi-hot or soft, in [0, 1]."""
+
+    def __init__(self, from_logits=False, label_smoothing=0.0, axis=-1, reduction="sum_over_batch_size",
+                 name="binary_crossentropy"):
+        if label_smoothing != 0.0:
+            raise NotImplementedError("label_smoothing is not built")
+        if axis != -1:
+            raise NotImplementedError("only axis=-1 is built")
+        if reduction not in ("sum_over_batch_size", "auto"):
+            raise NotImplementedError("only the default mean-over-batch reduction is built")
+        self.from_logits = from_logits
+        self.name = name
+
+    def __call__(self, y_true, y_pred):
+        torch = _lib.require_cuda()
+        y = _lib.as_tensor(y_true).to(device="cuda", dtype=torch.float32)
+        if self.from_logits:
+            logits = y_pred
+        elif getattr(y_pred, "_gcs_activation", None) == "sigmoid":
+            logits = y_pred._gcs_logits
+        else:
+            # probabilities of unknown origin: Keras' fallback (clip, then -(y log(p + eps) + (1 - y) log(1 - p + eps)))
+            eps = 1e-7
+            p = y_pred.clamp(eps, 1.0 - eps)
+            bce = y * (p + eps).log() + (1.0 - y) * (1.0 - p + eps).log()
+            return (-bce).mean(dim=-1).mean()
+        tape = getattr(y_pred, "_gcs_tape", None)
+        _, loss_acc, dlogits = ops.sigmoid_bce(logits, y, want_grad=tape is not None)
+        if tape is not None:
+            tape.loss_record = dict(dlogits=dlogits, loss_acc=loss_acc)
+        return loss_acc[0]
+
+
+def binary_accuracy(y_true, y_pred, threshold=0.5):
+    """Per-row mean over the columns of ``y_true == (y_pred > threshold)``, like tf.keras.metrics.binary_accuracy (the
+    comparison is on the float32 probabilities)."""
+    torch = _lib.require_cuda()
+    y = _lib.as_tensor(y_true).to(device="cuda", dtype=torch.float32)
+    pred = (_lib.as_tensor(y_pred) > threshold).to(torch.float32)
+    return (y == pred).to(torch.float32).mean(dim=-1)

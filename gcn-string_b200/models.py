@@ -265,6 +265,7 @@ class GeneralGNN:
         off = lib.gcs_model_logits_offset(self._c, batch.n_nodes, batch.n_graphs, int(training))
         logits = ws[off:off + out.numel() * 4].view(torch.float32).view(out.shape)
         out._gcs_logits = logits       # like Keras' `_keras_logits`: lets the loss use the logits
+        out._gcs_activation = self.cfg.activation
         if tape is not None:
             tape.model = self
             tape.ctx = dict(batch=batch, keep=keep, ws=ws, out=out)
@@ -279,7 +280,8 @@ class GeneralGNN:
                                      ptr(ctx["ws"]), ctx["ws"].numel(), stream_ptr()), "gcs_model_backward")
 
     def train_step_grads(self, inputs, target, grad_scale: Optional[float] = None, comm=None, sync_bn: bool = False):
-        """Fused training-mode forward + categorical cross-entropy + backward (one C call).
+        """Fused training-mode forward + loss + backward (one C call): categorical cross-entropy with
+        activation='softmax', binary cross-entropy (mean over the C columns, then the rows) with activation='sigmoid'.
         Leaves the gradients in ``self.grads``; returns (loss_acc [2] device tensor = {loss,
         accuracy}, probs [B, C]).  ``grad_scale`` defaults to 1/B (mean loss, gcn.py:335).
         ``comm`` (distributed.NativeComm): the data-parallel form - the gradients are SUM all-reduced over the

@@ -561,6 +561,31 @@ def softmax_xent(logits, y=None, grad_scale: Optional[float] = None, want_grad=F
     return probs, loss_acc, dlogits
 
 
+def sigmoid_bce(logits, y=None, grad_scale: Optional[float] = None, want_grad=False):
+    """Returns (probs, loss_acc[2] or None, dlogits or None) of gcs_sigmoid_bce: probs = sigmoid(logits), loss_acc =
+    {binary cross-entropy (mean over the columns, then the rows), binary accuracy}, dlogits = (probs - y) * grad_scale / C
+    (``grad_scale`` defaults to 1 / rows)."""
+    torch = _t()
+    lib = _lib.load()
+    logits, _ = _mat(logits, "logits")
+    logits = logits.contiguous()
+    b, c = logits.shape
+    if y is not None:
+        y, _ = _mat(y, "y")
+        if tuple(y.shape) != (b, c):
+            raise ValueError(f"y must be [{b}, {c}], got {tuple(y.shape)}")
+        y = y.contiguous()
+    probs = torch.empty_like(logits)
+    loss_acc = torch.empty(2, dtype=torch.float32, device="cuda") if y is not None else None
+    dlogits = torch.empty_like(logits) if (want_grad and y is not None) else None
+    gs = (1.0 / b if b else 0.0) if grad_scale is None else grad_scale
+    nbytes = int(lib.gcs_sigmoid_bce_workspace_bytes(b, c))
+    ws = torch.empty(nbytes, dtype=torch.uint8, device="cuda") if nbytes > 0 else None
+    check(lib.gcs_sigmoid_bce(ptr(logits), ptr(y), b, c, ptr(probs), ptr(loss_acc), ptr(dlogits), gs, ptr(ws), nbytes,
+                              stream_ptr()), "gcs_sigmoid_bce")
+    return probs, loss_acc, dlogits
+
+
 def sgd_step(w, g, lr: float, grad_scale: float = 1.0):
     lib = _lib.load()
     check(lib.gcs_sgd_step(ptr(w), ptr(g), w.numel(), lr, grad_scale, stream_ptr()), "gcs_sgd_step")

@@ -22,7 +22,7 @@ from typing import List, Optional, Tuple
 
 CONNECTIVITY = {None: 0, "cat": 1, "sum": 2}
 POOL = {None: 0, "sum": 1, "avg": 2, "attn_sum": 3}   # spektral GlobalSumPool / GlobalAvgPool / GlobalAttnSumPool
-FINAL_ACT = {None: 0, "linear": 0, "softmax": 1}
+FINAL_ACT = {None: 0, "linear": 0, "softmax": 1, "sigmoid": 2}
 AGGREGATE = {"sum": 0, "mean": 1, "max": 2}          # spektral scatter_sum / scatter_mean / scatter_max
 
 
@@ -62,7 +62,7 @@ class GNNConfig:
         if not self.batch_norm:
             raise NotImplementedError("native path implements batch_norm=True only")
         if self.activation not in FINAL_ACT:
-            raise NotImplementedError("final activation must be None/'linear'/'softmax'")
+            raise NotImplementedError("final activation must be None/'linear'/'softmax'/'sigmoid'")
         if self.pre_process < 1 or self.post_process < 1 or self.message_passing < 1:
             raise NotImplementedError("pre_process, post_process, message_passing must be >= 1")
         if min(self.in_features, self.output, self.hidden) < 1:

@@ -304,6 +304,24 @@ int gcs_softmax_xent_ws(const float* logits, const float* y, int32_t B, int32_t 
                         float* dlogits, float grad_scale, void* workspace, int64_t workspace_bytes, gcs_stream stream);
 
 /* ---------------------------------------------------------------------------------
+ * K5b  sigmoid + BinaryCrossentropy + binary_accuracy: the head of GeneralGNN(C, activation="sigmoid") trained with
+ * tf.keras.losses.BinaryCrossentropy() and tf.keras.metrics.binary_accuracy (binary and multi-label targets, graph- or
+ * node-level).  Per element l = max(z, 0) - z*y + log1p(exp(-|z|)) (tf.nn.sigmoid_cross_entropy_with_logits);
+ *   probs[rows,C] = sigmoid(logits) (NULL-able);
+ *   loss_acc[2] = {mean over rows of the mean over the C columns of l, mean of y == (probs > 0.5)} (NULL-able);
+ *   dlogits (NULL-able) = (probs - y) * grad_scale / C  (grad_scale = 1/rows for the mean loss; 1/global_rows under
+ *   data parallelism).
+ * Labels y may be multi-hot or soft, in [0, 1]; y may be NULL when only probs is asked for.  Any C, rows = 0 gives
+ * loss_acc = {0, 0}.  A grid-wide elementwise kernel leaves per-block fp64 loss sums and integer hit counts in the
+ * workspace and a second launch adds them in a fixed order (bit-identical run to run; the grid depends on rows * C
+ * alone).  workspace: gcs_sigmoid_bce_workspace_bytes(rows, C) bytes, 8-byte aligned (only read when loss_acc != NULL;
+ * 0 bytes when rows * C <= 1024).
+ * --------------------------------------------------------------------------------- */
+int64_t gcs_sigmoid_bce_workspace_bytes(int64_t rows, int32_t C);
+int gcs_sigmoid_bce(const float* logits, const float* y, int64_t rows, int32_t C, float* probs, float* loss_acc,
+                    float* dlogits, float grad_scale, void* workspace, int64_t workspace_bytes, gcs_stream stream);
+
+/* ---------------------------------------------------------------------------------
  * K11  Residue contact maps of a batch of chains (SURVEY.md 8 f4).  Replaces
  * GraphMaker.calculate_residue_dist / calculate_dist_matrix / generate_proximity_matrix
  * (src/utilities/gcn_utills.py:161-238): d = sqrt(sum((ca_i - ca_j)^2)) in float32 with NumPy's operation order
@@ -379,7 +397,7 @@ typedef struct gcs_model_config {
   int32_t connectivity;     /* 0 = None (out = z), 1 = 'cat' (out = concat[z, out]), 2 = 'sum' (out = z + out) */
   int32_t pool;             /* 0 = None (node-level output), 1 = 'sum', 2 = 'avg', 3 = 'attn_sum' (adds the trainable
                                attn_kernel [H*(L+1) or H] after the last post block) */
-  int32_t final_activation; /* 0 = linear, 1 = softmax */
+  int32_t final_activation; /* 0 = linear, 1 = softmax (C <= 64), 2 = sigmoid (any C) */
   float bn_momentum;        /* 0.99 */
   float bn_epsilon;         /* 1e-3 */
   int32_t aggregate;        /* GeneralConv aggregate: 0 = 'sum' (the reference's), 1 = 'mean', 2 = 'max' */
@@ -415,7 +433,7 @@ int64_t gcs_model_num_params(const gcs_model_config* cfg);
 int64_t gcs_model_num_state(const gcs_model_config* cfg);
 int64_t gcs_model_workspace_bytes(const gcs_model_config* cfg, int64_t n_nodes, int64_t nnz,
                                   int32_t n_graphs, int32_t training);
-/* Inference / training-mode forward.  out: [B, C] (or [N, C] when pool == 0).  With
+/* Inference / training-mode forward.  out: [B, C] (or [N, C] when pool == 0), after the final activation.  With
  * training != 0 BatchNorm uses batch statistics and updates `state` in place. */
 int gcs_model_forward(const gcs_model_config* cfg, const float* params, float* state,
                       const gcs_batch* batch, int32_t training, float* out, void* workspace,
@@ -424,7 +442,10 @@ int gcs_model_forward(const gcs_model_config* cfg, const float* params, float* s
  * loss_acc[2] = {mean categorical cross-entropy over this batch, accuracy}; probs [B,C] ([N,C] when pool == 0: the
  * loss is then the mean over nodes).  grad_scale multiplies dLoss (1/B - 1/N node-level - reproduces the reference; use
  * 1/global_B or 1/global_N when the gradients are then summed across data-parallel ranks).  The loss runs through
- * gcs_softmax_xent_ws; gcs_model_workspace_bytes includes its workspace. */
+ * gcs_softmax_xent_ws; gcs_model_workspace_bytes includes its workspace.  With final_activation = 2 (sigmoid) the loss
+ * is binary cross-entropy through gcs_sigmoid_bce instead: probs = sigmoid(logits), loss_acc = {mean binary
+ * cross-entropy, binary accuracy}, and grad_scale keeps its meaning (the 1/C of the per-row mean is applied inside).
+ * final_activation = 0 (linear) has no loss and is refused. */
 int gcs_model_train_step(const gcs_model_config* cfg, const float* params, float* state,
                          const gcs_batch* batch, float grad_scale, float* grads, float* probs,
                          float* loss_acc, void* workspace, int64_t workspace_bytes,
