@@ -14,6 +14,7 @@ from .params import GNNConfig, block_specs, init_params, n_state, n_trainable, n
 from .data import Dataset, DisjointLoader, Graph, SparseAdjacency  # noqa: F401,E402
 from .layers import GeneralConv, GlobalAttnSumPool, GlobalAvgPool, GlobalSumPool, MLP  # noqa: F401,E402
 from .losses import BinaryCrossentropy, CategoricalCrossentropy, binary_accuracy, categorical_accuracy  # noqa: F401,E402
+from .losses import Huber, MeanAbsoluteError, MeanSquaredError, mean_absolute_error, mean_squared_error  # noqa: F401,E402
 from .models import GeneralGNN, GradientTape  # noqa: F401,E402
 from . import optimizers  # noqa: F401,E402
 from . import shards  # noqa: F401,E402

@@ -22,7 +22,8 @@ class ModelConfig(Structure):
     _fields_ = [("in_features", c_int32), ("output", c_int32), ("hidden", c_int32),
                 ("message_passing", c_int32), ("pre_process", c_int32), ("post_process", c_int32),
                 ("connectivity", c_int32), ("pool", c_int32), ("final_activation", c_int32),
-                ("bn_momentum", c_float), ("bn_epsilon", c_float), ("aggregate", c_int32)]
+                ("bn_momentum", c_float), ("bn_epsilon", c_float), ("aggregate", c_int32),
+                ("loss", c_int32), ("huber_delta", c_float)]
 
 
 class Batch(Structure):
@@ -86,6 +87,8 @@ PROTOTYPES = {
     "gcs_softmax_xent_ws": (c_int32, [P, P, I32, I32, P, P, P, F32, P, I64, P]),
     "gcs_sigmoid_bce_workspace_bytes": (c_int64, [I64, I32]),
     "gcs_sigmoid_bce": (c_int32, [P, P, I64, I32, P, P, P, F32, P, I64, P]),
+    "gcs_regression_loss_workspace_bytes": (c_int64, [I64, I32]),
+    "gcs_regression_loss": (c_int32, [I32, F32, P, P, I64, I32, P, P, P, F32, P, I64, P]),
     "gcs_sgd_step": (c_int32, [P, P, I64, F32, F32, P]),
     "gcs_adam_step": (c_int32, [P, P, P, P, I64, F64, F64, F64, F64, I64, F32, P]),
     "gcs_comm_unique_id": (c_int32, [P]),
@@ -180,7 +183,7 @@ def model_config(cfg) -> ModelConfig:
     cfg.validate()
     return ModelConfig(cfg.in_features, cfg.output, cfg.hidden, cfg.message_passing, cfg.pre_process,
                        cfg.post_process, CONNECTIVITY[cfg.connectivity], POOL[cfg.pool],
-                       FINAL_ACT[cfg.activation], cfg.bn_momentum, cfg.bn_epsilon, AGGREGATE[cfg.aggregate])
+                       FINAL_ACT[cfg.activation], cfg.bn_momentum, cfg.bn_epsilon, AGGREGATE[cfg.aggregate], 0, 1.0)
 
 
 ALLREDUCE_FN = ctypes.CFUNCTYPE(c_int32, c_void_p, c_int64, c_void_p, c_void_p)

@@ -23,6 +23,7 @@
 // next layer and is needed again for its weight gradient), the skip operand is added in the aggregation's epilogue, and
 // the backward carries ONE running gradient g[N, H] = dLoss/d(out_k) that the input-gradient GEMM accumulates into.
 // The caller owns the workspace; nothing is allocated here.
+#include <cmath>
 #include <vector>
 
 #include "common.cuh"
@@ -101,6 +102,13 @@ static int check_config(const gcs_model_config* c) {
                                      "aggregation's own output, which the skip connection overwrites)");
   if (c->final_activation == 1 && c->output > 64)
     return fail(GCS_ERR_UNSUPPORTED, "model config: softmax over more than 64 classes is not built");
+  if (c->loss < 0 || c->loss > 3)
+    return fail(GCS_ERR_INVALID_ARGUMENT, "model config: loss must be 0 (the head's own), 1 (MSE), 2 (MAE) or 3 (Huber)");
+  if (c->loss != 0 && c->final_activation != 0)
+    return fail(GCS_ERR_UNSUPPORTED, "model config: the regression losses need a linear head (final_activation = 0)");
+  if (c->loss == 3 && !(std::isfinite(c->huber_delta) && c->huber_delta > 0.f))
+    return fail(GCS_ERR_INVALID_ARGUMENT, "model config: huber_delta must be finite and > 0, got %g",
+                static_cast<double>(c->huber_delta));
   return GCS_OK;
 }
 
@@ -148,8 +156,8 @@ struct Plan {
   int64_t bn_ws_bytes = 0;
   void* lin_ws = nullptr;       // split weights of the tensor-core GEMM in flight
   int64_t lin_ws_bytes = 0;
-  void* xent_ws = nullptr;      // loss partials of gcs_softmax_xent_ws (0 bytes up to its row threshold), or of
-                                // gcs_sigmoid_bce with final_activation = 2
+  void* xent_ws = nullptr;      // loss partials of gcs_softmax_xent_ws (0 bytes up to its row threshold), of
+                                // gcs_sigmoid_bce with final_activation = 2, or of gcs_regression_loss with 0
   int64_t xent_ws_bytes = 0;
   // backward
   float* gcat = nullptr;        // [N, Wc]  without pooling (node-level output) and for 'attn_sum': dLoss/d(emb(L)) in full
@@ -337,9 +345,10 @@ static void make_plan(const gcs_model_config& c, int64_t N, int B, bool training
     p.prep_ws_bytes = list_step_weights(c, p, nullptr, nullptr, nullptr, nullptr);
     p.prep_ws = a.take<char>(p.prep_ws_bytes);
   }
-  // last: graph-level softmax plans keep their layout
-  p.xent_ws_bytes = c.final_activation == 2 ? gcs_sigmoid_bce_workspace_bytes(p.rows_post, p.C)
-                                            : gcs_softmax_xent_workspace_bytes(p.rows_post, p.C);
+  // last: graph-level softmax plans keep their layout; the regression partials do not depend on c.loss
+  p.xent_ws_bytes = c.final_activation == 2   ? gcs_sigmoid_bce_workspace_bytes(p.rows_post, p.C)
+                    : c.final_activation == 0 ? gcs_regression_loss_workspace_bytes(p.rows_post, p.C)
+                                              : gcs_softmax_xent_workspace_bytes(p.rows_post, p.C);
   p.xent_ws = a.take<char>(p.xent_ws_bytes);
   *total = a.used;
 }
@@ -561,9 +570,13 @@ struct GradReady {
 };
 
 // The loss of the fused train step on p.logits: categorical cross-entropy on a softmax head, binary cross-entropy on a
-// sigmoid head; leaves dLoss/dlogits (scaled by grad_scale) in p.dlogits.
+// sigmoid head, the regression loss c.loss selects (MSE by default) on a linear head; leaves dLoss/dlogits (scaled by
+// grad_scale) in p.dlogits.
 static int run_loss(const gcs_model_config& c, const Plan& p, const float* y, float* probs, float* loss_acc,
                     float grad_scale, gcs_stream st) {
+  if (c.final_activation == 0)
+    return gcs_regression_loss(c.loss ? c.loss : 1, c.huber_delta, p.logits, y, p.rows_post, p.C, probs, loss_acc,
+                               p.dlogits, grad_scale, p.xent_ws, p.xent_ws_bytes, st);
   if (c.final_activation == 2)
     return gcs_sigmoid_bce(p.logits, y, p.rows_post, p.C, probs, loss_acc, p.dlogits, grad_scale, p.xent_ws,
                            p.xent_ws_bytes, st);
@@ -770,9 +783,6 @@ extern "C" int gcs_model_train_step(const gcs_model_config* cfg, const float* pa
                                     gcs_stream stream) {
   GCS_TRY(check_config(cfg));
   GCS_TRY(check_batch(*cfg, batch, true, true));
-  GCS_CHECK_ARG(cfg->final_activation == 1 || cfg->final_activation == 2,
-                "gcs_model_train_step: the loss is categorical cross-entropy on a softmax output or binary cross-entropy "
-                "on a sigmoid output");
   GCS_CHECK_ARG(params && state && grads && loss_acc && workspace, "gcs_model_train_step: null pointer");
   GCS_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 255u) == 0, "gcs_model_train_step: workspace must be 256-byte aligned");
   const gcs_model_config& c = *cfg;
@@ -839,9 +849,6 @@ extern "C" int gcs_model_train_step_dp(const gcs_model_config* cfg, const float*
                                        gcs_comm* comm, gcs_stream comm_stream, int32_t sync_batchnorm) {
   GCS_TRY(check_config(cfg));
   GCS_TRY(check_batch(*cfg, batch, true, true));
-  GCS_CHECK_ARG(cfg->final_activation == 1 || cfg->final_activation == 2,
-                "gcs_model_train_step_dp: the loss is categorical cross-entropy on a softmax output or binary "
-                "cross-entropy on a sigmoid output");
   GCS_CHECK_ARG(params && state && grads && loss_acc && workspace && comm, "gcs_model_train_step_dp: null pointer");
   GCS_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 255u) == 0, "gcs_model_train_step_dp: workspace must be 256-byte aligned");
   GCS_CHECK_ARG(comm_stream != stream, "gcs_model_train_step_dp: the collective needs its own stream");

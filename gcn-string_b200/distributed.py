@@ -147,11 +147,12 @@ class DataParallelTrainer:
     3H+1 in the backward): the step then equals ONE single-device step on the union of the shards - same loss
     gradient, same BatchNorm state on every rank - instead of a count-weighted average of per-shard steps."""
 
-    def __init__(self, model, optimizer, group=None, sync_bn: bool = False, native_comm: bool = False):
+    def __init__(self, model, optimizer, group=None, sync_bn: bool = False, native_comm: bool = False, loss=None):
         """``native_comm=True``: the gradient all-reduce goes through the library's own NCCL communicator and is
         started bucket by bucket during the backward (gcs_model_train_step_dp) instead of one torch.distributed
-        all-reduce after it."""
-        self.model, self.optimizer, self.group = model, optimizer, group
+        all-reduce after it.  ``loss``: what ``GeneralGNN.train_step_grads`` runs (None = the head's own loss;
+        ``MeanSquaredError()``, ``MeanAbsoluteError()`` or ``Huber(delta)`` for a linear head)."""
+        self.model, self.optimizer, self.group, self.loss = model, optimizer, group, loss
         self.sync_bn = bool(sync_bn)
         self._synced = False
         self.comm = NativeComm(group) if native_comm and world()[1] > 1 else None
@@ -183,9 +184,10 @@ class DataParallelTrainer:
             global_batch = getattr(a, key, None) or target.shape[0] * ws
         if self.comm is not None:                 # the library's own communicator: collectives (and synchronised BatchNorm) per call
             loss_acc, probs = self.model.train_step_grads(inputs, target, grad_scale=1.0 / float(global_batch), comm=self.comm,
-                                                          sync_bn=self.sync_bn)
+                                                          sync_bn=self.sync_bn, loss=self.loss)
         else:
-            step = lambda: self.model.train_step_grads(inputs, target, grad_scale=1.0 / float(global_batch))   # noqa: E731
+            step = lambda: self.model.train_step_grads(inputs, target, grad_scale=1.0 / float(global_batch),   # noqa: E731
+                                                       loss=self.loss)
             loss_acc, probs = self._hooked(step)
         if self.comm is None:
             allreduce_gradients(self.model.grads, self.group)

@@ -15,18 +15,22 @@ from __future__ import annotations
 import numpy as np
 
 from . import _lib
-from .losses import BinaryCrossentropy, CategoricalCrossentropy, binary_accuracy, categorical_accuracy
+from .losses import (BinaryCrossentropy, CategoricalCrossentropy, Huber, MeanAbsoluteError, MeanSquaredError,
+                     binary_accuracy, categorical_accuracy, mean_absolute_error)
 
 
-def evaluate(model, loader, loss_fn=None):
+def evaluate(model, loader, loss_fn=None, metric=None):
     """One pass over ``loader`` -> (np.array([loss, acc]) weighted by batch size, [pred per batch]).
     Mirrors gcn.py:342-362; the only host transfers are the two scalars per batch.  The loss and accuracy default to
     BinaryCrossentropy / binary_accuracy for a model built with activation='sigmoid', to CategoricalCrossentropy /
-    categorical_accuracy otherwise."""
+    categorical_accuracy otherwise.  ``metric(y_true, y_pred)`` -> per-row values replaces the accuracy; with a
+    regression ``loss_fn`` (MeanSquaredError, MeanAbsoluteError, Huber) it defaults to mean_absolute_error."""
     torch = _lib.require_cuda()
     sigmoid = getattr(model, "config", {}).get("activation") == "sigmoid"
+    if metric is None and isinstance(loss_fn, (MeanSquaredError, MeanAbsoluteError, Huber)):
+        metric = mean_absolute_error
     loss_fn = loss_fn or (BinaryCrossentropy() if sigmoid else CategoricalCrossentropy())
-    metric = binary_accuracy if sigmoid else categorical_accuracy
+    metric = metric or (binary_accuracy if sigmoid else categorical_accuracy)
     stats, preds = [], []
     step = 0
     while step < loader.steps_per_epoch:

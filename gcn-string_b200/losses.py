@@ -7,7 +7,11 @@ launch (csrc/loss.cu).  Reduction is the Keras default: mean over the batch.
 
 ``BinaryCrossentropy`` and ``binary_accuracy`` are the Keras pair for a sigmoid head (binary and multi-label targets):
 on the logits of a ``GeneralGNN(activation='sigmoid')`` output, or with ``from_logits=True``, they run the fused kernel
-of csrc/loss_bce.cu."""
+of csrc/loss_bce.cu.
+
+``MeanSquaredError``, ``MeanAbsoluteError`` and ``Huber`` are the Keras regression losses for the linear head of a
+default ``GeneralGNN(C)`` (activation=None); with ``mean_squared_error`` / ``mean_absolute_error`` they run the fused
+kernel of csrc/loss_reg.cu."""
 from __future__ import annotations
 
 from . import _lib, ops
@@ -86,3 +90,86 @@ def binary_accuracy(y_true, y_pred, threshold=0.5):
     y = _lib.as_tensor(y_true).to(device="cuda", dtype=torch.float32)
     pred = (_lib.as_tensor(y_pred) > threshold).to(torch.float32)
     return (y == pred).to(torch.float32).mean(dim=-1)
+
+
+class _RegressionLoss:
+    """Shared body of the Keras regression losses: the mean over the last axis, then over the rows, of the element loss
+    of e = y_pred - y_true, on the predictions of a linear head (the logits the model attached to its output) or on
+    ``y_pred`` itself.  Under an active ``GradientTape`` it records dLoss/dlogits for the model's backward."""
+    kind = ""         # ops.regression_loss name
+    code = 0          # gcs_model_config.loss
+
+    def __init__(self, reduction, name, delta=1.0):
+        if reduction not in ("sum_over_batch_size", "auto"):
+            raise NotImplementedError("only the default mean-over-batch reduction is built")
+        self.name = name
+        self.delta = float(delta)
+
+    def __call__(self, y_true, y_pred):
+        torch = _lib.require_cuda()
+        y = _lib.as_tensor(y_true).to(device="cuda", dtype=torch.float32)
+        linear = getattr(y_pred, "_gcs_activation", None) in (None, "linear")
+        pred = y_pred._gcs_logits if linear and hasattr(y_pred, "_gcs_logits") else y_pred
+        tape = getattr(y_pred, "_gcs_tape", None)
+        if tape is not None and not linear:
+            raise NotImplementedError(f"{type(self).__name__} is built for a linear head (activation=None); the model's "
+                                      f"output has activation={y_pred._gcs_activation!r}")
+        loss_acc, dlogits = ops.regression_loss(pred, y, self.kind, self.delta, want_grad=tape is not None)
+        if tape is not None:
+            tape.loss_record = dict(dlogits=dlogits, loss_acc=loss_acc)
+        return loss_acc[0]
+
+
+class MeanSquaredError(_RegressionLoss):
+    """tf.keras.losses.MeanSquaredError: mean of (y_pred - y_true)^2."""
+    kind, code = "mse", 1
+
+    def __init__(self, reduction="sum_over_batch_size", name="mean_squared_error"):
+        super().__init__(reduction, name)
+
+
+class MeanAbsoluteError(_RegressionLoss):
+    """tf.keras.losses.MeanAbsoluteError: mean of |y_pred - y_true|; its gradient at an exact tie is 0, as in TF."""
+    kind, code = "mae", 2
+
+    def __init__(self, reduction="sum_over_batch_size", name="mean_absolute_error"):
+        super().__init__(reduction, name)
+
+
+class Huber(_RegressionLoss):
+    """tf.keras.losses.Huber: 0.5 e^2 where |e| <= delta, delta |e| - 0.5 delta^2 elsewhere."""
+    kind, code = "huber", 3
+
+    def __init__(self, delta=1.0, reduction="sum_over_batch_size", name="huber_loss"):
+        delta = float(delta)
+        if not (0.0 < delta < float("inf")):
+            raise ValueError(f"Huber: delta must be finite and > 0, got {delta}")
+        super().__init__(reduction, name, delta)
+
+
+def mean_squared_error(y_true, y_pred):
+    """Per-row mean over the columns of (y_pred - y_true)^2, like tf.keras.metrics.mean_squared_error."""
+    torch = _lib.require_cuda()
+    y = _lib.as_tensor(y_true).to(device="cuda", dtype=torch.float32)
+    return (_lib.as_tensor(y_pred) - y).square().mean(dim=-1)
+
+
+def mean_absolute_error(y_true, y_pred):
+    """Per-row mean over the columns of |y_pred - y_true|, like tf.keras.metrics.mean_absolute_error."""
+    torch = _lib.require_cuda()
+    y = _lib.as_tensor(y_true).to(device="cuda", dtype=torch.float32)
+    return (_lib.as_tensor(y_pred) - y).abs().mean(dim=-1)
+
+
+def fused_loss_fields(loss, activation):
+    """(gcs_model_config.loss, .huber_delta) for the fused train step of a head with ``activation``: ``None`` gives
+    (0, 1.0), the head's own loss; a regression loss needs a linear head."""
+    if loss is None:
+        return 0, 1.0
+    if not isinstance(loss, _RegressionLoss):
+        raise NotImplementedError(f"the fused train step takes loss=None (the head's own loss) or MeanSquaredError, "
+                                  f"MeanAbsoluteError or Huber, not {type(loss).__name__}")
+    if activation not in (None, "linear"):
+        raise NotImplementedError(f"{type(loss).__name__} is built for a linear head (activation=None), not "
+                                  f"activation={activation!r}")
+    return loss.code, loss.delta

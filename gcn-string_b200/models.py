@@ -18,6 +18,7 @@ import numpy as np
 from . import _lib, ops
 from ._lib import check, ptr, stream_ptr
 from .data import SparseAdjacency
+from .losses import fused_loss_fields
 from .params import GNNConfig, block_specs, init_params, n_state, n_trainable, named_slices
 
 _tape_stack = threading.local()
@@ -279,17 +280,26 @@ class GeneralGNN:
         check(lib.gcs_model_backward(self._c, ptr(self.params), ctx["batch"], ptr(dlogits), ptr(self.grads),
                                      ptr(ctx["ws"]), ctx["ws"].numel(), stream_ptr()), "gcs_model_backward")
 
-    def train_step_grads(self, inputs, target, grad_scale: Optional[float] = None, comm=None, sync_bn: bool = False):
+    def train_step_grads(self, inputs, target, grad_scale: Optional[float] = None, comm=None, sync_bn: bool = False,
+                         loss=None):
         """Fused training-mode forward + loss + backward (one C call): categorical cross-entropy with
-        activation='softmax', binary cross-entropy (mean over the C columns, then the rows) with activation='sigmoid'.
+        activation='softmax', binary cross-entropy (mean over the C columns, then the rows) with activation='sigmoid',
+        and with the linear head (activation=None) the regression loss ``loss`` - ``MeanSquaredError()`` (the default),
+        ``MeanAbsoluteError()`` or ``Huber(delta)``.
         Leaves the gradients in ``self.grads``; returns (loss_acc [2] device tensor = {loss,
-        accuracy}, probs [B, C]).  ``grad_scale`` defaults to 1/B (mean loss, gcn.py:335).
+        accuracy} - {loss, mean absolute error} for a regression loss -, probs [B, C] - the predictions of a linear
+        head).  ``grad_scale`` defaults to 1/B (mean loss, gcn.py:335).
         ``comm`` (distributed.NativeComm): the data-parallel form - the gradients are SUM all-reduced over the
         communicator, bucket by bucket on its own stream while the backward is still running
         (gcs_model_train_step_dp); the current stream waits for the reductions."""
         torch = _lib.require_cuda()
         lib = _lib.load()
+        code, delta = fused_loss_fields(loss, self.config["activation"])
         batch, keep = self._prepare(inputs, need_transpose=True)
+        c = self._c
+        if code:                                         # for this call only: the layout never depends on the loss
+            c = _lib.ModelConfig.from_buffer_copy(self._c)
+            c.loss, c.huber_delta = code, delta
         y = _lib.as_tensor(target)
         y = y.to(device="cuda", dtype=torch.float32).contiguous()
         rows = self._rows_out(batch)
@@ -301,11 +311,11 @@ class GeneralGNN:
         loss_acc = torch.empty(2, dtype=torch.float32, device="cuda")
         gs = 1.0 / rows if grad_scale is None else float(grad_scale)
         if comm is not None:
-            check(lib.gcs_model_train_step_dp(self._c, ptr(self.params), ptr(self.state), batch, gs, ptr(self.grads),
+            check(lib.gcs_model_train_step_dp(c, ptr(self.params), ptr(self.state), batch, gs, ptr(self.grads),
                                               ptr(probs), ptr(loss_acc), ptr(ws), ws.numel(), stream_ptr(), comm.handle,
                                               comm.stream.cuda_stream, int(bool(sync_bn))), "gcs_model_train_step_dp")
         else:
-            check(lib.gcs_model_train_step(self._c, ptr(self.params), ptr(self.state), batch, gs, ptr(self.grads),
+            check(lib.gcs_model_train_step(c, ptr(self.params), ptr(self.state), batch, gs, ptr(self.grads),
                                            ptr(probs), ptr(loss_acc), ptr(ws), ws.numel(), stream_ptr()),
                   "gcs_model_train_step")
         self._keep = (keep, y)

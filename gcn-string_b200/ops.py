@@ -586,6 +586,34 @@ def sigmoid_bce(logits, y=None, grad_scale: Optional[float] = None, want_grad=Fa
     return probs, loss_acc, dlogits
 
 
+REGRESSION_KIND = {"mse": 1, "mae": 2, "huber": 3}
+
+
+def regression_loss(pred, y, loss: str = "mse", delta: float = 1.0, want_grad=False, grad_scale: Optional[float] = None):
+    """Returns (loss_acc[2], dlogits or None) of gcs_regression_loss on the predictions of a linear head: loss_acc =
+    {``loss`` ('mse', 'mae' or 'huber' with ``delta``; mean over the columns, then the rows), mean absolute error},
+    dlogits = dLoss/dpred * grad_scale / C (``grad_scale`` defaults to 1 / rows)."""
+    torch = _t()
+    lib = _lib.load()
+    if loss not in REGRESSION_KIND:
+        raise ValueError(f"loss must be one of {sorted(REGRESSION_KIND)}, got {loss!r}")
+    pred, _ = _mat(pred, "pred")
+    pred = pred.contiguous()
+    b, c = pred.shape
+    y, _ = _mat(y, "y")
+    if tuple(y.shape) != (b, c):
+        raise ValueError(f"y must be [{b}, {c}], got {tuple(y.shape)}")
+    y = y.contiguous()
+    loss_acc = torch.empty(2, dtype=torch.float32, device="cuda")
+    dlogits = torch.empty_like(pred) if want_grad else None
+    gs = (1.0 / b if b else 0.0) if grad_scale is None else grad_scale
+    nbytes = int(lib.gcs_regression_loss_workspace_bytes(b, c))
+    ws = torch.empty(nbytes, dtype=torch.uint8, device="cuda") if nbytes > 0 else None
+    check(lib.gcs_regression_loss(REGRESSION_KIND[loss], float(delta), ptr(pred), ptr(y), b, c, None, ptr(loss_acc),
+                                  ptr(dlogits), gs, ptr(ws), nbytes, stream_ptr()), "gcs_regression_loss")
+    return loss_acc, dlogits
+
+
 def sgd_step(w, g, lr: float, grad_scale: float = 1.0):
     lib = _lib.load()
     check(lib.gcs_sgd_step(ptr(w), ptr(g), w.numel(), lr, grad_scale, stream_ptr()), "gcs_sgd_step")

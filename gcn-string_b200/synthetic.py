@@ -14,7 +14,9 @@ What the reference's offline generator emits per protein pair, restated as a sam
     mostly probabilities -> U[0,1); width F is a parameter (BASELINE.json uses 32);
   * labels one-hot [0,1] positive / [1,0] negative, balanced (src/scripts/gcn.py:259,262);
     ``node_level=True`` instead labels every residue (a per-residue task such as interface residues): one-hot of the
-    argmax of a fixed random projection of the summed neighbour features, which a GeneralGNN can learn.
+    argmax of a fixed random projection of the summed neighbour features, which a GeneralGNN can learn;
+    ``task='regression'`` gives continuous targets instead: tanh of that projection per residue, or its mean over
+    each graph (a continuous score per protein pair).
 
 Everything is NumPy with ``default_rng(seed + graph_id)`` so any graph can be
 regenerated alone.  The output is the packed layout the device batching kernel consumes
@@ -119,30 +121,61 @@ def make_graph(seed: int, graph_id: int, n_mean: int = 500, deg: int = 12, n_fea
     return rowptr, c, x
 
 
-def node_labels(packed: PackedGraphs, n_classes: int, seed: int) -> np.ndarray:
-    """One-hot [sum N, C] node labels of a packed dataset: row n is one-hot at argmax_c of
-    (sum over the stored neighbours j of n of (x_j - 1/2)) . V[:, c], with V [F, C] standard normal from
-    ``default_rng(seed)`` - a function of the graph that one aggregation step can express."""
+def neighbour_scores(packed: PackedGraphs, n_out: int, seed: int) -> np.ndarray:
+    """float64 [sum N, n_out] score of every node of a packed dataset: (sum over the stored neighbours j of n of
+    (x_j - 1/2)) . V, with V [F, n_out] standard normal from ``default_rng(seed)`` - a function of the graph that one
+    aggregation step can express."""
     import scipy.sparse as sp
     n = int(packed.node_off[-1])
     rows = np.repeat(np.arange(n, dtype=np.int64), np.diff(packed.rowptr))
     cols = packed.col.astype(np.int64) + np.repeat(packed.node_off[:-1], packed.n_nodes)[rows]
     a = sp.csr_matrix((np.ones(rows.shape[0]), (rows, cols)), shape=(n, n))
-    v = np.random.default_rng(seed).standard_normal((packed.x.shape[1], n_classes))
-    score = (a @ (np.asarray(packed.x, dtype=np.float64) - 0.5)) @ v
+    v = np.random.default_rng(seed).standard_normal((packed.x.shape[1], n_out))
+    return (a @ (np.asarray(packed.x, dtype=np.float64) - 0.5)) @ v
+
+
+def node_labels(packed: PackedGraphs, n_classes: int, seed: int) -> np.ndarray:
+    """One-hot [sum N, C] node labels of a packed dataset: row n is one-hot at argmax_c of its ``neighbour_scores``."""
+    score = neighbour_scores(packed, n_classes, seed)
+    n = score.shape[0]
     y = np.zeros((n, n_classes), dtype=np.float32)
     y[np.arange(n), np.argmax(score, axis=1)] = 1.0
     return y
+
+
+def regression_targets(packed: PackedGraphs, n_out: int, seed: int, node_level: bool) -> np.ndarray:
+    """Continuous float32 targets in (-1, 1): tanh of the ``neighbour_scores``, per node [sum N, n_out] with
+    ``node_level``, else their mean over each graph's nodes [G, n_out] (what a sum or average pool can express)."""
+    t = np.tanh(neighbour_scores(packed, n_out, seed))
+    if node_level:
+        return t.astype(np.float32)
+    counts = packed.n_nodes
+    seg = np.repeat(np.arange(packed.n_graphs, dtype=np.int64), counts)
+    sums = np.stack([np.bincount(seg, weights=t[:, k], minlength=packed.n_graphs) for k in range(n_out)], axis=1)
+    return (sums / np.maximum(counts, 1)[:, None]).astype(np.float32)
 
 
 def _with_node_labels(p: PackedGraphs, n_classes: int, seed: int) -> PackedGraphs:
     return PackedGraphs(p.node_off, p.rowptr, p.col, p.x, node_labels(p, n_classes, seed + 0x5EED), node_level=True)
 
 
+def _with_regression_targets(p: PackedGraphs, n_out: int, seed: int, node_level: bool) -> PackedGraphs:
+    return PackedGraphs(p.node_off, p.rowptr, p.col, p.x, regression_targets(p, n_out, seed + 0x5EED, node_level),
+                        node_level=node_level)
+
+
+TASKS = ("classification", "regression")
+
+
 def make_dataset(n_graphs: int, seed: int = 0, n_mean: int = 500, deg: int = 12,
-                 n_feat: int = 32, n_classes: int = 2, node_level: bool = False) -> PackedGraphs:
+                 n_feat: int = 32, n_classes: int = 2, node_level: bool = False,
+                 task: str = "classification") -> PackedGraphs:
     """G(seed, n_mean, deg, F) of SURVEY.md §8d, packed.  ``node_level=True``: per-node labels (``node_labels``, one
-    projection for the whole dataset) instead of the balanced graph labels; the graphs themselves are the same."""
+    projection for the whole dataset) instead of the balanced graph labels; the graphs themselves are the same.
+    ``task='regression'``: ``n_classes`` continuous targets per graph or per node (``regression_targets``) instead of
+    one-hot labels."""
+    if task not in TASKS:
+        raise ValueError(f"task must be one of {TASKS}, got {task!r}")
     rps: List[np.ndarray] = []
     cols: List[np.ndarray] = []
     xs: List[np.ndarray] = []
@@ -158,6 +191,9 @@ def make_dataset(n_graphs: int, seed: int = 0, n_mean: int = 500, deg: int = 12,
     rowptr = np.concatenate(rps + [np.array([e_off], dtype=np.int64)]) if n_graphs else np.zeros(1, np.int64)
     col = np.concatenate(cols) if n_graphs else np.zeros(0, np.int32)
     x = np.concatenate(xs) if n_graphs else np.zeros((0, n_feat), np.float32)
+    if task == "regression":
+        return _with_regression_targets(PackedGraphs(node_off, rowptr, col, x, np.zeros((0, n_classes), np.float32)),
+                                        n_classes, seed, node_level)
     if node_level:
         return _with_node_labels(PackedGraphs(node_off, rowptr, col, x, np.zeros((0, n_classes), np.float32)), n_classes,
                                  seed)

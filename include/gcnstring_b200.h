@@ -322,6 +322,27 @@ int gcs_sigmoid_bce(const float* logits, const float* y, int64_t rows, int32_t C
                     float* dlogits, float grad_scale, void* workspace, int64_t workspace_bytes, gcs_stream stream);
 
 /* ---------------------------------------------------------------------------------
+ * K5c  Regression losses of a linear head: GeneralGNN(C) (activation=None) trained with tf.keras.losses
+ * MeanSquaredError(), MeanAbsoluteError() or Huber(delta), and tf.keras.metrics.mean_absolute_error.  kind: 1 = MSE,
+ * 2 = MAE, 3 = Huber (huber_delta finite and > 0; ignored otherwise).  Per element, e = pred - y in float32:
+ *   MSE l = e^2, dl = 2e;  MAE l = |e|, dl = sign(e) (sign(0) = 0);
+ *   Huber l = 0.5 e^2 if |e| <= delta, else delta |e| - 0.5 delta^2;  dl = e, or delta sign(e).
+ *   loss_acc[2] = {mean over rows of the mean over the C columns of l, mean of |e|} (NULL-able);
+ *   probs[rows,C] (NULL-able) = pred (the predictions of a linear head are its logits);
+ *   dlogits (NULL-able) = dl * grad_scale / C  (grad_scale = 1/rows for the mean loss; 1/global_rows under data
+ *   parallelism).
+ * y may be NULL when only probs is asked for (a copy, nothing else is computed).  Any C, rows = 0 gives
+ * loss_acc = {0, 0}.  A grid-wide elementwise kernel leaves per-block fp64 sums in the workspace and a second launch adds
+ * them in a fixed order (bit-identical run to run; the grid depends on rows * C alone).  workspace:
+ * gcs_regression_loss_workspace_bytes(rows, C) bytes, 8-byte aligned (only read when loss_acc != NULL; 0 bytes when
+ * rows * C <= 1024).
+ * --------------------------------------------------------------------------------- */
+int64_t gcs_regression_loss_workspace_bytes(int64_t rows, int32_t C);
+int gcs_regression_loss(int32_t kind, float huber_delta, const float* pred, const float* y, int64_t rows, int32_t C,
+                        float* probs, float* loss_acc, float* dlogits, float grad_scale, void* workspace,
+                        int64_t workspace_bytes, gcs_stream stream);
+
+/* ---------------------------------------------------------------------------------
  * K11  Residue contact maps of a batch of chains (SURVEY.md 8 f4).  Replaces
  * GraphMaker.calculate_residue_dist / calculate_dist_matrix / generate_proximity_matrix
  * (src/utilities/gcn_utills.py:161-238): d = sqrt(sum((ca_i - ca_j)^2)) in float32 with NumPy's operation order
@@ -401,6 +422,10 @@ typedef struct gcs_model_config {
   float bn_momentum;        /* 0.99 */
   float bn_epsilon;         /* 1e-3 */
   int32_t aggregate;        /* GeneralConv aggregate: 0 = 'sum' (the reference's), 1 = 'mean', 2 = 'max' */
+  int32_t loss;             /* loss of the fused train steps: 0 = the head's own (categorical cross-entropy for softmax,
+                               binary cross-entropy for sigmoid, MSE for linear); 1 = MSE, 2 = MAE, 3 = Huber, with
+                               final_activation = 0 only.  Does not change the parameter or workspace layout. */
+  float huber_delta;        /* Huber's delta when loss = 3: finite and > 0 */
 } gcs_model_config;
 
 typedef struct gcs_batch {
@@ -445,7 +470,9 @@ int gcs_model_forward(const gcs_model_config* cfg, const float* params, float* s
  * gcs_softmax_xent_ws; gcs_model_workspace_bytes includes its workspace.  With final_activation = 2 (sigmoid) the loss
  * is binary cross-entropy through gcs_sigmoid_bce instead: probs = sigmoid(logits), loss_acc = {mean binary
  * cross-entropy, binary accuracy}, and grad_scale keeps its meaning (the 1/C of the per-row mean is applied inside).
- * final_activation = 0 (linear) has no loss and is refused. */
+ * With final_activation = 0 (linear) the loss is the regression loss cfg->loss selects (0 or 1 = MSE, 2 = MAE, 3 =
+ * Huber with cfg->huber_delta) through gcs_regression_loss: probs = the predictions (the logits), loss_acc = {mean
+ * loss, mean absolute error}, and grad_scale keeps its meaning the same way. */
 int gcs_model_train_step(const gcs_model_config* cfg, const float* params, float* state,
                          const gcs_batch* batch, float grad_scale, float* grads, float* probs,
                          float* loss_acc, void* workspace, int64_t workspace_bytes,
