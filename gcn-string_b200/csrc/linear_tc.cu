@@ -18,6 +18,8 @@
 //   linear_tc_pair_kernel   forward and input gradient: persistent CTA pairs (cta_group::2), A operand
 //                           split by converter warps straight into TENSOR MEMORY (TS-mode MMA), weight
 //                           tiles split across the pair, TMA-store / reduce-add epilogue
+//   linear_f16_pass256_kernel  its fp16 form for output widths that are multiples of 256: 256 columns per pass, the
+//                           split A operand in shared memory (SS-mode MMA), one fetch and split of A per pass
 //   wgrad_tc_kernel         weight gradient: reduction over the rows, A^T gathered into tensor memory,
 //                           dH split in shared memory as an MN-major operand
 #include <cuda.h>
@@ -580,6 +582,285 @@ __global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kF16 ? kHThreads : k
     }
     if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");           // every box written before the CTA exits
     if (kF16) amax_commit(out_max, amax_out);
+  }
+  tc_fence_before();
+  cluster_sync_all();              // the peer's tensor core may still read this CTA's shared memory until its commits land
+  if (warp == 1) {
+    tc_fence_after();
+    asm volatile("tcgen05.dealloc.cta_group::2.sync.aligned.b32 %0, %1;" ::"r"(tmem_base), "n"(kTmemCols));
+  }
+}
+
+// ---------------------------------------------------------------------------------------------
+// fp16 forward / dX kernel for widths that are multiples of 256: one CTA pair computes a 256 x 256 tile per pass.
+//
+// linear_tc_pair_kernel<true> computes 256 x 128 tiles, so a 256-wide output fetches every raw fp32 A row from L2 twice
+// and splits it twice: per CTA and K block of 64, 2 x (32 KB raw A + 16 KB weight halves) = 96 KB of L2 -> SM ingest,
+// the bound of that kernel.  Here both 128-column halves come out of one pass over A: 32 KB raw A + 32 KB weight halves
+// = 64 KB per K block, for the same tensor work.  Tensor memory then holds nothing but the two accumulators, so the
+// split A operand lives in shared memory (SS-form MMAs):
+//   TMEM (each CTA, its 128 rows):  MAIN = A_hi.B_hi in columns [0, 256), CORR = A_hi.B_lo + A_lo.B_hi in [256, 512)
+//   (both correction products carry the same 2^11, so one accumulator takes both; the epilogue adds CORR * 2^-11).
+//   Per CTA and stage: [A raw box k0..k0+31 | A raw box k0+32..k0+63 | B_hi 128 x 64 | B_lo 128 x 64]  = 64 KB
+//   (rank r holds output columns [128 r, 128 r + 128) of the pass: cta_group::2 takes N = 256 as two halves).
+// The converters split A IN PLACE: A_hi over raw box 0 and A_lo over raw box 1, each a K-major SWIZZLE_128B fp16
+// operand of 128 rows x 128 B (the layout TMA gives the weight tiles).  Row r of both the raw boxes and the split
+// operands is the 128 B at r * 128, and only the four converter warps of r's lane quarter touch it: they meet at a
+// named barrier between reading their raw chunks and writing the split ones.  The stage is released by the MMA commit.
+// Three 64 KB stages + 16 x 2 KB of epilogue staging fit the 227 KB; there is no room for a second accumulator set,
+// so (as in linear_tc_pair_kernel) the converters write a tile out before they feed the next one.
+constexpr int kSStages = 3;
+constexpr uint32_t S_B_BYTES = 128 * BKH * 2;                         // 16 KB: 128 weight rows of one half
+constexpr uint32_t S_STAGE_BYTES = 2 * A_RAW_BYTES + 2 * S_B_BYTES;   // 64 KB
+constexpr uint32_t S_OUT_BYTES = 32 * 16 * 4;                         // per converter warp: one 32 x 16 output box
+constexpr uint32_t kSSmemBytes = kSStages * S_STAGE_BYTES + kHConvWarps * S_OUT_BYTES + 1024 + 256;
+static_assert(kSSmemBytes <= 232448, "fp16 256-column kernel exceeds the 227 KB of shared memory per CTA");
+constexpr uint32_t S_MAIN = 0, S_CORR = 256;
+
+__device__ __forceinline__ void mma_f16_ss_pair(uint32_t d_tmem, uint64_t a_desc, uint64_t b_desc, uint32_t idesc, uint32_t accumulate) {
+  asm volatile(
+      "{\n\t.reg .pred p;\n\t"
+      "setp.ne.b32 p, %4, 0;\n\t"
+      "tcgen05.mma.cta_group::2.kind::f16 [%0], %1, %2, %3, p;\n\t}"
+      ::"r"(d_tmem), "l"(a_desc), "l"(b_desc), "r"(idesc), "r"(accumulate) : "memory");
+}
+
+__global__ void __cluster_dims__(2, 1, 1) __launch_bounds__(kHThreads, 1) linear_f16_pass256_kernel(
+    const __grid_constant__ CUtensorMap map_a, const __grid_constant__ CUtensorMap map_b_hi,
+    const __grid_constant__ CUtensorMap map_b_lo, const __grid_constant__ CUtensorMap map_c,
+    const float* __restrict__ bias, int64_t M, int K, int N, int num_tiles, int accumulate,
+    const float* __restrict__ rowbias, int64_t ld_rowbias, const int64_t* __restrict__ seg,
+    const float* __restrict__ a_amax, const float* __restrict__ b_scale_inv, const float* __restrict__ alpha,
+    float* __restrict__ amax_out, float* __restrict__ stats_part) {
+  extern __shared__ uint8_t smem_dyn[];
+  const uint32_t base = (smem_u32(smem_dyn) + 1023u) & ~1023u;
+  const uint32_t out_stage = base + kSStages * S_STAGE_BYTES;     // 1024 B aligned
+  const uint32_t bars = out_stage + kHConvWarps * S_OUT_BYTES;
+  // barriers (8 B each): full[3] | smem_empty[3] | a_ready[3] | acc_full | tmem ptr
+  auto full = [&](int s) { return bars + 8u * s; };
+  auto smem_empty = [&](int s) { return bars + 24u + 8u * s; };
+  auto a_ready = [&](int s) { return bars + 48u + 8u * s; };
+  const uint32_t acc_full = bars + 72u;
+  const uint32_t tmem_slot = bars + 80u;
+
+  const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+  const int rank = blockIdx.x;
+  const int num_kb = K / BKH;
+  const int n_pass = N / 256;
+  // persistent walk as in linear_tc_pair_kernel: tile -> (row pair, 256-column pass), the passes of a row pair adjacent
+
+  if (warp == 0 && lane == 0) {
+    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_a));
+    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_b_hi));
+    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_b_lo));
+    asm volatile("prefetch.tensormap [%0];" ::"l"(&map_c));
+    for (int s = 0; s < kSStages; ++s) {
+      mbar_init(full(s), 1);
+      mbar_init(smem_empty(s), 1);                 // the multicast tcgen05.commit: the split A is read by the MMAs alone
+      mbar_init(a_ready(s), 2 * kHConvWarps);      // converter warps of both CTAs (only the leader's copy is used)
+    }
+    mbar_init(acc_full, 1);
+    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
+  }
+  if (warp == 1) {
+    asm volatile("tcgen05.alloc.cta_group::2.sync.aligned.shared::cta.b32 [%0], %1;" ::"r"(tmem_slot), "n"(kTmemCols));
+    asm volatile("tcgen05.relinquish_alloc_permit.cta_group::2.sync.aligned;");
+  }
+  tc_fence_before();
+  cluster_sync_all();
+  tc_fence_after();
+  uint32_t tmem_base;
+  asm volatile("ld.shared.u32 %0, [%1];" : "=r"(tmem_base) : "r"(tmem_slot));
+
+  if (warp == 0) {
+    // ------------------------------------------------------------ TMA producer
+    if (lane == 0) {
+      uint32_t it = 0;
+      for (int tile = blockIdx.y; tile < num_tiles; tile += gridDim.y) {
+        const int n0 = (tile % n_pass) * 256;
+        const int m0 = ((tile / n_pass) * 2 + rank) * BM;
+        for (int kb = 0; kb < num_kb; ++kb, ++it) {
+          const int s = it % kSStages;
+          mbar_wait(smem_empty(s), ((it / kSStages) & 1) ^ 1);
+          const uint32_t st = base + s * S_STAGE_BYTES;
+          mbar_arrive_expect_tx(full(s), S_STAGE_BYTES);
+          tma_load_2d(st, &map_a, kb * BKH, m0, full(s));
+          tma_load_2d(st + A_RAW_BYTES, &map_a, kb * BKH + 32, m0, full(s));
+          tma_load_2d(st + 2 * A_RAW_BYTES, &map_b_hi, kb * BKH, n0 + 128 * rank, full(s));
+          tma_load_2d(st + 2 * A_RAW_BYTES + S_B_BYTES, &map_b_lo, kb * BKH, n0 + 128 * rank, full(s));
+        }
+      }
+    }
+  } else if (warp == 1) {
+    // ------------------------------------------------------------ MMA issuer (leader CTA only; converged warp, one elected lane)
+    if (rank == 0) {
+      const uint32_t leader = elect_one();
+      uint32_t it = 0;
+      for (int tile = blockIdx.y; tile < num_tiles; tile += gridDim.y) {
+        for (int kb = 0; kb < num_kb; ++kb, ++it) {
+          const int s = it % kSStages;
+          const uint32_t ph = (it / kSStages) & 1;
+          mbar_wait(full(s), ph);
+          // both CTAs: stage landed and split; for kb == 0 also: the previous tile's accumulators have been read
+          mbar_wait(a_ready(s), ph);
+          tc_fence_after();
+          if (leader) {
+            const uint32_t st = base + s * S_STAGE_BYTES;
+            const uint64_t d_ahi = make_kmajor_sw128_desc(st);
+            const uint64_t d_alo = make_kmajor_sw128_desc(st + A_RAW_BYTES);
+            const uint64_t d_bhi = make_kmajor_sw128_desc(st + 2 * A_RAW_BYTES);
+            const uint64_t d_blo = make_kmajor_sw128_desc(st + 2 * A_RAW_BYTES + S_B_BYTES);
+#pragma unroll
+            for (int k = 0; k < 4; ++k) {               // K = 16 per instruction: 32 B of each 128 B operand row
+              const uint64_t koff = static_cast<uint64_t>((k * 32) >> 4);
+              const uint32_t acc = (kb > 0 || k > 0) ? 1u : 0u;
+              mma_f16_ss_pair(tmem_base + S_MAIN, d_ahi + koff, d_bhi + koff, kPairDesc256H, acc);
+              mma_f16_ss_pair(tmem_base + S_CORR, d_ahi + koff, d_blo + koff, kPairDesc256H, acc);
+              mma_f16_ss_pair(tmem_base + S_CORR, d_alo + koff, d_bhi + koff, kPairDesc256H, 1u);
+            }
+            tc_commit_pair(smem_empty(s));
+            if (kb == num_kb - 1) tc_commit_pair(acc_full);
+          }
+          __syncwarp();
+        }
+      }
+    }
+  } else {
+    // ------------------------------------------------------------ converters, then epilogue, per tile
+    const int quarter = warp & 3;
+    const int half = (warp - 2) >> 2;                  // 0..3: which 16 of the 64 K elements; which 64 output columns
+    const int r = quarter * 32 + lane;
+    const uint32_t lane_addr = static_cast<uint32_t>(quarter * 32) << 16;
+    uint32_t it = 0, tile_iter = 0;
+    const float a_scale = f16_scale(__ldg(a_amax));
+    const float out_scale = (1.f / a_scale) * __ldg(b_scale_inv);     // powers of two: exact
+    float out_max = 0.f;
+    for (int tile = blockIdx.y; tile < num_tiles; tile += gridDim.y, ++tile_iter) {
+      const int n0 = (tile % n_pass) * 256;
+      const int64_t m0 = (static_cast<int64_t>(tile / n_pass) * 2 + rank) * BM;
+      for (int kb = 0; kb < num_kb; ++kb, ++it) {
+        const int s = it % kSStages;
+        mbar_wait(full(s), (it / kSStages) & 1);
+        const uint32_t st = base + s * S_STAGE_BYTES;
+        uint32_t hi[8], lo[8];
+        // the row's swizzled addresses are recomputed per K block (a few integer instructions): hoisted out of the
+        // tile loops, ptxas kept them in local memory
+        uint32_t rr7;
+        asm volatile("and.b32 %0, %1, 7;" : "=r"(rr7) : "r"(r));
+        const uint32_t raw_row = st + (half >> 1) * A_RAW_BYTES + r * 128;
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+          float4 v;
+          const uint32_t addr = raw_row + (((4 * (half & 1) + c) ^ rr7) << 4);          // undo the 128 B TMA swizzle
+          asm volatile("ld.shared.v4.f32 {%0, %1, %2, %3}, [%4];" : "=f"(v.x), "=f"(v.y), "=f"(v.z), "=f"(v.w) : "r"(addr));
+          split_f16x2(v.x * a_scale, v.y * a_scale, hi[2 * c], lo[2 * c]);
+          split_f16x2(v.z * a_scale, v.w * a_scale, hi[2 * c + 1], lo[2 * c + 1]);
+        }
+        // the four warps of this lane quarter have read rows r of both raw boxes before any of them overwrites them
+        asm volatile("bar.sync %0, 128;" ::"r"(1 + quarter) : "memory");
+        // K elements 16 * half .. + 15 are the 16 B chunks 2 * half, 2 * half + 1 of the fp16 row (SWIZZLE_128B)
+#pragma unroll
+        for (int j = 0; j < 2; ++j) {
+          const uint32_t off = r * 128 + (((2 * half + j) ^ rr7) << 4);
+          asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};"
+                       ::"r"(st + off), "r"(hi[4 * j]), "r"(hi[4 * j + 1]), "r"(hi[4 * j + 2]), "r"(hi[4 * j + 3]) : "memory");
+          asm volatile("st.shared.v4.b32 [%0], {%1, %2, %3, %4};"
+                       ::"r"(st + A_RAW_BYTES + off), "r"(lo[4 * j]), "r"(lo[4 * j + 1]), "r"(lo[4 * j + 2]), "r"(lo[4 * j + 3]) : "memory");
+        }
+        // Hand-off of the split operand to the tensor core.  Each SM of the pair reads the A rows of its OWN CTA's shared
+        // memory (cta_group::2 splits M = 256 into the two CTAs' 128 rows), so every converter orders its generic-proxy
+        // stores before async-proxy reads of its own CTA's shared memory with fence.proxy.async.shared::cta, and only the
+        // signal crosses the pair: the arrive below (a default, i.e. .release.cta, remote arrive, as for the tensor-memory
+        // A of linear_tc_pair_kernel) is program-ordered after the fence, the leader issues the MMAs only after the phase
+        // completed, and the MMA's reads of this CTA's rows are performed by this SM's tensor core, through the proxy the
+        // fence has already made the stores visible to.  No generic-proxy data crosses the CTA boundary, so no
+        // cluster-scope release is needed (it costs a MEMBAR.ALL.GPU per arrive: see mbar_arrive_leader).
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        __syncwarp();
+        if (lane == 0) mbar_arrive_leader(a_ready(s));
+      }
+      mbar_wait(acc_full, tile_iter & 1);
+      tc_fence_after();
+      const int64_t row = m0 + r;
+      const float* rb = (rowbias && row < M) ? rowbias + __ldg(seg + row) * ld_rowbias + n0 : nullptr;
+      const int crow = static_cast<int>(m0) + quarter * 32;
+      const int64_t grow = m0 + quarter * 32;
+      // 64 output columns per warp as four 32 x 16 boxes through a 2 KB staging buffer and TMA stores (SWIZZLE_64B: the
+      // 16 B chunk index XOR bits 1-2 of the row, so the row-per-lane stores are conflict-free)
+      const uint32_t sbuf = out_stage + (warp - 2) * S_OUT_BYTES;
+#pragma unroll 1
+      for (int b = 0; b < 4; ++b) {
+        const int c0 = half * 64 + b * 16;
+        uint32_t v[16], w[16];
+        tmem_ld16(tmem_base + lane_addr + S_MAIN + c0, v);
+        tmem_ld16(tmem_base + lane_addr + S_CORR + c0, w);
+        asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
+        float4 o[4];
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          // the correction accumulator carries the 2^11 of the low parts; then undo the operand scales
+          o[q] = make_float4(fmaf(__uint_as_float(w[4 * q]), 1.f / 2048.f, __uint_as_float(v[4 * q])) * out_scale,
+                             fmaf(__uint_as_float(w[4 * q + 1]), 1.f / 2048.f, __uint_as_float(v[4 * q + 1])) * out_scale,
+                             fmaf(__uint_as_float(w[4 * q + 2]), 1.f / 2048.f, __uint_as_float(v[4 * q + 2])) * out_scale,
+                             fmaf(__uint_as_float(w[4 * q + 3]), 1.f / 2048.f, __uint_as_float(v[4 * q + 3])) * out_scale);
+          if (bias) {
+            const float4 bb = __ldg(reinterpret_cast<const float4*>(bias + n0 + c0) + q);
+            o[q].x += bb.x; o[q].y += bb.y; o[q].z += bb.z; o[q].w += bb.w;
+          }
+          if (rb) {
+            const float4 bb = __ldg(reinterpret_cast<const float4*>(rb + c0) + q);
+            o[q].x += bb.x; o[q].y += bb.y; o[q].z += bb.z; o[q].w += bb.w;
+          }
+          if (alpha) {                                       // inference: BatchNorm is folded into W / bias, PReLU here
+            const float4 al = __ldg(reinterpret_cast<const float4*>(alpha + n0 + c0) + q);
+            o[q].x = o[q].x > 0.f ? o[q].x : al.x * o[q].x; o[q].y = o[q].y > 0.f ? o[q].y : al.y * o[q].y;
+            o[q].z = o[q].z > 0.f ? o[q].z : al.z * o[q].z; o[q].w = o[q].w > 0.f ? o[q].w : al.w * o[q].w;
+          }
+          if (amax_out && row < M) out_max = amax4(out_max, o[q]);
+        }
+        if (lane == 0) asm volatile("cp.async.bulk.wait_group.read 0;" ::: "memory");   // the previous box has left the buffer
+        __syncwarp();
+#pragma unroll
+        for (int q = 0; q < 4; ++q) {
+          const uint32_t dst = sbuf + lane * 64 + ((q ^ ((lane >> 1) & 3)) << 4);      // SWIZZLE_64B box layout
+          asm volatile("st.shared.v4.f32 [%0], {%1, %2, %3, %4};" ::"r"(dst), "f"(o[q].x), "f"(o[q].y), "f"(o[q].z), "f"(o[q].w) : "memory");
+        }
+        asm volatile("fence.proxy.async.shared::cta;" ::: "memory");
+        __syncwarp();
+        if (lane == 0) {
+          if (crow < M) {
+            if (accumulate) tma_reduce_add_2d(&map_c, sbuf, n0 + c0, crow);
+            else tma_store_2d(&map_c, sbuf, n0 + c0, crow);
+          }
+          asm volatile("cp.async.bulk.commit_group;" ::: "memory");
+        }
+        // BatchNorm statistics of the box's 32-row group, pivot-shifted as in linear_tc_pair_kernel: lane c < 16 reduces
+        // column c (the same order of sums as there)
+        if (stats_part && grow < M && lane < 16) {
+          float ssum = 0.f, ssq = 0.f, pivot = 0.f;
+#pragma unroll 8
+          for (int rr = 0; rr < 32; ++rr) {
+            float hv;
+            const uint32_t src = sbuf + rr * 64 + (((lane >> 2) ^ ((rr >> 1) & 3)) << 4) + (lane & 3) * 4;
+            asm volatile("ld.shared.f32 %0, [%1];" : "=f"(hv) : "r"(src));
+            if (rr == 0) pivot = hv;
+            if (grow + rr < M) {
+              const float d = hv - pivot;
+              ssum += d;
+              ssq = fmaf(d, d, ssq);
+            }
+          }
+          const float cnt = static_cast<float>(M - grow < 32 ? M - grow : 32);
+          const float dm = ssum / cnt;
+          reinterpret_cast<float2*>(stats_part)[(grow >> 5) * static_cast<int64_t>(N) + n0 + c0 + lane] =
+              make_float2(pivot + dm, fmaxf(ssq - ssum * dm, 0.f));
+        }
+        __syncwarp();
+      }
+      tc_fence_before();          // accumulator reads ordered before this warp's next a_ready arrive
+    }
+    if (lane == 0) asm volatile("cp.async.bulk.wait_group 0;" ::: "memory");           // every box written before the CTA exits
+    amax_commit(out_max, amax_out);
   }
   tc_fence_before();
   cluster_sync_all();              // the peer's tensor core may still read this CTA's shared memory until its commits land
@@ -1357,6 +1638,34 @@ int launch_f16(const float* A, int64_t lda, const void* Bt_hi, const void* Bt_lo
   if ((alpha || amax_out || stats_part) && K > g_max_chain_k_f16)
     return fail(GCS_ERR_UNSUPPORTED, "launch_f16: the PReLU / |max| / statistics epilogue needs the reduction in one chain");
   alignas(64) CUtensorMap ma, mh, ml, mc;
+  const __half* bh = static_cast<const __half*>(Bt_hi);
+  const __half* bl = static_cast<const __half*>(Bt_lo);
+  // chains as in launch(): a K = 16 step adds into the accumulator with the same truncation, half as many steps per K
+  const int kMaxChainK = g_max_chain_k_f16;
+  if (N % 256 == 0) {
+    // one pass over A per 256 output columns (linear_f16_pass256_kernel); output boxes of 32 rows x 16 columns
+    GCS_TRY(make_map(&mc, C, M, N, ldc, 32, 16, CU_TENSOR_MAP_SWIZZLE_64B));
+    static bool attr256 = false;
+    if (!attr256) {
+      GCS_CUDA(cudaFuncSetAttribute(linear_f16_pass256_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, kSSmemBytes));
+      attr256 = true;
+    }
+    const int num_tiles = static_cast<int>(ceil_div(M, 2 * BM)) * (N / 256);
+    const int pairs = num_tiles < sm_count() / 2 ? num_tiles : sm_count() / 2;
+    dim3 grid(2, pairs);
+    for (int k0 = 0; k0 < K; k0 += kMaxChainK) {
+      const int kc = K - k0 < kMaxChainK ? K - k0 : kMaxChainK;
+      GCS_TRY(make_map(&ma, A + k0, M, kc, lda, BM));
+      GCS_TRY(make_map_f16(&mh, bh + k0, N, kc, K, 128));
+      GCS_TRY(make_map_f16(&ml, bl + k0, N, kc, K, 128));
+      const bool first = k0 == 0;
+      linear_f16_pass256_kernel<<<grid, kHThreads, kSSmemBytes, st>>>(ma, mh, ml, mc, first ? bias : nullptr, M, kc, N, num_tiles,
+                                                                       first ? accumulate : 1, first ? rowbias : nullptr, ld_rowbias,
+                                                                       seg, a_amax, cells + 1, alpha, amax_out, stats_part);
+      GCS_CHECK_LAUNCH("linear_f16_pass256_kernel");
+    }
+    return GCS_OK;
+  }
   GCS_TRY(make_map(&mc, C, M, N, ldc, 32, 32));
   static bool attr = false;
   if (!attr) {
@@ -1367,10 +1676,6 @@ int launch_f16(const float* A, int64_t lda, const void* Bt_hi, const void* Bt_lo
   const int num_tiles = static_cast<int>(ceil_div(M, 2 * BM)) * n_tiles;
   const int pairs = num_tiles < sm_count() / 2 ? num_tiles : sm_count() / 2;
   dim3 grid(2, pairs);
-  const __half* bh = static_cast<const __half*>(Bt_hi);
-  const __half* bl = static_cast<const __half*>(Bt_lo);
-  // chains as in launch(): a K = 16 step adds into the accumulator with the same truncation, half as many steps per K
-  const int kMaxChainK = g_max_chain_k_f16;
   for (int k0 = 0; k0 < K; k0 += kMaxChainK) {
     const int kc = K - k0 < kMaxChainK ? K - k0 : kMaxChainK;
     GCS_TRY(make_map(&ma, A + k0, M, kc, lda, BM));
