@@ -1,31 +1,56 @@
-// K5 — softmax + CategoricalCrossentropy (mean) + categorical_accuracy, forward and the
-// gradient w.r.t. the logits (reference: src/scripts/gcn.py:326 loss_fn, :335 loss,
-// :339 accuracy; SURVEY.md §8 a10).  Keras recovers the logits of the softmax activation
-// and evaluates softmax_cross_entropy_with_logits:
-//   loss_b = logsumexp(z_b) * sum(y_b) - y_b . z_b ;  loss = mean_b loss_b
-//          (evaluated as log(sum exp(z - m)) * sum(y) - y . (z - m), m = max z)
-//   dz_b   = (softmax(z_b) * sum(y_b) - y_b) * grad_scale
-// Two kernels share the per-row code (xent_row), so probs / dlogits are bit-identical between them:
-//   softmax_xent_kernel       one CTA, fixed-order tree reduction.  Graph-level batches are tiny ([1024, 2]).
-//   softmax_xent_grid_kernel  a grid of CTAs for node-level batches (~508 k rows at the cfg3 shape, where one CTA
-//                             would walk ~500 rows per thread); per-CTA fp64 loss / int hit partials go to a workspace
-//                             and softmax_xent_finish_kernel adds them in a fixed order.  The grid size depends on the
-//                             row count alone: deterministic run to run.
-// gcs_softmax_xent_ws picks between them by row count (kXentGridThreshold).
+// K5 — the loss heads of the model, forward and the gradient w.r.t. the logits, with loss_acc = {loss, metric}:
+//   softmax + CategoricalCrossentropy + categorical_accuracy (reference: src/scripts/gcn.py:326 loss_fn, :335 loss,
+//   :339 accuracy; SURVEY.md §8 a10).  Keras recovers the logits of the softmax and evaluates
+//   softmax_cross_entropy_with_logits per row:
+//     loss_b = logsumexp(z_b) * sum(y_b) - y_b . z_b ;  loss = mean_b loss_b
+//            (evaluated as log(sum exp(z - m)) * sum(y) - y . (z - m), m = max z)
+//     dz_b   = (softmax(z_b) * sum(y_b) - y_b) * grad_scale
+//   sigmoid + BinaryCrossentropy + binary_accuracy (binary and multi-label targets), per element
+//   (sigmoid_cross_entropy_with_logits):
+//     l = max(z, 0) - z*y + log1p(exp(-|z|))   acc = mean(y == (p > 0.5))   dz = (p - y) * grad_scale / C
+//   MeanSquaredError / MeanAbsoluteError / Huber of a linear head, metric mean_absolute_error; with e = z - y:
+//     MSE    l = e^2                                              dl/dz = 2e
+//     MAE    l = |e|                                              dl/dz = sign(e)   (sign(0) = 0, as in TF)
+//     Huber  l = 0.5 e^2 if |e| <= delta, else delta|e| - 0.5 delta^2   dl/dz = e, or delta sign(e)
+//     mae = mean(|e|)   dz = dl/dz * grad_scale / C
+//   The elementwise losses are the mean over the C columns, then over the rows: sum(l) / (rows * C).
+// One kernel body serves every loss (loss_kernel<Policy>).  A thread walks its items grid-stride - a row for the
+// softmax, a unit of four elements of the flat [rows * C] array for the others - with fp32 math per item and fp64 sums
+// per thread; the block adds {loss, metric} in a fixed-order tree.  A grid of one block writes loss_acc itself;
+// otherwise the per-block partials go to a workspace that loss_finish_kernel adds in a fixed order.  The grid size
+// depends on the problem size alone and there are no atomics, so every result is bit-identical run to run.
+#include <cmath>
+
 #include "common.cuh"
 
 namespace gcs {
 
 constexpr int kMaxClasses = 64;
-constexpr int64_t kXentGridThreshold = 65536;   // rows above which gcs_softmax_xent_ws runs the grid kernel
-constexpr int kXentGridThreads = 256;
-constexpr int kXentMaxBlocks = 1024;            // = the finish kernel's block size: one partial per thread
+constexpr int64_t kXentGridThreshold = 65536;   // rows above which gcs_softmax_xent_ws runs a grid of blocks
+constexpr int kXentMaxBlocks = 1024;
+constexpr int kElemMaxBlocks = 6 * 148;         // one wave of 6 resident blocks per SM (at <= 40 registers) on a
+                                                // B200's 148 SMs; a constant, not the device's count
+constexpr int kFinishThreads = 1024;            // one partial per finish thread
+static_assert(kXentMaxBlocks <= kFinishThreads && kElemMaxBlocks <= kFinishThreads, "one partial per finish thread");
 
-// One row b: writes probs / dlogits, adds the row's loss and hit to *loss / *hit (when y != NULL).
-__device__ __forceinline__ void xent_row(const float* __restrict__ logits, const float* __restrict__ y, int64_t b, int C,
-                                         float* __restrict__ probs, float* __restrict__ dlogits, float grad_scale,
-                                         double* loss, int* hit) {
-  const float* z = logits + b * C;
+enum { kRegMse = 1, kRegMae = 2, kRegHuber = 3 };
+
+struct LossArgs {
+  const float* logits;
+  const float* y;         // NULL: probabilities / predictions only
+  float* probs;
+  float* dlogits;
+  int64_t n;              // what the loss is the mean over: rows for the softmax, rows * C elements otherwise
+  int C;
+  float scale;            // gradient scale: grad_scale for the softmax, grad_scale / C otherwise
+  float delta = 0.f;      // Huber's delta
+  bool vec = false;       // every pointer is 16-byte aligned: the unit walk uses 128-bit accesses (set by launch_loss)
+};
+
+// One row b: writes probs / dlogits, adds the row's loss and hit to loss / hit (when y != NULL).
+__device__ __forceinline__ void xent_row(const LossArgs& a, int64_t b, double& loss, int& hit) {
+  const int C = a.C;
+  const float* z = a.logits + b * C;
   float m = z[0];
   int arg_p = 0;
   for (int c = 1; c < C; ++c)
@@ -41,105 +66,285 @@ __device__ __forceinline__ void xent_row(const float* __restrict__ logits, const
   const float inv = 1.0f / sum;
   float ysum = 0.f, yz = 0.f, ymax = 0.f;
   int arg_y = 0;
-  if (y) {
-    const float* yy = y + b * C;
+  if (a.y) {
+    const float* yy = a.y + b * C;
     ymax = yy[0];
     for (int c = 0; c < C; ++c) {
       ysum += yy[c];
       yz = fmaf(yy[c], z[c] - m, yz);            // y . (z - m): no cancellation against lse
       if (c > 0 && yy[c] > ymax) { ymax = yy[c]; arg_y = c; }
     }
-    *loss += static_cast<double>(log_sum * ysum - yz);
-    *hit += (arg_y == arg_p);
+    loss += static_cast<double>(log_sum * ysum - yz);
+    hit += (arg_y == arg_p);
   }
   for (int c = 0; c < C; ++c) {
     const float p = e[c] * inv;
-    if (probs) probs[b * C + c] = p;
-    if (dlogits) dlogits[b * C + c] = (p * ysum - y[b * C + c]) * grad_scale;
+    if (a.probs) a.probs[b * C + c] = p;
+    if (a.dlogits) a.dlogits[b * C + c] = (p * ysum - a.y[b * C + c]) * a.scale;
   }
 }
 
-__global__ void __launch_bounds__(1024) softmax_xent_kernel(
-    const float* __restrict__ logits, const float* __restrict__ y, int B, int C,
-    float* __restrict__ probs, float* __restrict__ loss_acc, float* __restrict__ dlogits,
-    float grad_scale) {
-  __shared__ double s_loss[1024];
-  __shared__ int s_hit[1024];
-  double loss = 0.0;
-  int hit = 0;
-  for (int b = threadIdx.x; b < B; b += blockDim.x)
-    xent_row(logits, y, b, C, probs, dlogits, grad_scale, &loss, &hit);
-  s_loss[threadIdx.x] = loss;
-  s_hit[threadIdx.x] = hit;
-  __syncthreads();
-  for (int off = blockDim.x >> 1; off > 0; off >>= 1) {
-    if (threadIdx.x < off) {
-      s_loss[threadIdx.x] += s_loss[threadIdx.x + off];
-      s_hit[threadIdx.x] += s_hit[threadIdx.x + off];
+// The metric of one unit of four, m[k] being element k's.  A hit count needs no order: the four elements add to one
+// counter.  fp32 values get a slot each and are added as (v0 + v1) + (v2 + v3), like the loss.
+struct UnitCount {
+  int n = 0;
+  __device__ int& operator[](int) { return n; }
+  __device__ int total() const { return n; }
+};
+struct UnitSum {
+  float v[4] = {0.f, 0.f, 0.f, 0.f};
+  __device__ float& operator[](int k) { return v[k]; }
+  __device__ float total() const { return (v[0] + v[1]) + (v[2] + v[3]); }
+};
+
+// One element of the sigmoid head: out = sigmoid(z); with labels also dz, the hit (added to hit) and the element's
+// loss (returned, 0 without labels).  One exp per element: e = exp(-|z|) gives both log1p(e) and p = 1/(1+e) or
+// e/(1+e), finite for any z.
+struct BceElem {
+  using Unit = UnitCount;
+  static constexpr bool kNeedsY = false;
+  __device__ __forceinline__ static float elem(float z, float yv, bool want_y, const LossArgs& a, float& out, float& dz,
+                                               int& hit) {
+    const float e = expf(-fabsf(z));
+    const float inv = 1.0f / (1.0f + e);
+    out = z >= 0.f ? inv : e * inv;
+    if (!want_y) return 0.f;
+    hit += (yv == (out > 0.5f ? 1.0f : 0.0f));
+    dz = (out - yv) * a.scale;
+    return fmaf(-z, yv, fmaxf(z, 0.f)) + log1pf(e);
+  }
+};
+
+// One element of a regression loss (only run with targets): out = z; returns the loss, leaves dz and |e| in ae.
+template <int KIND>
+struct RegElem {
+  using Unit = UnitSum;
+  static constexpr bool kNeedsY = true;            // the host copies the predictions itself when y is NULL
+  __device__ __forceinline__ static float elem(float z, float yv, bool, const LossArgs& a, float& out, float& dz,
+                                               float& ae) {
+    out = z;
+    const float e = z - yv;
+    const float abs_e = fabsf(e);
+    const float sgn = e > 0.f ? 1.f : (e < 0.f ? -1.f : 0.f);
+    ae = abs_e;
+    if (KIND == kRegMse) {
+      dz = (2.f * e) * a.scale;
+      return e * e;
     }
-    __syncthreads();
-  }
-  if (threadIdx.x == 0 && loss_acc) {
-    loss_acc[0] = B > 0 ? static_cast<float>(s_loss[0] / B) : 0.f;
-    loss_acc[1] = B > 0 ? static_cast<float>(s_hit[0]) / static_cast<float>(B) : 0.f;
-  }
-}
-
-// Rows b = blockIdx.x * blockDim.x + threadIdx.x + k * gridDim.x * blockDim.x; the CTA's loss / hit sums go to
-// part_loss[blockIdx.x] / part_hit[blockIdx.x].
-__global__ void __launch_bounds__(kXentGridThreads) softmax_xent_grid_kernel(
-    const float* __restrict__ logits, const float* __restrict__ y, int B, int C, float* __restrict__ probs,
-    float* __restrict__ dlogits, float grad_scale, double* __restrict__ part_loss, int* __restrict__ part_hit) {
-  __shared__ double s_loss[kXentGridThreads];
-  __shared__ int s_hit[kXentGridThreads];
-  double loss = 0.0;
-  int hit = 0;
-  const int64_t stride = static_cast<int64_t>(gridDim.x) * blockDim.x;
-  for (int64_t b = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x; b < B; b += stride)
-    xent_row(logits, y, b, C, probs, dlogits, grad_scale, &loss, &hit);
-  if (!part_loss) return;
-  s_loss[threadIdx.x] = loss;
-  s_hit[threadIdx.x] = hit;
-  __syncthreads();
-  for (int off = blockDim.x >> 1; off > 0; off >>= 1) {
-    if (threadIdx.x < off) {
-      s_loss[threadIdx.x] += s_loss[threadIdx.x + off];
-      s_hit[threadIdx.x] += s_hit[threadIdx.x + off];
+    if (KIND == kRegMae) {
+      dz = sgn * a.scale;
+      return abs_e;
     }
-    __syncthreads();
+    if (abs_e <= a.delta) {
+      dz = e * a.scale;
+      return 0.5f * e * e;
+    }
+    dz = (a.delta * sgn) * a.scale;
+    return a.delta * abs_e - 0.5f * a.delta * a.delta;
   }
-  if (threadIdx.x == 0) {
-    part_loss[blockIdx.x] = s_loss[0];
-    part_hit[blockIdx.x] = s_hit[0];
+};
+
+// Unit u = elements [4u, min(4u + 4, n)): one 128-bit access per operand when a.vec allows it, otherwise scalar
+// accesses of the same four elements, so the sums do not depend on alignment.  Each branch adds its own unit sums next
+// to the element math, which keeps the compiler's contraction of e.g. MSE's e0 * e0 + e1 * e1 into one FFMA.
+template <class E, class Metric>
+__device__ __forceinline__ void unit_walk(const LossArgs& a, int64_t u, double& loss, Metric& metric) {
+  const bool want_y = E::kNeedsY || a.y != nullptr;
+  const int64_t i0 = u << 2;
+  typename E::Unit m;
+  if (a.vec && i0 + 4 <= a.n) {
+    const float4 z = *reinterpret_cast<const float4*>(a.logits + i0);
+    const float4 yv = want_y ? *reinterpret_cast<const float4*>(a.y + i0) : make_float4(0.f, 0.f, 0.f, 0.f);
+    float4 o, d;
+    const float l0 = E::elem(z.x, yv.x, want_y, a, o.x, d.x, m[0]);
+    const float l1 = E::elem(z.y, yv.y, want_y, a, o.y, d.y, m[1]);
+    const float l2 = E::elem(z.z, yv.z, want_y, a, o.z, d.z, m[2]);
+    const float l3 = E::elem(z.w, yv.w, want_y, a, o.w, d.w, m[3]);
+    loss += static_cast<double>((l0 + l1) + (l2 + l3));
+    metric += m.total();
+    if (a.probs) *reinterpret_cast<float4*>(a.probs + i0) = o;
+    if (a.dlogits) *reinterpret_cast<float4*>(a.dlogits + i0) = d;
+  } else {
+    float l[4] = {0.f, 0.f, 0.f, 0.f};               // the vector path's order of the four additions
+#pragma unroll
+    for (int k = 0; k < 4; ++k) {
+      if (i0 + k >= a.n) break;
+      float o, d;
+      l[k] = E::elem(a.logits[i0 + k], want_y ? a.y[i0 + k] : 0.f, want_y, a, o, d, m[k]);
+      if (a.probs) a.probs[i0 + k] = o;
+      if (a.dlogits) a.dlogits[i0 + k] = d;
+    }
+    loss += static_cast<double>((l[0] + l[1]) + (l[2] + l[3]));
+    metric += m.total();
   }
 }
 
-// One thread per partial (n_parts <= kXentMaxBlocks), fixed-order tree sum.
-__global__ void __launch_bounds__(kXentMaxBlocks) softmax_xent_finish_kernel(
-    const double* __restrict__ part_loss, const int* __restrict__ part_hit, int n_parts, int B, float* __restrict__ loss_acc) {
-  __shared__ double s_loss[kXentMaxBlocks];
-  __shared__ int s_hit[kXentMaxBlocks];
+// loss_acc from the block sums (n > 0).  The sums are taken by reference: thread 0 reads each from shared memory
+// where it is used, which keeps the kernels at their register counts.
+struct XentFinish {
+  using Metric = int;                              // hit count, per thread and per block
+  using Acc = int;
+  __device__ static void finish(const double& s, const int& hits, int64_t rows, float* loss_acc) {
+    loss_acc[0] = static_cast<float>(s / static_cast<double>(rows));
+    loss_acc[1] = static_cast<float>(hits) / static_cast<float>(rows);
+  }
+};
+
+template <class M, class A>                        // per block M, per thread A: hit counts (sigmoid) or sums of |e|
+struct MeanFinish {
+  using Metric = M;
+  using Acc = A;
+  __device__ static void finish(const double& s, const M& m, int64_t n, float* loss_acc) {
+    loss_acc[0] = static_cast<float>(s / static_cast<double>(n));
+    loss_acc[1] = static_cast<float>(static_cast<double>(m) / static_cast<double>(n));
+  }
+};
+
+// Policies of loss_kernel: block size, minimum resident blocks (0: no bound), most blocks of a grid, the elements of
+// an item (a row for the softmax, whose n counts rows), one item, and the finish.
+template <int THREADS, int MAX_BLOCKS>
+struct Xent {
+  static constexpr int kThreads = THREADS, kMinBlocks = 0, kMaxBlocks = MAX_BLOCKS, kItem = 1;
+  using Finish = XentFinish;
+  __device__ static void item(const LossArgs& a, int64_t b, double& loss, int& hit) { xent_row(a, b, loss, hit); }
+};
+using XentBlock = Xent<1024, 1>;                   // gcs_softmax_xent: one block for any row count
+using XentGrid = Xent<256, kXentMaxBlocks>;        // gcs_softmax_xent_ws above kXentGridThreshold rows
+
+template <class E, class F>
+struct Elementwise {
+  static constexpr int kThreads = 256, kMinBlocks = 6, kMaxBlocks = kElemMaxBlocks, kItem = 4;
+  using Finish = F;
+  __device__ static void item(const LossArgs& a, int64_t u, double& loss, typename F::Acc& m) {
+    unit_walk<E>(a, u, loss, m);
+  }
+};
+using Bce = Elementwise<BceElem, MeanFinish<long long, int>>;
+template <int KIND>
+using Reg = Elementwise<RegElem<KIND>, MeanFinish<double, double>>;
+
+template <int THREADS, class M>
+struct BlockSums {
+  double loss[THREADS];
+  M m[THREADS];
+};
+
+// Fixed-order tree over the block of {loss, m}; the block's sums end in loss[0], m[0].
+template <int THREADS, class M>
+__device__ __forceinline__ const BlockSums<THREADS, M>& block_reduce(double loss, M m) {
+  __shared__ BlockSums<THREADS, M> s;
   const int t = threadIdx.x;
-  s_loss[t] = t < n_parts ? part_loss[t] : 0.0;
-  s_hit[t] = t < n_parts ? part_hit[t] : 0;
+  s.loss[t] = loss;
+  s.m[t] = m;
   __syncthreads();
-  for (int off = kXentMaxBlocks >> 1; off > 0; off >>= 1) {
+  for (int off = THREADS >> 1; off > 0; off >>= 1) {
     if (t < off) {
-      s_loss[t] += s_loss[t + off];
-      s_hit[t] += s_hit[t + off];
+      s.loss[t] += s.loss[t + off];
+      s.m[t] += s.m[t + off];
     }
     __syncthreads();
   }
-  if (t == 0) {
-    loss_acc[0] = static_cast<float>(s_loss[0] / B);
-    loss_acc[1] = static_cast<float>(s_hit[0]) / static_cast<float>(B);
+  return s;
+}
+
+template <class F>
+__device__ __forceinline__ void write_loss_acc(const double& s, const typename F::Metric& m, int64_t n,
+                                               float* loss_acc) {
+  if (n > 0) {
+    F::finish(s, m, n, loss_acc);
+  } else {
+    loss_acc[0] = 0.f;
+    loss_acc[1] = 0.f;
   }
 }
 
-static int xent_grid_blocks(int64_t B) {
-  const int64_t blocks = ceil_div(B, static_cast<int64_t>(kXentGridThreads));
-  return static_cast<int>(blocks < kXentMaxBlocks ? blocks : kXentMaxBlocks);
+// Items i = blockIdx.x * blockDim.x + threadIdx.x + k * gridDim.x * blockDim.x, elements [i * kItem, ...).  The
+// block's sums go to loss_acc (a grid of one block) or to part_loss / part_m[blockIdx.x].
+template <class P>
+__global__ void __launch_bounds__(P::kThreads, P::kMinBlocks) loss_kernel(
+    const LossArgs a, double* __restrict__ part_loss, typename P::Finish::Metric* __restrict__ part_m,
+    float* __restrict__ loss_acc) {
+  double loss = 0.0;
+  typename P::Finish::Acc m = 0;
+  const int64_t stride = static_cast<int64_t>(gridDim.x) * P::kThreads;
+#pragma unroll 1                                   // unrolled, the one-block softmax kernel spills
+  for (int64_t i = static_cast<int64_t>(blockIdx.x) * P::kThreads + threadIdx.x; i * P::kItem < a.n; i += stride)
+    P::item(a, i, loss, m);
+  if (!part_loss && !loss_acc) return;
+  const auto& s = block_reduce<P::kThreads, typename P::Finish::Metric>(loss, m);
+  if (threadIdx.x == 0) {
+    if (loss_acc) {
+      write_loss_acc<typename P::Finish>(s.loss[0], s.m[0], a.n, loss_acc);
+    } else {
+      part_loss[blockIdx.x] = s.loss[0];
+      part_m[blockIdx.x] = s.m[0];
+    }
+  }
 }
+
+// One thread per partial (n_parts <= kFinishThreads), zero-padded, fixed-order tree sum; n = 0 gives {0, 0}.
+template <class F>
+__global__ void __launch_bounds__(kFinishThreads) loss_finish_kernel(
+    const double* __restrict__ part_loss, const typename F::Metric* __restrict__ part_m, int n_parts, int64_t n,
+    float* __restrict__ loss_acc) {
+  const int t = threadIdx.x;
+  const auto& s = block_reduce<kFinishThreads>(t < n_parts ? part_loss[t] : 0.0,
+                                               t < n_parts ? part_m[t] : typename F::Metric(0));
+  if (t == 0) write_loss_acc<F>(s.loss[0], s.m[0], n, loss_acc);
+}
+
+// The grid: a count that depends on n alone; 0 when there is nothing to walk, except that a policy of one block runs
+// its block for any n (gcs_softmax_xent writes loss_acc = {0, 0} for B = 0 from its own kernel).
+template <class P>
+static int grid_blocks(int64_t n) {
+  if (P::kMaxBlocks == 1) return 1;
+  const int64_t blocks = ceil_div(ceil_div(n, P::kItem), static_cast<int64_t>(P::kThreads));
+  return static_cast<int>(blocks < P::kMaxBlocks ? blocks : P::kMaxBlocks);
+}
+
+// Bytes of the partials: the fp64 loss sums of the grid's blocks, then their metrics; none for a grid of one block.
+template <class P>
+static int64_t partial_bytes(int64_t n) {
+  const int blocks = grid_blocks<P>(n);
+  return blocks > 1 ? static_cast<int64_t>(blocks) * (sizeof(double) + sizeof(typename P::Finish::Metric)) : 0;
+}
+
+// Runs loss_kernel<P> and, for a grid of several blocks with loss_acc requested, loss_finish_kernel<P> over the
+// partials in `workspace`; with nothing to walk only the finish kernel, for loss_acc = {0, 0}.
+template <class P>
+static int launch_loss(const char* who, LossArgs a, float* loss_acc, void* workspace, int64_t workspace_bytes,
+                       cudaStream_t st) {
+  const int blocks = grid_blocks<P>(a.n);
+  double* part_loss = nullptr;
+  using F = typename P::Finish;
+  typename F::Metric* part_m = nullptr;
+  if (loss_acc && blocks > 1) {
+    const int64_t need = partial_bytes<P>(a.n);
+    if (!workspace || workspace_bytes < need)
+      return fail(GCS_ERR_WORKSPACE, "%s: workspace %lld < %lld bytes", who, (long long)workspace_bytes,
+                  (long long)need);
+    GCS_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 7u) == 0, "%s: workspace must be 8-byte aligned", who);
+    part_loss = static_cast<double*>(workspace);
+    part_m = reinterpret_cast<typename F::Metric*>(part_loss + blocks);
+  }
+  if (blocks == 0) {
+    if (loss_acc) {
+      loss_finish_kernel<F><<<1, kFinishThreads, 0, st>>>(nullptr, nullptr, 0, 0, loss_acc);
+      GCS_CHECK_LAUNCH("loss_finish_kernel");
+    }
+    return GCS_OK;
+  }
+  a.vec = aligned16(a.logits) && aligned16(a.y) && aligned16(a.probs) && aligned16(a.dlogits);
+  loss_kernel<P><<<blocks, P::kThreads, 0, st>>>(a, part_loss, part_m, blocks == 1 ? loss_acc : nullptr);
+  GCS_CHECK_LAUNCH("loss_kernel");
+  if (part_loss) {
+    loss_finish_kernel<F><<<1, kFinishThreads, 0, st>>>(part_loss, part_m, blocks, a.n, loss_acc);
+    GCS_CHECK_LAUNCH("loss_finish_kernel");
+  }
+  return GCS_OK;
+}
+
+static bool elementwise_size_ok(int64_t rows, int32_t C) { return rows >= 0 && C >= 1 && rows <= INT64_MAX / C; }
 
 }  // namespace gcs
 
@@ -150,16 +355,14 @@ extern "C" int gcs_softmax_xent(const float* logits, const float* y, int32_t B, 
   GCS_CHECK_ARG(B >= 0 && C > 0 && C <= kMaxClasses, "gcs_softmax_xent: C=%d outside [1, %d]", C, kMaxClasses);
   GCS_CHECK_ARG(logits || B == 0, "gcs_softmax_xent: null logits");
   GCS_CHECK_ARG(y || (!dlogits && !loss_acc), "gcs_softmax_xent: loss / gradient requested without labels");
-  softmax_xent_kernel<<<1, 1024, 0, as_stream(stream)>>>(logits, y, B, C, probs, loss_acc, dlogits, grad_scale);
-  GCS_CHECK_LAUNCH("softmax_xent_kernel");
-  return GCS_OK;
+  return launch_loss<XentBlock>("gcs_softmax_xent", {logits, y, probs, dlogits, B, C, grad_scale}, loss_acc, nullptr, 0,
+                                as_stream(stream));
 }
 
 extern "C" int64_t gcs_softmax_xent_workspace_bytes(int64_t B, int32_t C) {
   (void)C;
   if (B < 0) return -1;
-  if (B <= kXentGridThreshold) return 0;
-  return static_cast<int64_t>(xent_grid_blocks(B)) * (sizeof(double) + sizeof(int));
+  return B <= kXentGridThreshold ? 0 : partial_bytes<XentGrid>(B);
 }
 
 extern "C" int gcs_softmax_xent_ws(const float* logits, const float* y, int32_t B, int32_t C, float* probs,
@@ -170,25 +373,47 @@ extern "C" int gcs_softmax_xent_ws(const float* logits, const float* y, int32_t 
   GCS_CHECK_ARG(C > 0 && C <= kMaxClasses, "gcs_softmax_xent_ws: C=%d outside [1, %d]", C, kMaxClasses);
   GCS_CHECK_ARG(logits, "gcs_softmax_xent_ws: null logits");
   GCS_CHECK_ARG(y || (!dlogits && !loss_acc), "gcs_softmax_xent_ws: loss / gradient requested without labels");
-  const int blocks = xent_grid_blocks(B);
-  double* part_loss = nullptr;
-  int* part_hit = nullptr;
-  if (loss_acc) {
-    const int64_t need = gcs_softmax_xent_workspace_bytes(B, C);
-    if (!workspace || workspace_bytes < need)
-      return fail(GCS_ERR_WORKSPACE, "gcs_softmax_xent_ws: workspace %lld < %lld bytes", (long long)workspace_bytes,
-                  (long long)need);
-    GCS_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 7u) == 0, "gcs_softmax_xent_ws: workspace must be 8-byte aligned");
-    part_loss = static_cast<double*>(workspace);
-    part_hit = reinterpret_cast<int*>(part_loss + blocks);
-  }
+  return launch_loss<XentGrid>("gcs_softmax_xent_ws", {logits, y, probs, dlogits, B, C, grad_scale}, loss_acc,
+                               workspace, workspace_bytes, as_stream(stream));
+}
+
+extern "C" int64_t gcs_sigmoid_bce_workspace_bytes(int64_t rows, int32_t C) {
+  return elementwise_size_ok(rows, C) ? partial_bytes<Bce>(rows * C) : -1;
+}
+
+extern "C" int gcs_sigmoid_bce(const float* logits, const float* y, int64_t rows, int32_t C, float* probs,
+                               float* loss_acc, float* dlogits, float grad_scale, void* workspace,
+                               int64_t workspace_bytes, gcs_stream stream) {
+  GCS_CHECK_ARG(elementwise_size_ok(rows, C), "gcs_sigmoid_bce: rows=%lld, C=%d", (long long)rows, C);
+  GCS_CHECK_ARG(logits || rows == 0, "gcs_sigmoid_bce: null logits");
+  GCS_CHECK_ARG(y || (!dlogits && !loss_acc), "gcs_sigmoid_bce: loss / gradient requested without labels");
+  const LossArgs a{logits, y, probs, dlogits, rows * C, C, grad_scale / static_cast<float>(C)};
+  return launch_loss<Bce>("gcs_sigmoid_bce", a, loss_acc, workspace, workspace_bytes, as_stream(stream));
+}
+
+extern "C" int64_t gcs_regression_loss_workspace_bytes(int64_t rows, int32_t C) {
+  return elementwise_size_ok(rows, C) ? partial_bytes<Reg<kRegMse>>(rows * C) : -1;   // the same for every kind
+}
+
+extern "C" int gcs_regression_loss(int32_t kind, float huber_delta, const float* pred, const float* y, int64_t rows,
+                                   int32_t C, float* probs, float* loss_acc, float* dlogits, float grad_scale,
+                                   void* workspace, int64_t workspace_bytes, gcs_stream stream) {
+  GCS_CHECK_ARG(kind >= kRegMse && kind <= kRegHuber, "gcs_regression_loss: kind=%d (1 = MSE, 2 = MAE, 3 = Huber)",
+                kind);
+  GCS_CHECK_ARG(kind != kRegHuber || (std::isfinite(huber_delta) && huber_delta > 0.f),
+                "gcs_regression_loss: huber_delta must be finite and > 0, got %g", static_cast<double>(huber_delta));
+  GCS_CHECK_ARG(elementwise_size_ok(rows, C), "gcs_regression_loss: rows=%lld, C=%d", (long long)rows, C);
+  GCS_CHECK_ARG(pred || rows == 0, "gcs_regression_loss: null predictions");
+  GCS_CHECK_ARG(y || (!dlogits && !loss_acc), "gcs_regression_loss: loss / gradient requested without targets");
+  const LossArgs a{pred, y, probs, dlogits, rows * C, C, grad_scale / static_cast<float>(C), huber_delta};
   cudaStream_t st = as_stream(stream);
-  softmax_xent_grid_kernel<<<blocks, kXentGridThreads, 0, st>>>(logits, y, B, C, probs, dlogits, grad_scale, part_loss,
-                                                                part_hit);
-  GCS_CHECK_LAUNCH("softmax_xent_grid_kernel");
-  if (loss_acc) {
-    softmax_xent_finish_kernel<<<1, kXentMaxBlocks, 0, st>>>(part_loss, part_hit, blocks, B, loss_acc);
-    GCS_CHECK_LAUNCH("softmax_xent_finish_kernel");
+  if (!y) {                                          // predictions only: a linear head's output is its input
+    if (probs && probs != pred && a.n > 0)
+      GCS_CUDA(cudaMemcpyAsync(probs, pred, sizeof(float) * a.n, cudaMemcpyDeviceToDevice, st));
+    return GCS_OK;
   }
-  return GCS_OK;
+  const char* who = "gcs_regression_loss";
+  if (kind == kRegMse) return launch_loss<Reg<kRegMse>>(who, a, loss_acc, workspace, workspace_bytes, st);
+  if (kind == kRegMae) return launch_loss<Reg<kRegMae>>(who, a, loss_acc, workspace, workspace_bytes, st);
+  return launch_loss<Reg<kRegHuber>>(who, a, loss_acc, workspace, workspace_bytes, st);
 }

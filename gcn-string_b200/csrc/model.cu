@@ -156,9 +156,8 @@ struct Plan {
   int64_t bn_ws_bytes = 0;
   void* lin_ws = nullptr;       // split weights of the tensor-core GEMM in flight
   int64_t lin_ws_bytes = 0;
-  void* xent_ws = nullptr;      // loss partials of gcs_softmax_xent_ws (0 bytes up to its row threshold), of
-                                // gcs_sigmoid_bce with final_activation = 2, or of gcs_regression_loss with 0
-  int64_t xent_ws_bytes = 0;
+  void* loss_ws = nullptr;      // partials of the head's loss (head_loss_workspace_bytes)
+  int64_t loss_ws_bytes = 0;
   // backward
   float* gcat = nullptr;        // [N, Wc]  without pooling (node-level output) and for 'attn_sum': dLoss/d(emb(L)) in full
   float* dhcat = nullptr;       // [N, H*L] dh of the conv blocks, block k at columns [kH, (k+1)H)
@@ -265,6 +264,13 @@ static int prepare_step_weights(const gcs_model_config& c, const Plan& p, const 
   return tc::split_f16_multi(jobs, as_stream(st));
 }
 
+// Workspace of head_loss on [rows, C] logits; the regression partials do not depend on c.loss.
+static int64_t head_loss_workspace_bytes(const gcs_model_config& c, int64_t rows, int C) {
+  if (c.final_activation == 0) return gcs_regression_loss_workspace_bytes(rows, C);
+  if (c.final_activation == 2) return gcs_sigmoid_bce_workspace_bytes(rows, C);
+  return gcs_softmax_xent_workspace_bytes(rows, C);
+}
+
 static void make_plan(const gcs_model_config& c, int64_t N, int B, bool training, void* ws, Plan& p, int64_t* total) {
   build_blocks(c, p.blocks);
   p.P = c.pre_process; p.L = c.message_passing; p.Q = c.post_process;
@@ -345,11 +351,9 @@ static void make_plan(const gcs_model_config& c, int64_t N, int B, bool training
     p.prep_ws_bytes = list_step_weights(c, p, nullptr, nullptr, nullptr, nullptr);
     p.prep_ws = a.take<char>(p.prep_ws_bytes);
   }
-  // last: graph-level softmax plans keep their layout; the regression partials do not depend on c.loss
-  p.xent_ws_bytes = c.final_activation == 2   ? gcs_sigmoid_bce_workspace_bytes(p.rows_post, p.C)
-                    : c.final_activation == 0 ? gcs_regression_loss_workspace_bytes(p.rows_post, p.C)
-                                              : gcs_softmax_xent_workspace_bytes(p.rows_post, p.C);
-  p.xent_ws = a.take<char>(p.xent_ws_bytes);
+  // last: graph-level softmax plans keep their layout
+  p.loss_ws_bytes = head_loss_workspace_bytes(c, p.rows_post, p.C);
+  p.loss_ws = a.take<char>(p.loss_ws_bytes);
   *total = a.used;
 }
 
@@ -569,19 +573,22 @@ struct GradReady {
   void* user;
 };
 
-// The loss of the fused train step on p.logits: categorical cross-entropy on a softmax head, binary cross-entropy on a
-// sigmoid head, the regression loss c.loss selects (MSE by default) on a linear head; leaves dLoss/dlogits (scaled by
-// grad_scale) in p.dlogits.
-static int run_loss(const gcs_model_config& c, const Plan& p, const float* y, float* probs, float* loss_acc,
-                    float grad_scale, gcs_stream st) {
+// The head on p.logits: softmax with categorical cross-entropy, sigmoid with binary cross-entropy, or a linear head
+// with the regression loss c.loss selects (MSE by default).  probs gets the head's output (the probabilities, or a copy
+// of a linear head's logits).  With labels y it also leaves loss_acc and dLoss/dlogits (scaled by grad_scale) in
+// p.dlogits; with y = NULL, only probs.
+static int head_loss(const gcs_model_config& c, const Plan& p, const float* y, float* probs, float* loss_acc,
+                     float grad_scale, gcs_stream st) {
+  float* dlogits = y ? p.dlogits : nullptr;
   if (c.final_activation == 0)
     return gcs_regression_loss(c.loss ? c.loss : 1, c.huber_delta, p.logits, y, p.rows_post, p.C, probs, loss_acc,
-                               p.dlogits, grad_scale, p.xent_ws, p.xent_ws_bytes, st);
+                               dlogits, grad_scale, p.loss_ws, p.loss_ws_bytes, st);
   if (c.final_activation == 2)
-    return gcs_sigmoid_bce(p.logits, y, p.rows_post, p.C, probs, loss_acc, p.dlogits, grad_scale, p.xent_ws,
-                           p.xent_ws_bytes, st);
-  return gcs_softmax_xent_ws(p.logits, y, static_cast<int32_t>(p.rows_post), p.C, probs, loss_acc, p.dlogits, grad_scale,
-                             p.xent_ws, p.xent_ws_bytes, st);
+    return gcs_sigmoid_bce(p.logits, y, p.rows_post, p.C, probs, loss_acc, dlogits, grad_scale, p.loss_ws,
+                           p.loss_ws_bytes, st);
+  GCS_CHECK_ARG(p.rows_post < INT32_MAX, "softmax head: too many output rows");
+  return gcs_softmax_xent_ws(p.logits, y, static_cast<int32_t>(p.rows_post), p.C, probs, loss_acc, dlogits, grad_scale,
+                             p.loss_ws, p.loss_ws_bytes, st);
 }
 
 // Reverse pass given dlogits = dLoss/d(logits) [rows_post, C]; needs the activations a
@@ -764,17 +771,7 @@ extern "C" int gcs_model_forward(const gcs_model_config* cfg, const float* param
   if (workspace_bytes < total)
     return fail(GCS_ERR_WORKSPACE, "gcs_model_forward: workspace %lld < %lld bytes", (long long)workspace_bytes, (long long)total);
   GCS_TRY(run_forward(*cfg, p, params, state, *batch, training != 0, stream));
-  if (cfg->final_activation == 2) {
-    GCS_TRY(gcs_sigmoid_bce(p.logits, nullptr, p.rows_post, p.C, out, nullptr, nullptr, 0.f, p.xent_ws, p.xent_ws_bytes,
-                            stream));
-  } else if (cfg->final_activation == 1) {
-    GCS_CHECK_ARG(p.rows_post < INT32_MAX, "gcs_model_forward: too many output rows");
-    GCS_TRY(gcs_softmax_xent_ws(p.logits, nullptr, static_cast<int32_t>(p.rows_post), p.C, out, nullptr, nullptr, 0.f,
-                                p.xent_ws, p.xent_ws_bytes, stream));
-  } else {
-    GCS_CUDA(cudaMemcpyAsync(out, p.logits, sizeof(float) * p.rows_post * p.C, cudaMemcpyDeviceToDevice, as_stream(stream)));
-  }
-  return GCS_OK;
+  return head_loss(*cfg, p, nullptr, out, nullptr, 0.f, stream);
 }
 
 extern "C" int gcs_model_train_step(const gcs_model_config* cfg, const float* params, float* state,
@@ -797,7 +794,7 @@ extern "C" int gcs_model_train_step(const gcs_model_config* cfg, const float* pa
   GCS_TRY(prepare_step_weights(c, p, params, &prepared, stream));
   PreparedScope prepared_scope(&prepared);
   GCS_TRY(run_forward(c, p, params, state, bt, true, stream));
-  GCS_TRY(run_loss(c, p, bt.y, probs, loss_acc, grad_scale, stream));
+  GCS_TRY(head_loss(c, p, bt.y, probs, loss_acc, grad_scale, stream));
 
   return run_backward(c, p, params, grads, bt, p.dlogits, stream);
 }
@@ -865,7 +862,7 @@ extern "C" int gcs_model_train_step_dp(const gcs_model_config* cfg, const float*
   GCS_TRY(prepare_step_weights(c, p, params, &prepared, stream));
   PreparedScope prepared_scope(&prepared);
   GCS_TRY(run_forward(c, p, params, state, bt, true, stream));
-  GCS_TRY(run_loss(c, p, bt.y, probs, loss_acc, grad_scale, stream));
+  GCS_TRY(head_loss(c, p, bt.y, probs, loss_acc, grad_scale, stream));
   cudaEvent_t* ev = dp_events();
   DpSync sync{comm, grads, as_stream(stream), as_stream(comm_stream), {}, 0};
   for (int i = 0; i < 8; ++i) sync.ev[i] = ev[i];

@@ -7,11 +7,11 @@ launch (csrc/loss.cu).  Reduction is the Keras default: mean over the batch.
 
 ``BinaryCrossentropy`` and ``binary_accuracy`` are the Keras pair for a sigmoid head (binary and multi-label targets):
 on the logits of a ``GeneralGNN(activation='sigmoid')`` output, or with ``from_logits=True``, they run the fused kernel
-of csrc/loss_bce.cu.
+of csrc/loss.cu.
 
 ``MeanSquaredError``, ``MeanAbsoluteError`` and ``Huber`` are the Keras regression losses for the linear head of a
 default ``GeneralGNN(C)`` (activation=None); with ``mean_squared_error`` / ``mean_absolute_error`` they run the fused
-kernel of csrc/loss_reg.cu."""
+kernel of csrc/loss.cu."""
 from __future__ import annotations
 
 from . import _lib, ops

@@ -539,35 +539,13 @@ def attn_sum_pool_bwd(dout, x, kernel, graph_ptr, out, scores, gstats, dx=None):
 
 
 # ------------------------------------------------------------------ loss (K5) / optimizers (K10)
-def softmax_xent(logits, y=None, grad_scale: Optional[float] = None, want_grad=False):
-    """Returns (probs, loss_acc[2] or None, dlogits or None).  gcs_softmax_xent_ws: one thread block up to 65 536 rows,
-    a grid above - the same rule as the model's fused train step, so both give the same bits."""
+def _head_loss(entry, ws_bytes, logits, y, grad_scale, want_grad, want_probs=True, args=(), name="logits"):
+    """Shared body of the loss wrappers: returns (probs, loss_acc[2] or None, dlogits or None) of
+    ``lib.<entry>(*args, logits, y, rows, C, probs, loss_acc, dlogits, grad_scale, workspace, bytes, stream)``, with y
+    checked to have the shape of the logits and ``grad_scale`` defaulting to 1 / rows."""
     torch = _t()
     lib = _lib.load()
-    logits, _ = _mat(logits, "logits")
-    logits = logits.contiguous()
-    b, c = logits.shape
-    probs = torch.empty_like(logits)
-    loss_acc = torch.empty(2, dtype=torch.float32, device="cuda") if y is not None else None
-    dlogits = torch.empty_like(logits) if (want_grad and y is not None) else None
-    if y is not None:
-        y, _ = _mat(y, "y")
-        y = y.contiguous()
-    gs = (1.0 / b if b else 0.0) if grad_scale is None else grad_scale
-    nbytes = int(lib.gcs_softmax_xent_workspace_bytes(b, c))
-    ws = torch.empty(nbytes, dtype=torch.uint8, device="cuda") if nbytes > 0 else None
-    check(lib.gcs_softmax_xent_ws(ptr(logits), ptr(y), b, c, ptr(probs), ptr(loss_acc), ptr(dlogits), gs, ptr(ws), nbytes,
-                                  stream_ptr()), "gcs_softmax_xent_ws")
-    return probs, loss_acc, dlogits
-
-
-def sigmoid_bce(logits, y=None, grad_scale: Optional[float] = None, want_grad=False):
-    """Returns (probs, loss_acc[2] or None, dlogits or None) of gcs_sigmoid_bce: probs = sigmoid(logits), loss_acc =
-    {binary cross-entropy (mean over the columns, then the rows), binary accuracy}, dlogits = (probs - y) * grad_scale / C
-    (``grad_scale`` defaults to 1 / rows)."""
-    torch = _t()
-    lib = _lib.load()
-    logits, _ = _mat(logits, "logits")
+    logits, _ = _mat(logits, name)
     logits = logits.contiguous()
     b, c = logits.shape
     if y is not None:
@@ -575,15 +553,28 @@ def sigmoid_bce(logits, y=None, grad_scale: Optional[float] = None, want_grad=Fa
         if tuple(y.shape) != (b, c):
             raise ValueError(f"y must be [{b}, {c}], got {tuple(y.shape)}")
         y = y.contiguous()
-    probs = torch.empty_like(logits)
+    probs = torch.empty_like(logits) if want_probs else None
     loss_acc = torch.empty(2, dtype=torch.float32, device="cuda") if y is not None else None
     dlogits = torch.empty_like(logits) if (want_grad and y is not None) else None
     gs = (1.0 / b if b else 0.0) if grad_scale is None else grad_scale
-    nbytes = int(lib.gcs_sigmoid_bce_workspace_bytes(b, c))
+    nbytes = int(getattr(lib, ws_bytes)(b, c))
     ws = torch.empty(nbytes, dtype=torch.uint8, device="cuda") if nbytes > 0 else None
-    check(lib.gcs_sigmoid_bce(ptr(logits), ptr(y), b, c, ptr(probs), ptr(loss_acc), ptr(dlogits), gs, ptr(ws), nbytes,
-                              stream_ptr()), "gcs_sigmoid_bce")
+    check(getattr(lib, entry)(*args, ptr(logits), ptr(y), b, c, ptr(probs), ptr(loss_acc), ptr(dlogits), gs, ptr(ws),
+                              nbytes, stream_ptr()), entry)
     return probs, loss_acc, dlogits
+
+
+def softmax_xent(logits, y=None, grad_scale: Optional[float] = None, want_grad=False):
+    """Returns (probs, loss_acc[2] or None, dlogits or None).  gcs_softmax_xent_ws: one thread block up to 65 536 rows,
+    a grid above - the same rule as the model's fused train step, so both give the same bits."""
+    return _head_loss("gcs_softmax_xent_ws", "gcs_softmax_xent_workspace_bytes", logits, y, grad_scale, want_grad)
+
+
+def sigmoid_bce(logits, y=None, grad_scale: Optional[float] = None, want_grad=False):
+    """Returns (probs, loss_acc[2] or None, dlogits or None) of gcs_sigmoid_bce: probs = sigmoid(logits), loss_acc =
+    {binary cross-entropy (mean over the columns, then the rows), binary accuracy}, dlogits = (probs - y) * grad_scale / C
+    (``grad_scale`` defaults to 1 / rows)."""
+    return _head_loss("gcs_sigmoid_bce", "gcs_sigmoid_bce_workspace_bytes", logits, y, grad_scale, want_grad)
 
 
 REGRESSION_KIND = {"mse": 1, "mae": 2, "huber": 3}
@@ -593,24 +584,13 @@ def regression_loss(pred, y, loss: str = "mse", delta: float = 1.0, want_grad=Fa
     """Returns (loss_acc[2], dlogits or None) of gcs_regression_loss on the predictions of a linear head: loss_acc =
     {``loss`` ('mse', 'mae' or 'huber' with ``delta``; mean over the columns, then the rows), mean absolute error},
     dlogits = dLoss/dpred * grad_scale / C (``grad_scale`` defaults to 1 / rows)."""
-    torch = _t()
-    lib = _lib.load()
     if loss not in REGRESSION_KIND:
         raise ValueError(f"loss must be one of {sorted(REGRESSION_KIND)}, got {loss!r}")
-    pred, _ = _mat(pred, "pred")
-    pred = pred.contiguous()
-    b, c = pred.shape
-    y, _ = _mat(y, "y")
-    if tuple(y.shape) != (b, c):
-        raise ValueError(f"y must be [{b}, {c}], got {tuple(y.shape)}")
-    y = y.contiguous()
-    loss_acc = torch.empty(2, dtype=torch.float32, device="cuda")
-    dlogits = torch.empty_like(pred) if want_grad else None
-    gs = (1.0 / b if b else 0.0) if grad_scale is None else grad_scale
-    nbytes = int(lib.gcs_regression_loss_workspace_bytes(b, c))
-    ws = torch.empty(nbytes, dtype=torch.uint8, device="cuda") if nbytes > 0 else None
-    check(lib.gcs_regression_loss(REGRESSION_KIND[loss], float(delta), ptr(pred), ptr(y), b, c, None, ptr(loss_acc),
-                                  ptr(dlogits), gs, ptr(ws), nbytes, stream_ptr()), "gcs_regression_loss")
+    if y is None:
+        raise TypeError("regression_loss needs the targets y")
+    _, loss_acc, dlogits = _head_loss("gcs_regression_loss", "gcs_regression_loss_workspace_bytes", pred, y, grad_scale,
+                                      want_grad, want_probs=False, args=(REGRESSION_KIND[loss], float(delta)),
+                                      name="pred")
     return loss_acc, dlogits
 
 

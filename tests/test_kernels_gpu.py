@@ -653,6 +653,9 @@ def test_softmax_xent(B, C):
     assert rel_err(host(dlogits), (p - y) / B) < TOL
     p_only, none1, none2 = ops.softmax_xent(dev(z))
     assert none1 is None and none2 is None and torch.equal(p_only, probs)
+    for bad in (y[:-1], y[:, :-1]):                     # labels of another shape never reach the kernel
+        with pytest.raises(ValueError):
+            ops.softmax_xent(dev(z), dev(bad))
 
 
 def test_fused_optimizer_steps():
