@@ -15,6 +15,7 @@ _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libgcnstring_b200.so")
 
 GCS_OK = 0
+WORKSPACE_SAMPLE_WEIGHTS = 1          # gcs_model_workspace_bytes_ex flag (GCS_WORKSPACE_SAMPLE_WEIGHTS)
 _STATUS_EXC = {1: ValueError, 2: NotImplementedError, 3: MemoryError, 4: RuntimeError}
 
 
@@ -31,7 +32,8 @@ class Batch(Structure):
                 ("rowptr", c_void_p), ("colidx", c_void_p), ("rowptr_t", c_void_p), ("colidx_t", c_void_p),
                 ("graph_ptr", c_void_p), ("x", c_void_p), ("ldx", c_int64), ("y", c_void_p),
                 ("seg_ids", c_void_p), ("rb4_blk_ptr", c_void_p), ("rb4_ent", c_void_p), ("rb4_blk_ptr_t", c_void_p), ("rb4_ent_t", c_void_p),
-                ("max_graph_nodes", c_int32), ("reserved", c_int32), ("values", c_void_p), ("values_t", c_void_p)]
+                ("max_graph_nodes", c_int32), ("reserved", c_int32), ("values", c_void_p), ("values_t", c_void_p),
+                ("sample_weight", c_void_p)]
 
 
 P = c_void_p
@@ -89,6 +91,8 @@ PROTOTYPES = {
     "gcs_sigmoid_bce": (c_int32, [P, P, I64, I32, P, P, P, F32, P, I64, P]),
     "gcs_regression_loss_workspace_bytes": (c_int64, [I64, I32]),
     "gcs_regression_loss": (c_int32, [I32, F32, P, P, I64, I32, P, P, P, F32, P, I64, P]),
+    "gcs_weighted_loss_workspace_bytes": (c_int64, [I32, I64, I32]),
+    "gcs_weighted_loss": (c_int32, [I32, I32, F32, P, P, P, I64, I32, P, P, P, F32, P, I64, P]),
     "gcs_sgd_step": (c_int32, [P, P, I64, F32, F32, P]),
     "gcs_adam_step": (c_int32, [P, P, P, P, I64, F64, F64, F64, F64, I64, F32, P]),
     "gcs_comm_unique_id": (c_int32, [P]),
@@ -102,6 +106,7 @@ PROTOTYPES = {
     "gcs_model_num_params": (c_int64, [POINTER(ModelConfig)]),
     "gcs_model_num_state": (c_int64, [POINTER(ModelConfig)]),
     "gcs_model_workspace_bytes": (c_int64, [POINTER(ModelConfig), I64, I64, I32, I32]),
+    "gcs_model_workspace_bytes_ex": (c_int64, [POINTER(ModelConfig), I64, I64, I32, I32, I32]),
     "gcs_model_forward": (c_int32, [POINTER(ModelConfig), P, P, POINTER(Batch), I32, P, P, I64, P]),
     "gcs_model_train_step": (c_int32, [POINTER(ModelConfig), P, P, POINTER(Batch), F32, P, P, P, P, I64, P]),
     "gcs_model_logits_offset": (c_int64, [POINTER(ModelConfig), I64, I32, I32]),

@@ -19,6 +19,10 @@
 // per thread; the block adds {loss, metric} in a fixed-order tree.  A grid of one block writes loss_acc itself;
 // otherwise the per-block partials go to a workspace that loss_finish_kernel adds in a fixed order.  The grid size
 // depends on the problem size alone and there are no atomics, so every result is bit-identical run to run.
+// With per-row sample weights w (the weighted policies, gcs_weighted_loss), as Keras' sample_weight with the default
+// "sum_over_batch_size" reduction: loss = sum_r w_r l_r / rows, dz_r = w_r * dz_r, and the metric is the weighted mean
+// sum w m / sum w (0 when sum w = 0).  Each block then adds {sum w l, sum w m, sum w} in fp64 (WSums), in the same
+// fixed-order tree.
 #include <cmath>
 
 #include "common.cuh"
@@ -47,8 +51,16 @@ struct LossArgs {
   bool vec = false;       // every pointer is 16-byte aligned: the unit walk uses 128-bit accesses (set by launch_loss)
 };
 
-// One row b: writes probs / dlogits, adds the row's loss and hit to loss / hit (when y != NULL).
-__device__ __forceinline__ void xent_row(const LossArgs& a, int64_t b, double& loss, int& hit) {
+// The arguments of the weighted policies.  The weight pointer lives in this extension rather than in LossArgs itself, so
+// that the unweighted kernels keep their parameter layout and compiled code.
+struct WLossArgs : LossArgs {
+  const float* w;         // [rows] one weight per row (read with scalar loads; any alignment)
+};
+
+// One row b: writes probs / dlogits, adds the row's loss and hit to loss / hit (when y != NULL).  W: the row has weight
+// w, which multiplies its loss (in fp64) and its dlogits, after the unweighted expression (exact for w = 1).
+template <bool W = false>
+__device__ __forceinline__ void xent_row(const LossArgs& a, int64_t b, double& loss, int& hit, float w = 1.f) {
   const int C = a.C;
   const float* z = a.logits + b * C;
   float m = z[0];
@@ -74,13 +86,17 @@ __device__ __forceinline__ void xent_row(const LossArgs& a, int64_t b, double& l
       yz = fmaf(yy[c], z[c] - m, yz);            // y . (z - m): no cancellation against lse
       if (c > 0 && yy[c] > ymax) { ymax = yy[c]; arg_y = c; }
     }
-    loss += static_cast<double>(log_sum * ysum - yz);
+    if (W) loss += static_cast<double>(log_sum * ysum - yz) * static_cast<double>(w);
+    else loss += static_cast<double>(log_sum * ysum - yz);
     hit += (arg_y == arg_p);
   }
   for (int c = 0; c < C; ++c) {
     const float p = e[c] * inv;
     if (a.probs) a.probs[b * C + c] = p;
-    if (a.dlogits) a.dlogits[b * C + c] = (p * ysum - a.y[b * C + c]) * a.scale;
+    if (a.dlogits) {
+      if (W) a.dlogits[b * C + c] = (p * ysum - a.y[b * C + c]) * a.scale * w;
+      else a.dlogits[b * C + c] = (p * ysum - a.y[b * C + c]) * a.scale;
+    }
   }
 }
 
@@ -179,6 +195,64 @@ __device__ __forceinline__ void unit_walk(const LossArgs& a, int64_t u, double& 
   }
 }
 
+// {sum of w * metric, sum of w} of the weighted policies, per thread and per block (fp64).
+struct WSums {
+  double m, w;
+  WSums() = default;                               // trivial: block_reduce keeps an array of them in shared memory
+  __device__ WSums(int zero) : m(zero), w(zero) {}
+  __device__ WSums& operator+=(const WSums& o) {
+    m += o.m;
+    w += o.w;
+    return *this;
+  }
+};
+
+// The weighted unit u.  When its elements all carry the same weight w0 (every unit of a row when C % 4 == 0; any unit
+// when the weights agree) it is unit_walk itself on a gradient scale of scale * w0, and its sums times w0 in fp64: with
+// w0 = 1 loss, dlogits and metric are the unweighted kernel's bits.  A unit that spans rows of different weights takes
+// each element alone, with scalar accesses.
+template <class E, class Acc>
+__device__ __forceinline__ void unit_walk_weighted(const WLossArgs& a, int64_t u, double& loss, WSums& ws) {
+  const int64_t i0 = u << 2;
+  const int cnt = a.n - i0 < 4 ? static_cast<int>(a.n - i0) : 4;
+  const int64_t r0 = i0 / a.C;
+  const int c0 = static_cast<int>(i0 - r0 * a.C);
+  float w[4];
+  bool same = true;
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    w[k] = k < cnt ? a.w[r0 + (c0 + k) / a.C] : 0.f;
+    same = same && (k >= cnt || w[k] == w[0]);
+  }
+  if (same) {
+    LossArgs b = a;
+    b.scale = a.scale * w[0];
+    double l = 0.0;
+    Acc m = 0;
+    unit_walk<E>(b, u, l, m);
+    loss += l * static_cast<double>(w[0]);
+    ws.m += static_cast<double>(m) * static_cast<double>(w[0]);
+    ws.w += static_cast<double>(cnt) * static_cast<double>(w[0]);
+    return;
+  }
+  float wl[4] = {0.f, 0.f, 0.f, 0.f};
+#pragma unroll
+  for (int k = 0; k < 4; ++k) {
+    if (k >= cnt) break;
+    const int64_t i = i0 + k;
+    LossArgs b = a;
+    b.scale = a.scale * w[k];
+    typename E::Unit m;
+    float o, d;
+    wl[k] = E::elem(a.logits[i], a.y[i], true, b, o, d, m[0]) * w[k];
+    if (a.probs) a.probs[i] = o;
+    if (a.dlogits) a.dlogits[i] = d;
+    ws.m += static_cast<double>(m.total()) * static_cast<double>(w[k]);
+    ws.w += static_cast<double>(w[k]);
+  }
+  loss += static_cast<double>((wl[0] + wl[1]) + (wl[2] + wl[3]));
+}
+
 // loss_acc from the block sums (n > 0).  The sums are taken by reference: thread 0 reads each from shared memory
 // where it is used, which keeps the kernels at their register counts.
 struct XentFinish {
@@ -200,28 +274,69 @@ struct MeanFinish {
   }
 };
 
-// Policies of loss_kernel: block size, minimum resident blocks (0: no bound), most blocks of a grid, the elements of
-// an item (a row for the softmax, whose n counts rows), one item, and the finish.
-template <int THREADS, int MAX_BLOCKS>
+// The weighted policies: loss = sum w l / n (n = rows, or rows * C: the mean over the columns is inside), metric =
+// sum w m / sum w, or 0 when sum w = 0.
+struct WeightedFinish {
+  using Metric = WSums;
+  using Acc = WSums;
+  __device__ static void finish(const double& s, const WSums& m, int64_t n, float* loss_acc) {
+    loss_acc[0] = static_cast<float>(s / static_cast<double>(n));
+    loss_acc[1] = m.w != 0.0 ? static_cast<float>(m.m / m.w) : 0.f;
+  }
+};
+
+// Policies of loss_kernel: block size, minimum resident blocks (0: no bound), most blocks of a grid, the kernel's
+// arguments (Args), the elements of an item (a row for the softmax, whose n counts rows), one item, and the finish.
+// W selects the weighted form of a policy.
+template <int THREADS, int MAX_BLOCKS, bool W = false>
 struct Xent {
   static constexpr int kThreads = THREADS, kMinBlocks = 0, kMaxBlocks = MAX_BLOCKS, kItem = 1;
+  using Args = LossArgs;
   using Finish = XentFinish;
   __device__ static void item(const LossArgs& a, int64_t b, double& loss, int& hit) { xent_row(a, b, loss, hit); }
 };
+template <int THREADS, int MAX_BLOCKS>
+struct Xent<THREADS, MAX_BLOCKS, true> {
+  static constexpr int kThreads = THREADS, kMinBlocks = 0, kMaxBlocks = MAX_BLOCKS, kItem = 1;
+  using Args = WLossArgs;
+  using Finish = WeightedFinish;
+  __device__ static void item(const WLossArgs& a, int64_t b, double& loss, WSums& ws) {
+    const float w = a.w[b];
+    int hit = 0;
+    xent_row<true>(a, b, loss, hit, w);
+    if (hit) ws.m += static_cast<double>(w);
+    ws.w += static_cast<double>(w);
+  }
+};
 using XentBlock = Xent<1024, 1>;                   // gcs_softmax_xent: one block for any row count
 using XentGrid = Xent<256, kXentMaxBlocks>;        // gcs_softmax_xent_ws above kXentGridThreshold rows
+using XentBlockW = Xent<1024, 1, true>;            // gcs_weighted_loss, the same rule
+using XentGridW = Xent<256, kXentMaxBlocks, true>;
 
-template <class E, class F>
+template <class E, class F, bool W = false>
 struct Elementwise {
   static constexpr int kThreads = 256, kMinBlocks = 6, kMaxBlocks = kElemMaxBlocks, kItem = 4;
+  using Args = LossArgs;
   using Finish = F;
   __device__ static void item(const LossArgs& a, int64_t u, double& loss, typename F::Acc& m) {
     unit_walk<E>(a, u, loss, m);
   }
 };
+template <class E, class F>                        // F: the unweighted finish, whose per-thread metric a unit produces
+struct Elementwise<E, F, true> {
+  static constexpr int kThreads = 256, kMinBlocks = 0, kMaxBlocks = kElemMaxBlocks, kItem = 4;
+  using Args = WLossArgs;
+  using Finish = WeightedFinish;
+  __device__ static void item(const WLossArgs& a, int64_t u, double& loss, WSums& ws) {
+    unit_walk_weighted<E, typename F::Acc>(a, u, loss, ws);
+  }
+};
 using Bce = Elementwise<BceElem, MeanFinish<long long, int>>;
 template <int KIND>
 using Reg = Elementwise<RegElem<KIND>, MeanFinish<double, double>>;
+using BceW = Elementwise<BceElem, MeanFinish<long long, int>, true>;
+template <int KIND>
+using RegW = Elementwise<RegElem<KIND>, MeanFinish<double, double>, true>;
 
 template <int THREADS, class M>
 struct BlockSums {
@@ -262,7 +377,7 @@ __device__ __forceinline__ void write_loss_acc(const double& s, const typename F
 // block's sums go to loss_acc (a grid of one block) or to part_loss / part_m[blockIdx.x].
 template <class P>
 __global__ void __launch_bounds__(P::kThreads, P::kMinBlocks) loss_kernel(
-    const LossArgs a, double* __restrict__ part_loss, typename P::Finish::Metric* __restrict__ part_m,
+    const typename P::Args a, double* __restrict__ part_loss, typename P::Finish::Metric* __restrict__ part_m,
     float* __restrict__ loss_acc) {
   double loss = 0.0;
   typename P::Finish::Acc m = 0;
@@ -312,7 +427,7 @@ static int64_t partial_bytes(int64_t n) {
 // Runs loss_kernel<P> and, for a grid of several blocks with loss_acc requested, loss_finish_kernel<P> over the
 // partials in `workspace`; with nothing to walk only the finish kernel, for loss_acc = {0, 0}.
 template <class P>
-static int launch_loss(const char* who, LossArgs a, float* loss_acc, void* workspace, int64_t workspace_bytes,
+static int launch_loss(const char* who, typename P::Args a, float* loss_acc, void* workspace, int64_t workspace_bytes,
                        cudaStream_t st) {
   const int blocks = grid_blocks<P>(a.n);
   double* part_loss = nullptr;
@@ -416,4 +531,42 @@ extern "C" int gcs_regression_loss(int32_t kind, float huber_delta, const float*
   if (kind == kRegMse) return launch_loss<Reg<kRegMse>>(who, a, loss_acc, workspace, workspace_bytes, st);
   if (kind == kRegMae) return launch_loss<Reg<kRegMae>>(who, a, loss_acc, workspace, workspace_bytes, st);
   return launch_loss<Reg<kRegHuber>>(who, a, loss_acc, workspace, workspace_bytes, st);
+}
+
+// head: gcs_model_config.final_activation codes (0 = linear with a regression loss, 1 = softmax, 2 = sigmoid).
+extern "C" int64_t gcs_weighted_loss_workspace_bytes(int32_t head, int64_t rows, int32_t C) {
+  if (head < 0 || head > 2 || !elementwise_size_ok(rows, C)) return -1;
+  if (head == 1) return rows <= kXentGridThreshold ? 0 : partial_bytes<XentGridW>(rows);
+  return partial_bytes<BceW>(rows * C);                                  // the same for every elementwise head
+}
+
+extern "C" int gcs_weighted_loss(int32_t head, int32_t kind, float huber_delta, const float* logits, const float* y,
+                                 const float* sample_weight, int64_t rows, int32_t C, float* probs, float* loss_acc,
+                                 float* dlogits, float grad_scale, void* workspace, int64_t workspace_bytes,
+                                 gcs_stream stream) {
+  const char* who = "gcs_weighted_loss";
+  GCS_CHECK_ARG(head >= 0 && head <= 2, "%s: head=%d (0 = linear, 1 = softmax, 2 = sigmoid)", who, head);
+  GCS_CHECK_ARG(head != 0 || (kind >= kRegMse && kind <= kRegHuber), "%s: kind=%d (1 = MSE, 2 = MAE, 3 = Huber)", who,
+                kind);
+  GCS_CHECK_ARG(head != 0 || kind != kRegHuber || (std::isfinite(huber_delta) && huber_delta > 0.f),
+                "%s: huber_delta must be finite and > 0, got %g", who, static_cast<double>(huber_delta));
+  GCS_CHECK_ARG(elementwise_size_ok(rows, C), "%s: rows=%lld, C=%d", who, (long long)rows, C);
+  GCS_CHECK_ARG(head != 1 || C <= kMaxClasses, "%s: softmax C=%d outside [1, %d]", who, C, kMaxClasses);
+  GCS_CHECK_ARG(sample_weight, "%s: null sample_weight (the unweighted entry points take no weights)", who);
+  GCS_CHECK_ARG((logits && y) || rows == 0, "%s: null logits or labels", who);
+  cudaStream_t st = as_stream(stream);
+  WLossArgs a;
+  static_cast<LossArgs&>(a) = LossArgs{logits, y, probs, dlogits, rows, C, grad_scale};
+  a.w = sample_weight;
+  if (head == 1) {
+    if (rows <= kXentGridThreshold) return launch_loss<XentBlockW>(who, a, loss_acc, workspace, workspace_bytes, st);
+    return launch_loss<XentGridW>(who, a, loss_acc, workspace, workspace_bytes, st);
+  }
+  a.n = rows * C;
+  a.scale = grad_scale / static_cast<float>(C);
+  if (head == 2) return launch_loss<BceW>(who, a, loss_acc, workspace, workspace_bytes, st);
+  a.delta = huber_delta;
+  if (kind == kRegMse) return launch_loss<RegW<kRegMse>>(who, a, loss_acc, workspace, workspace_bytes, st);
+  if (kind == kRegMae) return launch_loss<RegW<kRegMae>>(who, a, loss_acc, workspace, workspace_bytes, st);
+  return launch_loss<RegW<kRegHuber>>(who, a, loss_acc, workspace, workspace_bytes, st);
 }

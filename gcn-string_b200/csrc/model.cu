@@ -264,14 +264,22 @@ static int prepare_step_weights(const gcs_model_config& c, const Plan& p, const 
   return tc::split_f16_multi(jobs, as_stream(st));
 }
 
-// Workspace of head_loss on [rows, C] logits; the regression partials do not depend on c.loss.
-static int64_t head_loss_workspace_bytes(const gcs_model_config& c, int64_t rows, int C) {
+// Workspace of head_loss on [rows, C] logits; the regression partials do not depend on c.loss.  With sample weights
+// (GCS_WORKSPACE_SAMPLE_WEIGHTS) the larger of the weighted and the unweighted partials, so that such a plan also serves
+// an unweighted step.
+static int64_t head_loss_workspace_bytes(const gcs_model_config& c, int64_t rows, int C, int flags = 0) {
+  if (flags & GCS_WORKSPACE_SAMPLE_WEIGHTS) {
+    const int64_t w = gcs_weighted_loss_workspace_bytes(c.final_activation, rows, C);
+    const int64_t u = head_loss_workspace_bytes(c, rows, C);
+    return w > u ? w : u;
+  }
   if (c.final_activation == 0) return gcs_regression_loss_workspace_bytes(rows, C);
   if (c.final_activation == 2) return gcs_sigmoid_bce_workspace_bytes(rows, C);
   return gcs_softmax_xent_workspace_bytes(rows, C);
 }
 
-static void make_plan(const gcs_model_config& c, int64_t N, int B, bool training, void* ws, Plan& p, int64_t* total) {
+static void make_plan(const gcs_model_config& c, int64_t N, int B, bool training, void* ws, Plan& p, int64_t* total,
+                      int flags = 0) {
   build_blocks(c, p.blocks);
   p.P = c.pre_process; p.L = c.message_passing; p.Q = c.post_process;
   p.H = c.hidden; p.Wc = c.connectivity == 1 ? c.hidden * (c.message_passing + 1) : c.hidden; p.C = c.output;
@@ -351,8 +359,8 @@ static void make_plan(const gcs_model_config& c, int64_t N, int B, bool training
     p.prep_ws_bytes = list_step_weights(c, p, nullptr, nullptr, nullptr, nullptr);
     p.prep_ws = a.take<char>(p.prep_ws_bytes);
   }
-  // last: graph-level softmax plans keep their layout
-  p.loss_ws_bytes = head_loss_workspace_bytes(c, p.rows_post, p.C);
+  // last: graph-level softmax plans keep their layout, and sample weights change no other offset
+  p.loss_ws_bytes = head_loss_workspace_bytes(c, p.rows_post, p.C, flags);
   p.loss_ws = a.take<char>(p.loss_ws_bytes);
   *total = a.used;
 }
@@ -576,10 +584,13 @@ struct GradReady {
 // The head on p.logits: softmax with categorical cross-entropy, sigmoid with binary cross-entropy, or a linear head
 // with the regression loss c.loss selects (MSE by default).  probs gets the head's output (the probabilities, or a copy
 // of a linear head's logits).  With labels y it also leaves loss_acc and dLoss/dlogits (scaled by grad_scale) in
-// p.dlogits; with y = NULL, only probs.
+// p.dlogits; with y = NULL, only probs.  Per-row weights w (with y) select the weighted form of the same head.
 static int head_loss(const gcs_model_config& c, const Plan& p, const float* y, float* probs, float* loss_acc,
-                     float grad_scale, gcs_stream st) {
+                     float grad_scale, gcs_stream st, const float* w = nullptr) {
   float* dlogits = y ? p.dlogits : nullptr;
+  if (y && w)
+    return gcs_weighted_loss(c.final_activation, c.loss ? c.loss : 1, c.huber_delta, p.logits, y, w, p.rows_post, p.C,
+                             probs, loss_acc, dlogits, grad_scale, p.loss_ws, p.loss_ws_bytes, st);
   if (c.final_activation == 0)
     return gcs_regression_loss(c.loss ? c.loss : 1, c.huber_delta, p.logits, y, p.rows_post, p.C, probs, loss_acc,
                                dlogits, grad_scale, p.loss_ws, p.loss_ws_bytes, st);
@@ -748,14 +759,19 @@ extern "C" int64_t gcs_model_num_state(const gcs_model_config* cfg) {
   return blocks.back().stat_off + 2LL * blocks.back().m_out;
 }
 
-extern "C" int64_t gcs_model_workspace_bytes(const gcs_model_config* cfg, int64_t n_nodes, int64_t nnz,
-                                             int32_t n_graphs, int32_t training) {
+extern "C" int64_t gcs_model_workspace_bytes_ex(const gcs_model_config* cfg, int64_t n_nodes, int64_t nnz,
+                                                int32_t n_graphs, int32_t training, int32_t flags) {
   (void)nnz;
-  if (check_config(cfg) != GCS_OK || n_nodes < 0 || n_graphs < 0) return -1;
+  if (check_config(cfg) != GCS_OK || n_nodes < 0 || n_graphs < 0 || (flags & ~GCS_WORKSPACE_SAMPLE_WEIGHTS)) return -1;
   Plan p;
   int64_t total = 0;
-  make_plan(*cfg, n_nodes, n_graphs, training != 0, nullptr, p, &total);
+  make_plan(*cfg, n_nodes, n_graphs, training != 0, nullptr, p, &total, flags);
   return total;
+}
+
+extern "C" int64_t gcs_model_workspace_bytes(const gcs_model_config* cfg, int64_t n_nodes, int64_t nnz,
+                                             int32_t n_graphs, int32_t training) {
+  return gcs_model_workspace_bytes_ex(cfg, n_nodes, nnz, n_graphs, training, 0);
 }
 
 extern "C" int gcs_model_forward(const gcs_model_config* cfg, const float* params, float* state,
@@ -786,7 +802,7 @@ extern "C" int gcs_model_train_step(const gcs_model_config* cfg, const float* pa
   const gcs_batch& bt = *batch;
   Plan p;
   int64_t total = 0;
-  make_plan(c, bt.n_nodes, bt.n_graphs, true, workspace, p, &total);
+  make_plan(c, bt.n_nodes, bt.n_graphs, true, workspace, p, &total, bt.sample_weight ? GCS_WORKSPACE_SAMPLE_WEIGHTS : 0);
   if (workspace_bytes < total)
     return fail(GCS_ERR_WORKSPACE, "gcs_model_train_step: workspace %lld < %lld bytes", (long long)workspace_bytes, (long long)total);
   GCS_CHECK_ARG(p.rows_post < INT32_MAX, "gcs_model_train_step: too many output rows");
@@ -794,7 +810,7 @@ extern "C" int gcs_model_train_step(const gcs_model_config* cfg, const float* pa
   GCS_TRY(prepare_step_weights(c, p, params, &prepared, stream));
   PreparedScope prepared_scope(&prepared);
   GCS_TRY(run_forward(c, p, params, state, bt, true, stream));
-  GCS_TRY(head_loss(c, p, bt.y, probs, loss_acc, grad_scale, stream));
+  GCS_TRY(head_loss(c, p, bt.y, probs, loss_acc, grad_scale, stream, bt.sample_weight));
 
   return run_backward(c, p, params, grads, bt, p.dlogits, stream);
 }
@@ -853,7 +869,7 @@ extern "C" int gcs_model_train_step_dp(const gcs_model_config* cfg, const float*
   const gcs_batch& bt = *batch;
   Plan p;
   int64_t total = 0;
-  make_plan(c, bt.n_nodes, bt.n_graphs, true, workspace, p, &total);
+  make_plan(c, bt.n_nodes, bt.n_graphs, true, workspace, p, &total, bt.sample_weight ? GCS_WORKSPACE_SAMPLE_WEIGHTS : 0);
   if (workspace_bytes < total)
     return fail(GCS_ERR_WORKSPACE, "gcs_model_train_step_dp: workspace %lld < %lld bytes", (long long)workspace_bytes, (long long)total);
   GCS_CHECK_ARG(p.rows_post < INT32_MAX, "gcs_model_train_step_dp: too many output rows");
@@ -862,7 +878,7 @@ extern "C" int gcs_model_train_step_dp(const gcs_model_config* cfg, const float*
   GCS_TRY(prepare_step_weights(c, p, params, &prepared, stream));
   PreparedScope prepared_scope(&prepared);
   GCS_TRY(run_forward(c, p, params, state, bt, true, stream));
-  GCS_TRY(head_loss(c, p, bt.y, probs, loss_acc, grad_scale, stream));
+  GCS_TRY(head_loss(c, p, bt.y, probs, loss_acc, grad_scale, stream, bt.sample_weight));
   cudaEvent_t* ev = dp_events();
   DpSync sync{comm, grads, as_stream(stream), as_stream(comm_stream), {}, 0};
   for (int i = 0; i < 8; ++i) sync.ev[i] = ev[i];

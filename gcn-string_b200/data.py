@@ -526,11 +526,18 @@ class DisjointLoader:
     graph across data-parallel ranks (rank r takes the r-th contiguous part of the slice); the adjacency carries the
     global slice's graph and node counts (``a.global_batch_graphs`` / ``a.global_batch_nodes``), the denominators of
     the graph- and node-level mean loss.
+
+    ``sample_weights`` (the name of Spektral's ``SingleLoader`` argument): a host array with one loss weight per graph,
+    or with ``node_level=True`` one per node in dataset order ([n] or [n, 1]).  Iterating then yields
+    ``((x, a, i), y, w)``, w [B] or [N] float32 on the device in batch order, for ``loss_fn(y, pred, sample_weight=w)``
+    or ``train_step_grads(..., sample_weight=w)``.  The weights are kept in HBM in every store mode (4 bytes per row) and
+    gathered per batch by the batch's graph ids: ``index_select`` per graph, ``gcs_gather_node_rows`` at width 1 per
+    node, into buffers of bucketed size.
     """
 
     def __init__(self, dataset, node_level=False, batch_size=1, epochs=None, shuffle=True, rank=0, world_size=1,
                  want_coo=False, symmetric=None, device_resident=True, prefetch=None, balance=None, zero_copy=False,
-                 device_gather=False):
+                 device_gather=False, sample_weights=None):
         node_level = bool(node_level)
         packed = dataset if isinstance(dataset, PackedGraphs) else pack_graphs(list(dataset), node_level=node_level)
         if packed.n_graphs == 0:
@@ -563,6 +570,16 @@ class DisjointLoader:
         self._order_dev = None
         self._order_epoch = -1
         self._ring = _PinnedRing(depth=4)
+        self._w, self._w_node_off = None, None
+        if sample_weights is not None:
+            torch = _lib.require_cuda()
+            rows = int(packed.node_off[-1]) if node_level else packed.n_graphs
+            w = np.asarray(sample_weights, dtype=np.float32)
+            ops.check_sample_weight_shape(w.shape, rows)
+            self._w = torch.from_numpy(np.ascontiguousarray(w.reshape(rows))).cuda()
+            if node_level:
+                self._w_node_off = (self.store.node_off if device_resident
+                                    else torch.from_numpy(np.ascontiguousarray(packed.node_off)).cuda())
         self._generator = self._generate()
 
     @property
@@ -588,8 +605,9 @@ class DisjointLoader:
     def tf_signature(self):
         """Shape/dtype contract of one batch (gcn.py:328): dynamic N, nnz, B."""
         f, c = self.store.n_feat, self.store.n_classes
-        return ((_Spec((None, f), "float32"), _Spec((None, None), "int64", sparse=True), _Spec((None,), "int64")),
+        spec = ((_Spec((None, f), "float32"), _Spec((None, None), "int64", sparse=True), _Spec((None,), "int64")),
                 _Spec((None, c), "float32"))
+        return spec + ((_Spec((None,), "float32"),) if self._w is not None else ())
 
     def _slices_of_rank(self, start, stop):
         """This rank's contiguous part of the global slice [start, stop)."""
@@ -643,31 +661,45 @@ class DisjointLoader:
                 ids_dev = self._order_dev[lo:hi]
             staged = None
             x, a, i, y = self.store.batch(ids_dev, ids_host, want_coo=self.want_coo)
+            w = self._batch_weights(ids_dev, a) if self._w is not None else None
             a.global_batch_graphs = global_count
             a.global_batch_nodes = global_nodes
             a._ids_keepalive = (ids_dev, staged)
             event = torch.cuda.Event()
             event.record(stream)
-        return (x, a, i, y), event
+        return (x, a, i, y, w), event
+
+    def _batch_weights(self, ids_dev, a):
+        """The batch's sample weights in batch order: the weights of its graphs, or of its nodes graph after graph at
+        the offsets the batching kernel wrote (a.graph_ptr)."""
+        torch = _lib.require_cuda()
+        b = int(ids_dev.shape[0])
+        if not self.node_level:
+            w = torch.empty(b, dtype=torch.float32, device="cuda")
+            return torch.index_select(self._w, 0, ids_dev, out=w)
+        w = ops.empty_bucketed(a.n_rows, dtype=torch.float32)
+        check(_lib.load().gcs_gather_node_rows(ptr(ids_dev), b, ptr(self._w_node_off), ptr(self._w), 1, ptr(a.graph_ptr),
+                                               ptr(w), stream_ptr()), "gcs_gather_node_rows")
+        return w
 
     def _generate(self):
         torch = _lib.require_cuda()
         it = self._slices()
         if not self.prefetch:
             for item in it:
-                (x, a, i, y), _ = self._launch(item, torch.cuda.current_stream())
-                yield (x, a, i), y
+                (x, a, i, y, w), _ = self._launch(item, torch.cuda.current_stream())
+                yield ((x, a, i), y, w) if w is not None else ((x, a, i), y)
             return
         side = torch.cuda.Stream()
         first = next(it, None)
         pending = self._launch(first, side) if first is not None else None
         while pending is not None:
-            (x, a, i, y), event = pending
+            (x, a, i, y, w), event = pending
             nxt = next(it, None)
             pending = self._launch(nxt, side) if nxt is not None else None      # step t+1 in flight
             main = torch.cuda.current_stream()
             main.wait_event(event)
-            for t in (x, i, y, a.rowptr, a.colidx, a.graph_ptr, a.edge_ptr, a.status, a._indices):
+            for t in (x, i, y, w, a.rowptr, a.colidx, a.graph_ptr, a.edge_ptr, a.status, a._indices):
                 if t is not None:
                     t.record_stream(main)       # allocated on the side stream, consumed on the main one
-            yield (x, a, i), y
+            yield ((x, a, i), y, w) if w is not None else ((x, a, i), y)

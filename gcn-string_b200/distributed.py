@@ -169,7 +169,9 @@ class DataParallelTrainer:
         finally:
             _lib.set_allreduce_hook(None)
 
-    def train_step(self, inputs, target, global_batch: Optional[int] = None):
+    def train_step(self, inputs, target, global_batch: Optional[int] = None, sample_weight=None):
+        """One step; ``sample_weight`` ([rows] or [rows, 1]): this rank's per-row loss weights.  With the 1/global_batch
+        scaling the summed gradient is that of sum w l / global_batch, Keras' weighted mean over the global batch."""
         rank, ws = world()
         if not self.model.built:                  # build before the first step: a dry run would move the BatchNorm statistics
             from . import _lib
@@ -184,10 +186,10 @@ class DataParallelTrainer:
             global_batch = getattr(a, key, None) or target.shape[0] * ws
         if self.comm is not None:                 # the library's own communicator: collectives (and synchronised BatchNorm) per call
             loss_acc, probs = self.model.train_step_grads(inputs, target, grad_scale=1.0 / float(global_batch), comm=self.comm,
-                                                          sync_bn=self.sync_bn, loss=self.loss)
+                                                          sync_bn=self.sync_bn, loss=self.loss, sample_weight=sample_weight)
         else:
             step = lambda: self.model.train_step_grads(inputs, target, grad_scale=1.0 / float(global_batch),   # noqa: E731
-                                                       loss=self.loss)
+                                                       loss=self.loss, sample_weight=sample_weight)
             loss_acc, probs = self._hooked(step)
         if self.comm is None:
             allreduce_gradients(self.model.grads, self.group)

@@ -24,7 +24,9 @@ def evaluate(model, loader, loss_fn=None, metric=None):
     Mirrors gcn.py:342-362; the only host transfers are the two scalars per batch.  The loss and accuracy default to
     BinaryCrossentropy / binary_accuracy for a model built with activation='sigmoid', to CategoricalCrossentropy /
     categorical_accuracy otherwise.  ``metric(y_true, y_pred)`` -> per-row values replaces the accuracy; with a
-    regression ``loss_fn`` (MeanSquaredError, MeanAbsoluteError, Huber) it defaults to mean_absolute_error."""
+    regression ``loss_fn`` (MeanSquaredError, MeanAbsoluteError, Huber) it defaults to mean_absolute_error.
+    A loader that yields ``(inputs, y, w)`` (DisjointLoader(sample_weights=...)) gives the weighted figures: the loss
+    is the sum over the pass of w * l over the total number of rows, the metric sum w * m / sum w (0 when sum w = 0)."""
     torch = _lib.require_cuda()
     sigmoid = getattr(model, "config", {}).get("activation") == "sigmoid"
     if metric is None and isinstance(loss_fn, (MeanSquaredError, MeanAbsoluteError, Huber)):
@@ -32,16 +34,29 @@ def evaluate(model, loader, loss_fn=None, metric=None):
     loss_fn = loss_fn or (BinaryCrossentropy() if sigmoid else CategoricalCrossentropy())
     metric = metric or (binary_accuracy if sigmoid else categorical_accuracy)
     stats, preds = [], []
+    weighted = False
     step = 0
     while step < loader.steps_per_epoch:
         step += 1
-        inputs, target = next(loader)
+        inputs, target, *w = next(loader)
         pred = model(inputs, training=False)
         preds.append(pred)
-        stats.append(torch.stack([loss_fn(target, pred).reshape(()), metric(target, pred).mean().reshape(()),
-                                  torch.tensor(float(target.shape[0]), device=pred.device)]))
+        rows = torch.tensor(float(target.shape[0]), device=pred.device)
+        if w:
+            weighted = True
+            w = w[0].reshape(-1).to(torch.float32)
+            loss = loss_fn(target, pred, sample_weight=w)
+            m = metric(target, pred).reshape(-1)
+            stats.append(torch.stack([loss.reshape(()), (w * m).sum(), w.sum(), rows]))
+        else:
+            stats.append(torch.stack([loss_fn(target, pred).reshape(()), metric(target, pred).mean().reshape(()), rows,
+                                      rows]))
     out = torch.stack(stats).cpu().numpy().astype(np.float64)
-    return np.average(out[:, :-1], 0, weights=out[:, -1]), preds
+    if not weighted:
+        return np.average(out[:, [0, 1]], 0, weights=out[:, -1]), preds
+    loss = np.average(out[:, 0], weights=out[:, -1])
+    wsum = out[:, 2].sum()
+    return np.array([loss, out[:, 1].sum() / wsum if wsum != 0 else 0.0]), preds
 
 
 def positive_scores(preds, column: int = 1):
@@ -59,14 +74,23 @@ def _as_torch(a, like=None):
     return t.to(like.device) if like is not None else t
 
 
-def roc_curve(y_true, y_score, drop_intermediate: bool = True):
+def roc_curve(y_true, y_score, drop_intermediate: bool = True, sample_weight=None):
     """``sklearn.metrics.roc_curve`` for binary labels in {0, 1} (positive = 1): returns
-    (fpr, tpr, thresholds) as NumPy arrays.  Sort and prefix sums run on the scores' device."""
+    (fpr, tpr, thresholds) as NumPy arrays.  Sort and prefix sums run on the scores' device.  ``sample_weight`` (one
+    per sample) as in scikit-learn: samples of weight 0 are left out, and the true and false positives are the
+    cumulative weights of the positive and negative samples."""
     import torch
     s = _as_torch(y_score).reshape(-1).to(torch.float64)
     y = _as_torch(y_true, like=s).reshape(-1).to(s.device).to(torch.float64)
     if y.shape[0] != s.shape[0]:
         raise ValueError(f"y_true has {y.shape[0]} entries, y_score {s.shape[0]}")
+    w = None
+    if sample_weight is not None:
+        w = _as_torch(sample_weight, like=s).reshape(-1).to(s.device).to(torch.float64)
+        if w.shape[0] != s.shape[0]:
+            raise ValueError(f"sample_weight has {w.shape[0]} entries, y_score {s.shape[0]}")
+        keep = w != 0
+        s, y, w = s[keep], y[keep], w[keep]
     if y.shape[0] == 0:
         raise ValueError("roc_curve needs at least one sample")
     order = torch.argsort(s, descending=True, stable=True)
@@ -74,8 +98,13 @@ def roc_curve(y_true, y_score, drop_intermediate: bool = True):
     n = s.shape[0]
     distinct = torch.nonzero(s[1:] != s[:-1]).reshape(-1)
     idx = torch.cat([distinct, torch.tensor([n - 1], device=s.device)])
-    tps = torch.cumsum(y, 0)[idx]
-    fps = (1 + idx).to(torch.float64) - tps
+    if w is None:
+        tps = torch.cumsum(y, 0)[idx]
+        fps = (1 + idx).to(torch.float64) - tps
+    else:
+        w = w[order]
+        tps = torch.cumsum(y * w, 0)[idx]
+        fps = torch.cumsum((1 - y) * w, 0)[idx]
     thr = s[idx]
     if drop_intermediate and idx.shape[0] > 2:
         d2f, d2t = torch.diff(fps, n=2), torch.diff(tps, n=2)

@@ -11,10 +11,42 @@ of csrc/loss.cu.
 
 ``MeanSquaredError``, ``MeanAbsoluteError`` and ``Huber`` are the Keras regression losses for the linear head of a
 default ``GeneralGNN(C)`` (activation=None); with ``mean_squared_error`` / ``mean_absolute_error`` they run the fused
-kernel of csrc/loss.cu."""
+kernel of csrc/loss.cu.
+
+Every loss takes Keras' ``sample_weight``: one weight per row (``[rows]`` or ``[rows, 1]``), with the default
+"sum_over_batch_size" reduction, so the loss is sum_r w_r l_r / rows (the number of rows, not sum w).  The fused paths
+run the weighted kernel (gcs_weighted_loss); the host fallbacks weight the same way in torch."""
 from __future__ import annotations
 
 from . import _lib, ops
+
+
+def _weighted_mean(per_row, sample_weight):
+    """Keras' "sum_over_batch_size" reduction of the per-row losses: sum(w * l) / rows (plain mean without weights)."""
+    if sample_weight is None:
+        return per_row.mean()
+    import torch
+    w = sample_weight if isinstance(sample_weight, torch.Tensor) else torch.as_tensor(sample_weight)
+    ops.check_sample_weight_shape(w.shape, per_row.shape[0])
+    w = w.to(device=per_row.device, dtype=per_row.dtype).reshape(-1)
+    return (w * per_row).sum() / per_row.shape[0]
+
+
+def categorical_crossentropy_from_probs(y, p, sample_weight=None):
+    """Keras' loss on probabilities of unknown origin: normalise, clip to [1e-7, 1 - 1e-7], -sum y log p per row, then
+    the (weighted) mean over the rows.  Runs on the tensors' device."""
+    p = p / p.sum(dim=-1, keepdim=True)
+    p = p.clamp(1e-7, 1.0 - 1e-7)
+    return _weighted_mean(-(y * p.log()).sum(dim=-1), sample_weight)
+
+
+def binary_crossentropy_from_probs(y, p, sample_weight=None):
+    """Keras' binary cross-entropy on probabilities: clip, -(y log(p + eps) + (1 - y) log(1 - p + eps)), the mean over
+    the last axis, then the (weighted) mean over the rows.  Runs on the tensors' device."""
+    eps = 1e-7
+    p = p.clamp(eps, 1.0 - eps)
+    bce = y * (p + eps).log() + (1.0 - y) * (1.0 - p + eps).log()
+    return _weighted_mean((-bce).mean(dim=-1), sample_weight)
 
 
 class CategoricalCrossentropy:
@@ -24,17 +56,15 @@ class CategoricalCrossentropy:
         self.from_logits = from_logits
         self.name = name
 
-    def __call__(self, y_true, y_pred):
+    def __call__(self, y_true, y_pred, sample_weight=None):
         torch = _lib.require_cuda()
         y = _lib.as_tensor(y_true).to(device="cuda", dtype=torch.float32)
         logits = y_pred if self.from_logits else getattr(y_pred, "_gcs_logits", None)
         if logits is None:
             # probabilities of unknown origin: Keras' fallback (normalise, clip, -sum y log p)
-            p = y_pred / y_pred.sum(dim=-1, keepdim=True)
-            p = p.clamp(1e-7, 1.0 - 1e-7)
-            return -(y * p.log()).sum(dim=-1).mean()
+            return categorical_crossentropy_from_probs(y, y_pred, sample_weight)
         tape = getattr(y_pred, "_gcs_tape", None)
-        _, loss_acc, dlogits = ops.softmax_xent(logits, y, want_grad=tape is not None)
+        _, loss_acc, dlogits = ops.softmax_xent(logits, y, want_grad=tape is not None, sample_weight=sample_weight)
         loss = loss_acc[0]
         if tape is not None:
             tape.loss_record = dict(dlogits=dlogits, loss_acc=loss_acc)
@@ -63,7 +93,7 @@ class BinaryCrossentropy:
         self.from_logits = from_logits
         self.name = name
 
-    def __call__(self, y_true, y_pred):
+    def __call__(self, y_true, y_pred, sample_weight=None):
         torch = _lib.require_cuda()
         y = _lib.as_tensor(y_true).to(device="cuda", dtype=torch.float32)
         if self.from_logits:
@@ -72,12 +102,9 @@ class BinaryCrossentropy:
             logits = y_pred._gcs_logits
         else:
             # probabilities of unknown origin: Keras' fallback (clip, then -(y log(p + eps) + (1 - y) log(1 - p + eps)))
-            eps = 1e-7
-            p = y_pred.clamp(eps, 1.0 - eps)
-            bce = y * (p + eps).log() + (1.0 - y) * (1.0 - p + eps).log()
-            return (-bce).mean(dim=-1).mean()
+            return binary_crossentropy_from_probs(y, y_pred, sample_weight)
         tape = getattr(y_pred, "_gcs_tape", None)
-        _, loss_acc, dlogits = ops.sigmoid_bce(logits, y, want_grad=tape is not None)
+        _, loss_acc, dlogits = ops.sigmoid_bce(logits, y, want_grad=tape is not None, sample_weight=sample_weight)
         if tape is not None:
             tape.loss_record = dict(dlogits=dlogits, loss_acc=loss_acc)
         return loss_acc[0]
@@ -105,7 +132,7 @@ class _RegressionLoss:
         self.name = name
         self.delta = float(delta)
 
-    def __call__(self, y_true, y_pred):
+    def __call__(self, y_true, y_pred, sample_weight=None):
         torch = _lib.require_cuda()
         y = _lib.as_tensor(y_true).to(device="cuda", dtype=torch.float32)
         linear = getattr(y_pred, "_gcs_activation", None) in (None, "linear")
@@ -114,7 +141,8 @@ class _RegressionLoss:
         if tape is not None and not linear:
             raise NotImplementedError(f"{type(self).__name__} is built for a linear head (activation=None); the model's "
                                       f"output has activation={y_pred._gcs_activation!r}")
-        loss_acc, dlogits = ops.regression_loss(pred, y, self.kind, self.delta, want_grad=tape is not None)
+        loss_acc, dlogits = ops.regression_loss(pred, y, self.kind, self.delta, want_grad=tape is not None,
+                                                sample_weight=sample_weight)
         if tape is not None:
             tape.loss_record = dict(dlogits=dlogits, loss_acc=loss_acc)
         return loss_acc[0]

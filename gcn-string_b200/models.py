@@ -242,7 +242,8 @@ class GeneralGNN:
     def _workspace(self, batch, training):
         torch = _lib.require_cuda()
         lib = _lib.load()
-        need = lib.gcs_model_workspace_bytes(self._c, batch.n_nodes, batch.nnz, batch.n_graphs, int(training))
+        flags = _lib.WORKSPACE_SAMPLE_WEIGHTS if batch.sample_weight else 0
+        need = lib.gcs_model_workspace_bytes_ex(self._c, batch.n_nodes, batch.nnz, batch.n_graphs, int(training), flags)
         if need < 0:
             raise RuntimeError("gcs_model_workspace_bytes failed: " + lib.gcs_last_error().decode())
         if self._ws is None or self._ws.numel() < need:
@@ -281,7 +282,7 @@ class GeneralGNN:
                                      ptr(ctx["ws"]), ctx["ws"].numel(), stream_ptr()), "gcs_model_backward")
 
     def train_step_grads(self, inputs, target, grad_scale: Optional[float] = None, comm=None, sync_bn: bool = False,
-                         loss=None):
+                         loss=None, sample_weight=None):
         """Fused training-mode forward + loss + backward (one C call): categorical cross-entropy with
         activation='softmax', binary cross-entropy (mean over the C columns, then the rows) with activation='sigmoid',
         and with the linear head (activation=None) the regression loss ``loss`` - ``MeanSquaredError()`` (the default),
@@ -291,7 +292,10 @@ class GeneralGNN:
         head).  ``grad_scale`` defaults to 1/B (mean loss, gcn.py:335).
         ``comm`` (distributed.NativeComm): the data-parallel form - the gradients are SUM all-reduced over the
         communicator, bucket by bucket on its own stream while the backward is still running
-        (gcs_model_train_step_dp); the current stream waits for the reductions."""
+        (gcs_model_train_step_dp); the current stream waits for the reductions.
+        ``sample_weight`` ([rows] or [rows, 1], one weight per graph - per node without pooling): Keras' per-row loss
+        weights; the loss is sum w l / rows, the metric the weighted mean, and each row's gradient is scaled by its
+        weight."""
         torch = _lib.require_cuda()
         lib = _lib.load()
         code, delta = fused_loss_fields(loss, self.config["activation"])
@@ -306,6 +310,8 @@ class GeneralGNN:
         if tuple(y.shape) != (rows, self.cfg.output):
             raise ValueError(f"target must be [{rows}, {self.cfg.output}], got {tuple(y.shape)}")
         batch.y = ptr(y)
+        w = ops.sample_weight_vector(sample_weight, rows) if sample_weight is not None else None
+        batch.sample_weight = ptr(w)
         ws = self._workspace(batch, True)
         probs = torch.empty(rows, self.cfg.output, dtype=torch.float32, device="cuda")
         loss_acc = torch.empty(2, dtype=torch.float32, device="cuda")
@@ -318,5 +324,5 @@ class GeneralGNN:
             check(lib.gcs_model_train_step(c, ptr(self.params), ptr(self.state), batch, gs, ptr(self.grads),
                                            ptr(probs), ptr(loss_acc), ptr(ws), ws.numel(), stream_ptr()),
                   "gcs_model_train_step")
-        self._keep = (keep, y)
+        self._keep = (keep, y, w)
         return loss_acc, probs

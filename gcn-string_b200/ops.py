@@ -539,10 +539,34 @@ def attn_sum_pool_bwd(dout, x, kernel, graph_ptr, out, scores, gstats, dx=None):
 
 
 # ------------------------------------------------------------------ loss (K5) / optimizers (K10)
-def _head_loss(entry, ws_bytes, logits, y, grad_scale, want_grad, want_probs=True, args=(), name="logits"):
+def check_sample_weight_shape(shape, rows: int) -> None:
+    """Raises ValueError unless ``shape`` is Keras' per-row weight shape: ``[rows]`` or ``[rows, 1]``."""
+    shape = tuple(int(d) for d in shape)
+    if shape not in ((rows,), (rows, 1)):
+        raise ValueError(f"sample_weight must be [{rows}] or [{rows}, 1] (one weight per row), got {list(shape)}")
+
+
+def sample_weight_vector(sample_weight, rows: int):
+    """``sample_weight`` (any array-like or tensor of shape [rows] or [rows, 1]) as a contiguous float32 [rows] CUDA
+    tensor; the shape is checked before anything is copied."""
+    torch = _t()
+    w = sample_weight
+    if not isinstance(w, torch.Tensor):
+        w = as_tensor(w) if hasattr(w, "__dlpack__") and not isinstance(w, np.ndarray) else torch.as_tensor(np.asarray(w))
+    check_sample_weight_shape(w.shape, rows)
+    return w.reshape(rows).to(device="cuda", dtype=torch.float32).contiguous()
+
+
+# gcs_weighted_loss's head codes (gcs_model_config.final_activation) of the unweighted entry points
+_WEIGHTED_HEAD = {"gcs_softmax_xent_ws": 1, "gcs_sigmoid_bce": 2, "gcs_regression_loss": 0}
+
+
+def _head_loss(entry, ws_bytes, logits, y, grad_scale, want_grad, want_probs=True, args=(), name="logits",
+               sample_weight=None):
     """Shared body of the loss wrappers: returns (probs, loss_acc[2] or None, dlogits or None) of
     ``lib.<entry>(*args, logits, y, rows, C, probs, loss_acc, dlogits, grad_scale, workspace, bytes, stream)``, with y
-    checked to have the shape of the logits and ``grad_scale`` defaulting to 1 / rows."""
+    checked to have the shape of the logits and ``grad_scale`` defaulting to 1 / rows.  With ``sample_weight`` the same
+    head runs through gcs_weighted_loss."""
     torch = _t()
     lib = _lib.load()
     logits, _ = _mat(logits, name)
@@ -553,44 +577,63 @@ def _head_loss(entry, ws_bytes, logits, y, grad_scale, want_grad, want_probs=Tru
         if tuple(y.shape) != (b, c):
             raise ValueError(f"y must be [{b}, {c}], got {tuple(y.shape)}")
         y = y.contiguous()
+    if sample_weight is not None:
+        if y is None:
+            raise ValueError("sample_weight needs the labels y")
+        sample_weight = sample_weight_vector(sample_weight, b)
     probs = torch.empty_like(logits) if want_probs else None
     loss_acc = torch.empty(2, dtype=torch.float32, device="cuda") if y is not None else None
     dlogits = torch.empty_like(logits) if (want_grad and y is not None) else None
     gs = (1.0 / b if b else 0.0) if grad_scale is None else grad_scale
-    nbytes = int(getattr(lib, ws_bytes)(b, c))
+    if sample_weight is None:
+        nbytes = int(getattr(lib, ws_bytes)(b, c))
+    else:
+        head = _WEIGHTED_HEAD[entry]
+        nbytes = int(lib.gcs_weighted_loss_workspace_bytes(head, b, c))
     ws = torch.empty(nbytes, dtype=torch.uint8, device="cuda") if nbytes > 0 else None
-    check(getattr(lib, entry)(*args, ptr(logits), ptr(y), b, c, ptr(probs), ptr(loss_acc), ptr(dlogits), gs, ptr(ws),
-                              nbytes, stream_ptr()), entry)
+    if sample_weight is None:
+        check(getattr(lib, entry)(*args, ptr(logits), ptr(y), b, c, ptr(probs), ptr(loss_acc), ptr(dlogits), gs, ptr(ws),
+                                  nbytes, stream_ptr()), entry)
+    else:
+        kind, delta = args if args else (0, 1.0)
+        check(lib.gcs_weighted_loss(head, kind, delta, ptr(logits), ptr(y), ptr(sample_weight), b, c, ptr(probs),
+                                    ptr(loss_acc), ptr(dlogits), gs, ptr(ws), nbytes, stream_ptr()), "gcs_weighted_loss")
     return probs, loss_acc, dlogits
 
 
-def softmax_xent(logits, y=None, grad_scale: Optional[float] = None, want_grad=False):
+def softmax_xent(logits, y=None, grad_scale: Optional[float] = None, want_grad=False, sample_weight=None):
     """Returns (probs, loss_acc[2] or None, dlogits or None).  gcs_softmax_xent_ws: one thread block up to 65 536 rows,
-    a grid above - the same rule as the model's fused train step, so both give the same bits."""
-    return _head_loss("gcs_softmax_xent_ws", "gcs_softmax_xent_workspace_bytes", logits, y, grad_scale, want_grad)
+    a grid above - the same rule as the model's fused train step, so both give the same bits.  ``sample_weight``
+    ([rows] or [rows, 1]): Keras' per-row weights, through gcs_weighted_loss (loss = sum w l / rows, accuracy = the
+    weighted mean, dlogits scaled per row)."""
+    return _head_loss("gcs_softmax_xent_ws", "gcs_softmax_xent_workspace_bytes", logits, y, grad_scale, want_grad,
+                      sample_weight=sample_weight)
 
 
-def sigmoid_bce(logits, y=None, grad_scale: Optional[float] = None, want_grad=False):
+def sigmoid_bce(logits, y=None, grad_scale: Optional[float] = None, want_grad=False, sample_weight=None):
     """Returns (probs, loss_acc[2] or None, dlogits or None) of gcs_sigmoid_bce: probs = sigmoid(logits), loss_acc =
     {binary cross-entropy (mean over the columns, then the rows), binary accuracy}, dlogits = (probs - y) * grad_scale / C
-    (``grad_scale`` defaults to 1 / rows)."""
-    return _head_loss("gcs_sigmoid_bce", "gcs_sigmoid_bce_workspace_bytes", logits, y, grad_scale, want_grad)
+    (``grad_scale`` defaults to 1 / rows).  ``sample_weight`` as in softmax_xent."""
+    return _head_loss("gcs_sigmoid_bce", "gcs_sigmoid_bce_workspace_bytes", logits, y, grad_scale, want_grad,
+                      sample_weight=sample_weight)
 
 
 REGRESSION_KIND = {"mse": 1, "mae": 2, "huber": 3}
 
 
-def regression_loss(pred, y, loss: str = "mse", delta: float = 1.0, want_grad=False, grad_scale: Optional[float] = None):
+def regression_loss(pred, y, loss: str = "mse", delta: float = 1.0, want_grad=False, grad_scale: Optional[float] = None,
+                    sample_weight=None):
     """Returns (loss_acc[2], dlogits or None) of gcs_regression_loss on the predictions of a linear head: loss_acc =
     {``loss`` ('mse', 'mae' or 'huber' with ``delta``; mean over the columns, then the rows), mean absolute error},
-    dlogits = dLoss/dpred * grad_scale / C (``grad_scale`` defaults to 1 / rows)."""
+    dlogits = dLoss/dpred * grad_scale / C (``grad_scale`` defaults to 1 / rows).  ``sample_weight`` as in
+    softmax_xent."""
     if loss not in REGRESSION_KIND:
         raise ValueError(f"loss must be one of {sorted(REGRESSION_KIND)}, got {loss!r}")
     if y is None:
         raise TypeError("regression_loss needs the targets y")
     _, loss_acc, dlogits = _head_loss("gcs_regression_loss", "gcs_regression_loss_workspace_bytes", pred, y, grad_scale,
                                       want_grad, want_probs=False, args=(REGRESSION_KIND[loss], float(delta)),
-                                      name="pred")
+                                      name="pred", sample_weight=sample_weight)
     return loss_acc, dlogits
 
 

@@ -343,6 +343,27 @@ int gcs_regression_loss(int32_t kind, float huber_delta, const float* pred, cons
                         int64_t workspace_bytes, gcs_stream stream);
 
 /* ---------------------------------------------------------------------------------
+ * K5d  The three heads above with one weight per row: Keras' loss(y, pred, sample_weight=w) with the default
+ * "sum_over_batch_size" reduction, and the sample-weighted metric.  head: 1 = softmax + categorical cross-entropy
+ * (C <= 64), 2 = sigmoid + binary cross-entropy, 0 = linear head with the regression loss `kind` (1 = MSE, 2 = MAE,
+ * 3 = Huber with huber_delta; kind is ignored for the other heads).  sample_weight [rows] (device, required: the entry
+ * points above are the unweighted path) may hold any finite values, 0 included; nothing is validated on the device.
+ * With l_r the row loss and m_r the row metric of the unweighted entry point:
+ *   loss_acc[0] = sum_r w_r l_r / rows   (divided by the row count, not by sum w);
+ *   loss_acc[1] = sum_r w_r m_r / sum_r w_r, 0 when sum w = 0;
+ *   dlogits     = w_r * (the unweighted dlogits of row r), so grad_scale keeps its meaning (1/rows, 1/global_rows).
+ * probs as the unweighted entry point.  With every weight 1, loss_acc[0], probs and dlogits are bit-identical to the
+ * unweighted entry point's, and loss_acc[1] is within one float ulp.  The grid follows the unweighted rule (rows alone
+ * for the softmax, rows * C otherwise), so results are bit-identical run to run.  workspace:
+ * gcs_weighted_loss_workspace_bytes(head, rows, C) bytes, 8-byte aligned (24 bytes per block of the grid; only read
+ * when loss_acc != NULL).
+ * --------------------------------------------------------------------------------- */
+int64_t gcs_weighted_loss_workspace_bytes(int32_t head, int64_t rows, int32_t C);
+int gcs_weighted_loss(int32_t head, int32_t kind, float huber_delta, const float* logits, const float* y,
+                      const float* sample_weight, int64_t rows, int32_t C, float* probs, float* loss_acc,
+                      float* dlogits, float grad_scale, void* workspace, int64_t workspace_bytes, gcs_stream stream);
+
+/* ---------------------------------------------------------------------------------
  * K11  Residue contact maps of a batch of chains (SURVEY.md 8 f4).  Replaces
  * GraphMaker.calculate_residue_dist / calculate_dist_matrix / generate_proximity_matrix
  * (src/utilities/gcn_utills.py:161-238): d = sqrt(sum((ca_i - ca_j)^2)) in float32 with NumPy's operation order
@@ -451,6 +472,9 @@ typedef struct gcs_batch {
   const float* values;          /* optional per-entry weights w_ij in CSR order (the `use_edge_data` switch of gcn.py:73-80);
                                    NULL = pattern only, as GeneralConv aggregates */
   const float* values_t;        /* the same weights in the order of (rowptr_t, colidx_t); backward only */
+  const float* sample_weight;   /* [rows_post] one loss weight per output row (per graph, or per node when pool == 0),
+                                   read by the train steps (gcs_weighted_loss); NULL = unweighted.  The workspace must
+                                   then be sized with GCS_WORKSPACE_SAMPLE_WEIGHTS.  gcs_model_forward ignores it. */
 } gcs_batch;
 
 /* Number of floats in the flat trainable / state buffers (layout: gcn-string_b200/params.py). */
@@ -458,6 +482,12 @@ int64_t gcs_model_num_params(const gcs_model_config* cfg);
 int64_t gcs_model_num_state(const gcs_model_config* cfg);
 int64_t gcs_model_workspace_bytes(const gcs_model_config* cfg, int64_t n_nodes, int64_t nnz,
                                   int32_t n_graphs, int32_t training);
+/* The same with flags: GCS_WORKSPACE_SAMPLE_WEIGHTS sizes the plan for a batch with sample_weight set.  Only the last
+ * slot of the plan (the loss partials) grows, so every other offset - gcs_model_logits_offset included - is the
+ * unweighted plan's.  flags = 0 is gcs_model_workspace_bytes; unknown bits give -1. */
+#define GCS_WORKSPACE_SAMPLE_WEIGHTS 1
+int64_t gcs_model_workspace_bytes_ex(const gcs_model_config* cfg, int64_t n_nodes, int64_t nnz, int32_t n_graphs,
+                                     int32_t training, int32_t flags);
 /* Inference / training-mode forward.  out: [B, C] (or [N, C] when pool == 0), after the final activation.  With
  * training != 0 BatchNorm uses batch statistics and updates `state` in place. */
 int gcs_model_forward(const gcs_model_config* cfg, const float* params, float* state,
@@ -472,7 +502,10 @@ int gcs_model_forward(const gcs_model_config* cfg, const float* params, float* s
  * cross-entropy, binary accuracy}, and grad_scale keeps its meaning (the 1/C of the per-row mean is applied inside).
  * With final_activation = 0 (linear) the loss is the regression loss cfg->loss selects (0 or 1 = MSE, 2 = MAE, 3 =
  * Huber with cfg->huber_delta) through gcs_regression_loss: probs = the predictions (the logits), loss_acc = {mean
- * loss, mean absolute error}, and grad_scale keeps its meaning the same way. */
+ * loss, mean absolute error}, and grad_scale keeps its meaning the same way.  With batch->sample_weight set, every head
+ * runs through gcs_weighted_loss instead (loss = sum w l / rows, the weighted mean metric, dlogits scaled per row), and
+ * the workspace must be gcs_model_workspace_bytes_ex(..., GCS_WORKSPACE_SAMPLE_WEIGHTS) bytes: with less the call
+ * fails with GCS_ERR_WORKSPACE. */
 int gcs_model_train_step(const gcs_model_config* cfg, const float* params, float* state,
                          const gcs_batch* batch, float grad_scale, float* grads, float* probs,
                          float* loss_acc, void* workspace, int64_t workspace_bytes,
