@@ -36,6 +36,14 @@ class Batch(Structure):
                 ("sample_weight", c_void_p)]
 
 
+class GradClip(Structure):
+    """gcs_grad_clip: clipping options and the device chunk table of one optimizer call."""
+    _fields_ = [("mode", c_int32), ("clipvalue", c_float), ("clipnorm", c_float), ("n_chunks", c_int32),
+                ("chunks", c_void_p), ("partials", c_void_p), ("chunk_base", c_int32), ("n_partials", c_int32)]
+
+
+CLIP_VALUE, CLIP_NORM, CLIP_GLOBAL_NORM, CLIP_PARTIALS_READY = 1, 2, 4, 8     # gcs_clip_mode
+
 P = c_void_p
 I32, I64, F32, F64 = c_int32, c_int64, c_float, ctypes.c_double
 
@@ -95,6 +103,9 @@ PROTOTYPES = {
     "gcs_weighted_loss": (c_int32, [I32, I32, F32, P, P, P, I64, I32, P, P, P, F32, P, I64, P]),
     "gcs_sgd_step": (c_int32, [P, P, I64, F32, F32, P]),
     "gcs_adam_step": (c_int32, [P, P, P, P, I64, F64, F64, F64, F64, I64, F32, P]),
+    "gcs_sgd_step_ex": (c_int32, [P, P, P, I64, F32, F32, I32, F32, POINTER(GradClip), P]),
+    "gcs_adam_step_ex": (c_int32, [P, P, P, P, P, I64, F64, F64, F64, F64, I64, F32, POINTER(GradClip), P]),
+    "gcs_grad_clip_partials": (c_int32, [P, I64, F32, POINTER(GradClip), P]),
     "gcs_comm_unique_id": (c_int32, [P]),
     "gcs_comm_init": (c_int32, [P, I32, I32, POINTER(c_void_p)]),
     "gcs_comm_destroy": (c_int32, [P]),

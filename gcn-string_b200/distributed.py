@@ -193,5 +193,5 @@ class DataParallelTrainer:
             loss_acc, probs = self._hooked(step)
         if self.comm is None:
             allreduce_gradients(self.model.grads, self.group)
-        self.optimizer.apply_flat(self.model.params, self.model.grads)
+        self.optimizer.apply_flat(self.model.params, self.model.grads, variables=self.model.trainable_variables)
         return loss_acc, probs

@@ -646,3 +646,31 @@ def adam_step(w, g, m, v, step: int, lr: float, beta1=0.9, beta2=0.999, eps=1e-7
     lib = _lib.load()
     check(lib.gcs_adam_step(ptr(w), ptr(g), ptr(m), ptr(v), w.numel(), lr, beta1, beta2, eps, step, grad_scale,
                             stream_ptr()), "gcs_adam_step")
+
+
+def sgd_step_ex(w, g, accum, lr: float, momentum: float = 0.0, nesterov: bool = False, grad_scale: float = 1.0,
+                clip=None):
+    """gcs_sgd_step_ex: SGD with momentum (slot ``accum``, None for momentum 0) or Nesterov, and the clipping options
+    of ``clip`` (a ``_lib.GradClip`` whose chunk table and partials are already on the device, or None)."""
+    import ctypes
+    lib = _lib.load()
+    check(lib.gcs_sgd_step_ex(ptr(w), ptr(g), ptr(accum), w.numel(), lr, momentum, int(bool(nesterov)), grad_scale,
+                              None if clip is None else ctypes.byref(clip), stream_ptr()), "gcs_sgd_step_ex")
+
+
+def adam_step_ex(w, g, m, v, vhat, step: int, lr: float, beta1=0.9, beta2=0.999, eps=1e-7, grad_scale: float = 1.0,
+                 clip=None):
+    """gcs_adam_step_ex: Adam, amsgrad when ``vhat`` is given, with the clipping options of ``clip`` (as sgd_step_ex)."""
+    import ctypes
+    lib = _lib.load()
+    check(lib.gcs_adam_step_ex(ptr(w), ptr(g), ptr(m), ptr(v), ptr(vhat), w.numel(), lr, beta1, beta2, eps, step,
+                               grad_scale, None if clip is None else ctypes.byref(clip), stream_ptr()),
+          "gcs_adam_step_ex")
+
+
+def grad_clip_partials(g, clip, grad_scale: float = 1.0):
+    """gcs_grad_clip_partials: the norm pass alone (per-chunk fp64 sums of squares into ``clip.partials``)."""
+    import ctypes
+    lib = _lib.load()
+    check(lib.gcs_grad_clip_partials(ptr(g), g.numel(), grad_scale, ctypes.byref(clip), stream_ptr()),
+          "gcs_grad_clip_partials")

@@ -401,10 +401,50 @@ int gcs_link_pairs(const int64_t* chain_rowptr, const int32_t* chain_col, const 
  * K10  Fused multi-tensor optimizer steps over the flat parameter buffer.
  *   sgd:  w -= lr * (g * grad_scale)          (tf.keras.optimizers.SGD, gcn.py:325,338)
  *   adam: Keras Adam, lr_t = lr*sqrt(1-b2^t)/(1-b1^t), w -= lr_t*m/(sqrt(v)+eps)
+ * The _ex forms add Keras' options; with every option off they run the same kernel as the plain entry points.
+ *   gcs_sgd_step_ex:  momentum in [0, 1] (slot accum, NULL allowed only for momentum 0, which is plain SGD):
+ *                     accum = momentum*accum - lr*g; w += accum, or with nesterov w += momentum*accum - lr*g.
+ *   gcs_adam_step_ex: vhat != NULL is amsgrad: vhat = max(vhat, v), w -= lr_t*m/(sqrt(vhat)+eps).
+ *   clip (NULL: none) acts on g*grad_scale: GCS_CLIP_VALUE clamps each element to [-clipvalue, clipvalue] (NaN stays
+ *   NaN); then GCS_CLIP_NORM (per tensor) or GCS_CLIP_GLOBAL_NORM (all tensors) scales by clipnorm/||g|| where
+ *   ||g|| > clipnorm and by exactly 1 otherwise; a non-finite global norm gives NaN everywhere.
+ *   The norms come from a chunk table over the buffer: `chunks` is device int64 [n_chunks][4] = {begin, end, lo, hi},
+ *   element range [begin, end) of w / g (no chunk crosses a tensor), and [lo, hi) the indices in `partials` of the
+ *   chunks of the same tensor.  Row k of a call writes its fp64 sum of squares to partials[chunk_base + k]; the global
+ *   norm sums partials[0, n_partials).  A norm-clipped step is two launches (one block per chunk each): the norm pass,
+ *   then the update, whose blocks each form their factor from the partials in a fixed order.  No atomics: the step is
+ *   bit-identical from run to run.  GCS_CLIP_PARTIALS_READY skips the norm pass when gcs_grad_clip_partials already
+ *   wrote this step's partials (tensors that are not one buffer: every tensor's pass first, then every update).
  * --------------------------------------------------------------------------------- */
 int gcs_sgd_step(float* w, const float* g, int64_t n, float lr, float grad_scale, gcs_stream stream);
 int gcs_adam_step(float* w, const float* g, float* m, float* v, int64_t n, double lr, double beta1,
                   double beta2, double eps, int64_t step, float grad_scale, gcs_stream stream);
+
+enum gcs_clip_mode {
+  GCS_CLIP_VALUE = 1,
+  GCS_CLIP_NORM = 2,
+  GCS_CLIP_GLOBAL_NORM = 4,
+  GCS_CLIP_PARTIALS_READY = 8
+};
+typedef struct gcs_grad_clip {
+  int32_t mode;            /* gcs_clip_mode bits; NORM and GLOBAL_NORM exclude each other */
+  float clipvalue;         /* >= 0 */
+  float clipnorm;          /* >= 0, the threshold of NORM or GLOBAL_NORM */
+  int32_t n_chunks;        /* rows of `chunks` this call covers (NORM / GLOBAL_NORM) */
+  const int64_t* chunks;   /* device [n_chunks][4] */
+  double* partials;        /* device [n_partials] */
+  int32_t chunk_base;
+  int32_t n_partials;
+} gcs_grad_clip;
+
+int gcs_sgd_step_ex(float* w, const float* g, float* accum, int64_t n, float lr, float momentum, int32_t nesterov,
+                    float grad_scale, const gcs_grad_clip* clip, gcs_stream stream);
+int gcs_adam_step_ex(float* w, const float* g, float* m, float* v, float* vhat, int64_t n, double lr, double beta1,
+                     double beta2, double eps, int64_t step, float grad_scale, const gcs_grad_clip* clip,
+                     gcs_stream stream);
+/* The norm pass alone: partials[chunk_base + k] = sum of squares of clipvalue(g*grad_scale) over row k. */
+int gcs_grad_clip_partials(const float* g, int64_t n, float grad_scale, const gcs_grad_clip* clip,
+                           gcs_stream stream);
 
 /* ---------------------------------------------------------------------------------
  * C1  Data-parallel collective (SURVEY.md 8b / 8e; the reference is single-process, this is the sharding the north star
