@@ -9,7 +9,7 @@ from __future__ import annotations
 
 import ctypes
 import os
-from ctypes import POINTER, Structure, c_char_p, c_float, c_int32, c_int64, c_void_p
+from ctypes import POINTER, Structure, c_char_p, c_float, c_int32, c_int64, c_uint32, c_uint64, c_void_p
 
 _HERE = os.path.dirname(os.path.abspath(__file__))
 LIB_PATH = os.path.join(_HERE, "libgcnstring_b200.so")
@@ -25,6 +25,11 @@ class ModelConfig(Structure):
                 ("connectivity", c_int32), ("pool", c_int32), ("final_activation", c_int32),
                 ("bn_momentum", c_float), ("bn_epsilon", c_float), ("aggregate", c_int32),
                 ("loss", c_int32), ("huber_delta", c_float)]
+
+
+class Dropout(Structure):
+    """gcs_dropout: the dropout of one training-mode model call (csrc/dropout.cuh)."""
+    _fields_ = [("rate", c_float), ("_pad", c_uint32), ("seed", c_uint64), ("step", c_uint64)]
 
 
 class Batch(Structure):
@@ -122,6 +127,12 @@ PROTOTYPES = {
     "gcs_model_train_step": (c_int32, [POINTER(ModelConfig), P, P, POINTER(Batch), F32, P, P, P, P, I64, P]),
     "gcs_model_logits_offset": (c_int64, [POINTER(ModelConfig), I64, I32, I32]),
     "gcs_model_backward": (c_int32, [POINTER(ModelConfig), P, POINTER(Batch), P, P, P, I64, P]),
+    "gcs_model_forward_ex": (c_int32, [POINTER(ModelConfig), P, P, POINTER(Batch), I32, P, P, I64, P, POINTER(Dropout)]),
+    "gcs_model_train_step_ex": (c_int32, [POINTER(ModelConfig), P, P, POINTER(Batch), F32, P, P, P, P, I64, P,
+                                          POINTER(Dropout)]),
+    "gcs_model_train_step_dp_ex": (c_int32, [POINTER(ModelConfig), P, P, POINTER(Batch), F32, P, P, P, P, I64, P, P, P,
+                                             I32, POINTER(Dropout)]),
+    "gcs_model_backward_ex": (c_int32, [POINTER(ModelConfig), P, POINTER(Batch), P, P, P, I64, P, POINTER(Dropout)]),
 }
 # test/sweep hook, not part of the header
 _DEBUG = {"gcs_debug_set_spmm_mode": (None, [I32]),
@@ -132,6 +143,7 @@ _DEBUG = {"gcs_debug_set_spmm_mode": (None, [I32]),
           "gcs_debug_profile_end": (c_int32, [ctypes.c_char_p, c_int32]),
           "gcs_debug_slab_timing": (None, [P]),
           "gcs_debug_prelu_branch": (c_int32, [P, I64, P, P, P, P, F32, I64, I32, P, P]),
+          "gcs_debug_dropout_keep": (c_int32, [c_uint64, c_uint64, I32, I64, I32, F32, P, P]),
           "gcs_model_debug_block_buffers": (c_int32, [POINTER(ModelConfig), I64, I32, I32, POINTER(I64), POINTER(I64),
                                                       POINTER(I64), POINTER(I32)])}
 

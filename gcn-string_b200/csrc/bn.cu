@@ -12,6 +12,7 @@
 // in fp64 E[h^2] - mean^2 reproduces the two-pass variance to fp32 rounding.  Partials are
 // written per row-split and combined in a fixed order: deterministic, no atomics.
 #include "common.cuh"
+#include "dropout.cuh"
 
 namespace gcs {
 
@@ -202,11 +203,12 @@ __global__ void bn_fold_kernel(const float* __restrict__ mean, const float* __re
   }
 }
 
-template <int VEC>
+// DROP: Keras Dropout between the BatchNorm and the activation, out = prelu(m * scale * bn(h)) (dropout.cuh).
+template <int VEC, bool DROP>
 __global__ void __launch_bounds__(256) bn_prelu_fwd_kernel(
     const float* __restrict__ h, int64_t ldh, const float* __restrict__ scale,
     const float* __restrict__ shift, const float* __restrict__ alpha, float* __restrict__ out,
-    int64_t ldo, int64_t M, int C, float* __restrict__ amax) {
+    int64_t ldo, int64_t M, int C, float* __restrict__ amax, Dropout d) {
   const int cpr = (C + VEC - 1) / VEC;   // column groups per row
   const int64_t total = M * cpr;
   float mx = 0.f;
@@ -214,7 +216,24 @@ __global__ void __launch_bounds__(256) bn_prelu_fwd_kernel(
        idx += static_cast<int64_t>(gridDim.x) * blockDim.x) {
     const int64_t r = idx / cpr;
     const int c = static_cast<int>(idx - r * cpr) * VEC;
-    if (VEC == 4) {
+    if (DROP) {
+      const unsigned bits = dropout_keep4(d, r, c >> 2) >> (c & 3);
+      float v[VEC];
+      if (VEC == 4) {
+        const float4 t = __ldg(reinterpret_cast<const float4*>(h + r * ldh + c));
+        v[0] = t.x; v[1] = t.y; v[2] = t.z; v[3] = t.w;
+      } else {
+        v[0] = __ldg(h + r * ldh + c);
+      }
+#pragma unroll
+      for (int k = 0; k < VEC; ++k) {
+        const float z = dropout_apply(d, bits, k, fmaf(v[k], __ldg(scale + c + k), __ldg(shift + c + k)));
+        v[k] = alpha ? (z > 0.f ? z : __ldg(alpha + c + k) * z) : z;
+        mx = fmaxf(mx, fabsf(v[k]));
+      }
+      if (VEC == 4) *reinterpret_cast<float4*>(out + r * ldo + c) = make_float4(v[0], v[1], v[2], v[3]);
+      else out[r * ldo + c] = v[0];
+    } else if (VEC == 4) {
       float4 v = __ldg(reinterpret_cast<const float4*>(h + r * ldh + c));
       const float4 sc = __ldg(reinterpret_cast<const float4*>(scale + c));
       const float4 sh = __ldg(reinterpret_cast<const float4*>(shift + c));
@@ -239,13 +258,14 @@ __global__ void __launch_bounds__(256) bn_prelu_fwd_kernel(
 }
 
 // Backward pass 1: per column S1 = sum dz, S2 = sum dz*xhat, S3 = sum da*min(z,0), with
-// z = gamma*xhat + beta, dz = da * slope(z).
-template <int VEC>
+// z = gamma*xhat + beta, dz = da * slope(z).  DROP: with zd = m*scale*z the block's output is prelu(zd), so
+// dz = m*scale*slope(zd)*da and S3 sums da*min(zd,0); m is regenerated from the mask function.
+template <int VEC, bool DROP>
 __global__ void __launch_bounds__(kBnThreads) bn_bwd_partial_kernel(
     const float* __restrict__ da, int64_t ldda, const float* __restrict__ h, int64_t ldh,
     const float* __restrict__ mean, const float* __restrict__ var, const float* __restrict__ gamma,
     const float* __restrict__ beta, const float* __restrict__ alpha, float eps, int64_t M, int C,
-    int64_t rows_per_split, double* __restrict__ ws) {
+    int64_t rows_per_split, double* __restrict__ ws, Dropout d) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int c = (blockIdx.x * 32 + lane) * VEC;
   const int64_t rb = blockIdx.y * rows_per_split;
@@ -268,23 +288,27 @@ __global__ void __launch_bounds__(kBnThreads) bn_bwd_partial_kernel(
     // accumulators once per step.  One F2F + DADD/DFMA per element made this pass conversion-bound (331 us for
     // 1.06 GB = 3.2 TB/s; the fp64-accumulating statistics pass with a third of the conversions runs at 7.3 TB/s);
     // a four-term fp32 partial sum costs ~1e-7 relative, far inside the 1e-5 budget.
-    auto term = [&](float hvk, float gvk, int k, float& t1, float& t2, float& t3) {
+    auto term = [&](float hvk, float gvk, int k, unsigned bits, float& t1, float& t2, float& t3) {
       const float xhat = (hvk - mu[k]) * rs[k];
-      const float z = fmaf(ga[k], xhat, be[k]);
+      float z = fmaf(ga[k], xhat, be[k]);
+      if (DROP) z = dropout_apply(d, bits, k, z);
       float dz = gvk;
       t3 = 0.f;
       if (alpha) {
         dz = z > 0.f ? gvk : (z < 0.f ? gvk * al[k] : 0.f);
         t3 = gvk * fminf(z, 0.f);
       }
+      if (DROP) dz = dropout_apply(d, bits, k, dz);
       t1 = dz;
       t2 = dz * xhat;
     };
     int64_t r = rb + warp;
     for (; r + 24 < re; r += 32) {
       float hv[4][VEC], gv[4][VEC];
+      unsigned bits[4] = {0u, 0u, 0u, 0u};
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
+        if (DROP) bits[u] = dropout_keep4(d, r + 8 * u, c >> 2) >> (c & 3);
         if (VEC == 4) {
           const float4 t = __ldg(reinterpret_cast<const float4*>(h + (r + 8 * u) * ldh + c));
           const float4 g = __ldg(reinterpret_cast<const float4*>(da + (r + 8 * u) * ldda + c));
@@ -299,7 +323,7 @@ __global__ void __launch_bounds__(kBnThreads) bn_bwd_partial_kernel(
       for (int k = 0; k < VEC; ++k) {
         float a1[4], a2[4], a3[4];
 #pragma unroll
-        for (int u = 0; u < 4; ++u) term(hv[u][k], gv[u][k], k, a1[u], a2[u], a3[u]);
+        for (int u = 0; u < 4; ++u) term(hv[u][k], gv[u][k], k, bits[u], a1[u], a2[u], a3[u]);
         acc[3 * k] += static_cast<double>((a1[0] + a1[1]) + (a1[2] + a1[3]));
         acc[3 * k + 1] += static_cast<double>((a2[0] + a2[1]) + (a2[2] + a2[3]));
         if (alpha) acc[3 * k + 2] += static_cast<double>((a3[0] + a3[1]) + (a3[2] + a3[3]));
@@ -307,6 +331,7 @@ __global__ void __launch_bounds__(kBnThreads) bn_bwd_partial_kernel(
     }
     for (; r < re; r += 8) {
       float hv[VEC], gv[VEC];
+      const unsigned bits = DROP ? dropout_keep4(d, r, c >> 2) >> (c & 3) : 0u;
       if (VEC == 4) {
         const float4 t = __ldg(reinterpret_cast<const float4*>(h + r * ldh + c));
         const float4 u = __ldg(reinterpret_cast<const float4*>(da + r * ldda + c));
@@ -319,7 +344,7 @@ __global__ void __launch_bounds__(kBnThreads) bn_bwd_partial_kernel(
 #pragma unroll
       for (int k = 0; k < VEC; ++k) {
         float t1, t2, t3;
-        term(hv[k], gv[k], k, t1, t2, t3);
+        term(hv[k], gv[k], k, bits, t1, t2, t3);
         acc[3 * k] += static_cast<double>(t1);
         acc[3 * k + 1] += static_cast<double>(t2);
         if (alpha) acc[3 * k + 2] += static_cast<double>(t3);
@@ -397,13 +422,13 @@ __global__ void bn_bwd_finish_kernel(const double* __restrict__ sums, int C, dou
 
 // Backward pass 2: dh = gamma*rstd*(dz - S1/M - xhat*S2/M).  Same thread->column mapping as the
 // reduction pass (lane = VEC columns, 8 row warps per block, grid.y row splits), so the per-column
-// coefficients stay in registers for the whole row loop.
-template <int VEC>
+// coefficients stay in registers for the whole row loop.  DROP: dz as in bn_bwd_partial_kernel.
+template <int VEC, bool DROP>
 __global__ void __launch_bounds__(kBnThreads) bn_bwd_apply_kernel(
     const float* __restrict__ da, int64_t ldda, const float* __restrict__ h, int64_t ldh,
     const float* __restrict__ mean, const float* __restrict__ gamma, const float* __restrict__ beta,
     const float* __restrict__ alpha, const float* __restrict__ coef, float* __restrict__ dh, int64_t lddh,
-    int64_t M, int C, int64_t rows_per_split, double* __restrict__ colsum_ws, float* __restrict__ amax) {
+    int64_t M, int C, int64_t rows_per_split, double* __restrict__ colsum_ws, float* __restrict__ amax, Dropout d) {
   const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
   const int c = (blockIdx.x * 32 + lane) * VEC;
   const bool valid = c < C;
@@ -429,18 +454,22 @@ __global__ void __launch_bounds__(kBnThreads) bn_bwd_apply_kernel(
       rs[k] = __ldg(coef + 4 * (c + k) + 2);
       gr[k] = __ldg(coef + 4 * (c + k) + 3);
     }
-    auto out = [&](float hvk, float gvk, int k) {
+    auto out = [&](float hvk, float gvk, int k, unsigned bits) {
       const float xhat = (hvk - mu[k]) * rs[k];
-      const float z = fmaf(ga[k], xhat, be[k]);
+      float z = fmaf(ga[k], xhat, be[k]);
+      if (DROP) z = dropout_apply(d, bits, k, z);
       float dz = gvk;
       if (alpha) dz = z > 0.f ? gvk : (z < 0.f ? gvk * al[k] : 0.f);
+      if (DROP) dz = dropout_apply(d, bits, k, dz);
       return gr[k] * (dz - c1[k] - xhat * c2[k]);
     };
     int64_t r = rb + warp;
     for (; r + 24 < re; r += 32) {                       // four rows per step: eight 128-bit loads in flight
       float hv[4][VEC], gv[4][VEC], o[4][VEC];
+      unsigned bits[4] = {0u, 0u, 0u, 0u};
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
+        if (DROP) bits[u] = dropout_keep4(d, r + 8 * u, c >> 2) >> (c & 3);
         if (VEC == 4) {
           const float4 t = __ldg(reinterpret_cast<const float4*>(h + (r + 8 * u) * ldh + c));
           const float4 g = __ldg(reinterpret_cast<const float4*>(da + (r + 8 * u) * ldda + c));
@@ -454,7 +483,7 @@ __global__ void __launch_bounds__(kBnThreads) bn_bwd_apply_kernel(
 #pragma unroll
       for (int u = 0; u < 4; ++u) {
 #pragma unroll
-        for (int k = 0; k < VEC; ++k) { o[u][k] = out(hv[u][k], gv[u][k], k); mx = fmaxf(mx, fabsf(o[u][k])); }
+        for (int k = 0; k < VEC; ++k) { o[u][k] = out(hv[u][k], gv[u][k], k, bits[u]); mx = fmaxf(mx, fabsf(o[u][k])); }
         if (VEC == 4) *reinterpret_cast<float4*>(dh + (r + 8 * u) * lddh + c) = make_float4(o[u][0], o[u][1], o[u][2], o[u][3]);
         else dh[(r + 8 * u) * lddh + c] = o[u][0];
       }
@@ -465,6 +494,7 @@ __global__ void __launch_bounds__(kBnThreads) bn_bwd_apply_kernel(
     }
     for (; r < re; r += 8) {
       float hv[VEC], gv[VEC], o[VEC];
+      const unsigned bits = DROP ? dropout_keep4(d, r, c >> 2) >> (c & 3) : 0u;
       if (VEC == 4) {
         const float4 t = __ldg(reinterpret_cast<const float4*>(h + r * ldh + c));
         const float4 u = __ldg(reinterpret_cast<const float4*>(da + r * ldda + c));
@@ -475,7 +505,7 @@ __global__ void __launch_bounds__(kBnThreads) bn_bwd_apply_kernel(
         gv[0] = __ldg(da + r * ldda + c);
       }
 #pragma unroll
-      for (int k = 0; k < VEC; ++k) { o[k] = out(hv[k], gv[k], k); mx = fmaxf(mx, fabsf(o[k])); }
+      for (int k = 0; k < VEC; ++k) { o[k] = out(hv[k], gv[k], k, bits); mx = fmaxf(mx, fabsf(o[k])); }
       if (VEC == 4) *reinterpret_cast<float4*>(dh + r * lddh + c) = make_float4(o[0], o[1], o[2], o[3]);
       else dh[r * lddh + c] = o[0];
       if (colsum_ws) {
@@ -582,26 +612,42 @@ extern "C" int gcs_bn_fold(const float* mean, const float* var, const float* gam
   return GCS_OK;
 }
 
-extern "C" int gcs_bn_prelu_fwd(const float* h, int64_t ldh, const float* scale, const float* shift,
-                                const float* alpha, float* out, int64_t ldo, int64_t M, int32_t C,
-                                gcs_stream stream) {
+namespace gcs {
+// gcs_bn_prelu_fwd with the block's dropout (drop == NULL or threshold 0: none).
+int bn_prelu_fwd(const float* h, int64_t ldh, const float* scale, const float* shift, const float* alpha, float* out,
+                 int64_t ldo, int64_t M, int32_t C, const Dropout* drop, gcs_stream stream) {
   GCS_CHECK_ARG(M >= 0 && C > 0, "gcs_bn_prelu_fwd: bad size");
   if (M == 0) return GCS_OK;
   GCS_CHECK_ARG(h && scale && shift && out && ldh >= C && ldo >= C, "gcs_bn_prelu_fwd: bad pointer / leading dimension");
   const bool vec = (C % 4 == 0) && (ldh % 4 == 0) && (ldo % 4 == 0) && aligned16(h) && aligned16(out) &&
                    aligned16(scale) && aligned16(shift) && (!alpha || aligned16(alpha));
   cudaStream_t st = as_stream(stream);
-  if (vec) bn_prelu_fwd_kernel<4><<<static_cast<unsigned>(elementwise_blocks(M * (C / 4))), 256, 0, st>>>(h, ldh, scale, shift, alpha, out, ldo, M, C, amax_sink().produce);
-  else bn_prelu_fwd_kernel<1><<<static_cast<unsigned>(elementwise_blocks(M * C)), 256, 0, st>>>(h, ldh, scale, shift, alpha, out, ldo, M, C, amax_sink().produce);
+  const unsigned b4 = static_cast<unsigned>(elementwise_blocks(M * (C / 4))), b1 = static_cast<unsigned>(elementwise_blocks(M * C));
+  float* amax = amax_sink().produce;
+  if (drop && drop->threshold) {
+    if (vec) bn_prelu_fwd_kernel<4, true><<<b4, 256, 0, st>>>(h, ldh, scale, shift, alpha, out, ldo, M, C, amax, *drop);
+    else bn_prelu_fwd_kernel<1, true><<<b1, 256, 0, st>>>(h, ldh, scale, shift, alpha, out, ldo, M, C, amax, *drop);
+  } else {
+    if (vec) bn_prelu_fwd_kernel<4, false><<<b4, 256, 0, st>>>(h, ldh, scale, shift, alpha, out, ldo, M, C, amax, Dropout{});
+    else bn_prelu_fwd_kernel<1, false><<<b1, 256, 0, st>>>(h, ldh, scale, shift, alpha, out, ldo, M, C, amax, Dropout{});
+  }
   GCS_CHECK_LAUNCH("bn_prelu_fwd_kernel");
   return GCS_OK;
 }
+}  // namespace gcs
 
-extern "C" int gcs_bn_prelu_bwd(const float* da, int64_t ldda, const float* h, int64_t ldh, const float* mean,
-                                const float* var, const float* gamma, const float* beta, const float* alpha,
-                                float eps, float* dh, int64_t lddh, float* dgamma, float* dbeta, float* dalpha,
-                                float* dbias, int64_t M, int32_t C, void* workspace, int64_t workspace_bytes,
+extern "C" int gcs_bn_prelu_fwd(const float* h, int64_t ldh, const float* scale, const float* shift,
+                                const float* alpha, float* out, int64_t ldo, int64_t M, int32_t C,
                                 gcs_stream stream) {
+  return gcs::bn_prelu_fwd(h, ldh, scale, shift, alpha, out, ldo, M, C, nullptr, stream);
+}
+
+namespace gcs {
+// gcs_bn_prelu_bwd of a block whose forward applied `drop` (NULL or threshold 0: none).
+int bn_prelu_bwd(const float* da, int64_t ldda, const float* h, int64_t ldh, const float* mean, const float* var,
+                 const float* gamma, const float* beta, const float* alpha, float eps, float* dh, int64_t lddh,
+                 float* dgamma, float* dbeta, float* dalpha, float* dbias, int64_t M, int32_t C, void* workspace,
+                 int64_t workspace_bytes, const Dropout* drop, gcs_stream stream) {
   GCS_CHECK_ARG(M > 0 && C > 0, "gcs_bn_prelu_bwd: needs at least one row");
   GCS_CHECK_ARG(da && h && mean && var && gamma && beta && dh && workspace, "gcs_bn_prelu_bwd: null pointer");
   GCS_CHECK_ARG(ldda >= C && ldh >= C && lddh >= C, "gcs_bn_prelu_bwd: leading dimension smaller than C");
@@ -617,8 +663,15 @@ extern "C" int gcs_bn_prelu_bwd(const float* da, int64_t ldda, const float* h, i
   float* coef = reinterpret_cast<float*>(static_cast<char*>(workspace) +
                                          round_up(bn_max_splits(M) * C * 3 * static_cast<int64_t>(sizeof(double)), 256));
   dim3 grid(g.col_blocks, g.splits);
-  if (vec) bn_bwd_partial_kernel<4><<<grid, kBnThreads, 0, st>>>(da, ldda, h, ldh, mean, var, gamma, beta, alpha, eps, M, C, g.rows_per_split, ws);
-  else bn_bwd_partial_kernel<1><<<grid, kBnThreads, 0, st>>>(da, ldda, h, ldh, mean, var, gamma, beta, alpha, eps, M, C, g.rows_per_split, ws);
+  const bool dr = drop && drop->threshold;
+  const Dropout dd = dr ? *drop : Dropout{};
+  if (dr) {
+    if (vec) bn_bwd_partial_kernel<4, true><<<grid, kBnThreads, 0, st>>>(da, ldda, h, ldh, mean, var, gamma, beta, alpha, eps, M, C, g.rows_per_split, ws, dd);
+    else bn_bwd_partial_kernel<1, true><<<grid, kBnThreads, 0, st>>>(da, ldda, h, ldh, mean, var, gamma, beta, alpha, eps, M, C, g.rows_per_split, ws, dd);
+  } else {
+    if (vec) bn_bwd_partial_kernel<4, false><<<grid, kBnThreads, 0, st>>>(da, ldda, h, ldh, mean, var, gamma, beta, alpha, eps, M, C, g.rows_per_split, ws, dd);
+    else bn_bwd_partial_kernel<1, false><<<grid, kBnThreads, 0, st>>>(da, ldda, h, ldh, mean, var, gamma, beta, alpha, eps, M, C, g.rows_per_split, ws, dd);
+  }
   GCS_CHECK_LAUNCH("bn_bwd_partial_kernel");
   const SyncHook& hook = sync_hook();
   if (hook.fn) {
@@ -633,14 +686,30 @@ extern "C" int gcs_bn_prelu_bwd(const float* da, int64_t ldda, const float* h, i
     GCS_CHECK_LAUNCH("bn_bwd_final_kernel");
   }
   double* cws = dbias ? ws : nullptr;          // the reduction partials are consumed: reuse their space
-  if (vec) bn_bwd_apply_kernel<4><<<grid, kBnThreads, 0, st>>>(da, ldda, h, ldh, mean, gamma, beta, alpha, coef, dh, lddh, M, C, g.rows_per_split, cws, amax_sink().produce);
-  else bn_bwd_apply_kernel<1><<<grid, kBnThreads, 0, st>>>(da, ldda, h, ldh, mean, gamma, beta, alpha, coef, dh, lddh, M, C, g.rows_per_split, cws, amax_sink().produce);
+  float* amax = amax_sink().produce;
+  if (dr) {
+    if (vec) bn_bwd_apply_kernel<4, true><<<grid, kBnThreads, 0, st>>>(da, ldda, h, ldh, mean, gamma, beta, alpha, coef, dh, lddh, M, C, g.rows_per_split, cws, amax, dd);
+    else bn_bwd_apply_kernel<1, true><<<grid, kBnThreads, 0, st>>>(da, ldda, h, ldh, mean, gamma, beta, alpha, coef, dh, lddh, M, C, g.rows_per_split, cws, amax, dd);
+  } else {
+    if (vec) bn_bwd_apply_kernel<4, false><<<grid, kBnThreads, 0, st>>>(da, ldda, h, ldh, mean, gamma, beta, alpha, coef, dh, lddh, M, C, g.rows_per_split, cws, amax, dd);
+    else bn_bwd_apply_kernel<1, false><<<grid, kBnThreads, 0, st>>>(da, ldda, h, ldh, mean, gamma, beta, alpha, coef, dh, lddh, M, C, g.rows_per_split, cws, amax, dd);
+  }
   GCS_CHECK_LAUNCH("bn_bwd_apply_kernel");
   if (dbias) {
     bn_bwd_dbias_final_kernel<<<static_cast<unsigned>(ceil_div(C, 8)), 256, 0, st>>>(ws, g.splits, C, dbias);
     GCS_CHECK_LAUNCH("bn_bwd_dbias_final_kernel");
   }
   return GCS_OK;
+}
+}  // namespace gcs
+
+extern "C" int gcs_bn_prelu_bwd(const float* da, int64_t ldda, const float* h, int64_t ldh, const float* mean,
+                                const float* var, const float* gamma, const float* beta, const float* alpha,
+                                float eps, float* dh, int64_t lddh, float* dgamma, float* dbeta, float* dalpha,
+                                float* dbias, int64_t M, int32_t C, void* workspace, int64_t workspace_bytes,
+                                gcs_stream stream) {
+  return gcs::bn_prelu_bwd(da, ldda, h, ldh, mean, var, gamma, beta, alpha, eps, dh, lddh, dgamma, dbeta, dalpha, dbias,
+                           M, C, workspace, workspace_bytes, nullptr, stream);
 }
 
 // Test hook (not part of the drop-in surface): the PReLU branch every element takes in the BatchNorm backward above,

@@ -27,6 +27,7 @@
 #include <vector>
 
 #include "common.cuh"
+#include "dropout.cuh"
 #include "prep.cuh"
 
 namespace gcs {
@@ -44,6 +45,12 @@ int linear_fwd_fused(const float* A, int64_t lda, const float* W, const float* b
 int bn_stats_from_partials(const float* part, int64_t M, int C, float* mean, float* var, void* workspace,
                            int64_t workspace_bytes, gcs_stream stream);
 namespace tc { int amax_merge(float* cell, const float* other, cudaStream_t st); }
+int bn_prelu_fwd(const float* h, int64_t ldh, const float* scale, const float* shift, const float* alpha, float* out,
+                 int64_t ldo, int64_t M, int32_t C, const Dropout* drop, gcs_stream stream);   // bn.cu
+int bn_prelu_bwd(const float* da, int64_t ldda, const float* h, int64_t ldh, const float* mean, const float* var,
+                 const float* gamma, const float* beta, const float* alpha, float eps, float* dh, int64_t lddh,
+                 float* dgamma, float* dbeta, float* dalpha, float* dbias, int64_t M, int32_t C, void* workspace,
+                 int64_t workspace_bytes, const Dropout* drop, gcs_stream stream);
 int segment_rows_div_count(float* D, int64_t ld, const int32_t* graph_ptr, int n_graphs, int W, gcs_stream stream);   // pool.cu
 
 enum { kPoolNone = 0, kPoolSum = 1, kPoolAvg = 2, kPoolAttnSum = 3 };
@@ -81,6 +88,34 @@ static void build_blocks(const gcs_model_config& c, std::vector<BlockDesc>& out)
     push(k, last ? c.output : c.hidden, !last);
     k = c.hidden;
   }
+}
+
+// The dropout of one training step (dropout.cuh): threshold and scale from the rate in double, here and nowhere else.
+// A rate below 2^-32 has threshold 0 and scale 1.0f: every element is kept unscaled, and the rate-0 kernels run.
+Dropout make_dropout(float rate, uint64_t seed, uint64_t step, int block) {
+  const double t = std::floor(static_cast<double>(rate) * 4294967296.0);
+  Dropout d;
+  d.threshold = static_cast<uint32_t>(t < 4294967295.0 ? t : 4294967295.0);
+  d.scale = static_cast<float>(1.0 / (1.0 - static_cast<double>(rate)));
+  d.seed = seed;
+  d.step = static_cast<uint32_t>(step);
+  d.block = block;
+  return d;
+}
+
+// The dropout of one training-mode call (block index filled in per block); threshold 0 without one, and in inference.
+static int step_dropout(const gcs_dropout* d, bool training, Dropout* out) {
+  *out = Dropout{};
+  if (!d) return GCS_OK;
+  if (!(d->rate >= 0.f && d->rate < 1.f))
+    return fail(GCS_ERR_INVALID_ARGUMENT, "dropout: rate must be in [0, 1), got %g", static_cast<double>(d->rate));
+  if (training) *out = make_dropout(d->rate, d->seed, d->step, 0);
+  return GCS_OK;
+}
+
+static Dropout block_dropout(Dropout d, int bi) {
+  d.block = bi;
+  return d;
 }
 
 static int check_config(const gcs_model_config* c) {
@@ -401,14 +436,29 @@ static int aggregate(const gcs_batch& bt, bool transposed, const float* X, int64
 }
 
 // dLoss/d(a_k) from dz = dLoss/d(z_k), z_k = agg(a_k): the transposed aggregation.  Z: the forward output z_k (max only).
+// With dropout the forward aggregated the materialised a = prelu(dropout(bn(h))) (run_forward); the kernels that read
+// f(X) again get the same a, rebuilt by the same kernel into `scratch` [N, H] (ld lds) and read with the transform off.
 static int aggregate_bwd(const gcs_model_config& c, const Plan& p, const gcs_batch& bt, int bi, const float* params,
-                         const float* dz, int64_t lddz, const float* Z, int64_t ldz, gcs_stream st) {
+                         const float* dz, int64_t lddz, const float* Z, int64_t ldz, const Dropout& drop, float* scratch,
+                         int64_t lds, gcs_stream st) {
   const int H = p.H;
   if (c.aggregate == 0 && !bt.values)
     return aggregate(bt, true, dz, lddz, nullptr, nullptr, nullptr, nullptr, 0, p.tmp_a, H, H, st);
   const float* scale = p.stat[bi] + 2 * H;
+  const float* X = p.h[bi];
+  int64_t ldx = H;
+  const float* alpha = params + p.blocks[bi].alpha();
+  if (drop.threshold) {
+    const Dropout d = block_dropout(drop, bi);
+    AmaxScope off(nullptr, amax_sink().consume, amax_sink().consume_act);
+    GCS_TIMED("dropout_act", bn_prelu_fwd(p.h[bi], H, scale, scale + H, alpha, scratch, lds, p.N, H, &d, st));
+    X = scratch;
+    ldx = lds;
+    scale = nullptr;
+    alpha = nullptr;
+  }
   return gcs_spmm_aggregate_bwd(bt.rowptr_t, bt.colidx_t, bt.values ? bt.values_t : nullptr, bt.rowptr, bt.colidx, bt.values,
-                                bt.n_nodes, dz, lddz, c.aggregate, p.h[bi], H, scale, scale + H, params + p.blocks[bi].alpha(), Z,
+                                bt.n_nodes, dz, lddz, c.aggregate, X, ldx, scale, scale ? scale + H : nullptr, alpha, Z,
                                 ldz, p.tmp_b, H, p.tmp_a, H, H, st);
 }
 
@@ -437,7 +487,7 @@ static int block_norm(const gcs_model_config& c, const Plan& p, int bi, const fl
 
 // Everything up to the logits ([rows_post, C] in p.logits).
 static int run_forward(const gcs_model_config& c, const Plan& p, const float* params, float* state,
-                       const gcs_batch& bt, bool training, gcs_stream st) {
+                       const gcs_batch& bt, bool training, const Dropout& drop, gcs_stream st) {
   const int H = p.H, Wc = p.Wc, L = p.L, P = p.P;
   const int64_t N = p.N;
   const bool cat = c.connectivity == 1;
@@ -477,7 +527,8 @@ static int run_forward(const gcs_model_config& c, const Plan& p, const float* pa
       if (!with_stats)
         GCS_TIMED("linear_fwd", gcs_linear_fwd(in, ld_in, params + b.kernel(), params + b.bias(), p.h[j], H, N, b.k_in, H, p.lin_ws, p.lin_ws_bytes, st));
       GCS_TRY(block_norm(c, p, j, params, state, p.h[j], H, N, training, st, with_stats ? p.stat_part : nullptr));
-      GCS_TIMED("bn_prelu_fwd", gcs_bn_prelu_fwd(p.h[j], H, scale, scale + H, params + b.alpha(), out, ld_out, N, H, st));
+      const Dropout d = block_dropout(drop, j);
+      GCS_TIMED("bn_prelu_fwd", bn_prelu_fwd(p.h[j], H, scale, scale + H, params + b.alpha(), out, ld_out, N, H, &d, st));
     }
     in = out;
     ld_in = ld_out;
@@ -510,8 +561,22 @@ static int run_forward(const gcs_model_config& c, const Plan& p, const float* pa
     if (!with_stats)
       GCS_TIMED("linear_fwd", gcs_linear_fwd(cin, ld_emb, params + b.kernel(), params + b.bias(), p.h[bi], H, N, b.k_in, H, p.lin_ws, p.lin_ws_bytes, st));
     GCS_TRY(block_norm(c, p, bi, params, state, p.h[bi], H, N, training, st, with_stats ? p.stat_part : nullptr));
+    const float* ax = p.h[bi];
+    const float* ascale = scale;
+    const float* aalpha = params + b.alpha();
+    if (drop.threshold) {
+      // dropout: a = prelu(dropout(bn(h))) written once per node and aggregated as it is, instead of one mask draw per
+      // gathered entry inside the aggregation kernels (DESIGN.md 3.12).  a is no GEMM operand: its |max| is not folded.
+      // tmp_a, a backward buffer of the training plan, is free during the forward.
+      const Dropout d = block_dropout(drop, bi);
+      AmaxScope off(nullptr, amax_sink().consume, amax_sink().consume_act);
+      GCS_TIMED("dropout_act", bn_prelu_fwd(p.h[bi], H, scale, scale + H, aalpha, p.tmp_a, H, N, H, &d, st));
+      ax = p.tmp_a;
+      ascale = nullptr;
+      aalpha = nullptr;
+    }
     // z_k is the leading block of out_{k+1} ('cat'), or out_{k+1} = z_k (+ out_k for 'sum') in the next slab
-    GCS_TIMED("spmm_fwd", aggregate(bt, false, p.h[bi], H, scale, scale + H, params + b.alpha(),
+    GCS_TIMED("spmm_fwd", aggregate(bt, false, ax, H, ascale, ascale ? ascale + H : nullptr, aalpha,
                                     c.connectivity == 2 ? emb(k) : nullptr, H, emb(k + 1), ld_emb, H, st, c.aggregate));
   }
   // global pool
@@ -535,13 +600,14 @@ static int run_forward(const gcs_model_config& c, const Plan& p, const float* pa
                            b.m_out, p.lin_ws, p.lin_ws_bytes, st));
     GCS_TRY(block_norm(c, p, bi, params, state, p.post_h[j], b.m_out, R, training, st));
     const float* scale = p.stat[bi] + 2 * b.m_out;
+    const Dropout d = block_dropout(drop, bi);     // the last block too: Keras' dropout acts on the logits
     if (j < p.Q - 1) {
-      GCS_TRY(gcs_bn_prelu_fwd(p.post_h[j], b.m_out, scale, scale + b.m_out, params + b.alpha(), p.post_a[j], H, R,
-                               b.m_out, st));
+      GCS_TRY(bn_prelu_fwd(p.post_h[j], b.m_out, scale, scale + b.m_out, params + b.alpha(), p.post_a[j], H, R,
+                           b.m_out, &d, st));
       pin = p.post_a[j];
       ld_pin = H;
     } else {
-      GCS_TRY(gcs_bn_prelu_fwd(p.post_h[j], b.m_out, scale, scale + b.m_out, nullptr, p.logits, p.C, R, p.C, st));
+      GCS_TRY(bn_prelu_fwd(p.post_h[j], b.m_out, scale, scale + b.m_out, nullptr, p.logits, p.C, R, p.C, &d, st));
     }
   }
   return GCS_OK;
@@ -552,17 +618,18 @@ static int run_forward(const gcs_model_config& c, const Plan& p, const float* pa
 static int block_backward(const gcs_model_config& c, const Plan& p, int bi, const float* params, float* grads,
                           const float* da, int64_t ldda, const float* h, int64_t ldh, int64_t rows,
                           const float* in, int64_t ld_in, float* dh, int64_t lddh, float* din, int64_t lddin,
-                          int accumulate, gcs_stream st) {
+                          int accumulate, const Dropout& drop, gcs_stream st) {
   const BlockDesc& b = p.blocks[bi];
+  const Dropout d = block_dropout(drop, bi);
   const float* mean = p.stat[bi];
   const float* var = mean + b.m_out;
   float* const dh_amax = const_cast<float*>(amax_sink().consume);      // set for the node-level blocks only
   amax_sink().produce = dh_amax;
-  GCS_TIMED("bn_prelu_bwd", gcs_bn_prelu_bwd(da, ldda, h, ldh, mean, var, params + b.gamma(), params + b.beta(),
-                                             b.has_alpha ? params + b.alpha() : nullptr, c.bn_epsilon, dh, lddh,
-                                             grads + b.gamma(), grads + b.beta(),
-                                             b.has_alpha ? grads + b.alpha() : nullptr, grads + b.bias(), rows, b.m_out,
-                                             p.bn_ws, p.bn_ws_bytes, st));
+  GCS_TIMED("bn_prelu_bwd", bn_prelu_bwd(da, ldda, h, ldh, mean, var, params + b.gamma(), params + b.beta(),
+                                         b.has_alpha ? params + b.alpha() : nullptr, c.bn_epsilon, dh, lddh,
+                                         grads + b.gamma(), grads + b.beta(),
+                                         b.has_alpha ? grads + b.alpha() : nullptr, grads + b.bias(), rows, b.m_out,
+                                         p.bn_ws, p.bn_ws_bytes, &d, st));
   amax_sink().produce = nullptr;
   // the bias gradient (column sums of dh) came out of the BatchNorm backward's apply pass
   GCS_TIMED("linear_bwd_weight", gcs_linear_bwd_weight(in, ld_in, dh, lddh, grads + b.kernel(), nullptr, rows,
@@ -605,7 +672,8 @@ static int head_loss(const gcs_model_config& c, const Plan& p, const float* y, f
 // Reverse pass given dlogits = dLoss/d(logits) [rows_post, C]; needs the activations a
 // training-mode run_forward left in the workspace.
 static int run_backward(const gcs_model_config& c, const Plan& p, const float* params, float* grads,
-                        const gcs_batch& bt, const float* dlogits, gcs_stream st, const GradReady* ready = nullptr) {
+                        const gcs_batch& bt, const float* dlogits, const Dropout& drop, gcs_stream st,
+                        const GradReady* ready = nullptr) {
   const int H = p.H, Wc = p.Wc, L = p.L, P = p.P, Q = p.Q;
   const int64_t N = p.N, R = p.rows_post;
   const bool cat = c.connectivity == 1;
@@ -627,7 +695,7 @@ static int run_backward(const gcs_model_config& c, const Plan& p, const float* p
     if (j == 0) { din = c.pool ? p.dpooled : p.gcat; lddin = Wc; }
     else { din = p.dpost_in; lddin = H; }
     GCS_TRY(block_backward(c, p, bi, params, grads, da, ldda, p.post_h[j], b.m_out, R, in, ld_in, p.dpost, b.m_out,
-                           din, lddin, 0, st));
+                           din, lddin, 0, drop, st));
     da = din;
     ldda = lddin;
   }
@@ -684,9 +752,11 @@ static int run_backward(const gcs_model_config& c, const Plan& p, const float* p
       dz = blk;
       lddz = Wc;
     }
-    GCS_TIMED("spmm_bwd", aggregate_bwd(c, p, bt, bi, params, dz, lddz, p.cat + static_cast<int64_t>(L - 1 - k) * H, Wc, st));
+    // the dh slot of block k is written by its block_backward below: free scratch for the aggregation backward
+    GCS_TIMED("spmm_bwd", aggregate_bwd(c, p, bt, bi, params, dz, lddz, p.cat + static_cast<int64_t>(L - 1 - k) * H, Wc, drop,
+                                        p.dhcat + static_cast<int64_t>(k) * H, ldd, st));
     GCS_TRY(block_backward(c, p, bi, params, grads, p.tmp_a, H, p.h[bi], H, N, p.cat + static_cast<int64_t>(L - k) * H, Wc,
-                           p.dhcat + static_cast<int64_t>(k) * H, ldd, nullptr, 0, 0, st));
+                           p.dhcat + static_cast<int64_t>(k) * H, ldd, nullptr, 0, 0, drop, st));
     if (k == L - 1 || k == (L - 1) / 2) GCS_TRY(notify(bi));   // two buckets inside the message-passing stack
   }
   // ---- pre-processing MLP: its output block (last H columns of cat) is read by the pool and by
@@ -705,9 +775,9 @@ static int run_backward(const gcs_model_config& c, const Plan& p, const float* p
       g = p.tmp_c;
     }
     for (int k = L - 1; k >= 0; --k) {
-      GCS_TIMED("spmm_bwd", aggregate_bwd(c, p, bt, P + k, params, g, H, emb(k + 1), H, st));
+      GCS_TIMED("spmm_bwd", aggregate_bwd(c, p, bt, P + k, params, g, H, emb(k + 1), H, drop, p.dhcat, H, st));
       GCS_TRY(block_backward(c, p, P + k, params, grads, p.tmp_a, H, p.h[P + k], H, N, emb(k), ld_emb, p.dhcat, H, g, H,
-                             c.connectivity == 2 ? 1 : 0, st));
+                             c.connectivity == 2 ? 1 : 0, drop, st));
       if (k == L - 1 || k == (L - 1) / 2) GCS_TRY(notify(P + k));
     }
     da_pre = g;
@@ -732,7 +802,7 @@ static int run_backward(const gcs_model_config& c, const Plan& p, const float* p
     const float* in = j == 0 ? bt.x : p.act[j - 1];
     const int64_t ld_in = j == 0 ? bt.ldx : H;
     GCS_TRY(block_backward(c, p, j, params, grads, da, ldda, p.h[j], H, N, in, ld_in, p.tmp_b, H,
-                           j > 0 ? p.tmp_a : nullptr, H, 0, st));
+                           j > 0 ? p.tmp_a : nullptr, H, 0, drop, st));
     da = p.tmp_a;
     ldda = H;
   }
@@ -774,10 +844,12 @@ extern "C" int64_t gcs_model_workspace_bytes(const gcs_model_config* cfg, int64_
   return gcs_model_workspace_bytes_ex(cfg, n_nodes, nnz, n_graphs, training, 0);
 }
 
-extern "C" int gcs_model_forward(const gcs_model_config* cfg, const float* params, float* state,
-                                 const gcs_batch* batch, int32_t training, float* out, void* workspace,
-                                 int64_t workspace_bytes, gcs_stream stream) {
+extern "C" int gcs_model_forward_ex(const gcs_model_config* cfg, const float* params, float* state,
+                                    const gcs_batch* batch, int32_t training, float* out, void* workspace,
+                                    int64_t workspace_bytes, gcs_stream stream, const gcs_dropout* dropout) {
   GCS_TRY(check_config(cfg));
+  Dropout drop;
+  GCS_TRY(step_dropout(dropout, training != 0, &drop));
   GCS_TRY(check_batch(*cfg, batch, false, false));
   GCS_CHECK_ARG(params && state && out && workspace, "gcs_model_forward: null pointer");
   GCS_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 255u) == 0, "gcs_model_forward: workspace must be 256-byte aligned");
@@ -786,15 +858,23 @@ extern "C" int gcs_model_forward(const gcs_model_config* cfg, const float* param
   make_plan(*cfg, batch->n_nodes, batch->n_graphs, training != 0, workspace, p, &total);
   if (workspace_bytes < total)
     return fail(GCS_ERR_WORKSPACE, "gcs_model_forward: workspace %lld < %lld bytes", (long long)workspace_bytes, (long long)total);
-  GCS_TRY(run_forward(*cfg, p, params, state, *batch, training != 0, stream));
+  GCS_TRY(run_forward(*cfg, p, params, state, *batch, training != 0, drop, stream));
   return head_loss(*cfg, p, nullptr, out, nullptr, 0.f, stream);
 }
 
-extern "C" int gcs_model_train_step(const gcs_model_config* cfg, const float* params, float* state,
-                                    const gcs_batch* batch, float grad_scale, float* grads, float* probs,
-                                    float* loss_acc, void* workspace, int64_t workspace_bytes,
-                                    gcs_stream stream) {
+extern "C" int gcs_model_forward(const gcs_model_config* cfg, const float* params, float* state,
+                                 const gcs_batch* batch, int32_t training, float* out, void* workspace,
+                                 int64_t workspace_bytes, gcs_stream stream) {
+  return gcs_model_forward_ex(cfg, params, state, batch, training, out, workspace, workspace_bytes, stream, nullptr);
+}
+
+extern "C" int gcs_model_train_step_ex(const gcs_model_config* cfg, const float* params, float* state,
+                                       const gcs_batch* batch, float grad_scale, float* grads, float* probs,
+                                       float* loss_acc, void* workspace, int64_t workspace_bytes,
+                                       gcs_stream stream, const gcs_dropout* dropout) {
   GCS_TRY(check_config(cfg));
+  Dropout drop;
+  GCS_TRY(step_dropout(dropout, true, &drop));
   GCS_TRY(check_batch(*cfg, batch, true, true));
   GCS_CHECK_ARG(params && state && grads && loss_acc && workspace, "gcs_model_train_step: null pointer");
   GCS_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 255u) == 0, "gcs_model_train_step: workspace must be 256-byte aligned");
@@ -809,10 +889,18 @@ extern "C" int gcs_model_train_step(const gcs_model_config* cfg, const float* pa
   PreparedTable prepared;
   GCS_TRY(prepare_step_weights(c, p, params, &prepared, stream));
   PreparedScope prepared_scope(&prepared);
-  GCS_TRY(run_forward(c, p, params, state, bt, true, stream));
+  GCS_TRY(run_forward(c, p, params, state, bt, true, drop, stream));
   GCS_TRY(head_loss(c, p, bt.y, probs, loss_acc, grad_scale, stream, bt.sample_weight));
 
-  return run_backward(c, p, params, grads, bt, p.dlogits, stream);
+  return run_backward(c, p, params, grads, bt, p.dlogits, drop, stream);
+}
+
+extern "C" int gcs_model_train_step(const gcs_model_config* cfg, const float* params, float* state,
+                                    const gcs_batch* batch, float grad_scale, float* grads, float* probs,
+                                    float* loss_acc, void* workspace, int64_t workspace_bytes,
+                                    gcs_stream stream) {
+  return gcs_model_train_step_ex(cfg, params, state, batch, grad_scale, grads, probs, loss_acc, workspace,
+                                 workspace_bytes, stream, nullptr);
 }
 
 // Data-parallel train step: gcs_model_train_step + the gradient all-reduce, started bucket by bucket on comm_stream as
@@ -856,11 +944,14 @@ struct HookScope {                                                        // cal
 };
 }  // namespace
 
-extern "C" int gcs_model_train_step_dp(const gcs_model_config* cfg, const float* params, float* state,
-                                       const gcs_batch* batch, float grad_scale, float* grads, float* probs,
-                                       float* loss_acc, void* workspace, int64_t workspace_bytes, gcs_stream stream,
-                                       gcs_comm* comm, gcs_stream comm_stream, int32_t sync_batchnorm) {
+extern "C" int gcs_model_train_step_dp_ex(const gcs_model_config* cfg, const float* params, float* state,
+                                          const gcs_batch* batch, float grad_scale, float* grads, float* probs,
+                                          float* loss_acc, void* workspace, int64_t workspace_bytes, gcs_stream stream,
+                                          gcs_comm* comm, gcs_stream comm_stream, int32_t sync_batchnorm,
+                                          const gcs_dropout* dropout) {
   GCS_TRY(check_config(cfg));
+  Dropout drop;
+  GCS_TRY(step_dropout(dropout, true, &drop));
   GCS_TRY(check_batch(*cfg, batch, true, true));
   GCS_CHECK_ARG(params && state && grads && loss_acc && workspace && comm, "gcs_model_train_step_dp: null pointer");
   GCS_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 255u) == 0, "gcs_model_train_step_dp: workspace must be 256-byte aligned");
@@ -877,16 +968,24 @@ extern "C" int gcs_model_train_step_dp(const gcs_model_config* cfg, const float*
   PreparedTable prepared;
   GCS_TRY(prepare_step_weights(c, p, params, &prepared, stream));
   PreparedScope prepared_scope(&prepared);
-  GCS_TRY(run_forward(c, p, params, state, bt, true, stream));
+  GCS_TRY(run_forward(c, p, params, state, bt, true, drop, stream));
   GCS_TRY(head_loss(c, p, bt.y, probs, loss_acc, grad_scale, stream, bt.sample_weight));
   cudaEvent_t* ev = dp_events();
   DpSync sync{comm, grads, as_stream(stream), as_stream(comm_stream), {}, 0};
   for (int i = 0; i < 8; ++i) sync.ev[i] = ev[i];
   GradReady ready{dp_bucket, &sync};
-  GCS_TRY(run_backward(c, p, params, grads, bt, p.dlogits, stream, &ready));
+  GCS_TRY(run_backward(c, p, params, grads, bt, p.dlogits, drop, stream, &ready));
   GCS_CUDA(cudaEventRecord(ev[8], as_stream(comm_stream)));
   GCS_CUDA(cudaStreamWaitEvent(as_stream(stream), ev[8], 0));
   return GCS_OK;
+}
+
+extern "C" int gcs_model_train_step_dp(const gcs_model_config* cfg, const float* params, float* state,
+                                       const gcs_batch* batch, float grad_scale, float* grads, float* probs,
+                                       float* loss_acc, void* workspace, int64_t workspace_bytes, gcs_stream stream,
+                                       gcs_comm* comm, gcs_stream comm_stream, int32_t sync_batchnorm) {
+  return gcs_model_train_step_dp_ex(cfg, params, state, batch, grad_scale, grads, probs, loss_acc, workspace,
+                                    workspace_bytes, stream, comm, comm_stream, sync_batchnorm, nullptr);
 }
 
 extern "C" int64_t gcs_model_logits_offset(const gcs_model_config* cfg, int64_t n_nodes, int32_t n_graphs,
@@ -899,10 +998,12 @@ extern "C" int64_t gcs_model_logits_offset(const gcs_model_config* cfg, int64_t 
   return reinterpret_cast<char*>(p.logits) - reinterpret_cast<char*>(256);
 }
 
-extern "C" int gcs_model_backward(const gcs_model_config* cfg, const float* params, const gcs_batch* batch,
-                                  const float* dlogits, float* grads, void* workspace, int64_t workspace_bytes,
-                                  gcs_stream stream) {
+extern "C" int gcs_model_backward_ex(const gcs_model_config* cfg, const float* params, const gcs_batch* batch,
+                                     const float* dlogits, float* grads, void* workspace, int64_t workspace_bytes,
+                                     gcs_stream stream, const gcs_dropout* dropout) {
   GCS_TRY(check_config(cfg));
+  Dropout drop;
+  GCS_TRY(step_dropout(dropout, true, &drop));
   GCS_TRY(check_batch(*cfg, batch, false, true));
   GCS_CHECK_ARG(params && dlogits && grads && workspace, "gcs_model_backward: null pointer");
   GCS_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 255u) == 0, "gcs_model_backward: workspace must be 256-byte aligned");
@@ -911,7 +1012,13 @@ extern "C" int gcs_model_backward(const gcs_model_config* cfg, const float* para
   make_plan(*cfg, batch->n_nodes, batch->n_graphs, true, workspace, p, &total);
   if (workspace_bytes < total)
     return fail(GCS_ERR_WORKSPACE, "gcs_model_backward: workspace %lld < %lld bytes", (long long)workspace_bytes, (long long)total);
-  return run_backward(*cfg, p, params, grads, *batch, dlogits, stream);
+  return run_backward(*cfg, p, params, grads, *batch, dlogits, drop, stream);
+}
+
+extern "C" int gcs_model_backward(const gcs_model_config* cfg, const float* params, const gcs_batch* batch,
+                                  const float* dlogits, float* grads, void* workspace, int64_t workspace_bytes,
+                                  gcs_stream stream) {
+  return gcs_model_backward_ex(cfg, params, batch, dlogits, grads, workspace, workspace_bytes, stream, nullptr);
 }
 
 // Test hook (not part of the drop-in surface): where a training-mode forward leaves block `block`'s pre-BatchNorm output
@@ -934,3 +1041,26 @@ extern "C" int gcs_model_debug_block_buffers(const gcs_model_config* cfg, int64_
   return GCS_OK;
 }
 
+// Test hook (not part of the drop-in surface): the keep mask of dense block `block` in step `step`, out[r, c] = 1 where
+// element (r, c) is kept, from the same device function the kernels apply (dropout.cuh).  threshold = 0 for rate 0.
+namespace gcs {
+__global__ void dropout_keep_kernel(Dropout d, int64_t M, int C, uint8_t* __restrict__ out) {
+  const int64_t i = static_cast<int64_t>(blockIdx.x) * blockDim.x + threadIdx.x;
+  if (i >= M * C) return;
+  const int64_t r = i / C;
+  const int c = static_cast<int>(i - r * C);
+  out[i] = static_cast<uint8_t>((dropout_keep4(d, r, c >> 2) >> (c & 3)) & 1u);
+}
+}  // namespace gcs
+
+extern "C" int gcs_debug_dropout_keep(uint64_t seed, uint64_t step, int32_t block, int64_t rows, int32_t cols, float rate,
+                                      uint8_t* out, gcs_stream stream) {
+  GCS_CHECK_ARG(out && rows >= 0 && cols > 0 && block >= 0, "gcs_debug_dropout_keep: bad argument");
+  GCS_CHECK_ARG(rate >= 0.f && rate < 1.f, "gcs_debug_dropout_keep: rate must be in [0, 1)");
+  if (rows == 0) return GCS_OK;
+  const gcs::Dropout d = gcs::make_dropout(rate, seed, step, block);
+  const int64_t n = rows * cols;
+  gcs::dropout_keep_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, gcs::as_stream(stream)>>>(d, rows, cols, out);
+  GCS_CHECK_LAUNCH("dropout_keep_kernel");
+  return GCS_OK;
+}

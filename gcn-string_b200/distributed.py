@@ -173,6 +173,8 @@ class DataParallelTrainer:
         """One step; ``sample_weight`` ([rows] or [rows, 1]): this rank's per-row loss weights.  With the 1/global_batch
         scaling the summed gradient is that of sum w l / global_batch, Keras' weighted mean over the global batch."""
         rank, ws = world()
+        self.model.dropout_rank = rank            # per-rank dropout masks (params.dropout_seed); the all-reduce keeps
+                                                  # the parameters identical
         if not self.model.built:                  # build before the first step: a dry run would move the BatchNorm statistics
             from . import _lib
             self.model.build(int(_lib.as_tensor(inputs[0]).shape[1]))

@@ -6,7 +6,8 @@ dropout=0.0, aggregate='sum', activation='prelu', use_bias=True)([x, a]) -> [N, 
 ``GlobalAttnSumPool()``; ``[x]`` alone pools over all nodes, keepdims), ``MLP(output, hidden=256, layers=2, batch_norm=True,
 dropout=0.0, activation='prelu', final_activation=None)(x)``.  They are inference/forward
 building blocks over the same kernels GeneralGNN uses (the reference only ever reaches them
-through GeneralGNN, src/scripts/gcn.py:320); training goes through the model entry points.
+through GeneralGNN, src/scripts/gcn.py:320); training goes through the model entry points.  ``dropout`` is Keras'
+rate: the identity in inference, as in Keras; a training-mode call with ``dropout > 0`` raises (GeneralGNN trains it).
 """
 from __future__ import annotations
 
@@ -14,6 +15,13 @@ import numpy as np
 
 from . import _lib, ops
 from .data import SparseAdjacency
+from .params import check_dropout_rate
+
+
+def _check_training_dropout(layer, rate, training):
+    if training and rate > 0.0:
+        raise NotImplementedError(f"{layer}(dropout={rate}) is forward-only in training mode: train dropout through "
+                                  "GeneralGNN(dropout=...), whose fused train step applies and differentiates the masks")
 
 
 def _param(arr):
@@ -64,16 +72,16 @@ class GeneralConv:
                  use_bias=True, seed=0, **kwargs):
         if aggregate not in ops.AGGREGATE:
             raise NotImplementedError("native path implements aggregate in {'sum', 'mean', 'max'}")
-        if dropout != 0.0:
-            raise NotImplementedError("native path implements dropout=0.0 only")
+        check_dropout_rate(dropout)
         if activation not in ("prelu", None, "linear"):
             raise NotImplementedError("native path implements activation in {'prelu', None}")
-        self.aggregate = aggregate
+        self.aggregate, self.dropout = aggregate, dropout
         self.channels, self.use_batch_norm, self.activation, self.use_bias = channels, batch_norm, activation, use_bias
         self.seed = seed
         self.block = None
 
     def __call__(self, inputs, training=False):
+        _check_training_dropout("GeneralConv", self.dropout, training)
         torch = _lib.require_cuda()
         x, a = inputs[0], inputs[1]
         x = _lib.as_tensor(x)
@@ -137,18 +145,18 @@ class GlobalAttnSumPool:
 class MLP:
     def __init__(self, output, hidden=256, layers=2, batch_norm=True, dropout=0.0, activation="prelu",
                  final_activation=None, seed=0):
-        if dropout != 0.0:
-            raise NotImplementedError("native path implements dropout=0.0 only")
+        check_dropout_rate(dropout)
         if activation != "prelu":
             raise NotImplementedError("native path implements activation='prelu' only")
         if final_activation not in (None, "linear", "softmax", "sigmoid", "prelu"):
             raise NotImplementedError("final_activation must be None, 'prelu', 'softmax' or 'sigmoid'")
         self.output, self.hidden, self.layers, self.batch_norm = output, hidden, layers, batch_norm
-        self.final_activation = final_activation
+        self.final_activation, self.dropout = final_activation, dropout
         self.seed = seed
         self.blocks = None
 
     def __call__(self, x, training=False):
+        _check_training_dropout("MLP", self.dropout, training)
         x = _lib.as_tensor(x)
         if self.blocks is None:
             rng = np.random.default_rng(self.seed)

@@ -19,7 +19,8 @@ from . import _lib, ops
 from ._lib import check, ptr, stream_ptr
 from .data import SparseAdjacency
 from .losses import fused_loss_fields
-from .params import GNNConfig, block_specs, init_params, n_state, n_trainable, named_slices
+from .params import (GNNConfig, block_specs, check_dropout_rate, dropout_seed, init_params, n_state, n_trainable,
+                     named_slices)
 
 _tape_stack = threading.local()
 
@@ -38,7 +39,8 @@ class GradientTape:
         gradients = tape.gradient(loss, model.trainable_variables)
 
     The tape records the training-mode forward (whose activations stay in the model's
-    workspace) and the loss; ``gradient`` runs the native backward."""
+    workspace), the dropout of that call (its step, so that the backward regenerates the forward's masks) and the
+    loss; ``gradient`` runs the native backward."""
 
     def __init__(self, persistent=False):
         self.model = None
@@ -93,13 +95,19 @@ class GeneralGNN:
     def __init__(self, output, activation=None, hidden=256, message_passing=4, pre_process=2, post_process=2,
                  connectivity="cat", batch_norm=True, dropout=0.0, aggregate="sum", hidden_activation="prelu",
                  pool="sum", seed: Optional[int] = None, use_edge_weights: bool = False):
+        # the layout keywords (params.GNNConfig); Keras' dropout rate changes no layout and is kept apart
         self.config = dict(output=output, activation=activation, hidden=hidden, message_passing=message_passing,
                            pre_process=pre_process, post_process=post_process, connectivity=connectivity,
-                           batch_norm=batch_norm, dropout=dropout, aggregate=aggregate,
-                           hidden_activation=hidden_activation, pool=pool)
+                           batch_norm=batch_norm, aggregate=aggregate, hidden_activation=hidden_activation, pool=pool)
+        check_dropout_rate(dropout)
+        self.dropout = float(dropout)
         # validate everything that does not depend on the input width now (no silent fallback)
         GNNConfig(in_features=1, **self.config).validate()
         self.seed = seed
+        # dropout: every training-mode call (train_step_grads, model(inputs, training=True)) consumes one step of the
+        # mask stream; the stream's key comes from the model's seed and, under DataParallelTrainer, the rank
+        self.dropout_step = 0
+        self.dropout_rank = 0
         # GeneralConv ignores adjacency values (SURVEY.md 8 a5); the reference's `use_edge_data` switch (gcn.py:73-80)
         # wanted them: with use_edge_weights=True the aggregation weights every message by a.edge_weight[entry]
         self.use_edge_weights = bool(use_edge_weights)
@@ -119,6 +127,7 @@ class GeneralGNN:
         if lib.gcs_model_num_params(self._c) != nw or lib.gcs_model_num_state(self._c) != ns:
             raise RuntimeError("parameter layout mismatch between params.py and csrc/model.cu")
         seed = self.seed if self.seed is not None else int(np.random.randint(0, 2**31 - 1))
+        self._seed = seed
         w, s = init_params(self.cfg, seed)
         self.params = torch.from_numpy(w).cuda()
         self.state = torch.from_numpy(s).cuda()
@@ -251,6 +260,15 @@ class GeneralGNN:
             self._ws = torch.empty(int(need * 1.08) + 256, dtype=torch.uint8, device="cuda")
         return self._ws
 
+    def _call_dropout(self, training):
+        """The gcs_dropout of one call: a training-mode call consumes the next step of the mask stream, keyed by the
+        model's seed and rank (host values only: no device synchronisation); inference draws nothing (None)."""
+        if not training:
+            return None
+        d = _lib.Dropout(self.dropout, 0, dropout_seed(self._seed, self.dropout_rank), self.dropout_step)
+        self.dropout_step += 1
+        return d
+
     def _rows_out(self, batch):
         return batch.n_graphs if self.cfg.pool is not None else batch.n_nodes
 
@@ -261,16 +279,17 @@ class GeneralGNN:
         tape = _active_tape() if training else None
         batch, keep = self._prepare(inputs, need_transpose=tape is not None)
         ws = self._workspace(batch, training)
+        drop = self._call_dropout(training)
         out = torch.empty(self._rows_out(batch), self.cfg.output, dtype=torch.float32, device="cuda")
-        check(lib.gcs_model_forward(self._c, ptr(self.params), ptr(self.state), batch, int(training), ptr(out),
-                                    ptr(ws), ws.numel(), stream_ptr()), "gcs_model_forward")
+        check(lib.gcs_model_forward_ex(self._c, ptr(self.params), ptr(self.state), batch, int(training), ptr(out),
+                                       ptr(ws), ws.numel(), stream_ptr(), drop), "gcs_model_forward")
         off = lib.gcs_model_logits_offset(self._c, batch.n_nodes, batch.n_graphs, int(training))
         logits = ws[off:off + out.numel() * 4].view(torch.float32).view(out.shape)
         out._gcs_logits = logits       # like Keras' `_keras_logits`: lets the loss use the logits
         out._gcs_activation = self.cfg.activation
         if tape is not None:
             tape.model = self
-            tape.ctx = dict(batch=batch, keep=keep, ws=ws, out=out)
+            tape.ctx = dict(batch=batch, keep=keep, ws=ws, out=out, dropout=drop)
             out._gcs_tape = tape
         return out
 
@@ -278,8 +297,9 @@ class GeneralGNN:
 
     def _backward(self, ctx, dlogits):
         lib = _lib.load()
-        check(lib.gcs_model_backward(self._c, ptr(self.params), ctx["batch"], ptr(dlogits), ptr(self.grads),
-                                     ptr(ctx["ws"]), ctx["ws"].numel(), stream_ptr()), "gcs_model_backward")
+        check(lib.gcs_model_backward_ex(self._c, ptr(self.params), ctx["batch"], ptr(dlogits), ptr(self.grads),
+                                        ptr(ctx["ws"]), ctx["ws"].numel(), stream_ptr(), ctx["dropout"]),
+              "gcs_model_backward")
 
     def train_step_grads(self, inputs, target, grad_scale: Optional[float] = None, comm=None, sync_bn: bool = False,
                          loss=None, sample_weight=None):
@@ -304,6 +324,7 @@ class GeneralGNN:
         if code:                                         # for this call only: the layout never depends on the loss
             c = _lib.ModelConfig.from_buffer_copy(self._c)
             c.loss, c.huber_delta = code, delta
+        drop = self._call_dropout(True)
         y = _lib.as_tensor(target)
         y = y.to(device="cuda", dtype=torch.float32).contiguous()
         rows = self._rows_out(batch)
@@ -317,12 +338,13 @@ class GeneralGNN:
         loss_acc = torch.empty(2, dtype=torch.float32, device="cuda")
         gs = 1.0 / rows if grad_scale is None else float(grad_scale)
         if comm is not None:
-            check(lib.gcs_model_train_step_dp(c, ptr(self.params), ptr(self.state), batch, gs, ptr(self.grads),
-                                              ptr(probs), ptr(loss_acc), ptr(ws), ws.numel(), stream_ptr(), comm.handle,
-                                              comm.stream.cuda_stream, int(bool(sync_bn))), "gcs_model_train_step_dp")
+            check(lib.gcs_model_train_step_dp_ex(c, ptr(self.params), ptr(self.state), batch, gs, ptr(self.grads),
+                                                 ptr(probs), ptr(loss_acc), ptr(ws), ws.numel(), stream_ptr(),
+                                                 comm.handle, comm.stream.cuda_stream, int(bool(sync_bn)), drop),
+                  "gcs_model_train_step_dp")
         else:
-            check(lib.gcs_model_train_step(c, ptr(self.params), ptr(self.state), batch, gs, ptr(self.grads),
-                                           ptr(probs), ptr(loss_acc), ptr(ws), ws.numel(), stream_ptr()),
+            check(lib.gcs_model_train_step_ex(c, ptr(self.params), ptr(self.state), batch, gs, ptr(self.grads),
+                                              ptr(probs), ptr(loss_acc), ptr(ws), ws.numel(), stream_ptr(), drop),
                   "gcs_model_train_step")
         self._keep = (keep, y, w)
         return loss_acc, probs

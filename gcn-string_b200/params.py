@@ -6,7 +6,8 @@ instantiates it (reference: src/scripts/gcn.py:320 — only ``output`` and
 ``activation`` are passed, everything else is the Spektral default; SURVEY.md §8 a2).
 
 A "dense block" is the unit every stage is made of (SURVEY.md §8 a3/a4):
-``Dense/K.dot + bias -> BatchNormalization -> Dropout(0) -> PReLU | final activation``.
+``Dense/K.dot + bias -> BatchNormalization -> Dropout(rate) -> PReLU | final activation`` (the rate is GeneralGNN's,
+not part of this layout).
 Blocks, in order: ``pre.0 .. pre.{P-1}``, ``gnn.0 .. gnn.{L-1}``, ``post.0 .. post.{Q-1}``.
 Per block the trainable tensors are laid out ``kernel[K,M], bias[M], gamma[M], beta[M],
 alpha[M]`` (no ``alpha`` on the last post block: its activation is the model's final
@@ -56,7 +57,9 @@ class GNNConfig:
         if self.connectivity not in CONNECTIVITY:
             raise ValueError("connectivity must be 'cat', 'sum' or None")
         if self.dropout != 0.0:
-            raise NotImplementedError("native path implements dropout=0.0 only")
+            # the rate changes no parameter, state or workspace layout: GeneralGNN carries it into its training calls
+            raise NotImplementedError("GNNConfig describes the layout, which dropout does not change: pass the rate as "
+                                      "GeneralGNN(dropout=rate)")
         if self.hidden_activation != "prelu":
             raise NotImplementedError("native path implements hidden_activation='prelu' only")
         if not self.batch_norm:
@@ -74,6 +77,26 @@ class GNNConfig:
         if self.connectivity == "cat":
             return self.hidden * (self.message_passing + 1)
         return self.hidden
+
+
+def check_dropout_rate(rate) -> None:
+    """Keras Dropout: ``0 <= rate < 1``; anything else (NaN included) is a ValueError."""
+    if isinstance(rate, bool) or not isinstance(rate, (int, float)) or not (0.0 <= rate < 1.0):
+        raise ValueError(f"dropout rate must be a number in [0, 1), got {rate!r}")
+
+
+_U64 = (1 << 64) - 1
+
+
+def dropout_seed(seed: int, rank: int = 0) -> int:
+    """Key of the dropout mask stream of data-parallel rank ``rank`` for a model seeded with ``seed``: the splitmix64
+    finaliser of ``seed + rank * 0x9E3779B97F4A7C15`` (mod 2^64).  The finaliser is a bijection and the odd increment
+    makes ``seed + rank * inc`` distinct for every rank, so ranks draw independent masks; rank 0 is the single-device
+    stream."""
+    z = (int(seed) + int(rank) * 0x9E3779B97F4A7C15) & _U64
+    z = ((z ^ (z >> 30)) * 0xBF58476D1CE4E5B9) & _U64
+    z = ((z ^ (z >> 27)) * 0x94D049BB133111EB) & _U64
+    return z ^ (z >> 31)
 
 
 @dataclass(frozen=True)

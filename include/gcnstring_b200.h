@@ -489,6 +489,20 @@ typedef struct gcs_model_config {
   float huber_delta;        /* Huber's delta when loss = 3: finite and > 0 */
 } gcs_model_config;
 
+/* Keras Dropout(rate) between the BatchNorm and the activation of every dense block, the last post block included (it
+ * acts on the logits), for ONE training-mode call: the `_ex` entry points below take it as their last argument (NULL, or
+ * rate 0: no dropout; the entry points without `_ex` are these with NULL).  Inference ignores it.  0 <= rate < 1;
+ * anything else, NaN included, is GCS_ERR_INVALID_ARGUMENT.  The keep mask is a function of (seed, step, block, row,
+ * column) only (format: csrc/dropout.cuh), so a training-mode gcs_model_forward_ex and the gcs_model_backward_ex that
+ * follows it regenerate the same masks when they pass the same struct.  Each training step should pass a new step
+ * value.  No extra workspace: the workspace sizes above hold. */
+typedef struct gcs_dropout {
+  float rate;
+  uint32_t _pad;
+  uint64_t seed;            /* key of the mask stream */
+  uint64_t step;            /* training step (its low 32 bits enter the mask counter) */
+} gcs_dropout;
+
 typedef struct gcs_batch {
   int64_t n_nodes;
   int64_t nnz;
@@ -573,6 +587,20 @@ int64_t gcs_model_logits_offset(const gcs_model_config* cfg, int64_t n_nodes, in
 int gcs_model_backward(const gcs_model_config* cfg, const float* params, const gcs_batch* batch,
                        const float* dlogits, float* grads, void* workspace, int64_t workspace_bytes,
                        gcs_stream stream);
+/* The four model entry points above with the dropout of the call (gcs_dropout; NULL = none). */
+int gcs_model_forward_ex(const gcs_model_config* cfg, const float* params, float* state, const gcs_batch* batch,
+                         int32_t training, float* out, void* workspace, int64_t workspace_bytes, gcs_stream stream,
+                         const gcs_dropout* dropout);
+int gcs_model_train_step_ex(const gcs_model_config* cfg, const float* params, float* state, const gcs_batch* batch,
+                            float grad_scale, float* grads, float* probs, float* loss_acc, void* workspace,
+                            int64_t workspace_bytes, gcs_stream stream, const gcs_dropout* dropout);
+int gcs_model_train_step_dp_ex(const gcs_model_config* cfg, const float* params, float* state, const gcs_batch* batch,
+                               float grad_scale, float* grads, float* probs, float* loss_acc, void* workspace,
+                               int64_t workspace_bytes, gcs_stream stream, gcs_comm* comm, gcs_stream comm_stream,
+                               int32_t sync_batchnorm, const gcs_dropout* dropout);
+int gcs_model_backward_ex(const gcs_model_config* cfg, const float* params, const gcs_batch* batch,
+                          const float* dlogits, float* grads, void* workspace, int64_t workspace_bytes,
+                          gcs_stream stream, const gcs_dropout* dropout);
 
 #ifdef __cplusplus
 }
