@@ -11,6 +11,8 @@ import pytest
 import gcn_string_b200 as g
 from gcn_string_b200.params import GNNConfig, block_specs, check_dropout_rate, dropout_seed
 
+from oracle import model_ref_np as O1
+
 import dropout_ref as D
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
@@ -176,19 +178,20 @@ def test_float64_restatement_with_dropout_matches_finite_differences(pool, conne
     y = np.eye(2)[rng.integers(0, 2, r_out)] if act else rng.standard_normal((r_out, 2))
     ew = rng.uniform(0.5, 1.5, rows.shape[0]) if aggregate == "mean" else None
     masks = D.model_masks(specs, cfg, n, r_out, 0.4, seed=5, step=1)
-    args = (cfg, specs, w, s, x, rows, cols, seg, y, B, masks, 0.4)
-    ref = D.loss_and_grads(*args, loss=loss, delta=0.5, edge_weight=ew)
+    args = (cfg, specs, w, s, x, rows, cols, seg, y, B)
+    kw = dict(masks=masks, rate=0.4, loss=loss, delta=0.5, edge_weight=ew)
+    ref = O1.loss_and_grads(*args, **kw)
     eps = 1e-6
     idx = rng.choice(w.shape[0], 60, replace=False)
     for k in idx:
         wp, wm = w.copy(), w.copy()
         wp[k] += eps
         wm[k] -= eps
-        fd = (D.loss_at(cfg, specs, wp, s, x, rows, cols, seg, y, B, masks, 0.4, loss, None, 0.5, ew) -
-              D.loss_at(cfg, specs, wm, s, x, rows, cols, seg, y, B, masks, 0.4, loss, None, 0.5, ew)) / (2 * eps)
+        fd = (O1.loss_at(cfg, specs, wp, s, x, rows, cols, seg, y, B, **kw) -
+              O1.loss_at(cfg, specs, wm, s, x, rows, cols, seg, y, B, **kw)) / (2 * eps)
         assert abs(fd - ref["grads"][k]) <= 1e-5 * max(1.0, abs(fd)), (k, fd, ref["grads"][k])
     # dropped elements are exactly zero after the activation, and kept ones are scaled by 1 / (1 - rate)
-    z, ctx = D.forward(cfg, specs, w, s, x, rows, cols, seg, B, masks, 0.4, ew)
+    z, ctx = O1.forward(cfg, specs, w, s, x, rows, cols, seg, B, training=True, edge_weight=ew, masks=masks, rate=0.4)
     c0 = ctx["caches"][0]
     assert not c0["zd"][~masks[0]].any()
     np.testing.assert_allclose(c0["zd"][masks[0]], c0["z"][masks[0]] * float(D.scale(0.4)))

@@ -14,6 +14,8 @@ import gcn_string_b200 as g
 from gcn_string_b200 import _lib, synthetic
 from gcn_string_b200.params import GNNConfig, block_specs, dropout_seed
 
+from oracle import model_ref_np as O1
+
 import dropout_ref as D
 
 from conftest import rel_err
@@ -89,8 +91,8 @@ def step_vs_oracle(cfg, rate, ds, batch_size, head="softmax", weighted=False, ew
                                              sample_weight=None if sw is None else torch.from_numpy(sw).cuda())
     masks = D.model_masks(specs, cfg, n, r_out, rate, dropout_seed(3, 0), step)
     branches = gpu_prelu_branches(model, cfg, n, B)
-    ref = D.loss_and_grads(cfg, specs, w, s, xr, rows, cols, seg, y, B, masks, rate, loss=head if head in LOSS else None,
-                           sw=sw, prelu_branch=branches, edge_weight=ew)
+    ref = O1.loss_and_grads(cfg, specs, w, s, xr, rows, cols, seg, y, B, masks=masks, rate=rate,
+                            loss=head if head in LOSS else None, sample_weight=sw, prelu_branch=branches, edge_weight=ew)
     got = host(loss_acc)
     assert abs(got[0] - ref["loss"]) < tol * max(abs(ref["loss"]), 1e-3), (got[0], ref["loss"])
     assert rel_err(host(model.state), ref["new_state"]) < tol

@@ -11,9 +11,7 @@ torch = pytest.importorskip("torch")
 import gcn_string_b200 as g
 from gcn_string_b200 import ops, synthetic
 from gcn_string_b200.params import GNNConfig, block_specs, pool_kernel_slice
-from oracle import batching_ref, model_ref_np as O1
-
-import pool_ref as R
+from oracle import batching_ref, model_ref_np as O1, model_ref_torch as O2
 
 from conftest import rel_err
 from test_model_gpu import TOL, _Sparse, gpu_prelu_branches, grad_errors, host, make_model
@@ -44,7 +42,7 @@ def test_segment_mean_kernels(W, ld_pad, col_off):
     gp = _graph_ptr(sizes)
     seg = np.repeat(np.arange(len(sizes)), sizes)
     out = ops.segment_mean_fwd(x, gp)
-    assert rel_err(host(out), R.segment_mean(x64, seg, len(sizes))) < 1e-6
+    assert rel_err(host(out), O1.segment_mean(x64, seg, len(sizes))) < 1e-6
     assert np.array_equal(host(out)[[0, 5]], np.zeros((2, W), dtype=np.float32))
     dout = torch.randn(len(sizes), W, device="cuda")
     dx = ops.segment_mean_bwd(dout, gp, x.shape[0])
@@ -63,7 +61,7 @@ def _attn_check(sizes, W, seed, scale, ld_pad=0, col_off=0, tol=1e-5):
     B = len(sizes)
     seg = np.repeat(np.arange(B), sizes)
     out, scores, gstats = ops.attn_sum_pool_fwd(x, kern, gp)
-    ref, ctx = R.attn_sum_pool(x64, a.astype(np.float64), seg, B)
+    ref, ctx = O1.attn_sum_pool(x64, a.astype(np.float64), seg, B)
     e_out = rel_err(host(out), ref)
     assert e_out < tol, e_out
     assert rel_err(host(scores), ctx["scores"]) < 1e-6
@@ -80,7 +78,7 @@ def _attn_check(sizes, W, seed, scale, ld_pad=0, col_off=0, tol=1e-5):
     den = np.zeros(B)
     np.add.at(den, seg, e)
     gctx = dict(p=e / (den[seg] + 1e-9), out=host(out).astype(np.float64))
-    dx_ref, dk_ref = R.attn_sum_pool_bwd(x64, a.astype(np.float64), seg, host(dout).astype(np.float64), gctx)
+    dx_ref, dk_ref = O1.attn_sum_pool_bwd(x64, a.astype(np.float64), seg, host(dout).astype(np.float64), gctx)
     e_dx, e_dk = rel_err(host(dx), dx_ref), rel_err(host(dk), dk_ref)
     assert e_dx < tol and e_dk < 2 * tol, (e_dx, e_dk)
     # bit-identical run to run
@@ -123,8 +121,8 @@ def _model_parity(cfg, w, s, inputs, y, args, n_nodes, n_graphs, tol=TOL, with_o
     model = make_model(cfg, w, s)
     loss_acc, probs = model.train_step_grads(inputs, y)
     branches = gpu_prelu_branches(model, cfg, n_nodes, n_graphs)
-    ref = R.loss_and_grads(*args, prelu_branch=branches)
-    o2 = R.torch_loss_and_grads(*args)["grads"] if with_o2 else None
+    ref = O1.loss_and_grads(*args, prelu_branch=branches)
+    o2 = O2.loss_and_grads(*args)["grads"] if with_o2 else None
     assert abs(host(loss_acc)[0] - ref["loss"]) < tol * abs(ref["loss"])
     assert rel_err(host(probs), ref["probs"]) < tol
     assert rel_err(host(model.state), ref["new_state"]) < tol
@@ -159,7 +157,7 @@ def test_train_step_and_inference_match_oracle(small_case, pool, connectivity, h
     model.train_step_grads([x, a, i], y)
     assert torch.equal(g1, model.grads)                       # deterministic
     model.load_flat(w, s)
-    p_inf, _ = R.forward(cfg, specs, w, s, c["x"], c["idx"][:, 0], c["idx"][:, 1], c["seg"], 8, False)
+    p_inf, _ = O1.forward(cfg, specs, w, s, c["x"], c["idx"][:, 0], c["idx"][:, 1], c["seg"], 8, False)
     assert rel_err(host(model([x, a, i], training=False)), p_inf) < TOL
 
 
@@ -216,22 +214,22 @@ def test_single_mode_layers_and_evaluate(small_case, pool):
     xs = torch.from_numpy(c["x"].astype(np.float32)).cuda()
     a = _Sparse(c["idx"], n)
     one = model([xs, a])                                                   # [x, a]: one graph of all nodes
-    ref1, _ = R.forward(cfg, specs, w, s, c["x"].astype(np.float32), rows, cols, np.zeros(n, dtype=np.int64), 1, False)
+    ref1, _ = O1.forward(cfg, specs, w, s, c["x"].astype(np.float32), rows, cols, np.zeros(n, dtype=np.int64), 1, False)
     assert one.shape == (1, 2) and rel_err(host(one), ref1) < TOL
     # the pooling layers on their own, disjoint ([x, i]) and single ([x]) mode
     i = torch.from_numpy(c["seg"]).cuda()
     x64 = c["x"].astype(np.float32).astype(np.float64)
     if pool == "avg":
         layer = g.GlobalAvgPool()
-        assert rel_err(host(layer([xs, i])), R.segment_mean(x64, c["seg"], 8)) < 1e-6
+        assert rel_err(host(layer([xs, i])), O1.segment_mean(x64, c["seg"], 8)) < 1e-6
         assert rel_err(host(layer([xs])), x64.mean(0, keepdims=True)) < 1e-6
     else:
         layer = g.GlobalAttnSumPool(seed=3)
         out = layer([xs, i])
         k = host(layer.attn_kernel).astype(np.float64)[:, 0]
         assert layer.attn_kernel.shape == (12, 1)
-        assert rel_err(host(out), R.attn_sum_pool(x64, k, c["seg"], 8)[0]) < TOL
-        assert rel_err(host(layer(xs)), R.attn_sum_pool(x64, k, np.zeros(n, dtype=np.int64), 1)[0]) < TOL
+        assert rel_err(host(out), O1.attn_sum_pool(x64, k, c["seg"], 8)[0]) < TOL
+        assert rel_err(host(layer(xs)), O1.attn_sum_pool(x64, k, np.zeros(n, dtype=np.int64), 1)[0]) < TOL
     # evaluate(): inference over batches of 3, 3, 2 graphs
     loader = g.DisjointLoader(c["ds"], batch_size=3, epochs=None, shuffle=False)
     (loss, acc), preds = evaluate(model, loader)
@@ -239,7 +237,7 @@ def test_single_mode_layers_and_evaluate(small_case, pool):
     for b0 in range(0, 8, 3):
         ids = list(range(b0, min(b0 + 3, 8)))
         (xr, (idx, _, _), seg), yr = batching_ref.collate([c["ds"].graph(k) for k in ids])
-        probs, cache = R.forward(cfg, specs, w, s, xr, idx[:, 0], idx[:, 1], seg, len(ids), training=False)
+        probs, cache = O1.forward(cfg, specs, w, s, xr, idx[:, 0], idx[:, 1], seg, len(ids), training=False)
         probs_ref.append(probs)
         losses.append(O1.xent_from_logits(cache["logits"], yr.astype(np.float64))[0])
         sizes.append(len(ids))

@@ -11,7 +11,7 @@ import gcn_string_b200 as g
 from gcn_string_b200 import losses, synthetic
 from gcn_string_b200.params import GNNConfig, block_specs, n_state, n_trainable, named_slices
 
-import reg_ref as R
+from oracle import model_ref_np as O1, model_ref_torch as O2
 
 from conftest import rel_err
 
@@ -124,22 +124,22 @@ def _case(small_case, pool, connectivity, c_out=2, seed=71):
     return cfg, specs, w, s, args
 
 
-@pytest.mark.parametrize("kind", R.LOSSES)
+@pytest.mark.parametrize("kind", O1.LOSSES)
 @pytest.mark.parametrize("pool", POOLS)
 @pytest.mark.parametrize("connectivity", ["cat", "sum", None])
 def test_float64_and_autograd_restatements_agree(small_case, kind, pool, connectivity):
     cfg, specs, w, s, args = _case(small_case, pool, connectivity)
     delta = 0.7
-    r1 = R.loss_and_grads(*args, kind=kind, delta=delta)
-    r2 = R.torch_loss_and_grads(*args, kind=kind, delta=delta)
-    assert r1["pred"].shape == args[8].shape
+    r1 = O1.loss_and_grads(*args, loss=kind, delta=delta)
+    r2 = O2.loss_and_grads(*args, loss=kind, delta=delta)
+    assert r1["logits"].shape == args[8].shape
     assert abs(r1["loss"] - r2["loss"]) < 1e-5 * abs(r1["loss"])
-    assert rel_err(r2["pred"], r1["pred"]) < 1e-5
+    assert rel_err(r2["logits"], r1["logits"]) < 1e-5
     assert rel_err(r2["grads"], r1["grads"]) < 2e-5
     assert rel_err(r2["new_state"], r1["new_state"]) < 1e-5
 
 
-@pytest.mark.parametrize("kind", R.LOSSES)
+@pytest.mark.parametrize("kind", O1.LOSSES)
 @pytest.mark.parametrize("pool", POOLS)
 def test_manual_backward_matches_finite_differences(small_case, kind, pool):
     c = small_case
@@ -148,16 +148,15 @@ def test_manual_backward_matches_finite_differences(small_case, kind, pool):
     delta = 0.7
     # targets that keep every element away from the kinks (MAE at e = 0, Huber at |e| = delta), half of them on each
     # Huber branch, so that finite differences see one smooth piece
-    z0, _ = R.forward(cfg, specs, w, s, c["x"], rows, cols, c["seg"], 8, training=True)
+    z0, _ = O1.forward(cfg, specs, w, s, c["x"], rows, cols, c["seg"], 8, training=True)
     rng = np.random.default_rng(5)
     mag = np.where(rng.random(z0.shape) < 0.5, rng.uniform(0.2, 0.5, z0.shape), rng.uniform(0.9, 1.5, z0.shape))
     y = z0 - np.where(rng.random(z0.shape) < 0.5, -1.0, 1.0) * mag
     args = args[:8] + (y,) + args[9:]
-    r = R.loss_and_grads(*args, kind=kind, delta=delta)
+    r = O1.loss_and_grads(*args, loss=kind, delta=delta)
 
     def loss_at(wv):
-        z, _ = R.forward(cfg, specs, wv, s, c["x"], rows, cols, c["seg"], 8, training=True)
-        return R.regression_loss(kind, z, y, delta)
+        return O1.loss_at(cfg, specs, wv, s, c["x"], rows, cols, c["seg"], y, 8, loss=kind, delta=delta)
 
     rng = np.random.default_rng(17)
     picks = list(rng.integers(0, w.shape[0], 10))
@@ -176,14 +175,14 @@ def test_manual_backward_matches_finite_differences(small_case, kind, pool):
 def test_keras_documentation_values():
     y_true = np.array([[0.0, 1.0], [0.0, 0.0]])
     y_pred = np.array([[1.0, 1.0], [1.0, 0.0]])
-    assert R.regression_loss("mse", y_pred, y_true) == pytest.approx(0.5, abs=1e-15)
-    assert R.regression_loss("mae", y_pred, y_true) == pytest.approx(0.5, abs=1e-15)
-    assert R.regression_loss("huber", np.array([[0.6, 0.4], [0.4, 0.6]]), y_true) == pytest.approx(0.155, abs=1e-12)
+    assert O1.regression_loss("mse", y_pred, y_true) == pytest.approx(0.5, abs=1e-15)
+    assert O1.regression_loss("mae", y_pred, y_true) == pytest.approx(0.5, abs=1e-15)
+    assert O1.regression_loss("huber", np.array([[0.6, 0.4], [0.4, 0.6]]), y_true) == pytest.approx(0.155, abs=1e-12)
     # the branches: |e| == delta is quadratic, above it linear; sign(0) = 0
     e = np.array([-3.0, -1.0, 0.0, 0.5, 1.0, 2.0])
-    assert R.element_loss("huber", e).tolist() == [2.5, 0.5, 0.0, 0.125, 0.5, 1.5]
-    assert R.element_grad("huber", e).tolist() == [-1.0, -1.0, 0.0, 0.5, 1.0, 1.0]
-    assert R.element_grad("mae", e).tolist() == [-1.0, -1.0, 0.0, 1.0, 1.0, 1.0]
+    assert O1.element_loss("huber", e).tolist() == [2.5, 0.5, 0.0, 0.125, 0.5, 1.5]
+    assert O1.element_grad("huber", e).tolist() == [-1.0, -1.0, 0.0, 0.5, 1.0, 1.0]
+    assert O1.element_grad("mae", e).tolist() == [-1.0, -1.0, 0.0, 1.0, 1.0, 1.0]
     # torch's huber_loss is Keras' form, value and gradient at |e| = delta included
     import torch
     z = torch.tensor([0.0, 2.0, 4.5], requires_grad=True)
@@ -191,8 +190,8 @@ def test_keras_documentation_values():
     loss = torch.nn.functional.huber_loss(z, t, delta=1.5, reduction="sum")
     loss.backward()
     ez = (z.detach() - t).numpy().astype(np.float64)
-    assert float(loss.detach()) == pytest.approx(R.element_loss("huber", ez, 1.5).sum())
-    assert z.grad.numpy().tolist() == pytest.approx(R.element_grad("huber", ez, 1.5).tolist())
+    assert float(loss.detach()) == pytest.approx(O1.element_loss("huber", ez, 1.5).sum())
+    assert z.grad.numpy().tolist() == pytest.approx(O1.element_grad("huber", ez, 1.5).tolist())
 
 
 def test_unsupported_arguments_raise():

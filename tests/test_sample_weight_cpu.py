@@ -12,6 +12,7 @@ import gcn_string_b200 as g
 from gcn_string_b200 import losses, ops
 from gcn_string_b200.evaluate import roc_curve
 from gcn_string_b200.params import GNNConfig, block_specs
+from oracle import model_ref_np as O1, model_ref_torch as O2
 
 import sw_ref as S
 
@@ -33,8 +34,8 @@ def test_keras_documentation_values():
              ("huber", y2, [[0.6, 0.4], [0.4, 0.6]], [1.0, 0.0], 0.155, 0.09),
              ("sigmoid", y2, [[-18.6, 0.51], [2.94, -12.8]], [0.8, 0.2], 0.86546, 0.24364)]
     for head, y, z, w, plain, weighted in cases:
-        assert S.weighted_loss(head, z, y, np.ones(2))[0] == pytest.approx(plain, rel=1e-4), head
-        assert S.weighted_loss(head, z, y, w)[0] == pytest.approx(weighted, rel=1e-4), head
+        assert O1.weighted_loss(head, z, y, np.ones(2))[0] == pytest.approx(plain, rel=1e-4), head
+        assert O1.weighted_loss(head, z, y, w)[0] == pytest.approx(weighted, rel=1e-4), head
     # the host fallbacks of the losses, on probabilities of unknown origin
     y3 = torch.tensor([[0.0, 1.0, 0.0], [0.0, 0.0, 1.0]], dtype=torch.float64)
     p3 = torch.tensor([[0.05, 0.95, 0.0], [0.1, 0.8, 0.1]], dtype=torch.float64)
@@ -50,17 +51,17 @@ def test_keras_documentation_values():
 def test_weighted_metric_is_the_weighted_mean_and_zero_without_weight():
     rng = np.random.default_rng(0)
     z, y = rng.standard_normal((6, 3)), (rng.random((6, 3)) > 0.5).astype(float)
-    for head in S.HEADS:
-        _, m1, _ = S.weighted_loss(head, z, y, np.ones(6))
-        _, mw, d0 = S.weighted_loss(head, z, y, np.zeros(6))
+    for head in O1.HEADS:
+        _, m1, _ = O1.weighted_loss(head, z, y, np.ones(6))
+        _, mw, d0 = O1.weighted_loss(head, z, y, np.zeros(6))
         assert mw == 0.0 and not d0.any()
-        l, m, _ = S.row_terms(head, z, y)
+        l, m, _ = O1.row_terms(head, z, y)
         assert m1 == pytest.approx(m.mean())
 
 
 def _case(small_case, pool, head, c_out=3, seed=81):
     c = small_case
-    cfg = GNNConfig(in_features=12, output=c_out, activation=S.activation(head), hidden=16, message_passing=3, pool=pool)
+    cfg = GNNConfig(in_features=12, output=c_out, activation=O1.activation(head), hidden=16, message_passing=3, pool=pool)
     specs = block_specs(cfg)
     w, s = g.init_params(cfg, seed=seed, perturb=True)
     rows = c["x"].shape[0] if pool is None else 8
@@ -73,16 +74,16 @@ def _case(small_case, pool, head, c_out=3, seed=81):
         y = rng.standard_normal((rows, c_out)).astype(np.float32)
     # half the rows masked, the rest with fractional weights
     sw = np.where(rng.random(rows) < 0.5, 0.0, rng.uniform(0.25, 2.0, rows))
-    args = (cfg, specs, w, s, c["x"], c["idx"][:, 0], c["idx"][:, 1], c["seg"], y, 8, sw, head)
-    return args
+    args = (cfg, specs, w, s, c["x"], c["idx"][:, 0], c["idx"][:, 1], c["seg"], y, 8)
+    return args, dict(loss=head, sample_weight=sw)
 
 
-@pytest.mark.parametrize("head", S.HEADS)
+@pytest.mark.parametrize("head", O1.HEADS)
 @pytest.mark.parametrize("pool", ["sum", None])
 def test_float64_and_autograd_restatements_agree(small_case, head, pool):
-    args = _case(small_case, pool, head)
-    r1 = S.loss_and_grads(*args, delta=0.7)
-    r2 = S.torch_loss_and_grads(*args, delta=0.7)
+    args, kw = _case(small_case, pool, head)
+    r1 = O1.loss_and_grads(*args, **kw, delta=0.7)
+    r2 = O2.loss_and_grads(*args, **kw, delta=0.7)
     assert abs(r1["loss"] - r2["loss"]) < 1e-5 * abs(r1["loss"])
     assert rel_err(r2["grads"], r1["grads"]) < 2e-5
 
@@ -90,8 +91,8 @@ def test_float64_and_autograd_restatements_agree(small_case, head, pool):
 @pytest.mark.parametrize("head", ["softmax", "sigmoid", "mse"])
 @pytest.mark.parametrize("pool", ["avg", None])
 def test_manual_backward_matches_finite_differences(small_case, head, pool):
-    args = _case(small_case, pool, head, seed=83)
-    r = S.loss_and_grads(*args)
+    args, kw = _case(small_case, pool, head, seed=83)
+    r = O1.loss_and_grads(*args, **kw)
     w = args[2]
     rng = np.random.default_rng(19)
     scale = np.abs(r["grads"]).max()
@@ -100,7 +101,7 @@ def test_manual_backward_matches_finite_differences(small_case, head, pool):
         wm = wp.copy()
         wp[j] += 1e-6
         wm[j] -= 1e-6
-        fd = (S.loss_at(args[0], args[1], wp, *args[3:]) - S.loss_at(args[0], args[1], wm, *args[3:])) / 2e-6
+        fd = (O1.loss_at(args[0], args[1], wp, *args[3:], **kw) - O1.loss_at(args[0], args[1], wm, *args[3:], **kw)) / 2e-6
         assert abs(fd - r["grads"][j]) < 2e-6 * scale + 1e-9, j
 
 

@@ -12,6 +12,7 @@ import gcn_string_b200 as g
 from gcn_string_b200 import _lib, ops, synthetic
 from gcn_string_b200.evaluate import evaluate
 from gcn_string_b200.params import GNNConfig, block_specs
+from oracle import model_ref_np as O1, model_ref_torch as O2
 
 import sw_ref as S
 
@@ -94,7 +95,7 @@ def _gpu_row_metric(head, z, y, probs):
 def test_weighted_kernel_against_float64(head, rows, c):
     z, y, w = _case(head, rows, c, seed=rows % 997 + c)
     probs, la, dl = _run(head, z, y, w)
-    loss, _, dref = S.weighted_loss(head, z, y, w, DELTA)
+    loss, _, dref = O1.weighted_loss(head, z, y, w, DELTA)
     assert abs(la[0] - loss) <= 1e-5 * max(abs(loss), 1e-30) + 1e-7, (la[0], loss)
     m = _gpu_row_metric(head, z, y, probs)
     metric = (w * m).sum() / w.sum() if w.sum() else 0.0
@@ -172,14 +173,15 @@ def _weights(rows, node_level, seed):
 @pytest.mark.parametrize("connectivity", ["cat", "sum", None])
 def test_weighted_train_step_matches_float64(small_case, head, pool, connectivity):
     c = small_case
-    cfg = GNNConfig(in_features=12, output=2, activation=S.activation(head), hidden=16, message_passing=3,
+    cfg = GNNConfig(in_features=12, output=2, activation=O1.activation(head), hidden=16, message_passing=3,
                     connectivity=connectivity, pool=pool)
     specs = block_specs(cfg)
     w, s = g.init_params(cfg, seed=91, perturb=True)
     (x, a, i), _ = next(g.DisjointLoader(c["ds"], batch_size=8, epochs=1, shuffle=False))
     n = c["x"].shape[0]
     base = (cfg, specs, w, s, c["x"], c["idx"][:, 0], c["idx"][:, 1], c["seg"])
-    z0 = S.loss_and_grads(*base, np.zeros((n if pool is None else 8, 2)), 8, np.ones(n if pool is None else 8), "mse")["logits"]
+    z0 = O1.loss_and_grads(*base, np.zeros((n if pool is None else 8, 2)), 8, sample_weight=np.ones(n if pool is None else 8),
+                           loss="mse")["logits"]
     y = _labels(head, z0, seed=n)
     sw = _weights(y.shape[0], pool is None, seed=5)
     model = make_model(cfg, w, s)
@@ -187,8 +189,8 @@ def test_weighted_train_step_matches_float64(small_case, head, pool, connectivit
     loss_acc, probs = model.train_step_grads((x, a, i), torch.from_numpy(y).cuda(), loss=loss,
                                              sample_weight=torch.from_numpy(sw).cuda())
     branches = gpu_prelu_branches(model, cfg, n, 8)
-    ref = S.loss_and_grads(*base, y, 8, sw, head, DELTA, prelu_branch=branches)
-    o2 = S.torch_loss_and_grads(*base, y, 8, sw, head, DELTA)["grads"]
+    ref = O1.loss_and_grads(*base, y, 8, sample_weight=sw, loss=head, delta=DELTA, prelu_branch=branches)
+    o2 = O2.loss_and_grads(*base, y, 8, sample_weight=sw, loss=head, delta=DELTA)["grads"]
     got = host(loss_acc)
     assert abs(got[0] - ref["loss"]) < TOL * abs(ref["loss"])
     regression = head in ("mse", "mae", "huber")
@@ -216,7 +218,7 @@ def test_tape_and_data_parallel_routes_equal_the_fused_step(head, pool):
     sw = torch.from_numpy(_weights(y.shape[0], node_level, seed=2)).cuda()
     models = []
     for _ in range(3):
-        m = g.GeneralGNN(3, activation=S.activation(head), hidden=64, message_passing=2, seed=0, pool=pool)
+        m = g.GeneralGNN(3, activation=O1.activation(head), hidden=64, message_passing=2, seed=0, pool=pool)
         m.build(8)
         wv, sv = g.init_params(m.cfg, seed=5, perturb=True)
         m.load_flat(wv, sv)
@@ -329,7 +331,7 @@ def test_evaluate_and_roc_curve_with_weights(small_case):
     # the loss is on the logits (no clipping of the probabilities): the same forward again, logits kept per batch
     plain = g.DisjointLoader(small_case["ds"], batch_size=3, epochs=1, shuffle=False)
     z = np.concatenate([host(model(inputs)._gcs_logits) for inputs, _ in plain])
-    l_rows = S.row_terms("softmax", z, y)[0]
+    l_rows = O1.row_terms("softmax", z, y)[0]
     assert loss == pytest.approx((sw * l_rows).sum() / 8, rel=1e-5)
     hit = (y.argmax(axis=1) == p.argmax(axis=1)).astype(np.float64)
     assert acc == pytest.approx((sw * hit).sum() / sw.sum(), rel=1e-6)

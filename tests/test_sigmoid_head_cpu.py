@@ -9,7 +9,7 @@ import pytest
 import gcn_string_b200 as g
 from gcn_string_b200.params import FINAL_ACT, GNNConfig, block_specs, n_state, n_trainable, named_slices
 
-import bce_ref as R
+from oracle import model_ref_np as O1, model_ref_torch as O2
 
 from conftest import rel_err
 
@@ -85,7 +85,7 @@ def _case(small_case, pool, connectivity, c_out=3, seed=51, soft=False):
 @pytest.mark.parametrize("connectivity", ["cat", "sum", None])
 def test_float64_and_autograd_restatements_agree(small_case, pool, connectivity):
     cfg, specs, w, s, args = _case(small_case, pool, connectivity, soft=True)
-    r1, r2 = R.loss_and_grads(*args), R.torch_loss_and_grads(*args)
+    r1, r2 = O1.loss_and_grads(*args), O2.loss_and_grads(*args)
     assert r1["probs"].shape == args[8].shape
     assert abs(r1["loss"] - r2["loss"]) < 1e-5 * abs(r1["loss"])
     assert rel_err(r2["probs"], r1["probs"]) < 1e-5
@@ -99,11 +99,10 @@ def test_manual_backward_matches_finite_differences(small_case, pool):
     cfg, specs, w, s, args = _case(small_case, pool, "cat", seed=53, soft=True)
     y = args[8].astype(np.float64)
     rows, cols = c["idx"][:, 0], c["idx"][:, 1]
-    r = R.loss_and_grads(*args)
+    r = O1.loss_and_grads(*args)
 
     def loss_at(wv):
-        _, ctx = R.forward(cfg, specs, wv, s, c["x"], rows, cols, c["seg"], 8, training=True)
-        return R.bce_from_logits(ctx["logits"], y)
+        return O1.loss_at(cfg, specs, wv, s, c["x"], rows, cols, c["seg"], y, 8)
 
     rng = np.random.default_rng(13)
     picks = list(rng.integers(0, w.shape[0], 10))
@@ -127,22 +126,22 @@ def test_keras_cases_by_hand():
     l01 = 2.0 + np.log1p(np.exp(-2.0))                    # y = 0: softplus(z)
     l10 = np.log1p(np.exp(-1.0))                          # y = 0, z < 0: softplus(-1)
     l11 = np.log1p(np.exp(-30.0))                         # y = 1: softplus(-z)
-    assert abs(R.bce_from_logits(z, y) - ((l00 + l01) / 2 + (l10 + l11) / 2) / 2) < 1e-15
+    assert abs(O1.bce_from_logits(z, y) - ((l00 + l01) / 2 + (l10 + l11) / 2) / 2) < 1e-15
     # a row-wise mean differs from a flat mean only through ragged weights: a 1-row case pins the column mean
-    assert abs(R.bce_from_logits(z[:1], y[:1]) - (l00 + l01) / 2) < 1e-15
+    assert abs(O1.bce_from_logits(z[:1], y[:1]) - (l00 + l01) / 2) < 1e-15
     # Keras' fallback on probabilities: clip to [1e-7, 1 - 1e-7], then log(p + 1e-7) and log(1 - p + 1e-7)
     p = np.array([[1.0, 0.0, 0.25]])
     t = np.array([[1.0, 1.0, 0.5]])
     hi, lo = 1.0 - 1e-7, 1e-7
     ref = -np.mean([np.log(hi + 1e-7), np.log(lo + 1e-7), 0.5 * np.log(0.25 + 1e-7) + 0.5 * np.log(0.75 + 1e-7)])
-    assert abs(R.bce_from_probs(p, t) - ref) < 1e-12
+    assert abs(O1.bce_from_probs(p, t) - ref) < 1e-12
     # the sigmoid is stable for both signs, and the loss finite at |z| = 100
-    assert R.sigmoid(np.array([-800.0]))[0] == 0.0 and R.sigmoid(np.array([800.0]))[0] == 1.0
-    assert abs(R.bce_from_logits(np.array([[100.0, -100.0]]), np.array([[0.0, 1.0]])) - 100.0) < 1e-12
+    assert O1.sigmoid(np.array([-800.0]))[0] == 0.0 and O1.sigmoid(np.array([800.0]))[0] == 1.0
+    assert abs(O1.bce_from_logits(np.array([[100.0, -100.0]]), np.array([[0.0, 1.0]])) - 100.0) < 1e-12
     # binary_accuracy: p == 0.5 predicts 0; soft labels never equal a 0/1 prediction
-    assert R.binary_accuracy(np.array([[0.0, 1.0]]), np.array([[0.5, 0.5]], np.float32))[0] == 0.5
-    assert R.binary_accuracy(np.array([[0.3, 1.0, 0.0]]), np.array([[0.2, 0.9, 0.1]], np.float32))[0] == pytest.approx(2 / 3)
-    assert R.binary_accuracy(np.array([[1.0], [0.0]]), np.array([[0.51], [0.49]], np.float32)).tolist() == [1.0, 1.0]
+    assert O1.binary_accuracy(np.array([[0.0, 1.0]]), np.array([[0.5, 0.5]], np.float32))[0] == 0.5
+    assert O1.binary_accuracy(np.array([[0.3, 1.0, 0.0]]), np.array([[0.2, 0.9, 0.1]], np.float32))[0] == pytest.approx(2 / 3)
+    assert O1.binary_accuracy(np.array([[1.0], [0.0]]), np.array([[0.51], [0.49]], np.float32)).tolist() == [1.0, 1.0]
 
 
 def test_unsupported_loss_arguments_raise():

@@ -14,9 +14,7 @@ import gcn_string_b200 as g
 from gcn_string_b200 import _lib, ops, synthetic
 from gcn_string_b200.data import Graph
 from gcn_string_b200.params import GNNConfig, block_specs
-from oracle import batching_ref
-
-import bce_ref as R
+from oracle import batching_ref, model_ref_np as O1, model_ref_torch as O2
 
 from conftest import rel_err
 from test_model_gpu import TOL, gpu_prelu_branches, grad_errors, host, make_model
@@ -43,15 +41,15 @@ def _bce_case(rows, c, seed):
 def _check_kernel(z, y, probs, la, dl, grad_scale=None):
     rows, c = z.shape
     z64, y64 = z.astype(np.float64), y.astype(np.float64)
-    p64 = R.sigmoid(z64)
-    loss = R.bce_from_logits(z64, y64)
+    p64 = O1.sigmoid(z64)
+    loss = O1.bce_from_logits(z64, y64)
     got = host(la)
     assert np.isfinite(got).all()
     assert abs(got[0] - loss) <= 1e-6 * max(1.0, abs(loss)), (got[0], loss)
     p = host(probs)
     assert np.abs(p - p64).max() < 1e-6
     # the accuracy counts y == (p > 0.5) on the kernel's own float32 probabilities
-    assert abs(got[1] - R.binary_accuracy(y, p).mean()) <= 1e-6
+    assert abs(got[1] - O1.binary_accuracy(y, p).mean()) <= 1e-6
     gs = 1.0 / rows if grad_scale is None else grad_scale
     assert rel_err(host(dl), (p64 - y64) * gs / c) < 1e-5
 
@@ -119,13 +117,13 @@ def _parity(cfg, w, s, inputs, y, args, n_nodes, n_graphs, tol=TOL, inference=Tr
     yt = torch.from_numpy(y).cuda()
     loss_acc, probs = model.train_step_grads(inputs, yt)
     branches = gpu_prelu_branches(model, cfg, n_nodes, n_graphs)
-    ref = R.loss_and_grads(*args, prelu_branch=branches)
-    o2 = R.torch_loss_and_grads(*args)["grads"]
+    ref = O1.loss_and_grads(*args, prelu_branch=branches)
+    o2 = O2.loss_and_grads(*args)["grads"]
     got = host(loss_acc)
     assert probs.shape == y.shape
     assert abs(got[0] - ref["loss"]) < tol * abs(ref["loss"])
-    assert abs(got[1] - R.binary_accuracy(y, host(probs)).mean()) < 1e-6
-    assert abs(got[1] - ref["acc"]) <= 2.0 / y.size                        # at most a tie at p = 0.5 apart
+    assert abs(got[1] - O1.binary_accuracy(y, host(probs)).mean()) < 1e-6
+    assert abs(got[1] - ref["metric"]) <= 2.0 / y.size                       # at most a tie at p = 0.5 apart
     assert rel_err(host(probs), ref["probs"]) < tol
     assert rel_err(host(model.state), ref["new_state"]) < tol
     e_gpu = grad_errors(host(model.grads), ref["grads"], cfg)
@@ -139,17 +137,18 @@ def _parity(cfg, w, s, inputs, y, args, n_nodes, n_graphs, tol=TOL, inference=Tr
     assert torch.equal(g1, model.grads) and torch.equal(p1, p2) and torch.equal(la1, la2)
     if inference:
         model.load_flat(w, s)
-        p_inf, cache = R.forward(*args[:8], args[9], training=False)
+        p_inf, cache = O1.forward(*args[:8], args[9], training=False)
         out = model(list(inputs), training=False)
         assert out._gcs_activation == "sigmoid"
         z = host(out._gcs_logits).astype(np.float64)
         assert rel_err(z, cache["logits"]) < TOL
-        assert np.abs(host(out) - R.sigmoid(z)).max() < 1e-6              # the kernel's sigmoid of its own logits
+        assert np.abs(host(out) - O1.sigmoid(z)).max() < 1e-6             # the kernel's sigmoid of its own logits
         # On the moving statistics of perturbed parameters the logits reach |z| ~ 1 500 (C = 130), where the float32
         # rounding of a logit near 0 alone moves its probability by ~4e-5: the probabilities are held to 1e-5 or 4x the
         # error of the float32 CPU restatement, whose logits carry the same rounding
         with torch.no_grad():
-            z32, _, _ = R.torch_logits(*args[:8], args[9], False, requires_grad=False)
+            z32 = O2.forward(cfg, O2.unpack(args[1], w, s, requires_grad=False), *O2.tensors(*args[4:8]), args[9], False,
+                             attn=O2.attn_leaf(cfg, args[1], w, requires_grad=False))
         e32 = rel_err(torch.sigmoid(z32).numpy(), p_inf)
         assert rel_err(host(out), p_inf) < max(TOL, 4 * e32), (rel_err(host(out), p_inf), e32)
     return model
@@ -228,7 +227,7 @@ def test_gradient_tape_route_equals_fused_step(pool):
     assert torch.equal(fused.grads, taped.grads) and torch.equal(fused.state, taped.state)
     # an output without sigmoid logits is taken as probabilities (Keras' clip + eps fallback)
     plain = pred.detach().clone()
-    ref = R.bce_from_probs(host(plain).astype(np.float64), host(y).astype(np.float64))
+    ref = O1.bce_from_probs(host(plain).astype(np.float64), host(y).astype(np.float64))
     assert abs(float(g.BinaryCrossentropy()(y, plain)) - ref) < 1e-5 * ref
 
 
@@ -254,10 +253,10 @@ def test_evaluate_with_multi_hot_node_labels(small_case):
         ids = list(range(b0, min(b0 + 3, 8)))
         (xr, (idx, _, _), _), yr = batching_ref.collate([parts[k] for k in ids])
         yr = yr.astype(np.float64)
-        probs, cache = R.forward(cfg, specs, w, s, xr, idx[:, 0], idx[:, 1], None, len(ids), training=False)
+        probs, cache = O1.forward(cfg, specs, w, s, xr, idx[:, 0], idx[:, 1], None, len(ids), training=False)
         probs_ref.append(probs)
-        losses.append(R.bce_from_logits(cache["logits"], yr))
-        accs.append(R.binary_accuracy(yr, probs.astype(np.float32)).mean())
+        losses.append(O1.bce_from_logits(cache["logits"], yr))
+        accs.append(O1.binary_accuracy(yr, probs.astype(np.float32)).mean())
         sizes.append(yr.shape[0])
     ref_loss = np.average(losses, weights=sizes)
     assert abs(loss - ref_loss) < TOL * abs(ref_loss)
