@@ -133,6 +133,11 @@ PROTOTYPES = {
     "gcs_model_train_step_dp_ex": (c_int32, [POINTER(ModelConfig), P, P, POINTER(Batch), F32, P, P, P, P, I64, P, P, P,
                                              I32, POINTER(Dropout)]),
     "gcs_model_backward_ex": (c_int32, [POINTER(ModelConfig), P, POINTER(Batch), P, P, P, I64, P, POINTER(Dropout)]),
+    "gcs_spmm_edge_grad": (c_int32, [P, P, P, I64, P, I64, I32, P, I64, P, P, P, P, I64, P, I64, I32, P, I32, P]),
+    "gcs_model_forward_attr": (c_int32, [POINTER(ModelConfig), P, P, POINTER(Batch), P, P, I64, P]),
+    "gcs_model_input_grad": (c_int32, [POINTER(ModelConfig), P, POINTER(Batch), I32, P, P, I64, P, P, P, I64, P,
+                                       POINTER(Dropout)]),
+    "gcs_output_grad": (c_int32, [I32, P, P, I64, I32, P, P]),
 }
 # test/sweep hook, not part of the header
 _DEBUG = {"gcs_debug_set_spmm_mode": (None, [I32]),

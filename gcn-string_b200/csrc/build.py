@@ -19,7 +19,7 @@ ROOT = os.path.dirname(PKG)
 OUT = os.path.join(PKG, "libgcnstring_b200.so")
 OBJ = os.path.join(HERE, "build")
 NVCC = os.environ.get("NVCC", "/usr/local/cuda/bin/nvcc")
-SOURCES = ["api.cu", "batching.cu", "spmm.cu", "spmm_slab.cu", "linear.cu", "linear_tc.cu", "bn.cu", "pool.cu", "pool_attn.cu", "loss.cu", "optim.cu", "model.cu", "contact.cu", "comm.cu"]
+SOURCES = ["api.cu", "batching.cu", "spmm.cu", "spmm_slab.cu", "linear.cu", "linear_tc.cu", "bn.cu", "pool.cu", "pool_attn.cu", "loss.cu", "optim.cu", "model.cu", "attr.cu", "contact.cu", "comm.cu"]
 FLAGS = ["-gencode", "arch=compute_100a,code=sm_100a", "-O3", "-lineinfo", "-std=c++17",
          "-Xcompiler", "-fPIC", "--expt-relaxed-constexpr"]
 

@@ -52,6 +52,10 @@ int bn_prelu_bwd(const float* da, int64_t ldda, const float* h, int64_t ldh, con
                  float* dgamma, float* dbeta, float* dalpha, float* dbias, int64_t M, int32_t C, void* workspace,
                  int64_t workspace_bytes, const Dropout* drop, gcs_stream stream);
 int segment_rows_div_count(float* D, int64_t ld, const int32_t* graph_ptr, int n_graphs, int W, gcs_stream stream);   // pool.cu
+int dense_dx_thin(const float* dH, int64_t ldh, const float* W, int K, int N, float* dX, int64_t lddx, int64_t M,
+                  cudaStream_t st);                                                                                 // attr.cu
+int bn_prelu_bwd_frozen(const float* da, int64_t ldda, const float* h, int64_t ldh, const float* scale, const float* shift,
+                        const float* alpha, float* dh, int64_t lddh, int64_t M, int C, cudaStream_t st);            // attr.cu
 
 enum { kPoolNone = 0, kPoolSum = 1, kPoolAvg = 2, kPoolAttnSum = 3 };
 
@@ -485,9 +489,11 @@ static int block_norm(const gcs_model_config& c, const Plan& p, int bi, const fl
   return GCS_OK;
 }
 
-// Everything up to the logits ([rows_post, C] in p.logits).
+// Everything up to the logits ([rows_post, C] in p.logits).  keep (inference only, on a training plan): the
+// attribution forward - moving statistics and no dropout as in inference, but every dense block runs unfused, so that
+// h, the activations and the pool state stay in the workspace for gcs_model_input_grad.
 static int run_forward(const gcs_model_config& c, const Plan& p, const float* params, float* state,
-                       const gcs_batch& bt, bool training, const Dropout& drop, gcs_stream st) {
+                       const gcs_batch& bt, bool training, const Dropout& drop, gcs_stream st, bool keep = false) {
   const int H = p.H, Wc = p.Wc, L = p.L, P = p.P;
   const int64_t N = p.N;
   const bool cat = c.connectivity == 1;
@@ -508,7 +514,7 @@ static int run_forward(const gcs_model_config& c, const Plan& p, const float* pa
     const int64_t ld_out = j < P - 1 ? H : ld_emb;
     const float* scale = p.stat[j] + 2 * H;
     int fused = 0;
-    if (!training) {
+    if (!training && !keep) {
       // inference: moving-statistics BatchNorm folded into the GEMM, PReLU in its epilogue (one pass instead of three);
       // the |max| of the result goes through a scratch cell so that the GEMM does not raise the cell it reads
       GCS_TRY(block_norm(c, p, j, params, state, nullptr, H, N, false, st));
@@ -541,7 +547,7 @@ static int run_forward(const gcs_model_config& c, const Plan& p, const float* pa
     const float* cin = emb(k);
     const float* scale = p.stat[bi] + 2 * H;
     int fused = 0;
-    if (!training) {
+    if (!training && !keep) {
       // inference: p.h[bi] receives prelu(bn(out . W + b)) straight from the GEMM; the aggregation is a plain gather
       GCS_TRY(block_norm(c, p, bi, params, state, nullptr, H, N, false, st));
       GCS_TIMED("linear_fwd", linear_fwd_fused(cin, ld_emb, params + b.kernel(), params + b.bias(), scale, scale + H,
@@ -614,26 +620,35 @@ static int run_forward(const gcs_model_config& c, const Plan& p, const float* pa
 }
 
 // Backward of one dense block given da = dLoss/d(block output): parameter gradients into
-// `grads`, dh left in `dh`; optionally the input gradient.
+// `grads`, dh left in `dh`; optionally the input gradient.  frozen (inference-mode attributions): BatchNorm on the
+// moving statistics the forward folded into p.stat's scale / shift, no parameter gradients (grads unused).
 static int block_backward(const gcs_model_config& c, const Plan& p, int bi, const float* params, float* grads,
                           const float* da, int64_t ldda, const float* h, int64_t ldh, int64_t rows,
                           const float* in, int64_t ld_in, float* dh, int64_t lddh, float* din, int64_t lddin,
-                          int accumulate, const Dropout& drop, gcs_stream st) {
+                          int accumulate, const Dropout& drop, gcs_stream st, bool frozen = false) {
   const BlockDesc& b = p.blocks[bi];
   const Dropout d = block_dropout(drop, bi);
   const float* mean = p.stat[bi];
   const float* var = mean + b.m_out;
   float* const dh_amax = const_cast<float*>(amax_sink().consume);      // set for the node-level blocks only
   amax_sink().produce = dh_amax;
-  GCS_TIMED("bn_prelu_bwd", bn_prelu_bwd(da, ldda, h, ldh, mean, var, params + b.gamma(), params + b.beta(),
-                                         b.has_alpha ? params + b.alpha() : nullptr, c.bn_epsilon, dh, lddh,
-                                         grads + b.gamma(), grads + b.beta(),
-                                         b.has_alpha ? grads + b.alpha() : nullptr, grads + b.bias(), rows, b.m_out,
-                                         p.bn_ws, p.bn_ws_bytes, &d, st));
-  amax_sink().produce = nullptr;
-  // the bias gradient (column sums of dh) came out of the BatchNorm backward's apply pass
-  GCS_TIMED("linear_bwd_weight", gcs_linear_bwd_weight(in, ld_in, dh, lddh, grads + b.kernel(), nullptr, rows,
-                                                       b.k_in, b.m_out, p.lw_ws, p.lw_ws_bytes, st));
+  if (frozen) {
+    const float* scale = mean + 2 * b.m_out;
+    GCS_TIMED("bn_prelu_bwd_frozen", bn_prelu_bwd_frozen(da, ldda, h, ldh, scale, scale + b.m_out,
+                                                         b.has_alpha ? params + b.alpha() : nullptr, dh, lddh, rows,
+                                                         b.m_out, as_stream(st)));
+    amax_sink().produce = nullptr;
+  } else {
+    GCS_TIMED("bn_prelu_bwd", bn_prelu_bwd(da, ldda, h, ldh, mean, var, params + b.gamma(), params + b.beta(),
+                                           b.has_alpha ? params + b.alpha() : nullptr, c.bn_epsilon, dh, lddh,
+                                           grads + b.gamma(), grads + b.beta(),
+                                           b.has_alpha ? grads + b.alpha() : nullptr, grads + b.bias(), rows, b.m_out,
+                                           p.bn_ws, p.bn_ws_bytes, &d, st));
+    amax_sink().produce = nullptr;
+    // the bias gradient (column sums of dh) came out of the BatchNorm backward's apply pass
+    GCS_TIMED("linear_bwd_weight", gcs_linear_bwd_weight(in, ld_in, dh, lddh, grads + b.kernel(), nullptr, rows,
+                                                         b.k_in, b.m_out, p.lw_ws, p.lw_ws_bytes, st));
+  }
   if (din)
     GCS_TIMED("linear_bwd_input", gcs_linear_bwd_input(dh, lddh, params + b.kernel(), din, lddin, rows, b.k_in,
                                                        b.m_out, accumulate, p.lin_ws, p.lin_ws_bytes, st));
@@ -669,11 +684,42 @@ static int head_loss(const gcs_model_config& c, const Plan& p, const float* y, f
                              p.loss_ws, p.loss_ws_bytes, st);
 }
 
+// What gcs_model_input_grad asks of run_backward besides (or, frozen, instead of) the parameter gradients.
+struct InputGrad {
+  bool frozen;          // inference mode: BatchNorm on moving statistics, no parameter gradients
+  float* dx;            // dLoss/dx [N, F] (ld lddx), or NULL
+  int64_t lddx;
+  float* dvalues;       // dLoss/d(edge weights) [nnz] in forward CSR order, or NULL
+};
+
+// dLoss/d(edge weights) of conv block bi from dz = dLoss/dz_k (gcs_spmm_edge_grad), accumulated onto the later layers'
+// part unless this is the last layer.  Runs right after aggregate_bwd, while what that call left is valid: the tie
+// counts of max aggregation in tmp_b, and under dropout the materialised activations in `scratch`.
+static int edge_grad(const gcs_model_config& c, const Plan& p, const gcs_batch& bt, int bi, const float* params,
+                     const float* dz, int64_t lddz, const float* Z, int64_t ldz, const Dropout& drop, const float* scratch,
+                     int64_t lds, float* dvalues, int accumulate, gcs_stream st) {
+  const int H = p.H;
+  const float* X = p.h[bi];
+  int64_t ldx = H;
+  const float* scale = p.stat[bi] + 2 * H;
+  const float* alpha = params + p.blocks[bi].alpha();
+  if (drop.threshold) {
+    X = scratch;
+    ldx = lds;
+    scale = nullptr;
+    alpha = nullptr;
+  }
+  return gcs_spmm_edge_grad(bt.rowptr, bt.colidx, bt.values, bt.n_nodes, dz, lddz, c.aggregate, X, ldx, scale,
+                            scale ? scale + H : nullptr, alpha, Z, ldz, p.tmp_b, H, H, dvalues, accumulate, st);
+}
+
 // Reverse pass given dlogits = dLoss/d(logits) [rows_post, C]; needs the activations a
-// training-mode run_forward left in the workspace.
+// training-mode run_forward (or the attribution forward, with ig->frozen) left in the workspace.
 static int run_backward(const gcs_model_config& c, const Plan& p, const float* params, float* grads,
                         const gcs_batch& bt, const float* dlogits, const Dropout& drop, gcs_stream st,
-                        const GradReady* ready = nullptr) {
+                        const GradReady* ready = nullptr, const InputGrad* ig = nullptr) {
+  const bool frozen = ig && ig->frozen;
+  float* const dvalues = ig ? ig->dvalues : nullptr;
   const int H = p.H, Wc = p.Wc, L = p.L, P = p.P, Q = p.Q;
   const int64_t N = p.N, R = p.rows_post;
   const bool cat = c.connectivity == 1;
@@ -695,7 +741,7 @@ static int run_backward(const gcs_model_config& c, const Plan& p, const float* p
     if (j == 0) { din = c.pool ? p.dpooled : p.gcat; lddin = Wc; }
     else { din = p.dpost_in; lddin = H; }
     GCS_TRY(block_backward(c, p, bi, params, grads, da, ldda, p.post_h[j], b.m_out, R, in, ld_in, p.dpost, b.m_out,
-                           din, lddin, 0, drop, st));
+                           din, lddin, 0, drop, st, frozen));
     da = din;
     ldda = lddin;
   }
@@ -706,8 +752,9 @@ static int run_backward(const gcs_model_config& c, const Plan& p, const float* p
     GCS_TIMED("pool_bwd", segment_rows_div_count(p.dpooled, Wc, bt.graph_ptr, bt.n_graphs, Wc, st));
   else if (c.pool == kPoolAttnSum)
     GCS_TIMED("pool_bwd", gcs_attn_sum_pool_bwd(p.dpooled, Wc, emb(L), Wc, N, params + p.attn_off, bt.graph_ptr, bt.n_graphs, Wc,
-                                                p.pooled, Wc, p.scores, p.gstats, p.gcat, Wc, grads + p.attn_off, p.attn_ws,
-                                                p.attn_ws_bytes, st));
+                                                p.pooled, Wc, p.scores, p.gstats, p.gcat, Wc,
+                                                frozen ? static_cast<float*>(p.lw_ws) : grads + p.attn_off,   // frozen: scratch
+                                                p.attn_ws, p.attn_ws_bytes, st));
   int64_t grads_final_from = p.n_params;                    // everything from here on is final
   auto notify = [&](int first_block) -> int {                // blocks first_block .. have all been differentiated
     const int64_t begin = p.blocks[first_block].off;
@@ -755,8 +802,11 @@ static int run_backward(const gcs_model_config& c, const Plan& p, const float* p
     // the dh slot of block k is written by its block_backward below: free scratch for the aggregation backward
     GCS_TIMED("spmm_bwd", aggregate_bwd(c, p, bt, bi, params, dz, lddz, p.cat + static_cast<int64_t>(L - 1 - k) * H, Wc, drop,
                                         p.dhcat + static_cast<int64_t>(k) * H, ldd, st));
+    if (dvalues)
+      GCS_TIMED("edge_grad", edge_grad(c, p, bt, bi, params, dz, lddz, p.cat + static_cast<int64_t>(L - 1 - k) * H, Wc, drop,
+                                       p.dhcat + static_cast<int64_t>(k) * H, ldd, dvalues, k != L - 1, st));
     GCS_TRY(block_backward(c, p, bi, params, grads, p.tmp_a, H, p.h[bi], H, N, p.cat + static_cast<int64_t>(L - k) * H, Wc,
-                           p.dhcat + static_cast<int64_t>(k) * H, ldd, nullptr, 0, 0, drop, st));
+                           p.dhcat + static_cast<int64_t>(k) * H, ldd, nullptr, 0, 0, drop, st, frozen));
     if (k == L - 1 || k == (L - 1) / 2) GCS_TRY(notify(bi));   // two buckets inside the message-passing stack
   }
   // ---- pre-processing MLP: its output block (last H columns of cat) is read by the pool and by
@@ -776,8 +826,10 @@ static int run_backward(const gcs_model_config& c, const Plan& p, const float* p
     }
     for (int k = L - 1; k >= 0; --k) {
       GCS_TIMED("spmm_bwd", aggregate_bwd(c, p, bt, P + k, params, g, H, emb(k + 1), H, drop, p.dhcat, H, st));
+      if (dvalues)
+        GCS_TIMED("edge_grad", edge_grad(c, p, bt, P + k, params, g, H, emb(k + 1), H, drop, p.dhcat, H, dvalues, k != L - 1, st));
       GCS_TRY(block_backward(c, p, P + k, params, grads, p.tmp_a, H, p.h[P + k], H, N, emb(k), ld_emb, p.dhcat, H, g, H,
-                             c.connectivity == 2 ? 1 : 0, drop, st));
+                             c.connectivity == 2 ? 1 : 0, drop, st, frozen));
       if (k == L - 1 || k == (L - 1) / 2) GCS_TRY(notify(P + k));
     }
     da_pre = g;
@@ -802,9 +854,19 @@ static int run_backward(const gcs_model_config& c, const Plan& p, const float* p
     const float* in = j == 0 ? bt.x : p.act[j - 1];
     const int64_t ld_in = j == 0 ? bt.ldx : H;
     GCS_TRY(block_backward(c, p, j, params, grads, da, ldda, p.h[j], H, N, in, ld_in, p.tmp_b, H,
-                           j > 0 ? p.tmp_a : nullptr, H, 0, drop, st));
+                           j > 0 ? p.tmp_a : nullptr, H, 0, drop, st, frozen));
     da = p.tmp_a;
     ldda = H;
+  }
+  if (ig && ig->dx) {
+    // dX = dh_0 . W_0^T: a thin output (F columns), on its own kernel where the shape allows
+    const BlockDesc& b0 = p.blocks[0];
+    ::gcs::ScopedOpTimer timer__("linear_bwd_input_x", st);
+    int r = dense_dx_thin(p.tmp_b, H, params + b0.kernel(), b0.k_in, H, ig->dx, ig->lddx, N, cst);
+    if (r == GCS_ERR_UNSUPPORTED)
+      r = gcs_linear_bwd_input(p.tmp_b, H, params + b0.kernel(), ig->dx, ig->lddx, N, b0.k_in, H, 0, p.lin_ws,
+                               p.lin_ws_bytes, st);
+    GCS_TRY(r);
   }
   GCS_TRY(notify(0));
   return GCS_OK;
@@ -1019,6 +1081,48 @@ extern "C" int gcs_model_backward(const gcs_model_config* cfg, const float* para
                                   const float* dlogits, float* grads, void* workspace, int64_t workspace_bytes,
                                   gcs_stream stream) {
   return gcs_model_backward_ex(cfg, params, batch, dlogits, grads, workspace, workspace_bytes, stream, nullptr);
+}
+
+extern "C" int gcs_model_forward_attr(const gcs_model_config* cfg, const float* params, float* state,
+                                      const gcs_batch* batch, float* out, void* workspace, int64_t workspace_bytes,
+                                      gcs_stream stream) {
+  GCS_TRY(check_config(cfg));
+  GCS_TRY(check_batch(*cfg, batch, false, false));
+  GCS_CHECK_ARG(params && state && out && workspace, "gcs_model_forward_attr: null pointer");
+  GCS_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 255u) == 0, "gcs_model_forward_attr: workspace must be 256-byte aligned");
+  Plan p;
+  int64_t total = 0;
+  make_plan(*cfg, batch->n_nodes, batch->n_graphs, true, workspace, p, &total);
+  if (workspace_bytes < total)
+    return fail(GCS_ERR_WORKSPACE, "gcs_model_forward_attr: workspace %lld < %lld bytes", (long long)workspace_bytes, (long long)total);
+  GCS_TRY(run_forward(*cfg, p, params, state, *batch, false, Dropout{}, stream, true));
+  return head_loss(*cfg, p, nullptr, out, nullptr, 0.f, stream);
+}
+
+extern "C" int gcs_model_input_grad(const gcs_model_config* cfg, const float* params, const gcs_batch* batch,
+                                    int32_t training, const float* dlogits, float* dx, int64_t lddx, float* dvalues,
+                                    float* grads, void* workspace, int64_t workspace_bytes, gcs_stream stream,
+                                    const gcs_dropout* dropout) {
+  GCS_TRY(check_config(cfg));
+  Dropout drop;
+  GCS_TRY(step_dropout(dropout, training != 0, &drop));
+  GCS_TRY(check_batch(*cfg, batch, false, true));
+  GCS_CHECK_ARG(params && dlogits && workspace, "gcs_model_input_grad: null pointer");
+  GCS_CHECK_ARG((reinterpret_cast<uintptr_t>(workspace) & 255u) == 0, "gcs_model_input_grad: workspace must be 256-byte aligned");
+  GCS_CHECK_ARG(dx || dvalues || grads, "gcs_model_input_grad: nothing to compute (dx, dvalues and grads are NULL)");
+  GCS_CHECK_ARG(!dx || lddx >= cfg->in_features, "gcs_model_input_grad: lddx < in_features");
+  GCS_CHECK_ARG(!dvalues || batch->values,
+                "gcs_model_input_grad: the edge-weight gradient needs a weighted aggregation (batch values)");
+  if (!training && grads)
+    return fail(GCS_ERR_UNSUPPORTED, "gcs_model_input_grad: parameter gradients need a training-mode forward");
+  GCS_CHECK_ARG(!training || grads, "gcs_model_input_grad: a training-mode backward writes the parameter gradients (grads)");
+  Plan p;
+  int64_t total = 0;
+  make_plan(*cfg, batch->n_nodes, batch->n_graphs, true, workspace, p, &total);
+  if (workspace_bytes < total)
+    return fail(GCS_ERR_WORKSPACE, "gcs_model_input_grad: workspace %lld < %lld bytes", (long long)workspace_bytes, (long long)total);
+  const InputGrad ig{training == 0, dx, lddx, dvalues};
+  return run_backward(*cfg, p, params, grads, *batch, dlogits, drop, stream, nullptr, &ig);
 }
 
 // Test hook (not part of the drop-in surface): where a training-mode forward leaves block `block`'s pre-BatchNorm output

@@ -40,12 +40,31 @@ class GradientTape:
 
     The tape records the training-mode forward (whose activations stay in the model's
     workspace), the dropout of that call (its step, so that the backward regenerates the forward's masks) and the
-    loss; ``gradient`` runs the native backward."""
+    loss; ``gradient`` runs the native backward.
+
+    Attributions (the saliency pattern): ``tape.watch(x)`` on the node-feature tensor passed as ``inputs[0]``, and/or
+    ``tape.watch(a)`` (a ``SparseAdjacency``: its values) or ``tape.watch(a.edge_weight)``.  Under a tape that watches
+    something, ``model(inputs, training=False)`` runs the attribution forward (gcs_model_forward_attr, the inference
+    result on moving statistics) and records it; ``tape.gradient(target, [x, a], output_gradients=...)`` then returns
+    dtarget/dx and dtarget/d(edge weights).  ``target`` is a recorded loss or the model output itself (output_gradients
+    [rows, C], ones by default).  Sources the call did not read return None, as in TF; model variables are sources of a
+    training-mode call only."""
 
     def __init__(self, persistent=False):
         self.model = None
         self.ctx = None
         self.loss_record = None
+        self._watched = []
+
+    def watch(self, tensor):
+        """Mark a node-feature tensor, a SparseAdjacency or its edge_weight as a source of ``gradient``."""
+        items = tensor if isinstance(tensor, (list, tuple)) else [tensor]
+        for t in items:
+            if not any(t is w for w in self._watched):
+                self._watched.append(t)
+
+    def _is_watched(self, t):
+        return t is not None and any(t is w for w in self._watched)
 
     def __enter__(self):
         if not hasattr(_tape_stack, "stack"):
@@ -57,17 +76,42 @@ class GradientTape:
         _tape_stack.stack.pop()
         return False
 
-    def gradient(self, loss, variables):
+    def gradient(self, loss, variables, output_gradients=None):
+        single = not isinstance(variables, (list, tuple))
+        sources = [variables] if single else list(variables)
+        inputs = self.ctx.get("inputs") if self.ctx else None
+        if inputs is not None and any(inputs.kind(v) for v in sources):
+            out = self.model._input_grad(self, loss, sources, output_gradients)
+            return out[0] if single else out
+        if self.ctx and self.ctx.get("mode") == "inference":
+            raise NotImplementedError("GradientTape.gradient: parameter gradients of a training=False call are not "
+                                      "built; call the model with training=True for them")
         if self.model is None or self.loss_record is None:
             raise RuntimeError("GradientTape.gradient: no training-mode model call and loss were recorded")
         self.model._backward(self.ctx, self.loss_record["dlogits"])
         by_name = {v.name: v for v in self.model.trainable_variables}
         out = []
-        for v in variables:
+        for v in sources:
             if getattr(v, "name", None) not in by_name:
                 raise ValueError("GradientTape.gradient: variable does not belong to the recorded model")
             out.append(by_name[v.name].grad_view)
-        return out
+        return out[0] if single else out
+
+
+class _WatchedInputs:
+    """The inputs of one recorded model call a gradient can be taken with respect to: the node features as passed
+    (``x``, its dtype) and the adjacency and edge-weight objects, if the tape watched them."""
+
+    def __init__(self, x_obj, x_dtype, a_obj, ew_obj, uses_ew):
+        self.x_obj, self.x_dtype, self.a_obj, self.ew_obj, self.uses_ew = x_obj, x_dtype, a_obj, ew_obj, uses_ew
+
+    def kind(self, v):
+        """'x', 'ew' (read by the call), 'unconnected' (a watched input the call did not read) or None."""
+        if v is self.x_obj and v is not None:
+            return "x"
+        if v is not None and (v is self.a_obj or v is self.ew_obj):
+            return "ew" if self.uses_ew else "unconnected"
+        return None
 
 
 class Variable:
@@ -276,7 +320,11 @@ class GeneralGNN:
     def __call__(self, inputs, training=False):
         torch = _lib.require_cuda()
         lib = _lib.load()
-        tape = _active_tape() if training else None
+        tape = _active_tape()
+        watched = self._watched_inputs(tape, inputs)
+        if not training and watched is not None:
+            return self._call_attr(tape, inputs, watched)
+        tape = tape if training else None
         batch, keep = self._prepare(inputs, need_transpose=tape is not None)
         ws = self._workspace(batch, training)
         drop = self._call_dropout(training)
@@ -289,9 +337,98 @@ class GeneralGNN:
         out._gcs_activation = self.cfg.activation
         if tape is not None:
             tape.model = self
-            tape.ctx = dict(batch=batch, keep=keep, ws=ws, out=out, dropout=drop)
+            tape.ctx = dict(batch=batch, keep=keep, ws=ws, out=out, dropout=drop, mode="training", inputs=watched)
             out._gcs_tape = tape
         return out
+
+    # ------------------------------------------------------------------ attributions
+    def _watched_inputs(self, tape, inputs):
+        """What of ``inputs`` the active tape watches (_WatchedInputs), or None when it watches none of them."""
+        if tape is None or not isinstance(inputs, (list, tuple)) or len(inputs) < 2:
+            return None
+        x, a = inputs[0], inputs[1]
+        ew = getattr(a, "edge_weight", None)
+        wx = tape._is_watched(x)
+        wa = tape._is_watched(a) or tape._is_watched(ew)
+        if not (wx or wa):
+            return None
+        dtype = getattr(x, "dtype", None)
+        return _WatchedInputs(x if wx else None, dtype, a if tape._is_watched(a) else None,
+                              ew if tape._is_watched(ew) else None, self.use_edge_weights)
+
+    def _call_attr(self, tape, inputs, watched):
+        """model(inputs, training=False) under a tape watching an input: the attribution forward on a training-mode
+        workspace (the inference result; the activations stay for _input_grad)."""
+        torch = _lib.require_cuda()
+        lib = _lib.load()
+        batch, keep = self._prepare(inputs, need_transpose=True)
+        ws = self._workspace(batch, True)
+        out = torch.empty(self._rows_out(batch), self.cfg.output, dtype=torch.float32, device="cuda")
+        check(lib.gcs_model_forward_attr(self._c, ptr(self.params), ptr(self.state), batch, ptr(out), ptr(ws),
+                                         ws.numel(), stream_ptr()), "gcs_model_forward_attr")
+        off = lib.gcs_model_logits_offset(self._c, batch.n_nodes, batch.n_graphs, 1)
+        out._gcs_logits = ws[off:off + out.numel() * 4].view(torch.float32).view(out.shape)
+        out._gcs_activation = self.cfg.activation
+        out._gcs_tape = tape
+        tape.model = self
+        tape.loss_record = None
+        tape.ctx = dict(batch=batch, keep=keep, ws=ws, out=out, dropout=None, mode="inference", inputs=watched)
+        return out
+
+    def _input_grad(self, tape, target, sources, output_gradients):
+        """tape.gradient with watched inputs among the sources: one gcs_model_input_grad call."""
+        torch = _lib.require_cuda()
+        lib = _lib.load()
+        ctx = tape.ctx
+        inputs = ctx["inputs"]
+        training = ctx["mode"] == "training"
+        out = ctx["out"]
+        if target is out:
+            rows, C = out.shape
+            d = (torch.ones_like(out) if output_gradients is None
+                 else _lib.as_tensor(output_gradients).to(device="cuda", dtype=torch.float32).contiguous())
+            if tuple(d.shape) != (rows, C):
+                raise ValueError(f"output_gradients must be [{rows}, {C}], got {tuple(d.shape)}")
+            dlogits = torch.empty_like(out)
+            from .params import FINAL_ACT
+            check(lib.gcs_output_grad(FINAL_ACT[self.cfg.activation], ptr(out), ptr(d), rows, C, ptr(dlogits),
+                                      stream_ptr()), "gcs_output_grad")
+        else:
+            if output_gradients is not None:
+                raise ValueError("GradientTape.gradient: output_gradients applies to the model output, not a loss")
+            if tape.loss_record is None:
+                raise RuntimeError("GradientTape.gradient: the target is neither the recorded model output nor a "
+                                   "loss computed from it under this tape")
+            dlogits = tape.loss_record["dlogits"]
+        kinds = [inputs.kind(v) for v in sources]
+        by_name = {v.name: v for v in self.trainable_variables}
+        want_params = any(k is None and getattr(v, "name", None) in by_name for v, k in zip(sources, kinds))
+        if want_params and not training:
+            raise NotImplementedError("GradientTape.gradient: parameter gradients of a training=False call are not "
+                                      "built; call the model with training=True for them")
+        batch = ctx["batch"]
+        dx = (torch.empty(batch.n_nodes, self.cfg.in_features, dtype=torch.float32, device="cuda")
+              if "x" in kinds else None)
+        dv = torch.empty(batch.nnz, dtype=torch.float32, device="cuda") if "ew" in kinds else None
+        check(lib.gcs_model_input_grad(self._c, ptr(self.params), batch, int(training), ptr(dlogits), ptr(dx),
+                                       self.cfg.in_features, ptr(dv), ptr(self.grads) if training else None,
+                                       ptr(ctx["ws"]), ctx["ws"].numel(), stream_ptr(), ctx["dropout"]),
+              "gcs_model_input_grad")
+        if dx is not None and inputs.x_dtype == torch.float64:
+            dx = dx.double()                              # Keras autocast: the gradient in the input's dtype
+        res = []
+        for v, k in zip(sources, kinds):
+            if k == "x":
+                res.append(dx)
+            elif k == "ew":
+                res.append(dv)
+            elif k == "unconnected":
+                res.append(None)
+            elif getattr(v, "name", None) in by_name:
+                res.append(by_name[v.name].grad_view)
+            else:
+                res.append(None)                          # not watched and not a variable: unconnected, as in TF
+        return res
 
     call = __call__
 

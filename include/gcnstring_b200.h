@@ -249,6 +249,21 @@ int gcs_spmm_aggregate_bwd(const int32_t* rowptr_t, const int32_t* colidx_t, con
                            const float* scale, const float* shift, const float* alpha, const float* Z, int64_t ldz,
                            float* ties, int64_t ldt, float* dA, int64_t ldda, int32_t H, gcs_stream stream);
 
+/* Gradient of gcs_spmm_aggregate with respect to its per-entry weights (an SDDMM over the forward pattern): for stored
+ * entry e = (i, j) of row i, with a = f(X) the transformed rows the aggregation read,
+ *   sum : dvalues[e] = sum_c dZ[i, c] * a[j, c]          mean: the same / (entries of row i)
+ *   max : the same over the columns where values[e] * a[j, c] attains Z[i, c] only, each divided by the tie count
+ *         ties[i, c] that gcs_spmm_aggregate_bwd (aggregate = 2) left in its `ties` scratch - call it first, with the
+ *         same forward pattern, X, prologue and Z.
+ * Output in forward CSR order (the order of `values`); accumulate != 0 adds to dvalues.  One writer per entry, no
+ * atomics: bit-identical from run to run.  H <= 512.  The reference's tf.GradientTape.gradient(pred, a.values) for the
+ * edge weights of its `use_edge_data` switch (gcn.py:73-80). */
+int gcs_spmm_edge_grad(const int32_t* rowptr, const int32_t* colidx, const float* values, int64_t n_rows,
+                       const float* dZ, int64_t lddz, int32_t aggregate, const float* X, int64_t ldx,
+                       const float* scale, const float* shift, const float* alpha, const float* Z, int64_t ldz,
+                       const float* ties, int64_t ldt, int32_t H, float* dvalues, int32_t accumulate,
+                       gcs_stream stream);
+
 /* ---------------------------------------------------------------------------------
  * K4/K6  GlobalSumPool = tf.math.segment_sum(X, i) over sorted graph ids, and its
  * gradient dX[n] = dOut[i[n]].
@@ -601,6 +616,32 @@ int gcs_model_train_step_dp_ex(const gcs_model_config* cfg, const float* params,
 int gcs_model_backward_ex(const gcs_model_config* cfg, const float* params, const gcs_batch* batch,
                           const float* dlogits, float* grads, void* workspace, int64_t workspace_bytes,
                           gcs_stream stream, const gcs_dropout* dropout);
+
+/* Attributions: gradients with respect to the model's inputs, the saliency pattern of
+ *   with tf.GradientTape() as tape: tape.watch(x); pred = model([x, a, i], training=False)
+ *   tape.gradient(pred, [x, a.values], output_gradients=...)
+ * gcs_model_forward_attr: the inference forward (moving statistics, no dropout, no moving-statistics update) on a
+ * training-mode workspace (gcs_model_workspace_bytes(..., training = 1)), every dense block unfused so that the
+ * activations stay there for gcs_model_input_grad.  Its `out` equals gcs_model_forward(training = 0) to float32
+ * rounding (the plain inference path folds BatchNorm into the GEMM).
+ * gcs_model_input_grad: the reverse pass from dlogits [rows_out, C] after either forward, same workspace and batch
+ * (with the transposed CSR):
+ *   training = 0 (after gcs_model_forward_attr): BatchNorm on the moving statistics; grads must be NULL
+ *                (parameter gradients of an inference-mode call are not built: GCS_ERR_UNSUPPORTED);
+ *   training = 1 (after gcs_model_forward_ex(training = 1) with the same `dropout`): the parameter gradients into grads
+ *                (required) exactly as gcs_model_backward_ex computes them.
+ *   dx      [n_nodes, in_features] (ld lddx), optional: dLoss/dx;
+ *   dvalues [nnz], optional, only with batch->values: dLoss/d(edge weights) in forward CSR order, the L GeneralConv
+ *           layers summed in a fixed order (gcs_spmm_edge_grad).
+ * gcs_output_grad: dlogits = J^T dprobs of the head's activation on its output probs [rows, C] - softmax
+ * p * (d - p . d), sigmoid d * p (1 - p), linear d - for a gradient of the model output itself (output_gradients). */
+int gcs_model_forward_attr(const gcs_model_config* cfg, const float* params, float* state, const gcs_batch* batch,
+                           float* out, void* workspace, int64_t workspace_bytes, gcs_stream stream);
+int gcs_model_input_grad(const gcs_model_config* cfg, const float* params, const gcs_batch* batch, int32_t training,
+                         const float* dlogits, float* dx, int64_t lddx, float* dvalues, float* grads, void* workspace,
+                         int64_t workspace_bytes, gcs_stream stream, const gcs_dropout* dropout);
+int gcs_output_grad(int32_t final_activation, const float* probs, const float* dprobs, int64_t rows, int32_t C,
+                    float* dlogits, gcs_stream stream);
 
 #ifdef __cplusplus
 }
