@@ -269,34 +269,50 @@ class _PinnedRing:
         return dev
 
 
-class DeviceGraphStore:
-    """The packed dataset resident in HBM + the host-side per-graph sizes."""
+def _pin(a):
+    """A pinned host copy of the NumPy array ``a``."""
+    return _lib.require_cuda().from_numpy(np.ascontiguousarray(a)).pin_memory()
 
-    def __init__(self, packed: PackedGraphs, symmetric: Optional[bool] = None):
-        torch = _lib.require_cuda()
-        _lib.load()
+
+def _gather_node_rows(graph_ids, node_off, src, graph_ptr, out):
+    """``out[graph_ptr[k]:graph_ptr[k+1]] = src[node_off[g]:node_off[g+1]]`` for ``g = graph_ids[k]``: the per-node rows
+    (``src`` [*, width], or [*] at width 1) of a batch's graphs, in batch order."""
+    width = int(src.shape[1]) if src.dim() == 2 else 1
+    check(_lib.load().gcs_gather_node_rows(ptr(graph_ids), int(graph_ids.shape[0]), ptr(node_off), ptr(src), width,
+                                           ptr(graph_ptr), ptr(out), stream_ptr()), "gcs_gather_node_rows")
+    return out
+
+
+class _GraphStore:
+    """What both stores keep of a packed dataset: per-graph sizes on the host, ``node_off`` / ``rowptr`` / ``col`` /
+    ``x`` / ``y`` (``y`` None without labels) in memory the device can address, and the assembly of a batch from them
+    or from a per-step copy of part of them."""
+
+    def __init__(self, packed: PackedGraphs, symmetric: Optional[bool], to_device):
         self.n_graphs = packed.n_graphs
         self.n_feat = int(packed.x.shape[1])
         self.n_classes = int(packed.y.shape[1]) if packed.y.ndim == 2 else 0
         self.h_n_nodes = packed.n_nodes.astype(np.int64)
         self.h_n_edges = packed.n_edges.astype(np.int64)
-        self.node_off = torch.from_numpy(packed.node_off).cuda()
-        self.rowptr = torch.from_numpy(packed.rowptr).cuda()
-        self.col = torch.from_numpy(packed.col).cuda()
-        self.x = torch.from_numpy(np.ascontiguousarray(packed.x, dtype=np.float32)).cuda()
-        self.y = torch.from_numpy(np.ascontiguousarray(packed.y, dtype=np.float32)).cuda() if self.n_classes else None
         self.node_level = bool(packed.node_level)
         self.symmetric = symmetric
+        self.node_off, self.rowptr, self.col = to_device(packed.node_off), to_device(packed.rowptr), to_device(packed.col)
+        self.x = to_device(packed.x.astype(np.float32, copy=False))
+        self.y = to_device(packed.y.astype(np.float32, copy=False)) if self.n_classes else None
 
-    def batch(self, graph_ids_dev, graph_ids_host, want_coo=False, want_labels=True):
-        """Run K0 for the graphs ``graph_ids`` (device int64 tensor + the same ids on host); node labels are then
-        gathered by gcs_gather_node_rows at the graph offsets K0 wrote."""
+    def _assemble(self, ids_dev, ids_host, want_coo, src=None, base=(0, 0, 0), node_y=None, label_ids=None):
+        """Run K0 for one batch.  ``src`` = (node_off, rowptr, col, x, graph labels or None): the arrays the kernel
+        reads, by default the store's own; they hold the dataset from graph, node and entry ``base`` = (g0, n0, e0) on,
+        and ``ids_dev`` addresses their graphs by that numbering.  ``ids_host`` are the batch's dataset graph ids.  Node
+        labels are ``node_y`` when the caller has them in batch order already, else gathered from the store's own at the
+        graph offsets K0 wrote, for the dataset graph ids ``label_ids`` (default ``ids_dev``)."""
         torch = _lib.require_cuda()
-        lib = _lib.load()
-        b = int(graph_ids_host.shape[0])
-        n = int(self.h_n_nodes[graph_ids_host].sum())
-        nnz = int(self.h_n_edges[graph_ids_host].sum())
-        max_nodes = int(self.h_n_nodes[graph_ids_host].max()) if b else 0
+        s_node_off, s_rowptr, s_col, s_x, s_y = src or (self.node_off, self.rowptr, self.col, self.x,
+                                                        None if self.node_level else self.y)
+        b = int(ids_host.shape[0])
+        n = int(self.h_n_nodes[ids_host].sum())
+        nnz = int(self.h_n_edges[ids_host].sum())
+        max_nodes = int(self.h_n_nodes[ids_host].max()) if b else 0
         i32 = dict(dtype=torch.int32, device="cuda")
         graph_ptr = torch.empty(b + 1, **i32)
         edge_ptr = torch.empty(b + 1, **i32)
@@ -304,29 +320,45 @@ class DeviceGraphStore:
         colidx = ops.empty_bucketed(nnz, dtype=torch.int32)
         x = ops.empty_bucketed(n, self.n_feat, dtype=torch.float32)
         seg = ops.empty_bucketed(n, dtype=torch.int64)
-        y = None
-        if want_labels and self.y is not None:
-            y = (ops.empty_bucketed(n, self.n_classes, dtype=torch.float32) if self.node_level
-                 else torch.empty(b, self.n_classes, dtype=torch.float32, device="cuda"))
+        if not self.node_level:
+            y = torch.empty(b, self.n_classes, dtype=torch.float32, device="cuda") if s_y is not None else None
+        elif node_y is None and self.y is not None:
+            y = ops.empty_bucketed(n, self.n_classes, dtype=torch.float32)
+        else:
+            y = node_y
         coo = ops.empty_bucketed(nnz, 2, dtype=torch.int64) if want_coo else None
         flag = torch.zeros(1, **i32)
-        graph_y = None if self.node_level else self.y
-        check(lib.gcs_batch_disjoint(ptr(self.node_off), ptr(self.rowptr), ptr(self.col), ptr(self.x), ptr(graph_y),
-                                     self.n_feat, max(self.n_classes, 1), ptr(graph_ids_dev), b, n, nnz,
-                                     ptr(graph_ptr), ptr(edge_ptr), ptr(rowptr), ptr(colidx), ptr(x), ptr(seg),
-                                     None if self.node_level else ptr(y), ptr(coo), ptr(flag), stream_ptr()),
-              "gcs_batch_disjoint")
-        if self.node_level and y is not None:
-            check(lib.gcs_gather_node_rows(ptr(graph_ids_dev), b, ptr(self.node_off), ptr(self.y), self.n_classes,
-                                           ptr(graph_ptr), ptr(y), stream_ptr()), "gcs_gather_node_rows")
+        g0, n0, e0 = base
+        # rebased pointers instead of rebased index arrays: the kernel only touches graphs, nodes and entries of the batch
+        check(_lib.load().gcs_batch_disjoint(
+            ptr(s_node_off) - 8 * g0, ptr(s_rowptr) - 8 * n0, ptr(s_col) - 4 * e0, ptr(s_x) - 4 * self.n_feat * n0,
+            ptr(s_y) - 4 * self.n_classes * g0 if s_y is not None else None, self.n_feat, max(self.n_classes, 1),
+            ptr(ids_dev), b, n, nnz, ptr(graph_ptr), ptr(edge_ptr), ptr(rowptr), ptr(colidx), ptr(x), ptr(seg),
+            None if self.node_level else ptr(y), ptr(coo), ptr(flag), stream_ptr()), "gcs_batch_disjoint")
+        if self.node_level and node_y is None and y is not None:
+            _gather_node_rows(ids_dev if label_ids is None else label_ids, self.node_off, self.y, graph_ptr, y)
         a = SparseAdjacency(rowptr, colidx, n, graph_ptr=graph_ptr, max_graph_nodes=max_nodes, indices=coo,
                             symmetric=self.symmetric)
-        a.edge_ptr = edge_ptr
-        a.status = flag
+        a.edge_ptr, a.status = edge_ptr, flag
+        a._keep = (src, ids_dev)
         return x, a, seg, y
 
 
-class HostGraphStore:
+class DeviceGraphStore(_GraphStore):
+    """The packed dataset resident in HBM + the host-side per-graph sizes."""
+
+    def __init__(self, packed: PackedGraphs, symmetric: Optional[bool] = None):
+        torch = _lib.require_cuda()
+        _lib.load()
+        super().__init__(packed, symmetric, lambda a: torch.from_numpy(np.ascontiguousarray(a)).cuda())
+
+    def batch(self, graph_ids_dev, graph_ids_host, want_coo=False):
+        """Run K0 for the graphs ``graph_ids`` (device int64 tensor + the same ids on host); node labels are then
+        gathered by gcs_gather_node_rows at the graph offsets K0 wrote."""
+        return self._assemble(graph_ids_dev, graph_ids_host, want_coo)
+
+
+class HostGraphStore(_GraphStore):
     """Streaming variant: the packed dataset stays in PINNED host memory and every step moves only the graphs of its
     batch to the device, inside the step.
     ``zero_copy=False`` (default): consecutive graph ids (shuffle=False) are uploaded as slices with cudaMemcpyAsync; a
@@ -343,163 +375,78 @@ class HostGraphStore:
         # device_gather=True: a non-consecutive (shuffled) batch is gathered by gcs_gather_graphs - a kernel that copies
         # each selected graph's slices out of the pinned arrays in coalesced runs - instead of a Python loop on the host
         self.device_gather = bool(device_gather)
-        torch = _lib.require_cuda()
         _lib.load()
-        self.n_graphs = packed.n_graphs
-        self.n_feat = int(packed.x.shape[1])
-        self.n_classes = int(packed.y.shape[1]) if packed.y.ndim == 2 else 0
-        self.h_n_nodes = packed.n_nodes.astype(np.int64)
-        self.h_n_edges = packed.n_edges.astype(np.int64)
-        self.h_node_off = packed.node_off
-        self.h_rowptr = packed.rowptr
-        pin = lambda a: torch.from_numpy(np.ascontiguousarray(a)).pin_memory()   # noqa: E731
-        self.node_off, self.rowptr, self.col = pin(packed.node_off), pin(packed.rowptr), pin(packed.col)
-        self.x = pin(packed.x.astype(np.float32, copy=False))
-        self.y = pin(packed.y.astype(np.float32, copy=False)) if self.n_classes else None
-        self.node_level = bool(packed.node_level)
-        self.symmetric = symmetric
+        super().__init__(packed, symmetric, _pin)
+        # NumPy views of the pinned arrays: the host-side reads of a step never touch `packed`, which may be a memory map
+        no_y = np.zeros((int(packed.node_off[-1]) if self.node_level else self.n_graphs, 0), np.float32)
+        self._host = PackedGraphs(self.node_off.numpy(), self.rowptr.numpy(), self.col.numpy(), self.x.numpy(),
+                                  self.y.numpy() if self.y is not None else no_y, self.node_level)
         self.h2d_bytes_last = 0
         self._ring = _PinnedRing(depth=6)
 
-    def _gather(self, ids):
-        """Pack the graphs ``ids`` (any order) into a fresh pinned mini-dataset."""
-        torch = _lib.require_cuda()
-        sub = PackedGraphs(*_take_graphs(self, ids), node_level=self.node_level)
-        pin = lambda a: torch.from_numpy(np.ascontiguousarray(a)).pin_memory()   # noqa: E731
-        return pin(sub.node_off), pin(sub.rowptr), pin(sub.col), pin(sub.x), (pin(sub.y) if self.n_classes else None)
+    def _graph_bytes(self, b, n, nnz):
+        """Bytes a kernel pulls over the host link for b graphs of n nodes and nnz entries: per graph its node offsets,
+        row pointers, columns, features, labels."""
+        return 16 * b + 8 * (n + b) + 4 * nnz + 4 * self.n_feat * n + 4 * self.n_classes * (n if self.node_level else b)
 
-    def batch(self, graph_ids_dev, graph_ids_host, want_coo=False, want_labels=True):
+    def batch(self, graph_ids_dev, graph_ids_host, want_coo=False):
         torch = _lib.require_cuda()
-        lib = _lib.load()
         ids = np.asarray(graph_ids_host, dtype=np.int64)
         b = int(ids.shape[0])
         consecutive = b > 0 and np.array_equal(ids, np.arange(ids[0], ids[0] + b))
         if self.zero_copy:
-            parts = (self.node_off, self.rowptr, self.col, self.x, self.y)           # the pinned dataset itself
-            g0 = n0 = e0 = 0
-            ids_local = torch.from_numpy(ids)
-        elif consecutive:
-            g0, g1 = int(ids[0]), int(ids[0]) + b
-            n0, n1 = int(self.h_node_off[g0]), int(self.h_node_off[g1])
-            e0, e1 = int(self.h_rowptr[n0]), int(self.h_rowptr[n1])
-            y_rows = (n0, n1) if self.node_level else (g0, g1)        # node labels: one contiguous node range
-            parts = (self.node_off[g0:g1 + 1], self.rowptr[n0:n1 + 1], self.col[e0:e1], self.x[n0:n1],
-                     self.y[y_rows[0]:y_rows[1]] if self.y is not None else None)
-            ids_local = torch.arange(g0, g1, dtype=torch.int64)
-        elif self.device_gather:
-            parts = None
-            g0 = n0 = e0 = 0
-            ids_local = torch.arange(0, b, dtype=torch.int64)
-        else:
-            parts = self._gather(ids)
-            g0 = n0 = e0 = 0
-            ids_local = torch.arange(0, b, dtype=torch.int64)
-        n = int(self.h_n_nodes[ids].sum())
-        nnz = int(self.h_n_edges[ids].sum())
-        if self.zero_copy:
-            dev = list(parts)
             # uploaded on THIS stream: with prefetch the kernel runs on a side stream, which is not ordered after the
             # loader's asynchronous upload of the epoch order (graph_ids_dev)
-            ids_dev = self._ring.upload(ids_local.numpy())
-            # bytes the kernel pulls over the host link: per graph its node offsets, row pointers, columns, features, label
-            self.h2d_bytes_last = (16 * b + 8 * (n + b) + 4 * nnz + 4 * self.n_feat * n
-                                   + 4 * self.n_classes * (n if self.node_level else b) + 8 * b)
-        elif parts is None:
+            ids_dev = self._ring.upload(ids)
+            out = self._assemble(ids_dev, ids, want_coo)          # the kernel reads the pinned dataset itself
+            self.h2d_bytes_last = self._graph_bytes(b, out[1].n_rows, out[1].nnz) + 8 * b
+            return out
+        if self.device_gather and not consecutive:
             # the selected graphs' offsets in the mini-dataset (host knows the sizes), then one gather kernel
             off = np.zeros((3, b + 1), dtype=np.int64)
             np.cumsum(self.h_n_nodes[ids], out=off[0, 1:])
             np.cumsum(self.h_n_edges[ids], out=off[1, 1:])
             off[2, :b] = ids
+            n, nnz = int(off[0, b]), int(off[1, b])
             off_dev = self._ring.upload(off)
-            d_node_off = off_dev[0]
             d_rowptr = ops.empty_bucketed(n + 1, dtype=torch.int64)
             d_col = ops.empty_bucketed(max(nnz, 1), dtype=torch.int32)
             d_x = ops.empty_bucketed(max(n, 1), self.n_feat, dtype=torch.float32)
             # node labels are gathered straight into the batch after K0 (gcs_gather_node_rows), not into the mini-dataset
             graph_y = None if self.node_level else self.y
             d_y = torch.empty(b, self.n_classes, dtype=torch.float32, device="cuda") if graph_y is not None else None
-            check(lib.gcs_gather_graphs(ptr(off_dev[2]), b, ptr(self.node_off), ptr(self.rowptr), ptr(self.col), ptr(self.x),
-                                        ptr(graph_y), self.n_feat, self.n_classes, ptr(off_dev[0]), ptr(off_dev[1]),
-                                        ptr(d_rowptr), ptr(d_col), ptr(d_x), ptr(d_y), stream_ptr()), "gcs_gather_graphs")
-            dev = [d_node_off, d_rowptr, d_col, d_x, d_y]
-            ids_dev = self._ring.upload(ids_local.numpy())
-            self.h2d_bytes_last = (16 * b + 8 * (n + b) + 4 * nnz + 4 * self.n_feat * n
-                                   + 4 * self.n_classes * (n if self.node_level else b) + 24 * (b + 1))
+            check(_lib.load().gcs_gather_graphs(
+                ptr(off_dev[2]), b, ptr(self.node_off), ptr(self.rowptr), ptr(self.col), ptr(self.x), ptr(graph_y),
+                self.n_feat, self.n_classes, ptr(off_dev[0]), ptr(off_dev[1]), ptr(d_rowptr), ptr(d_col), ptr(d_x),
+                ptr(d_y), stream_ptr()), "gcs_gather_graphs")
+            ids_dev = self._ring.upload(np.arange(b, dtype=np.int64))
+            self.h2d_bytes_last = self._graph_bytes(b, n, nnz) + 24 * (b + 1)
+            return self._assemble(ids_dev, ids, want_coo, (off_dev[0], d_rowptr, d_col, d_x, d_y),
+                                  label_ids=off_dev[2, :b])
+        if consecutive:
+            g0, g1 = int(ids[0]), int(ids[0]) + b
+            n0, n1, e0, e1 = self._host.span(g0, g1)
+            y_rows = (n0, n1) if self.node_level else (g0, g1)        # node labels: one contiguous node range
+            parts = (self.node_off[g0:g1 + 1], self.rowptr[n0:n1 + 1], self.col[e0:e1], self.x[n0:n1],
+                     self.y[y_rows[0]:y_rows[1]] if self.y is not None else None)
+            base, ids_local = (g0, n0, e0), np.arange(g0, g1, dtype=np.int64)
         else:
-            dev = []
-            for t in parts:                              # pinned slices -> bucketed device buffers
-                if t is None:
-                    dev.append(None)
-                    continue
+            sub = self._host.take(ids)
+            parts = (_pin(sub.node_off), _pin(sub.rowptr), _pin(sub.col), _pin(sub.x), _pin(sub.y) if self.n_classes else None)
+            base, ids_local = (0, 0, 0), np.arange(b, dtype=np.int64)
+        dev = []
+        for t in parts:                              # pinned slices -> bucketed device buffers
+            d = None
+            if t is not None:
                 d = ops.empty_bucketed(t.shape[0], *t.shape[1:], dtype=t.dtype)
                 d.copy_(t, non_blocking=True)
-                dev.append(d)
-            ids_dev = self._ring.upload(ids_local.numpy())
-            self.h2d_bytes_last = sum(t.numel() * t.element_size() for t in parts if t is not None) + ids_local.numel() * 8
-        d_node_off, d_rowptr, d_col, d_x, d_y = dev
-        max_nodes = int(self.h_n_nodes[ids].max()) if b else 0
-        i32 = dict(dtype=torch.int32, device="cuda")
-        graph_ptr, edge_ptr = torch.empty(b + 1, **i32), torch.empty(b + 1, **i32)
-        rowptr, colidx = ops.empty_bucketed(n + 1, dtype=torch.int32), ops.empty_bucketed(nnz, dtype=torch.int32)
-        x = ops.empty_bucketed(n, self.n_feat, dtype=torch.float32)
-        seg = ops.empty_bucketed(n, dtype=torch.int64)
-        coo = ops.empty_bucketed(nnz, 2, dtype=torch.int64) if want_coo else None
-        flag = torch.zeros(1, **i32)
-        if self.node_level:
-            y, graph_y = None, None
-            if want_labels and self.y is not None:
-                if parts is not None and not self.zero_copy:
-                    y = d_y                      # the copied slice / staged rows are already the batch's rows, in order
-                else:
-                    y = ops.empty_bucketed(n, self.n_classes, dtype=torch.float32)
-        else:
-            y = torch.empty(b, self.n_classes, dtype=torch.float32, device="cuda") if (want_labels and d_y is not None) else None
-            graph_y = (ptr(d_y) - 4 * self.n_classes * g0) if d_y is not None else None
-        # the uploaded slices are addressed with DATASET-global ids: rebase the pointers instead
-        # of the index arrays (the kernel only touches [g0, g1], [n0, n1], [e0, e1))
-        check(lib.gcs_batch_disjoint(ptr(d_node_off) - 8 * g0, ptr(d_rowptr) - 8 * n0, ptr(d_col) - 4 * e0,
-                                     ptr(d_x) - 4 * self.n_feat * n0, graph_y,
-                                     self.n_feat, max(self.n_classes, 1), ptr(ids_dev), b, n, nnz, ptr(graph_ptr),
-                                     ptr(edge_ptr), ptr(rowptr), ptr(colidx), ptr(x), ptr(seg),
-                                     None if self.node_level else ptr(y), ptr(coo), ptr(flag), stream_ptr()),
-              "gcs_batch_disjoint")
-        if self.node_level and y is not None and y is not d_y:
-            # zero_copy: the batch's graph ids index the pinned dataset; device_gather: the same ids (off_dev[2])
-            gids = ids_dev if self.zero_copy else off_dev[2]
-            check(lib.gcs_gather_node_rows(ptr(gids), b, ptr(self.node_off), ptr(self.y), self.n_classes, ptr(graph_ptr),
-                                           ptr(y), stream_ptr()), "gcs_gather_node_rows")
-        a = SparseAdjacency(rowptr, colidx, n, graph_ptr=graph_ptr, max_graph_nodes=max_nodes, indices=coo,
-                            symmetric=self.symmetric)
-        a.edge_ptr, a.status = edge_ptr, flag
-        a._keep = (dev, ids_dev)
-        return x, a, seg, y
-
-
-def _take_graphs(store, ids):
-    """Host gather of whole graphs into a packed mini-dataset (node_off, rowptr, col, x, y)."""
-    node_off = np.zeros(len(ids) + 1, dtype=np.int64)
-    np.cumsum(store.h_n_nodes[ids], out=node_off[1:])
-    hn, hr = store.h_node_off, store.h_rowptr
-    col_np, x_np = store.col.numpy(), store.x.numpy()
-    rp_np = store.rowptr.numpy()
-    rps, cols, xs, ys = [], [], [], []
-    e_off = 0
-    y_np = store.y.numpy() if store.y is not None else None
-    for g in ids:
-        n0, n1 = int(hn[g]), int(hn[g + 1])
-        e0, e1 = int(hr[n0]), int(hr[n1])
-        rps.append(rp_np[n0:n1] - e0 + e_off)
-        cols.append(col_np[e0:e1])
-        xs.append(x_np[n0:n1])
-        if store.node_level and y_np is not None:
-            ys.append(y_np[n0:n1])
-        e_off += e1 - e0
-    rowptr = np.concatenate(rps + [np.array([e_off], dtype=np.int64)])
-    if y_np is None:
-        y = np.zeros((len(ids), 0), np.float32)
-    else:
-        y = np.concatenate(ys) if store.node_level else y_np[ids]
-    return node_off, rowptr, np.concatenate(cols), np.concatenate(xs), y
+            dev.append(d)
+        ids_dev = self._ring.upload(ids_local)
+        self.h2d_bytes_last = sum(t.numel() * t.element_size() for t in parts if t is not None) + 8 * b
+        d_y = dev[4]
+        # the copied slice / staged rows of node labels are already the batch's rows, in order
+        return self._assemble(ids_dev, ids, want_coo, dev[:4] + [None if self.node_level else d_y], base,
+                              node_y=d_y if self.node_level else None)
 
 
 class _Spec:
@@ -546,7 +493,7 @@ class DisjointLoader:
             raise ValueError(f"DisjointLoader(node_level={node_level}) got a dataset with "
                              f"{'node' if packed.node_level else 'graph'} labels")
         if symmetric is None:
-            symmetric = getattr(packed, "symmetric", None)      # recorded by the shard writer (shards.py)
+            symmetric = packed.symmetric                         # recorded by the shard writer (shards.py)
         self.dataset = dataset
         # device_resident=False keeps the dataset in pinned host memory and uploads per batch
         self.store = (DeviceGraphStore(packed, symmetric=symmetric) if device_resident
@@ -659,12 +606,10 @@ class DisjointLoader:
                     self._order_dev = self._ring.upload(order_host)
                     self._order_epoch = epoch
                 ids_dev = self._order_dev[lo:hi]
-            staged = None
             x, a, i, y = self.store.batch(ids_dev, ids_host, want_coo=self.want_coo)
             w = self._batch_weights(ids_dev, a) if self._w is not None else None
             a.global_batch_graphs = global_count
             a.global_batch_nodes = global_nodes
-            a._ids_keepalive = (ids_dev, staged)
             event = torch.cuda.Event()
             event.record(stream)
         return (x, a, i, y, w), event
@@ -677,10 +622,8 @@ class DisjointLoader:
         if not self.node_level:
             w = torch.empty(b, dtype=torch.float32, device="cuda")
             return torch.index_select(self._w, 0, ids_dev, out=w)
-        w = ops.empty_bucketed(a.n_rows, dtype=torch.float32)
-        check(_lib.load().gcs_gather_node_rows(ptr(ids_dev), b, ptr(self._w_node_off), ptr(self._w), 1, ptr(a.graph_ptr),
-                                               ptr(w), stream_ptr()), "gcs_gather_node_rows")
-        return w
+        return _gather_node_rows(ids_dev, self._w_node_off, self._w, a.graph_ptr,
+                                 ops.empty_bucketed(a.n_rows, dtype=torch.float32))
 
     def _generate(self):
         torch = _lib.require_cuda()

@@ -34,11 +34,11 @@ from __future__ import annotations
 import json
 import os
 import struct
-from typing import Iterable, List, Optional, Sequence
+from typing import Iterable, List, Optional
 
 import numpy as np
 
-from .synthetic import PackedGraphs, pack_graphs
+from .synthetic import PackedGraphs, concat_packed, pack_graphs
 
 MAGIC = b"GCSSHRD1"
 VERSION = 1                  # graph labels
@@ -96,7 +96,7 @@ def write_shard(path: str, packed: PackedGraphs, symmetric: Optional[bool] = Non
     if packed.rowptr.shape[0] != n + 1 or int(packed.rowptr[-1]) != nnz:
         raise ValueError("inconsistent PackedGraphs: rowptr does not match node_off / col")
     x = np.ascontiguousarray(packed.x, dtype="<f4").reshape(n, -1) if n else np.zeros((0, packed.x.shape[-1]), "<f4")
-    node_level = bool(getattr(packed, "node_level", False))
+    node_level = bool(packed.node_level)
     y = np.ascontiguousarray(packed.y, dtype="<f4").reshape(n if node_level else g, -1)
     if nnz and (packed.col.min() < 0 or (packed.col >= np.repeat(packed.n_nodes, packed.n_edges)).any()):
         raise ValueError("column index outside its graph")
@@ -164,34 +164,10 @@ def read_shard(path: str, mmap: bool = True, verify: bool = False) -> PackedGrap
         arrs[name] = buf[off:off + nbytes].view(dt).reshape(shape)
     if verify and _checksum([arrs[k] for k in ("node_off", "rowptr", "col", "x", "y")]) != h.checksum:
         raise ValueError(f"{path}: payload checksum mismatch")
-    p = PackedGraphs(arrs["node_off"], arrs["rowptr"], arrs["col"], arrs["x"], arrs["y"], h.node_level)
+    p = PackedGraphs(arrs["node_off"], arrs["rowptr"], arrs["col"], arrs["x"], arrs["y"], h.node_level, h.symmetric)
     if h.n_graphs and (int(p.node_off[-1]) != h.n_nodes or int(p.rowptr[-1]) != h.nnz or int(p.node_off[0]) != 0):
         raise ValueError(f"{path}: offsets disagree with the header")
-    p.symmetric = h.symmetric
     return p
-
-
-def concat_packed(parts: Sequence[PackedGraphs]) -> PackedGraphs:
-    """Concatenate packed datasets (graph order preserved, offsets rebased).  Graph- and node-labelled parts do not
-    mix."""
-    if len({bool(getattr(p, "node_level", False)) for p in parts}) > 1:
-        raise ValueError("cannot concatenate graph-labelled and node-labelled shards")
-    parts = [p for p in parts if p.n_graphs]
-    if not parts:
-        raise ValueError("nothing to concatenate")
-    if len(parts) == 1:
-        return parts[0]
-    node_off, rowptr = [np.zeros(1, np.int64)], [np.zeros(1, np.int64)]
-    n0 = e0 = 0
-    for p in parts:
-        node_off.append(np.asarray(p.node_off[1:], dtype=np.int64) + n0)
-        rowptr.append(np.asarray(p.rowptr[1:], dtype=np.int64) + e0)
-        n0 += int(p.node_off[-1])
-        e0 += int(p.rowptr[-1])
-    out = PackedGraphs(np.concatenate(node_off), np.concatenate(rowptr), np.concatenate([p.col for p in parts]),
-                       np.concatenate([p.x for p in parts]), np.concatenate([p.y for p in parts]), parts[0].node_level)
-    out.symmetric = all(getattr(p, "symmetric", False) for p in parts)
-    return out
 
 
 def write_dataset(graphs: Iterable, out_dir: str, graphs_per_shard: int = 4096, prefix: str = "shard",
@@ -236,7 +212,10 @@ def load_dataset(out_dir_or_paths, mmap: bool = True, verify: bool = False) -> P
         paths = [os.path.join(d, s["file"]) for s in idx["shards"]]
     else:
         paths = list(out_dir_or_paths)
-    return concat_packed([read_shard(p, mmap=mmap, verify=verify) for p in paths])
+    packed = concat_packed([read_shard(p, mmap=mmap, verify=verify) for p in paths])
+    if packed.n_graphs == 0:
+        raise ValueError("nothing to concatenate")
+    return packed
 
 
 def graph_from_networkx(G, label, feature_name: str = "x"):

@@ -24,8 +24,9 @@ regenerated alone.  The output is the packed layout the device batching kernel c
 """
 from __future__ import annotations
 
+import dataclasses
 from dataclasses import dataclass
-from typing import List
+from typing import Optional, Sequence
 
 import numpy as np
 
@@ -39,6 +40,8 @@ class PackedGraphs:
     col[sumNNZ]    int32  neighbour index LOCAL to the graph, ascending within a row
     x[sumN, F]     float32
     y[G, C]        float32 one-hot graph labels, or y[sumN, C] node labels (rows in node order) when node_level
+    symmetric      True when every graph's pattern equals its transpose (a shard header records it), False when some
+                   graph's does not, None when unknown: the loader then checks each batch's pattern on the device
     """
     node_off: np.ndarray
     rowptr: np.ndarray
@@ -46,6 +49,26 @@ class PackedGraphs:
     x: np.ndarray
     y: np.ndarray
     node_level: bool = False
+    symmetric: Optional[bool] = None
+
+    @classmethod
+    def from_graphs(cls, rowptrs, cols, xs, ys, node_level: bool = False, n_feat: int = 0, n_classes: int = 0,
+                    symmetric: Optional[bool] = None) -> "PackedGraphs":
+        """Pack per-graph pieces, in order: local ``rowptr [n+1]``, ``col [nnz]`` int32, ``x [n, F]`` float32, and a label
+        row ``y [C]`` per graph or, with ``node_level``, ``y [n, C]``, all float32.  ``n_feat`` / ``n_classes`` are the
+        widths of ``x`` / ``y`` when there are no graphs."""
+        node_off = np.zeros(len(xs) + 1, dtype=np.int64)
+        np.cumsum([x.shape[0] for x in xs], out=node_off[1:])
+        e_off = np.zeros(len(rowptrs) + 1, dtype=np.int64)
+        np.cumsum([rp[-1] for rp in rowptrs], out=e_off[1:])
+        rowptr = np.concatenate([np.asarray(rp[:-1], dtype=np.int64) + e for rp, e in zip(rowptrs, e_off)] + [e_off[-1:]])
+        col = np.concatenate(cols) if cols else np.zeros(0, np.int32)
+        x = np.concatenate(xs) if xs else np.zeros((0, n_feat), np.float32)
+        if not ys:
+            y = np.zeros((0, n_classes), np.float32)
+        else:
+            y = np.concatenate(ys) if node_level else np.stack(ys)
+        return cls(node_off, rowptr, col, x, y, node_level, symmetric)
 
     @property
     def n_graphs(self) -> int:
@@ -59,16 +82,56 @@ class PackedGraphs:
     def n_edges(self) -> np.ndarray:
         return self.rowptr[self.node_off[1:]] - self.rowptr[self.node_off[:-1]]
 
+    def span(self, g0: int, g1: int):
+        """(n0, n1, e0, e1): the graphs [g0, g1) hold the nodes [n0, n1) of ``x`` / ``rowptr`` and the entries [e0, e1) of
+        ``col``."""
+        n0, n1 = int(self.node_off[g0]), int(self.node_off[g1])
+        return n0, n1, int(self.rowptr[n0]), int(self.rowptr[n1])
+
     def graph(self, g: int):
         """(x[n,F], scipy CSR int64 ones [n,n], y[C]) for graph g — the per-graph objects
         the reference's MyDataset hands to Spektral (src/scripts/gcn.py:161-181)."""
         import scipy.sparse as sp
-        n0, n1 = int(self.node_off[g]), int(self.node_off[g + 1])
-        e0, e1 = int(self.rowptr[n0]), int(self.rowptr[n1])
+        n0, n1, e0, e1 = self.span(g, g + 1)
         n = n1 - n0
         a = sp.csr_matrix((np.ones(e1 - e0, dtype=np.int64), self.col[e0:e1].astype(np.int32),
                            (self.rowptr[n0:n1 + 1] - e0).astype(np.int32)), shape=(n, n))
         return self.x[n0:n1], a, (self.y[n0:n1] if self.node_level else self.y[g])
+
+    def take(self, ids) -> "PackedGraphs":
+        """A new pack of the graphs ``ids``, in that order (a graph may repeat)."""
+        spans = [self.span(g, g + 1) for g in ids]
+        return PackedGraphs.from_graphs(
+            [self.rowptr[n0:n1 + 1] - e0 for n0, n1, e0, _ in spans], [self.col[e0:e1] for _, _, e0, e1 in spans],
+            [self.x[n0:n1] for n0, n1, _, _ in spans],
+            [self.y[n0:n1] for n0, n1, _, _ in spans] if self.node_level else [self.y[g] for g in ids],
+            self.node_level, self.x.shape[1], self.y.shape[1], self.symmetric)
+
+
+def concat_packed(parts: Sequence[PackedGraphs]) -> PackedGraphs:
+    """Concatenate packed datasets (graph order = order of the parts, offsets rebased).  Graph- and node-labelled parts
+    do not mix.  Parts without graphs are skipped, and a single remaining part is returned itself, not a copy.  The
+    result is symmetric when every part is, not symmetric when any part is not, and unknown otherwise."""
+    if len({bool(p.node_level) for p in parts}) > 1:
+        raise ValueError("cannot concatenate graph-labelled and node-labelled datasets")
+    if not parts:
+        raise ValueError("nothing to concatenate")
+    parts = [p for p in parts if p.n_graphs] or list(parts[:1])
+    if len(parts) == 1:
+        return parts[0]
+    node_off, rowptr = [np.zeros(1, np.int64)], []
+    n0 = e0 = 0
+    for p in parts:
+        node_off.append(p.node_off[1:] + n0)
+        rowptr.append(p.rowptr[:-1] - p.rowptr[0] + e0)
+        n0 += int(p.node_off[-1])
+        e0 += int(p.rowptr[-1] - p.rowptr[0])
+    rowptr.append(np.array([e0], dtype=np.int64))
+    sym = [p.symmetric for p in parts]
+    symmetric = False if any(s is False for s in sym) else (True if all(sym) else None)
+    return PackedGraphs(np.concatenate(node_off), np.concatenate(rowptr), np.concatenate([p.col for p in parts]),
+                        np.concatenate([p.x for p in parts]), np.concatenate([p.y for p in parts]), parts[0].node_level,
+                        symmetric)
 
 
 def _protein_pairs(rng, n, deg):
@@ -155,13 +218,14 @@ def regression_targets(packed: PackedGraphs, n_out: int, seed: int, node_level: 
     return (sums / np.maximum(counts, 1)[:, None]).astype(np.float32)
 
 
-def _with_node_labels(p: PackedGraphs, n_classes: int, seed: int) -> PackedGraphs:
-    return PackedGraphs(p.node_off, p.rowptr, p.col, p.x, node_labels(p, n_classes, seed + 0x5EED), node_level=True)
-
-
-def _with_regression_targets(p: PackedGraphs, n_out: int, seed: int, node_level: bool) -> PackedGraphs:
-    return PackedGraphs(p.node_off, p.rowptr, p.col, p.x, regression_targets(p, n_out, seed + 0x5EED, node_level),
-                        node_level=node_level)
+def _labelled(p: PackedGraphs, n_classes: int, seed: int, node_level: bool, task: str) -> PackedGraphs:
+    """``p`` (graphs with their balanced graph labels) with the labels ``make_dataset`` gives for ``task`` /
+    ``node_level``."""
+    if task == "regression":
+        return dataclasses.replace(p, y=regression_targets(p, n_classes, seed + 0x5EED, node_level), node_level=node_level)
+    if node_level:
+        return dataclasses.replace(p, y=node_labels(p, n_classes, seed + 0x5EED), node_level=True)
+    return p
 
 
 TASKS = ("classification", "regression")
@@ -176,69 +240,16 @@ def make_dataset(n_graphs: int, seed: int = 0, n_mean: int = 500, deg: int = 12,
     one-hot labels."""
     if task not in TASKS:
         raise ValueError(f"task must be one of {TASKS}, got {task!r}")
-    rps: List[np.ndarray] = []
-    cols: List[np.ndarray] = []
-    xs: List[np.ndarray] = []
-    node_off = np.zeros(n_graphs + 1, dtype=np.int64)
-    e_off = 0
-    for g in range(n_graphs):
-        rp, c, x = make_graph(seed, g, n_mean, deg, n_feat)
-        node_off[g + 1] = node_off[g] + x.shape[0]
-        rps.append(rp[:-1] + e_off)
-        e_off += int(rp[-1])
-        cols.append(c)
-        xs.append(x)
-    rowptr = np.concatenate(rps + [np.array([e_off], dtype=np.int64)]) if n_graphs else np.zeros(1, np.int64)
-    col = np.concatenate(cols) if n_graphs else np.zeros(0, np.int32)
-    x = np.concatenate(xs) if n_graphs else np.zeros((0, n_feat), np.float32)
-    if task == "regression":
-        return _with_regression_targets(PackedGraphs(node_off, rowptr, col, x, np.zeros((0, n_classes), np.float32)),
-                                        n_classes, seed, node_level)
-    if node_level:
-        return _with_node_labels(PackedGraphs(node_off, rowptr, col, x, np.zeros((0, n_classes), np.float32)), n_classes,
-                                 seed)
-    y = np.zeros((n_graphs, n_classes), dtype=np.float32)
-    lab = np.arange(n_graphs) % n_classes          # balanced (gcn.py:265-266)
-    y[np.arange(n_graphs), lab] = 1.0
-    return PackedGraphs(node_off, rowptr, col, x, y)
-
-
-def concat_packed(parts: List[PackedGraphs]) -> PackedGraphs:
-    """Concatenate packed datasets (graph order = order of the parts).  Graph- and node-labelled parts do not mix."""
-    kinds = {bool(p.node_level) for p in parts}
-    if len(kinds) > 1:
-        raise ValueError("cannot concatenate graph-labelled and node-labelled datasets")
-    if len(parts) == 1:
-        return parts[0]
-    node_off = [np.zeros(1, dtype=np.int64)]
-    rowptr = []
-    n0, e0 = 0, 0
-    for p in parts:
-        node_off.append(p.node_off[1:] + n0)
-        rowptr.append(p.rowptr[:-1] + e0)
-        n0 += int(p.node_off[-1])
-        e0 += int(p.rowptr[-1])
-    rowptr.append(np.array([e0], dtype=np.int64))
-    return PackedGraphs(np.concatenate(node_off), np.concatenate(rowptr), np.concatenate([p.col for p in parts]),
-                        np.concatenate([p.x for p in parts]), np.concatenate([p.y for p in parts]), kinds.pop())
+    return _labelled(_make_range((seed, 0, n_graphs, n_mean, deg, n_feat, n_classes)), n_classes, seed, node_level, task)
 
 
 def _make_range(args):
+    """Graphs [g0, g1) with their balanced graph labels (gcn.py:265-266: graph g is of class g % n_classes)."""
     seed, g0, g1, n_mean, deg, n_feat, n_classes = args
-    rps, cols, xs = [], [], []
-    node_off = np.zeros(g1 - g0 + 1, dtype=np.int64)
-    e_off = 0
-    for k, gid in enumerate(range(g0, g1)):
-        rp, c, x = make_graph(seed, gid, n_mean, deg, n_feat)
-        node_off[k + 1] = node_off[k] + x.shape[0]
-        rps.append(rp[:-1] + e_off)
-        e_off += int(rp[-1])
-        cols.append(c)
-        xs.append(x)
-    y = np.zeros((g1 - g0, n_classes), dtype=np.float32)
-    y[np.arange(g1 - g0), np.arange(g0, g1) % n_classes] = 1.0
-    return PackedGraphs(node_off, np.concatenate(rps + [np.array([e_off], dtype=np.int64)]), np.concatenate(cols),
-                        np.concatenate(xs), y)
+    graphs = [make_graph(seed, g, n_mean, deg, n_feat) for g in range(g0, g1)]
+    eye = np.eye(n_classes, dtype=np.float32)
+    return PackedGraphs.from_graphs([rp for rp, _, _ in graphs], [c for _, c, _ in graphs], [x for _, _, x in graphs],
+                                    [eye[g % n_classes] for g in range(g0, g1)], n_feat=n_feat, n_classes=n_classes)
 
 
 def make_dataset_parallel(n_graphs: int, seed: int = 0, n_mean: int = 500, deg: int = 12, n_feat: int = 32,
@@ -254,8 +265,7 @@ def make_dataset_parallel(n_graphs: int, seed: int = 0, n_mean: int = 500, deg: 
     jobs = [(seed, g0, min(g0 + chunk, n_graphs), n_mean, deg, n_feat, n_classes) for g0 in range(0, n_graphs, chunk)]
     with mp.get_context("fork").Pool(workers) as pool:
         parts = pool.map(_make_range, jobs)
-    out = concat_packed(parts)
-    return _with_node_labels(out, n_classes, seed) if node_level else out
+    return _labelled(concat_packed(parts), n_classes, seed, node_level, "classification")
 
 
 def tile_dataset(packed: PackedGraphs, n_graphs: int) -> PackedGraphs:
@@ -266,10 +276,9 @@ def tile_dataset(packed: PackedGraphs, n_graphs: int) -> PackedGraphs:
     out = concat_packed([packed] * reps)
     if out.n_graphs == n_graphs:
         return out
-    n1 = int(out.node_off[n_graphs])
-    e1 = int(out.rowptr[n1])
+    _, n1, _, e1 = out.span(0, n_graphs)
     return PackedGraphs(out.node_off[:n_graphs + 1], out.rowptr[:n1 + 1], out.col[:e1], out.x[:n1],
-                        out.y[:n1] if out.node_level else out.y[:n_graphs], out.node_level)
+                        out.y[:n1] if out.node_level else out.y[:n_graphs], out.node_level, out.symmetric)
 
 
 def pack_graphs(graphs, node_level: bool = False) -> PackedGraphs:
@@ -280,23 +289,19 @@ def pack_graphs(graphs, node_level: bool = False) -> PackedGraphs:
     (a5: GeneralConv never reads them).  ``node_level=True``: every ``.y`` is [n_nodes, C] (one label row per node,
     all with the same C) and the rows are stacked in node order."""
     import scipy.sparse as sp
-    node_off = np.zeros(len(graphs) + 1, dtype=np.int64)
     rps, cols, xs, ys = [], [], [], []
-    e_off = 0
     for g, gr in enumerate(graphs):
         a = sp.csr_matrix(gr.a, copy=True)     # never mutate the caller's matrix
         a.sum_duplicates()
         a.eliminate_zeros()
         a.sort_indices()
         n = a.shape[0]
-        x = np.asarray(gr.x)
+        x = np.asarray(gr.x, dtype=np.float32)
         if x.shape[0] != n:
             raise ValueError(f"graph {g}: x has {x.shape[0]} rows but a is {a.shape}")
-        node_off[g + 1] = node_off[g] + n
-        rps.append(a.indptr[:-1].astype(np.int64) + e_off)
-        e_off += int(a.indptr[-1])
+        rps.append(a.indptr)
         cols.append(a.indices.astype(np.int32))
-        xs.append(x.astype(np.float32))
+        xs.append(x)
         if node_level:
             yg = np.asarray(gr.y, dtype=np.float32) if gr.y is not None else None
             if yg is None or yg.ndim != 2 or yg.shape[0] != n or (ys and yg.shape[1] != ys[0].shape[1]):
@@ -306,10 +311,4 @@ def pack_graphs(graphs, node_level: bool = False) -> PackedGraphs:
             ys.append(yg)
         else:
             ys.append(np.asarray(gr.y, dtype=np.float32).reshape(-1))
-    rowptr = np.concatenate(rps + [np.array([e_off], dtype=np.int64)]) if graphs else np.zeros(1, np.int64)
-    col = np.concatenate(cols) if graphs else np.zeros(0, np.int32)
-    x = np.concatenate(xs) if graphs else np.zeros((0, 0), np.float32)
-    if node_level:
-        return PackedGraphs(node_off, rowptr, col, x, np.concatenate(ys) if graphs else np.zeros((0, 0), np.float32), True)
-    y = np.stack(ys) if graphs else np.zeros((0, 0), np.float32)
-    return PackedGraphs(node_off, rowptr, col, x, y)
+    return PackedGraphs.from_graphs(rps, cols, xs, ys, node_level)

@@ -76,7 +76,7 @@ def test_concat_and_tile_carry_node_labels_and_refuse_to_mix():
     with pytest.raises(ValueError):
         synthetic.concat_packed([a, gl])
     with pytest.raises(ValueError):
-        shards.concat_packed([gl, a])
+        synthetic.concat_packed([gl, a])
 
 
 def _v1_bytes(p, symmetric):
